@@ -2,6 +2,7 @@
 """Benchmark of the wavelet + SSIM hot path (driver contract: ONE JSON line on stdout from rank 0).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload cfg2|cfg1|cfg3|sweep1024] [--impl reference]
+                    [--dump-outputs DIR]
 
 A "step" is one pass of the hot path over one batch of synthetic input:
   cfg2 (default, BASELINE.json configs[1]): DWTForward(J=3, db3, symmetric) -> DWTInverse -> backward through both,
@@ -23,6 +24,8 @@ reference_gpu = the UNMODIFIED reference modules (oracle/_ref, staged by `make -
 cpu_baseline = the reference's CPU path on the host cores: the unmodified reference (kind "reference") when it is
                staged, else the C/OpenMP port oracle/c/ref_port.c (kind "port").
 --impl reference times that CPU path only (rank 0) and prints the same line with "impl": "reference".
+--dump-outputs DIR writes what the last timed step of the headline workload returned (rank 0) as DIR/<name>.npy, so
+that two builds run with the same arguments, and therefore on the same seeded inputs, can be compared output for output.
 """
 import argparse
 import json
@@ -347,6 +350,40 @@ def build_step(cfg, dev, modules):
     return step, make_set, 2 * 4 * n * c * h * w, step_bytes, extras
 
 
+def step_output_names(cfg):
+    """Names of the tensors the step of build_step returns, in order."""
+    if cfg["kind"] == "ssim":
+        return ("ssim", "dx")
+    return ("rec", "dx") if cfg["grad"] else ("rec", "ssim")
+
+
+DUMP_BYTES = 60 * 1024 * 1024   # all dumped arrays together; the .npy headers stay well inside 64 MB
+
+
+def dump_outputs(out_dir, names, outputs):
+    """Writes each output tensor as out_dir/<name>.npy (float32 or float64).  An output larger than its share of
+    DUMP_BYTES is written as a fixed sample: the elements of its flattened array at the sorted indices that
+    numpy.random.default_rng(0).choice(numel, k, replace=False) draws.  Returns what was written."""
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    pairs = [(name, t.detach()) for name, t in zip(names, outputs) if t is not None]
+    written = {}
+    for name, t in pairs:
+        if t.dtype not in (torch.float32, torch.float64):
+            t = t.float()
+        flat = t.reshape(-1)
+        k = DUMP_BYTES // len(pairs) // flat.element_size()
+        entry = {"shape": list(t.shape), "dtype": str(t.dtype).replace("torch.", "")}
+        if flat.numel() > k:
+            idx = np.sort(np.random.default_rng(0).choice(flat.numel(), k, replace=False))
+            flat = flat[torch.from_numpy(idx).to(flat.device)]
+            entry["sampled"] = k
+        np.save(os.path.join(out_dir, name + ".npy"), flat.cpu().numpy() if "sampled" in entry else t.cpu().numpy())
+        written[name] = entry
+    return written
+
+
 def capture_graphs(step, sets):
     import torch
     graphs = []
@@ -484,10 +521,11 @@ def run_value(step, sets, steps, warmup, use_graph):
             graphs = None
 
     def run_step(i):
+        """Runs step i; returns its outputs (for a replay, the graph's output tensors, which it has just rewritten)."""
         if graphs is not None:
             graphs[i % nsets][0].replay()
-        else:
-            step(*sets[i % nsets])
+            return graphs[i % nsets][1]
+        return step(*sets[i % nsets])
     return run_step, graphs
 
 
@@ -540,7 +578,12 @@ def main():
     ap.add_argument("--e2e-chunks", type=int, default=1,
                     help="batch chunks of the host-buffer pipeline (e2e); consecutive steps already overlap their "
                          "uploads and downloads, and one chunk per step measured best (profiles/r01_notes.md)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the outputs of the last timed step of the headline workload as DIR/<name>.npy "
+                         "(a fixed sample of an output that does not fit %d MB)" % (DUMP_BYTES >> 20))
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3)
 
     rank = int(os.environ.get("RANK", "0"))
@@ -597,8 +640,9 @@ def main():
             return float(t.item())
         return ms
 
-    def measure(name, wcfg, steps, warmup, with_e2e):
-        """value (+ e2e) of one workload on every rank, max over ranks; the kernel rooflines on rank 0."""
+    def measure(name, wcfg, steps, warmup, with_e2e, dump_dir=None):
+        """value (+ e2e) of one workload on every rank, max over ranks; the kernel rooflines on rank 0; with dump_dir,
+        rank 0 writes the outputs of the last timed step there."""
         wn, wc, wh, ww = wcfg["shape"]
         step, make_set, set_bytes, step_bytes, extras = build_step(wcfg, dev, b200wave)
         nsets = max(2, -(-2 * L2_BYTES // set_bytes))  # inputs alone exceed 2x L2 across the rotation
@@ -621,10 +665,11 @@ def main():
         ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         ev0.record()
         for i in range(steps):
-            run_step(i)
+            out = run_step(i)
         ev1.record()
         barrier()
         ms = all_max(ev0.elapsed_time(ev1))
+        dumped = dump_outputs(dump_dir, step_output_names(wcfg), out) if dump_dir and rank == 0 else None
         res = {"desc": wcfg["desc"], "ms_per_step": ms / steps, "steps": steps,
                "value": world * wn * wc * wh * ww / 1e6 * steps / (ms / 1e3), "unit": UNIT,
                "step_algorithmic_bytes": step_bytes, "step_hbm_frac": (step_bytes / (ms / steps * 1e-3) / 1e9) / peak,
@@ -632,6 +677,8 @@ def main():
                "replay": "cuda-graph" if graphs is not None else "eager",
                "l2": "rotating %d input sets (%.0f MB) > 2x 126 MB L2; outputs re-allocated per set"
                      % (nsets, nsets * set_bytes / 1e6)}
+        if dumped is not None:
+            res["dump_outputs"] = dumped
         if with_e2e:
             # The public host-buffer call (b200wave.HostPipeline): every step copies that step's inputs from pinned
             # host memory, runs the same step, and copies the results back; H2D copy, kernels and D2H copy overlap
@@ -678,7 +725,7 @@ def main():
     sampler = ClockSampler(local_rank) if rank == 0 else None
     if sampler:
         sampler.start()
-    main_res = measure(args.workload, cfg, args.steps, args.warmup, True)
+    main_res = measure(args.workload, cfg, args.steps, args.warmup, True, args.dump_outputs)
     clocks = sampler.stop() if sampler else None
 
     # the other BASELINE configs, device-resident value + roofline each (every rank runs them so that the per-rank
@@ -725,6 +772,8 @@ def main():
             "workloads": others, "reference_gpu": ref_gpu, "cpu_baseline": cpu, "clocks": clocks,
             "library_build": _cabi.build_hash(),
         }
+        if "dump_outputs" in main_res:
+            line["dump_outputs"] = {"dir": args.dump_outputs, "arrays": main_res["dump_outputs"]}
         if saved_stdout is not None:
             sys.stdout.flush()
             os.dup2(saved_stdout, 1)

@@ -22,6 +22,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(os.path.dirname(HERE))
 REF = os.environ.get("B200W_REFERENCE", "/root/reference")
 sys.path.insert(0, ROOT)
+sys.path.insert(0, os.path.join(ROOT, "tests"))
 sys.path.insert(0, os.path.join(ROOT, "oracle", "pywt_standin"))
 sys.path.insert(0, os.path.join(REF, "pytorch_wavelets"))
 sys.path.insert(0, REF)
@@ -35,6 +36,7 @@ from pytorch_wavelets import DWTForward, DWTInverse  # noqa: E402  (the referenc
 import ssim as ref_ssim  # noqa: E402  (the reference)
 
 from oracle import dwt_oracle, ssim_oracle  # noqa: E402
+from helpers import save_golden  # noqa: E402  (keeps every golden file under 1 MB)
 
 # (name, wave, J, mode, (N, C, H, W))
 DWT_CASES = []
@@ -150,7 +152,7 @@ def main():
             bundle["c%02d/%s" % (i, k)] = v
         print("dwt case %02d %-14s J=%d %-14s %s  oracle-vs-ref %.2e" % (i, wave, J, mode, shape, worst))
     bundle["ncases"] = np.int64(len(DWT_CASES))
-    np.savez_compressed(os.path.join(HERE, "dwt_cases.npz"), **bundle)
+    save_golden("dwt_cases", bundle)
 
     sb = {}
     x = f32_valued(rng, (2, 3, 24, 31), "rand")
@@ -172,7 +174,7 @@ def main():
     print("ssim case %02d same val=%s" % (n, out["val"]))
     n += 1
     sb["ncases"] = np.int64(n)
-    np.savez_compressed(os.path.join(HERE, "ssim_cases.npz"), **sb)
+    save_golden("ssim_cases", sb)
     print("worst oracle-vs-reference deviation: %.3e" % worst_all)
     assert worst_all < 1e-10, worst_all
 

@@ -20,6 +20,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(os.path.dirname(HERE))
 REF = os.environ.get("B200W_REFERENCE", "/root/reference")
 sys.path.insert(0, ROOT)
+sys.path.insert(0, os.path.join(ROOT, "tests"))
 sys.path.insert(0, os.path.join(ROOT, "oracle", "pywt_standin"))
 sys.path.insert(0, os.path.join(REF, "pytorch_wavelets"))
 warnings.filterwarnings("ignore")
@@ -29,6 +30,7 @@ torch.set_default_dtype(torch.float64)
 from pytorch_wavelets.dwt.transform1d import DWT1DForward, DWT1DInverse  # noqa: E402  (the reference)
 
 from oracle import dwt_oracle  # noqa: E402
+from helpers import save_golden  # noqa: E402  (keeps every golden file under 1 MB)
 
 CASES = []
 for wave, J, mode in [("db1", 1, "zero"), ("db1", 3, "zero"), ("db3", 1, "symmetric"), ("db3", 2, "reflect"),
@@ -91,5 +93,5 @@ for k, (wave, J, mode, shape) in enumerate(CASES):
             r = r[..., :-1]
         r = dwt_oracle.sfb1d(r, hi, g0, g1, mode)
     worst = max(worst, float(np.abs(r - out[pre + "rec"]).max()))
-np.savez_compressed(os.path.join(HERE, "dwt1d_cases.npz"), **out)
+save_golden("dwt1d_cases", out)
 print("dwt1d cases: %d, worst |oracle - reference| = %.3e" % (len(CASES), worst))

@@ -1,6 +1,6 @@
 """Golden vectors for the Fourier-domain frequency split, from the UNMODIFIED reference ``utils.py``.
 
-    python tests/golden/make_golden_freq.py        # writes tests/golden/freq_cases.npz
+    python tests/golden/make_golden_freq.py        # writes tests/golden/freq_cases.*.npz
 
 Build container only (needs /root/reference).  ``utils.py`` imports packages that are not installed here (skimage,
 matplotlib, ...) and hard-codes ``.cuda()`` on the mask (``utils.py:97,110``); empty stand-in modules and a no-op
@@ -18,6 +18,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(os.path.dirname(HERE))
 REF = os.environ.get("B200W_REFERENCE", "/root/reference")
 sys.path.insert(0, ROOT)
+sys.path.insert(0, os.path.join(ROOT, "tests"))
 warnings.filterwarnings("ignore")
 import torch  # noqa: E402
 
@@ -47,6 +48,7 @@ sys.path.insert(0, REF)
 import utils as ref_utils  # noqa: E402  (the reference)
 
 from oracle import freq_oracle  # noqa: E402
+from helpers import save_golden  # noqa: E402  (keeps every golden file under 1 MB)
 
 CASES = [  # (H, W, radius, highpass) -- train.py:173-213 uses i = 10, 8, 5, 14 on 256x256
     (256, 256, 10, True), (256, 256, 8, False), (128, 128, 5, True), (128, 128, 14, False),
@@ -69,5 +71,4 @@ for k, (h, w, r, hp) in enumerate(CASES):
     out[pre + "radius"] = r
     out[pre + "highpass"] = int(hp)
 print("oracle (float64) vs reference (fp32 fft): worst rel err %.2e" % worst)
-np.savez_compressed(os.path.join(HERE, "freq_cases.npz"), **out)
-print("wrote", os.path.join(HERE, "freq_cases.npz"))
+print("wrote", save_golden("freq_cases", out))

@@ -20,6 +20,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(os.path.dirname(HERE))
 REF = os.environ.get("B200W_REFERENCE", "/root/reference")
 sys.path.insert(0, ROOT)
+sys.path.insert(0, os.path.join(ROOT, "tests"))
 sys.path.insert(0, os.path.join(ROOT, "oracle", "pywt_standin"))
 warnings.filterwarnings("ignore")
 import torch  # noqa: E402
@@ -53,6 +54,7 @@ import model as ref_model  # noqa: E402  (the reference)
 from pytorch_wavelets import DWTForward  # noqa: E402  (the reference)
 
 from oracle import fsd_oracle  # noqa: E402
+from helpers import save_golden  # noqa: E402  (keeps every golden file under 1 MB)
 
 # (variant, cs, norm, (N, C, H, W)); train.py feeds (N, 1, 256, 256) crops, FS_DiscriminatorA cs='sum', B cs='cat'
 CASES = [("A", "sum", True, (2, 1, 64, 64)), ("B", "cat", True, (2, 1, 64, 64)),
@@ -88,5 +90,5 @@ for k, (variant, cs, norm, shape) in enumerate(CASES):
     dxo = fsd_oracle.filter_wavelet_backward([g.numpy() for g in grads], shape, cs, norm, variant)
     worst = max(worst, float(np.abs(dxo - out[pre + "dx"]).max()))
 
-np.savez_compressed(os.path.join(HERE, "fsd_cases.npz"), **out)
+save_golden("fsd_cases", out)
 print("fsd cases: %d, worst |oracle - reference| = %.3e" % (len(CASES), worst))

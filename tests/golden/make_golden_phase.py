@@ -1,6 +1,6 @@
 """Golden vectors for phase_consistency_loss, from the UNMODIFIED reference ``model.py`` (:36-58).
 
-    python tests/golden/make_golden_phase.py        # writes tests/golden/phase_cases.npz
+    python tests/golden/make_golden_phase.py        # writes tests/golden/phase_cases.*.npz
 
 Build container only (needs /root/reference and the ``pywt`` stand-in).  ``model.py`` imports packages that are not
 installed here and hard-codes ``.cuda()`` on the mask (:50); empty stand-in modules and a no-op ``Tensor.cuda`` let the
@@ -18,6 +18,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(os.path.dirname(HERE))
 REF = os.environ.get("B200W_REFERENCE", "/root/reference")
 sys.path.insert(0, ROOT)
+sys.path.insert(0, os.path.join(ROOT, "tests"))
 sys.path.insert(0, os.path.join(ROOT, "oracle", "pywt_standin"))
 warnings.filterwarnings("ignore")
 import torch  # noqa: E402
@@ -52,6 +53,7 @@ torch.Tensor.float = lambda self, *a, **k: self     # ... after .float(): keep t
 import model as ref_model  # noqa: E402  (the reference)
 
 from oracle import phase_oracle  # noqa: E402
+from helpers import save_golden  # noqa: E402  (keeps every golden file under 1 MB)
 
 CASES = [(2, 1, 64, 64), (1, 1, 256, 256), (3, 2, 37, 41), (1, 3, 16, 50), (2, 1, 33, 8), (1, 1, 128, 96)]
 out = {"ncases": len(CASES)}
@@ -73,5 +75,5 @@ for k, shape in enumerate(CASES):
                       / np.abs(out[pre + "dx"]).max()),
                 float(np.abs(phase_oracle.phase_consistency_grad(xn, yn, 1) - out[pre + "dy"]).max()
                       / np.abs(out[pre + "dy"]).max()))
-np.savez_compressed(os.path.join(HERE, "phase_cases.npz"), **out)
+save_golden("phase_cases", out)
 print("phase cases: %d, worst |oracle - reference| = %.3e" % (len(CASES), worst))

@@ -17,6 +17,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(os.path.dirname(HERE))
 REF = os.environ.get("B200W_REFERENCE", "/root/reference")
 sys.path.insert(0, ROOT)
+sys.path.insert(0, os.path.join(ROOT, "tests"))
 sys.path.insert(0, os.path.join(ROOT, "oracle", "pywt_standin"))
 sys.path.insert(0, os.path.join(REF, "pytorch_wavelets"))
 warnings.filterwarnings("ignore")
@@ -28,6 +29,7 @@ from pytorch_wavelets.dwt import lowlevel  # noqa: E402  (the reference)
 from pytorch_wavelets.dwt.transform2d import SWTForward  # noqa: E402
 
 from oracle import swt_oracle  # noqa: E402
+from helpers import save_golden  # noqa: E402  (keeps every golden file under 1 MB)
 
 CASES = []
 for mode in ("zero", "symmetric", "reflect", "periodic"):
@@ -85,6 +87,6 @@ try:
     out["J2_error"] = ""
 except Exception as e:      # noqa: BLE001
     out["J2_error"] = "%s: %s" % (type(e).__name__, str(e)[:80])
-np.savez_compressed(os.path.join(HERE, "swt_cases.npz"), **out)
+save_golden("swt_cases", out)
 print("swt cases: %d, worst |oracle - reference| = %.3e; default mode -> %s; J=2 -> %s"
       % (out["ncases"], worst, out["default_mode_error"], out["J2_error"]))

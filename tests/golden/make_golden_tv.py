@@ -17,6 +17,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(os.path.dirname(HERE))
 REF = os.environ.get("B200W_REFERENCE", "/root/reference")
 sys.path.insert(0, ROOT)
+sys.path.insert(0, os.path.join(ROOT, "tests"))
 sys.path.insert(0, os.path.join(ROOT, "oracle", "pywt_standin"))
 warnings.filterwarnings("ignore")
 import torch  # noqa: E402
@@ -49,6 +50,7 @@ torch.set_default_dtype(torch.float64)
 import model as ref_model  # noqa: E402  (the reference)
 
 from oracle import tv_oracle  # noqa: E402
+from helpers import save_golden  # noqa: E402  (keeps every golden file under 1 MB)
 
 CASES = [((2, 1, 64, 64), 1), ((1, 1, 256, 256), 1), ((3, 2, 37, 41), 0.5), ((1, 3, 5, 300), 2), ((2, 1, 130, 7), 1),
          ((1, 1, 2, 2), 1)]
@@ -66,5 +68,5 @@ for k, (shape, weight) in enumerate(CASES):
     out[pre + "dx"] = x.grad.numpy()
     worst = max(worst, abs(tv_oracle.tv_loss(out[pre + "x"], weight) - float(loss)) / abs(float(loss)),
                 float(np.abs(tv_oracle.tv_loss_backward(out[pre + "x"], 1.0, weight) - out[pre + "dx"]).max()))
-np.savez_compressed(os.path.join(HERE, "tv_cases.npz"), **out)
+save_golden("tv_cases", out)
 print("tv cases: %d, worst |oracle - reference| = %.3e" % (len(CASES), worst))

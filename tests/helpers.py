@@ -1,4 +1,6 @@
 """Shared helpers for the test-suite (oracle access, golden-case loading, error metric)."""
+import glob
+import io
 import os
 
 import numpy as np
@@ -8,6 +10,58 @@ GOLDEN = os.path.join(ROOT, "tests", "golden")
 
 # north_star tolerance: 1e-5 relative (fp32), measured as max|a-b| / max|b| per tensor (BASELINE.md 5)
 RTOL_F32 = 1e-5
+
+# every golden file stays below 1 MB; a set that does not fit is written as several parts
+GOLDEN_FILE_BYTES = 1000 * 1000
+
+
+def _golden_paths(name):
+    single = os.path.join(GOLDEN, name + ".npz")
+    parts = glob.glob(os.path.join(GOLDEN, name + ".[0-9]*.npz"))
+    return [single] if os.path.exists(single) else sorted(parts, key=lambda p: int(p.rsplit(".", 2)[1]))
+
+
+def _npz_bytes(arrays):
+    buf = io.BytesIO()
+    np.savez_compressed(buf, **arrays)
+    return buf.tell()
+
+
+def save_golden(name, arrays):
+    """Writes the golden set ``name`` (a dict of arrays) as tests/golden/<name>.npz, or, when that file would not stay
+    under GOLDEN_FILE_BYTES, as <name>.1.npz, <name>.2.npz, ... each holding whole arrays.  load_golden reads either
+    form."""
+    for p in _golden_paths(name):
+        os.remove(p)
+    parts = [arrays]
+    if _npz_bytes(arrays) >= GOLDEN_FILE_BYTES:
+        parts, cur, cur_bytes = [], {}, 0
+        for key, value in arrays.items():
+            size = _npz_bytes({key: value})
+            if cur and cur_bytes + size > 0.9 * GOLDEN_FILE_BYTES:
+                parts.append(cur)
+                cur, cur_bytes = {}, 0
+            cur[key] = value
+            cur_bytes += size
+        parts.append(cur)
+    names = [name + ".npz"] if len(parts) == 1 else ["%s.%d.npz" % (name, i + 1) for i in range(len(parts))]
+    for fname, part in zip(names, parts):
+        path = os.path.join(GOLDEN, fname)
+        np.savez_compressed(path, **part)
+        assert os.path.getsize(path) < GOLDEN_FILE_BYTES, (path, "one array alone is too large for a golden file")
+    return names
+
+
+def load_golden(name):
+    """The arrays of the golden set ``name`` written by save_golden, as a dict."""
+    paths = _golden_paths(name)
+    if not paths:
+        raise FileNotFoundError("no golden set %r under %s" % (name, GOLDEN))
+    out = {}
+    for p in paths:
+        with np.load(p) as z:
+            out.update((k, z[k]) for k in z.files)
+    return out
 
 
 def rel_err(a, b):
@@ -21,12 +75,12 @@ def rel_err(a, b):
 
 
 def load_dwt_cases():
-    z = np.load(os.path.join(GOLDEN, "dwt_cases.npz"))
+    z = load_golden("dwt_cases")
     n = int(z["ncases"])
     cases = []
     for i in range(n):
         pre = "c%02d/" % i
-        case = {k[len(pre):]: z[k] for k in z.files if k.startswith(pre)}
+        case = {k[len(pre):]: z[k] for k in z if k.startswith(pre)}
         case["J"] = int(case["J"])
         case["mode"] = str(case["mode"])
         case["wave"] = str(case["wave"])
@@ -37,12 +91,12 @@ def load_dwt_cases():
 
 
 def load_ssim_cases():
-    z = np.load(os.path.join(GOLDEN, "ssim_cases.npz"))
+    z = load_golden("ssim_cases")
     n = int(z["ncases"])
     cases = []
     for i in range(n):
         pre = "s%02d/" % i
-        case = {k[len(pre):]: z[k] for k in z.files if k.startswith(pre)}
+        case = {k[len(pre):]: z[k] for k in z if k.startswith(pre)}
         case["size_average"] = bool(case["size_average"])
         case["id"] = "%02d-sa%d" % (i, case["size_average"])
         cases.append(case)
@@ -56,11 +110,11 @@ def case_filters(case):
 
 
 def load_freq_cases():
-    z = np.load(os.path.join(GOLDEN, "freq_cases.npz"))
+    z = load_golden("freq_cases")
     cases = []
     for i in range(int(z["ncases"])):
         pre = "f%02d/" % i
-        case = {k[len(pre):]: z[k] for k in z.files if k.startswith(pre)}
+        case = {k[len(pre):]: z[k] for k in z if k.startswith(pre)}
         case["radius"] = int(case["radius"])
         case["highpass"] = bool(case["highpass"])
         case["id"] = "%02d-%s-r%d-%dx%d" % (i, "high" if case["highpass"] else "low", case["radius"],
@@ -70,11 +124,11 @@ def load_freq_cases():
 
 
 def load_fsd_cases():
-    z = np.load(os.path.join(GOLDEN, "fsd_cases.npz"))
+    z = load_golden("fsd_cases")
     cases = []
     for i in range(int(z["ncases"])):
         pre = "w%02d/" % i
-        case = {k[len(pre):]: z[k] for k in z.files if k.startswith(pre)}
+        case = {k[len(pre):]: z[k] for k in z if k.startswith(pre)}
         case["variant"] = str(case["variant"])
         case["cs"] = str(case["cs"])
         case["norm"] = bool(case["norm"])
@@ -88,11 +142,11 @@ def load_fsd_cases():
 
 
 def load_tv_cases():
-    z = np.load(os.path.join(GOLDEN, "tv_cases.npz"))
+    z = load_golden("tv_cases")
     cases = []
     for i in range(int(z["ncases"])):
         pre = "t%02d/" % i
-        case = {k[len(pre):]: z[k] for k in z.files if k.startswith(pre)}
+        case = {k[len(pre):]: z[k] for k in z if k.startswith(pre)}
         case["weight"] = float(case["weight"])
         case["loss"] = float(case["loss"])
         case["id"] = "%02d-%s-w%g" % (i, "x".join(str(d) for d in case["x"].shape), case["weight"])
@@ -101,11 +155,11 @@ def load_tv_cases():
 
 
 def load_phase_cases():
-    z = np.load(os.path.join(GOLDEN, "phase_cases.npz"))
+    z = load_golden("phase_cases")
     cases = []
     for i in range(int(z["ncases"])):
         pre = "p%02d/" % i
-        case = {k[len(pre):]: z[k] for k in z.files if k.startswith(pre)}
+        case = {k[len(pre):]: z[k] for k in z if k.startswith(pre)}
         case["loss"] = float(case["loss"])
         case["id"] = "%02d-%s" % (i, "x".join(str(d) for d in case["x"].shape))
         cases.append(case)
@@ -113,11 +167,11 @@ def load_phase_cases():
 
 
 def load_dwt1d_cases():
-    z = np.load(os.path.join(GOLDEN, "dwt1d_cases.npz"))
+    z = load_golden("dwt1d_cases")
     cases = []
     for i in range(int(z["ncases"])):
         pre = "d%02d/" % i
-        case = {k[len(pre):]: z[k] for k in z.files if k.startswith(pre)}
+        case = {k[len(pre):]: z[k] for k in z if k.startswith(pre)}
         case["J"] = int(case["J"])
         case["mode"] = str(case["mode"])
         case["wave"] = str(case["wave"])
@@ -127,11 +181,11 @@ def load_dwt1d_cases():
 
 
 def load_swt_cases():
-    z = np.load(os.path.join(GOLDEN, "swt_cases.npz"))
+    z = load_golden("swt_cases")
     cases = []
-    pres = sorted({k.split("/")[0] for k in z.files if "/" in k})
+    pres = sorted({k.split("/")[0] for k in z if "/" in k})
     for pre in pres:
-        case = {k[len(pre) + 1:]: z[k] for k in z.files if k.startswith(pre + "/")}
+        case = {k[len(pre) + 1:]: z[k] for k in z if k.startswith(pre + "/")}
         case["mode"], case["wave"], case["dilation"] = str(case["mode"]), str(case["wave"]), int(case["dilation"])
         case["id"] = "%s-%s-%s-d%d-%dx%d" % (pre, case["wave"], case["mode"], case["dilation"], case["x"].shape[-2],
                                              case["x"].shape[-1])
