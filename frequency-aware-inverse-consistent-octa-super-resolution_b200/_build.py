@@ -27,9 +27,7 @@ NVCC_FLAGS = [
     "-O3", "-lineinfo", "-std=c++17",
     "-Xcompiler", "-fPIC", "-Xcompiler", "-O3",
     "-cudart", "static",
-] + (["-DB200W_TIMELINE"] if os.environ.get("B200W_TIMELINE") == "1" else []) \
-  + (["-DB200W_OWNER_NT=%d" % int(os.environ["B200W_OWNER_NT"])] if os.environ.get("B200W_OWNER_NT") else []) \
-  + ["-D" + d for d in os.environ.get("B200W_DEFINES", "").split()]
+]
 
 
 def find_nvcc():

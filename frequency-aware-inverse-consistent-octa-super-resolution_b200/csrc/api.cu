@@ -1,7 +1,9 @@
-// ABI bookkeeping: version, status names, last CUDA error (thread-local, diagnostics only).
+// ABI bookkeeping: version, status names, last CUDA error (thread-local, diagnostics only); the DWT kernel-family
+// switches.
+#include <algorithm>
 #include <atomic>
 #include <cstdlib>
-#include "common.cuh"
+#include "dwt_levels.cuh"
 #include "tma.cuh"
 
 namespace b200w {
@@ -11,13 +13,23 @@ int set_last_cuda_error(cudaError_t e) {
     g_last_cuda_error = (int)e;
     return B200W_ERR_LAUNCH;
 }
-bool pdl_enabled() {
-    static int v = -1;
-    if (v < 0) {
-        const char* e = getenv("B200W_PDL");
-        v = (e && e[0] == '0') ? 0 : 1;
-    }
-    return v == 1;
+const DwtPolicy& dwt_policy() {
+    static const DwtPolicy pol = [] {
+        auto flag = [](const char* name) { const char* e = getenv(name); return e && e[0] == '1'; };
+        auto count = [](const char* name) { const char* e = getenv(name); return e ? std::max(1, atoi(e)) : 0; };
+        const char* owner = getenv("B200W_OWNER");
+        const char* tma = getenv("B200W_TMA");
+        DwtPolicy p;
+        p.force_direct = flag("B200W_FORCE_DIRECT");
+        p.force_tiled = flag("B200W_FORCE_TILED");
+        p.owner = (owner && owner[0] >= '0' && owner[0] <= '2') ? owner[0] - '0' : 1;
+        p.tma = !(tma && tma[0] == '0');
+        p.tma_noboxes = getenv("B200W_TMA_NOBOXES") != nullptr;
+        p.tma_G = count("B200W_TMA_G");
+        p.tma_D = count("B200W_TMA_D");
+        return p;
+    }();
+    return pol;
 }
 EncodeTiledFn tma_encode_fn() {
     static std::atomic<void*> fn{nullptr};

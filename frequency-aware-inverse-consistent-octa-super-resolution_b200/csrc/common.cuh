@@ -194,7 +194,6 @@ __device__ __forceinline__ void cp_async_wait() { asm volatile("cp.async.wait_gr
 // lets the dependent grid be scheduled as soon as every CTA has issued it (or exited).  Both are no-ops for plain launches.
 __device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
 __device__ __forceinline__ void pdl_trigger() { asm volatile("griddepcontrol.launch_dependents;"); }
-bool pdl_enabled();   // B200W_PDL=0 switches the attribute off
 
 template <typename Kernel, typename Params>
 inline cudaError_t launch_pdl(Kernel kernel, unsigned grid, unsigned block, size_t smem, cudaStream_t st, const Params& prm) {
@@ -207,7 +206,7 @@ inline cudaError_t launch_pdl(Kernel kernel, unsigned grid, unsigned block, size
     attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
     attr[0].val.programmaticStreamSerializationAllowed = 1;
     cfg.attrs = attr;
-    cfg.numAttrs = pdl_enabled() ? 1 : 0;
+    cfg.numAttrs = 1;
     return cudaLaunchKernelEx(&cfg, kernel, prm);
 }
 

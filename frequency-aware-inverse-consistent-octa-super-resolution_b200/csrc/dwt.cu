@@ -638,43 +638,6 @@ __global__ void __launch_bounds__(kThreads) sfb2d_direct_kernel(const __grid_con
 // ------------------------------------------------------------------------------------------------
 // host side
 // ------------------------------------------------------------------------------------------------
-// B200W_FORCE_DIRECT=1: one-thread-per-output kernels; B200W_FORCE_TILED=1: shared-memory tile kernels instead of
-// the streaming kernels (both are on-device cross-checks of the default path, used by the tests)
-static int env_flag(const char* name) {
-    const char* e = getenv(name);
-    return (e && e[0] == '1') ? 1 : 0;
-}
-static bool force_direct() {
-    static int v = -1;
-    if (v < 0) v = env_flag("B200W_FORCE_DIRECT");
-    return v == 1;
-}
-static bool force_tiled() {
-    static int v = -1;
-    if (v < 0) v = env_flag("B200W_FORCE_TILED");
-    return v == 1;
-}
-// B200W_OWNER=0 switches the owner kernels off (chains of small planes then take the ticketed chain kernels);
-// B200W_OWNER_J0=n makes them start no earlier than level n (the levels before run as a chain launch).
-// B200W_OWNER=2 uses them whenever the shapes fit, however few planes there are (tests).
-static int owner_mode() {
-    static int v = -1;
-    if (v < 0) {
-        const char* e = getenv("B200W_OWNER");
-        v = (e && e[0] >= '0' && e[0] <= '2') ? e[0] - '0' : 1;
-    }
-    return v;
-}
-static int owner_j0_min() {
-    static int v = -1;
-    if (v < 0) {
-        const char* e = getenv("B200W_OWNER_J0");
-        v = (e && *e) ? atoi(e) : 0;
-        if (v < 0) v = 0;
-    }
-    return v;
-}
-
 static bool mode_supported(int mode) {
     return mode == B200W_MODE_ZERO || mode == B200W_MODE_SYMMETRIC || mode == B200W_MODE_PERIODIZATION ||
            mode == B200W_MODE_REFLECT || mode == B200W_MODE_PERIODIC;
@@ -842,22 +805,16 @@ static size_t direct_grid(size_t total) {
 }
 
 static bool templated_taps(int Lw, int Lh) {
-    return Lw == Lh && (Lw % 2) == 0 && Lw >= 2 && Lw <= 16 && !force_direct();
+    return Lw == Lh && (Lw % 2) == 0 && Lw >= 2 && Lw <= 16 && !dwt_policy().force_direct;
 }
 
 // ---- analysis chain --------------------------------------------------------------------------------
 static int run_afb_big_levels(AfbParams& p, int L, cudaStream_t st) {
-    if (!force_tiled() && afb_stream_supported(p, L)) return launch_afb_stream(p, L, device_info().sms, st);
-    switch (L) {
-        case 2: return launch_afb_chain<2>(p, st);
-        case 4: return launch_afb_chain<4>(p, st);
-        case 6: return launch_afb_chain<6>(p, st);
-        case 8: return launch_afb_chain<8>(p, st);
-        case 10: return launch_afb_chain<10>(p, st);
-        case 12: return launch_afb_chain<12>(p, st);
-        case 14: return launch_afb_chain<14>(p, st);
-        default: return launch_afb_chain<16>(p, st);
-    }
+    if (!dwt_policy().force_tiled && afb_stream_supported(p, L)) return launch_afb_stream(p, L, device_info().sms, st);
+#define X(LL) return launch_afb_chain<LL>(p, st)
+    B200W_FOR_EACH_L(X)
+#undef X
+    return B200W_ERR_BAD_TAPS;
 }
 
 // level sizes of the analysis chain; returns a status
@@ -960,25 +917,20 @@ static int run_afb_chain(const float* x, int64_t x_ps, int64_t x_rs, int planes,
         w = lv.Wo;
     }
     // the store epilogue lives in the stream and the direct kernels: other inputs (unaligned rows) take the direct one
-    if (templated_taps(Lw, Lh) && (plain || (!force_tiled() && afb_stream_supported(p, Lw)))) {
+    const DwtPolicy& pol = dwt_policy();
+    if (templated_taps(Lw, Lh) && (plain || (!pol.force_tiled && afb_stream_supported(p, Lw)))) {
         // chains of small planes: one CTA owns a part of a plane for all levels (TMA-staged owner kernel first, the
         // cp.async owner kernel for the shapes it declines); everything else goes through the ticketed stream chain
         // (or the tile chain when rows are unaligned)
-        if (J > 1 && plain && !force_tiled() && owner_mode() != 0) {
+        const bool owner = J > 1 && !pol.force_tiled && pol.owner != 0, force = pol.owner == 2;
+        if (owner && plain && pol.tma) {
             AfbTmaParams tp;
-            if (afb_tma_plan(p, Lw, device_info().sms, owner_mode() == 2, tp)) return launch_afb_tma(tp, Lw, st);
+            if (afb_tma_plan(p, Lw, device_info().sms, force, pol.tma_G, pol.tma_D, pol.tma_noboxes, tp))
+                return launch_afb_tma(tp, Lw, st);
         }
-        if (J > 1 && !force_tiled() && owner_mode() != 0) {
+        if (owner) {
             AfbOwnerParams op;
-            if (afb_owner_plan(p, Lw, device_info().sms, owner_j0_min(), owner_mode() == 2, op)) {
-                if (op.j0 > 0) {
-                    AfbParams head = p;
-                    head.J = op.j0;
-                    rc = run_afb_big_levels(head, Lw, st);
-                    if (rc) return rc;
-                }
-                return launch_afb_owner(op, Lw, st);
-            }
+            if (afb_owner_plan(p, Lw, device_info().sms, force, op)) return launch_afb_owner(op, Lw, st);
         }
         return run_afb_big_levels(p, Lw, st);
     }
@@ -1000,17 +952,11 @@ static int run_afb_chain(const float* x, int64_t x_ps, int64_t x_rs, int planes,
 
 // ---- synthesis chain -------------------------------------------------------------------------------
 static int run_sfb_big_levels(SfbParams& p, int L, cudaStream_t st) {
-    if (!force_tiled() && sfb_stream_supported(p, L)) return launch_sfb_stream(p, L, device_info().sms, st);
-    switch (L) {
-        case 2: return launch_sfb_chain<2>(p, st);
-        case 4: return launch_sfb_chain<4>(p, st);
-        case 6: return launch_sfb_chain<6>(p, st);
-        case 8: return launch_sfb_chain<8>(p, st);
-        case 10: return launch_sfb_chain<10>(p, st);
-        case 12: return launch_sfb_chain<12>(p, st);
-        case 14: return launch_sfb_chain<14>(p, st);
-        default: return launch_sfb_chain<16>(p, st);
-    }
+    if (!dwt_policy().force_tiled && sfb_stream_supported(p, L)) return launch_sfb_stream(p, L, device_info().sms, st);
+#define X(LL) return launch_sfb_chain<LL>(p, st)
+    B200W_FOR_EACH_L(X)
+#undef X
+    return B200W_ERR_BAD_TAPS;
 }
 
 static int sfb_check_dims(int planes, const int* hs, const int* ws, int Lw, int Lh, int mode, int J, const int* out_hs,
@@ -1096,13 +1042,15 @@ static int run_sfb_chain(const float* yl, int64_t yl_ps, int64_t yl_rs, const fl
         lv.y_vec = 1;
     }
     if (templated_taps(Lw, Lh)) {
-        if (J > 1 && !force_tiled() && owner_mode() != 0) {
+        const DwtPolicy& pol = dwt_policy();
+        const bool owner = J > 1 && !pol.force_tiled && pol.owner != 0, force = pol.owner == 2;
+        if (owner && pol.tma) {
             SfbTmaParams tp;
-            if (sfb_tma_plan(p, Lw, device_info().sms, owner_mode() == 2, tp)) return launch_sfb_tma(tp, Lw, st);
+            if (sfb_tma_plan(p, Lw, device_info().sms, force, pol.tma_G, pol.tma_D, tp)) return launch_sfb_tma(tp, Lw, st);
         }
-        if (J > 1 && !force_tiled() && owner_mode() != 0) {
+        if (owner) {
             SfbOwnerParams op;
-            if (sfb_owner_plan(p, Lw, device_info().sms, owner_mode() == 2, op)) return launch_sfb_owner(op, Lw, st);
+            if (sfb_owner_plan(p, Lw, device_info().sms, force, op)) return launch_sfb_owner(op, Lw, st);
         }
         return run_sfb_big_levels(p, Lw, st);
     }

@@ -66,14 +66,12 @@ struct AfbParams {
     Taps t;
 };
 
-// "Owner" kernels (small planes, J > 1): one CTA owns a horizontal part of one plane for ALL levels from j0 on.  The
-// first of them streams its input rows from global memory, the low-pass image of every level but the last stays in
-// the CTA's shared memory, so the dependent levels cost a block barrier instead of a trip through L2 and a
-// grid-wide dependency.  Parts of a plane overlap by the few rows the deeper levels need (recomputed, not shared).
+// "Owner" kernels (small planes, J > 1): one CTA owns a horizontal part of one plane for ALL levels.  The first level
+// streams its input rows from global memory, the low-pass image of every level but the last stays in the CTA's
+// shared memory, so the dependent levels cost a block barrier instead of a trip through L2 and a grid-wide
+// dependency.  Parts of a plane overlap by the few rows the deeper levels need (recomputed, not shared).
 constexpr int kMaxParts = 8;
-#ifndef B200W_OWNER_NT
-#define B200W_OWNER_NT 384   // threads of an owner CTA for filters up to 8 taps: 12 warps with up to 168 registers each (measured best of 256..512, profiles/r01_notes.md)
-#endif
+constexpr int kOwnerNT = 384;   // threads of an owner CTA for filters up to 8 taps: 12 warps with up to 168 registers each (measured best of 256..512, profiles/r01_notes.md)
 struct OwnerLevel {
     int R;                 // output rows per thread segment
     int pitch;             // row pitch (floats, multiple of 4) of this level's low-pass image in shared memory
@@ -85,7 +83,7 @@ struct OwnerLevel {
 struct AfbOwnerParams {
     AfbParams p;
     OwnerLevel ol[kMaxLevels];
-    int j0, parts;
+    int parts;
     int ring_floats;       // size of the staging rings that precede the maps and the low-pass area
     int map_ints;          // size of the extension-map area (all levels)
 };
@@ -145,10 +143,10 @@ int launch_afb_stream(AfbParams& p, int L, int sms, cudaStream_t st);
 bool sfb_stream_supported(const SfbParams& p, int L);
 int launch_sfb_stream(SfbParams& p, int L, int sms, cudaStream_t st);
 
-// owner kernel (dwt_stream_afb.cu): levels j0 .. J-1 of an analysis chain in one launch without grid-wide
-// dependencies.  afb_owner_plan fills `op` and returns true when the shapes qualify (low-pass images fit in shared
-// memory, enough planes x parts to occupy the device -- unless `force`); j0_min = first level it may start from.
-bool afb_owner_plan(const AfbParams& p, int L, int sms, int j0_min, bool force, AfbOwnerParams& op);
+// owner kernel (dwt_stream_afb.cu): all levels of an analysis chain in one launch without grid-wide dependencies.
+// afb_owner_plan fills `op` and returns true when the shapes qualify (low-pass images fit in shared memory, enough
+// planes x parts to occupy the device -- unless `force`).
+bool afb_owner_plan(const AfbParams& p, int L, int sms, bool force, AfbOwnerParams& op);
 int launch_afb_owner(const AfbOwnerParams& op, int L, cudaStream_t st);
 
 // synthesis owner kernel (dwt_stream_sfb.cu): all positions of a synthesis chain in one launch, the intermediate
@@ -191,5 +189,52 @@ static inline void sfb_register_bounds(const SfbParams&, cudaStream_t) {}
 
 static inline int ceil_div(int a, int b) { return (a + b - 1) / b; }
 static inline bool aligned_to(const void* p, size_t a) { return (reinterpret_cast<uintptr_t>(p) & (a - 1)) == 0; }
+
+// Kernel-family selection from the environment, read once per process (api.cu).  The switches run independently
+// written kernel families against each other on the same inputs; the defaults are what every other run takes.
+struct DwtPolicy {
+    bool force_direct;   // B200W_FORCE_DIRECT=1: one-thread-per-output kernels only
+    bool force_tiled;    // B200W_FORCE_TILED=1: shared-memory tile kernels instead of the stream and owner kernels
+    int owner;           // B200W_OWNER: 0 = no owner kernels (ticketed chains), 1 = where they pay off, 2 = whenever they fit
+    bool tma;            // B200W_TMA=0: cp.async owner kernels instead of the TMA-staged ones
+    bool tma_noboxes;    // B200W_TMA_NOBOXES: TMA analysis ring fetches every extension row from its source row
+    int tma_G, tma_D;    // B200W_TMA_G / B200W_TMA_D: row streams / ring stages of the TMA kernels (0 = the plan's choice)
+};
+const DwtPolicy& dwt_policy();
+
+// the owner kernels run one CTA per SM: a short last wave wastes too much of the device
+static inline bool short_last_wave(long long ctas, int sms) {
+    const long long waves = (ctas + sms - 1) / sms;
+    return ctas * 4 < waves * sms * 3 && waves > 1;
+}
+
+constexpr size_t kMaxDynSmem = 227 * 1024;   // dynamic shared memory of one CTA on sm_100a
+
+// lets `Kernel` use up to kMaxDynSmem of dynamic shared memory; the attribute is per device (a process may drive
+// several GPUs), so it is set once per device
+template <auto Kernel>
+static cudaError_t allow_max_dyn_smem() {
+    static bool attr_set[64] = {false};
+    int dev = 0;
+    cudaGetDevice(&dev);
+    if (dev >= 0 && dev < 64 && attr_set[dev]) return cudaSuccess;
+    const cudaError_t e = cudaFuncSetAttribute(Kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kMaxDynSmem);
+    if (e == cudaSuccess && dev >= 0 && dev < 64) attr_set[dev] = true;
+    return e;
+}
+
+// X(L) for each tap count the templated kernels are instantiated for; X returns, other L fall through
+#define B200W_FOR_EACH_L(X) \
+    switch (L) {             \
+        case 2: X(2);        \
+        case 4: X(4);        \
+        case 6: X(6);        \
+        case 8: X(8);        \
+        case 10: X(10);      \
+        case 12: X(12);      \
+        case 14: X(14);      \
+        case 16: X(16);      \
+        default: break;      \
+    }
 
 }  // namespace b200w

@@ -23,7 +23,6 @@
 // Segments overlap by L-2 input rows (re-read through L2).
 #include <algorithm>
 #include <cmath>
-#include <cstdio>
 #include "dwt_levels.cuh"
 
 namespace b200w {
@@ -111,19 +110,6 @@ __device__ __forceinline__ void afb_pair_fma(const Taps& t, const float (&v)[2][
     }
 }
 
-#ifdef B200W_TIMELINE
-// debug build only (B200W_TIMELINE=1 python -m b200wave._build): per-CTA timestamps of the last chained launch
-__device__ unsigned long long* g_timeline = nullptr;
-__device__ __forceinline__ unsigned long long gtime() {
-    unsigned long long t;
-    asm volatile("mov.u64 %0, %globaltimer;" : "=l"(t));
-    return t;
-}
-#define TL_MARK(slot) do { if (g_timeline && threadIdx.x == 0) g_timeline[(size_t)item * 16 + (slot)] = ((slot) == 0 || (slot) == 5) ? gtime() : (unsigned long long)clock64(); } while (0)
-#else
-#define TL_MARK(slot) do { } while (0)
-#endif
-
 // block until every CTA item of the previous level of this plane has been published (called by all threads,
 // after their index arithmetic so that the set-up overlaps the wait)
 __device__ __forceinline__ void chain_wait(const unsigned* ctr, unsigned need) {
@@ -160,8 +146,7 @@ __device__ __forceinline__ float4 lds128(unsigned addr) {
 // memory, so a lane reads its window straight from there and the ring is not used.
 template <int L, int S, bool OWNER = false, bool SMEM_SRC = false, int Q = 1>
 __device__ __forceinline__ void afb_ring_cta(const AfbParams& p, const AfbLevel& lv, int plane, int it, float4* ring_all,
-                                             const unsigned* wait_ctr, unsigned wait_need, unsigned item,
-                                             const OwnRows& own) {
+                                             const unsigned* wait_ctr, unsigned wait_need, const OwnRows& own) {
     using C = AfbStreamCfg<L, S>;
     constexpr int H2 = C::H2, NV = C::NV, NE = C::NE, D = C::depth(Q);
     constexpr int RP = C::rp(Q), STAGE = 2 * RP;
@@ -252,7 +237,6 @@ __device__ __forceinline__ void afb_ring_cta(const AfbParams& p, const AfbLevel&
     for (int o = 16; o > 0; o >>= 1) npw = max(npw, __shfl_xor_sync(0xffffffffu, npw, o));
 
     if (!OWNER) chain_wait(wait_ctr, wait_need);
-    TL_MARK(1);
     if (!SMEM_SRC) {
 #pragma unroll 1
         for (int s = 0; s < D - 1; ++s) {
@@ -260,7 +244,6 @@ __device__ __forceinline__ void afb_ring_cta(const AfbParams& p, const AfbLevel&
             cp_async_commit();
         }
     }
-    TL_MARK(14);
     // SMEM_SRC: shared address of this lane's window in source row 0
     const unsigned win_s = SMEM_SRC ? own.src_s + (unsigned)(cb - own.src_row0 * (int)rs) * 4u : 0u;
     int orow = i0;         // OWNER: output row the next store belongs to
@@ -276,7 +259,6 @@ __device__ __forceinline__ void afb_ring_cta(const AfbParams& p, const AfbLevel&
                 if (!SMEM_SRC) {
                     cp_async_wait<D - 2>();   // this lane's copies of pair q have landed ...
                     __syncwarp();             // ... and everybody's; all lanes are done reading pair q-1
-                    if (q < 4) TL_MARK(6 + 2 * q);
                     issue(q + D - 1, st_w);   // refill the stage pair q-1 was read from
                     cp_async_commit();
                     st_w = st_w + 1 == D ? 0 : st_w + 1;
@@ -362,7 +344,6 @@ __device__ __forceinline__ void afb_ring_cta(const AfbParams& p, const AfbLevel&
                     }
                 }
                 st_r = st_r + 1 == D ? 0 : st_r + 1;
-                if (q < 4) TL_MARK(7 + 2 * q);
             }
         }
     }
@@ -473,42 +454,30 @@ __global__ void __launch_bounds__(kStreamNT, AfbStreamCfg<L, S>::MINB) afb_strea
     const unsigned local = item - (unsigned)lv.cta_base;
     const int plane = (int)(local / (unsigned)lv.cpp);
     const int cta = (int)(local - (unsigned)plane * (unsigned)lv.cpp);
-    TL_MARK(0);
-    TL_MARK(15);
-#ifdef B200W_TIMELINE
-    if (g_timeline && tid == 0) {
-        g_timeline[(size_t)item * 16 + 3] = ((unsigned long long)level << 48) | ((unsigned long long)plane << 24) | (unsigned)cta;
-        unsigned smid;
-        asm volatile("mov.u32 %0, %smid;" : "=r"(smid));
-        g_timeline[(size_t)item * 16 + 4] = smid | ((unsigned long long)(cta < lv.cppA ? 0 : 1) << 32);
-    }
-#endif
     // the previous level of this plane must be complete before its low-pass image is read
     const unsigned* wait_ctr = level > 0 ? p.done + (size_t)(level - 1) * p.planes + plane : nullptr;
     const unsigned wait_need = level > 0 ? (unsigned)p.lv[level - 1].cpp : 0u;
     const OwnRows none{};
     if (cta < lv.cppA) {
-        afb_ring_cta<L, S>(p, lv, plane, cta * kStreamNT + tid, ring_all, wait_ctr, wait_need, item, none);
+        afb_ring_cta<L, S>(p, lv, plane, cta * kStreamNT + tid, ring_all, wait_ctr, wait_need, none);
     } else {
         const int it = (cta - lv.cppA) * kStreamNT + tid;
         afb_border_item<L, S>(p, lv, plane, it, it < lv.itemsB, wait_ctr, wait_need, none);
     }
-    TL_MARK(2);
     if (level + 1 < p.J) {
         __syncthreads();
         if (tid == 0) signal_done(p.done + (size_t)level * p.planes + plane);
     }
-    TL_MARK(5);
 }
 
-// ---- owner kernel: levels j0 .. J-1 of one (plane, part) in one CTA -------------------------------------------
+// ---- owner kernel: every level of one (plane, part) in one CTA ------------------------------------------------
 // The first level streams from global memory through the same per-warp rings as above; its low-pass rows land in
 // shared memory, where the next level reads its windows directly (SMEM_SRC), and so on.  No tickets, no counters:
 // the only synchronisation is one block barrier per level.
 template <int L>
 struct AfbOwnerCfg {
     // one CTA per SM; long filters need more than 128 registers per thread
-    static constexpr int NT = L <= 8 ? B200W_OWNER_NT : 256;
+    static constexpr int NT = L <= 8 ? kOwnerNT : 256;
     // column pairs per lane: two for the short filters (their accumulators fit the register budget twice)
     static constexpr int Q = 1;
 };
@@ -521,22 +490,13 @@ __global__ void __launch_bounds__(AfbOwnerCfg<L>::NT, 1) afb_owner_kernel(const 
     const int tid = threadIdx.x;
     const int plane = blockIdx.x / op.parts;
     const int part = blockIdx.x - plane * op.parts;
-#ifdef B200W_TIMELINE
-    // slot 0 / 14: %globaltimer at start / end; slot 15: clock at start; slots 1 + 3*(j-j0) + {0,1,2}: clock after the
-    // maps, the interior passes and the border passes of level j
-#define OWN_MARK(slot, v) do { if (g_timeline && tid == 0) g_timeline[(size_t)blockIdx.x * 16 + (slot)] = (v); } while (0)
-    OWN_MARK(0, gtime());
-    OWN_MARK(15, (unsigned long long)clock64());
-#else
-#define OWN_MARK(slot, v) do { } while (0)
-#endif
     pdl_trigger();   // the next kernel in the stream may be scheduled as SMs free up (it waits before touching memory)
     int* const maps = reinterpret_cast<int*>(reinterpret_cast<float*>(ring_all) + op.ring_floats);
     float* const ll_area = reinterpret_cast<float*>(maps) + op.map_ints;
     // extension maps of every level, built once: input rows 2*c0 - offH + [0, 2*nrows + L) and input columns
     // -offW + [0, 2*Wo + L) of level j at maps + map_off[j]
 #pragma unroll 1
-    for (int j = op.j0; j < p.J; ++j) {
+    for (int j = 0; j < p.J; ++j) {
         const AfbLevel& lv = p.lv[j];
         const OwnerLevel& ol = op.ol[j];
         const int c0 = ol.c0[part];
@@ -556,15 +516,14 @@ __global__ void __launch_bounds__(AfbOwnerCfg<L>::NT, 1) afb_owner_kernel(const 
     }
     pdl_wait();      // everything above used only the parameter block; from here on global memory is touched
     __syncthreads();
-    OWN_MARK(13, (unsigned long long)clock64());
 #pragma unroll 1
-    for (int j = op.j0; j < p.J; ++j) {
+    for (int j = 0; j < p.J; ++j) {
         AfbLevel lv = p.lv[j];
         const OwnerLevel& ol = op.ol[j];
         OwnRows own;
         own.c0 = ol.c0[part]; own.c1 = ol.c1[part]; own.h0 = ol.h0[part]; own.h1 = ol.h1[part];
         own.src_s = 0; own.src_row0 = 0;
-        const bool smem_src = j > op.j0;
+        const bool smem_src = j > 0;
         if (smem_src) {   // input = the previous level's low-pass rows [c0', c1') in shared memory
             const OwnerLevel& pv = op.ol[j - 1];
             float* buf = ll_area + pv.buf_off;
@@ -586,7 +545,6 @@ __global__ void __launch_bounds__(AfbOwnerCfg<L>::NT, 1) afb_owner_kernel(const 
         own.itemsA = ((nrows + lv.R - 1) / lv.R) * ((lv.ncpA + Q - 1) / Q);
         own.rmap = maps + ol.map_off;
         own.cmap = own.rmap + 2 * nrows + L;
-        OWN_MARK(1 + 3 * (j - op.j0), (unsigned long long)clock64());
         const int itemsB = nrows * (lv.Wo - 2 * lv.ncpA);
         const int padA = (own.itemsA + 31) & ~31;
         // When the interior segments leave warps free (the plan sizes them so), those warps evaluate the border
@@ -598,37 +556,18 @@ __global__ void __launch_bounds__(AfbOwnerCfg<L>::NT, 1) afb_owner_kernel(const 
             for (int base = 0; base < own.itemsA; base += ntA) {
                 __syncwarp();   // the warp's ring is reused from pass to pass
                 if (smem_src)
-                    afb_ring_cta<L, S, true, true, Q>(p, lv, plane, base + tid, ring_all, nullptr, 0u, 0u, own);
+                    afb_ring_cta<L, S, true, true, Q>(p, lv, plane, base + tid, ring_all, nullptr, 0u, own);
                 else
-                    afb_ring_cta<L, S, true, false, Q>(p, lv, plane, base + tid, ring_all, nullptr, 0u, 0u, own);
+                    afb_ring_cta<L, S, true, false, Q>(p, lv, plane, base + tid, ring_all, nullptr, 0u, own);
             }
         }
-#ifdef B200W_TIMELINE
-        if (!beside) __syncthreads();
-        OWN_MARK(2 + 3 * (j - op.j0), (unsigned long long)clock64());
-#endif
         if (!beside || tid >= padA) {
             const int nb = beside ? NT - padA : NT;
             for (int it = beside ? tid - padA : NT - 1 - tid; it < itemsB; it += nb)
                 afb_border_item<L, S, true>(p, lv, plane, it, true, nullptr, 0u, own);
         }
         __syncthreads();   // this level's low-pass rows are complete before the next level reads them
-        OWN_MARK(3 + 3 * (j - op.j0), (unsigned long long)clock64());
     }
-    OWN_MARK(14, gtime());
-}
-
-static int env_int(const char* name, int dflt) {
-    const char* e = getenv(name);
-    if (!e || !*e) return dflt;
-    const int v = atoi(e);
-    return v > 0 ? v : dflt;
-}
-// tuning knob (read once): rows per segment override
-static int stream_rows_override() {
-    static int v = -1;
-    if (v < 0) v = env_int("B200W_STREAM_ROWS", 0);
-    return v;
 }
 
 bool afb_stream_supported(const AfbParams& p, int L) {
@@ -643,6 +582,20 @@ bool afb_stream_supported(const AfbParams& p, int L) {
     return true;
 }
 
+// interior / border split of the output columns of a level (the same for the stream and the owner kernel)
+template <int L, int S>
+static void afb_stream_columns(AfbLevel& lv) {
+    using C = AfbStreamCfg<L, S>;
+    lv.ncp = ceil_div(lv.Wo, 2);
+    // interior column pairs: window [4cp - (offW+S), +NE) inside [0, Wreal) and both output columns valid
+    lv.cp0A = (lv.offW + S) / 4;
+    int cpR = (lv.Wreal + lv.offW + S - C::NE) / 4 + 1;   // first pair whose window leaves the image
+    if (lv.Wreal + lv.offW + S - C::NE < 0) cpR = 0;
+    if (cpR > lv.Wo / 2) cpR = lv.Wo / 2;
+    lv.ncpA = cpR - lv.cp0A;
+    if (lv.ncpA < kMinColPairs) lv.ncpA = 0;              // too narrow for the ring: all columns take the border path
+}
+
 template <int L, int S>
 static int launch_afb_stream_t(AfbParams& p, int sms, cudaStream_t st) {
     using C = AfbStreamCfg<L, S>;
@@ -653,7 +606,7 @@ static int launch_afb_stream_t(AfbParams& p, int sms, cudaStream_t st) {
     // the other): it gets shorter segments, down to 2 rows for the small dependent levels of a chain.
     // rows per work item of the first level.  Every item re-reads L/2 - 1 row pairs of warm-up, which favours long items
     // for long filters; short filters have (almost) no warm-up and balance better with short items.  Measured at
-    // 64 x 1024^2 (B200W_STREAM_ROWS sweep, profiles/r02_notes.md): haar 6 / 16 rows = 81.5 / 85.8 us, db2 92.8 (8 rows:
+    // 64 x 1024^2 (rows-per-item sweep, profiles/r02_notes.md): haar 6 / 16 rows = 81.5 / 85.8 us, db2 92.8 (8 rows:
     // 94.1) / 104.7 us; db3 gains 2 % at J = 1 with 10 rows but loses 1-3 % in chains (J >= 2), so it keeps 16 like
     // db4 and longer, where 16+ rows are best.
     const int rpref = H2 == 1 ? 6 : (H2 == 2 ? 8 : std::max(16, 4 * (H2 - 1)));
@@ -661,14 +614,7 @@ static int launch_afb_stream_t(AfbParams& p, int sms, cudaStream_t st) {
     long long base = 0;
     for (int j = 0; j < p.J; ++j) {
         AfbLevel& lv = p.lv[j];
-        lv.ncp = ceil_div(lv.Wo, 2);
-        // interior column pairs: window [4cp - (offW+S), +NE) inside [0, Wreal) and both output columns valid
-        lv.cp0A = (lv.offW + S) / 4;
-        int cpR = (lv.Wreal + lv.offW + S - C::NE) / 4 + 1;   // first pair whose window leaves the image
-        if (lv.Wreal + lv.offW + S - C::NE < 0) cpR = 0;
-        if (cpR > lv.Wo / 2) cpR = lv.Wo / 2;
-        lv.ncpA = cpR - lv.cp0A;
-        if (lv.ncpA < kMinColPairs) lv.ncpA = 0;              // too narrow for the ring: all columns take the border path
+        afb_stream_columns<L, S>(lv);
         // the first level keeps the preferred length (measured best even when it leaves CTA slots empty; an
         // SM-balancing search over R was tried and was not better, profiles/r01_notes.md); the dependent levels of a
         // chain shrink until they fill the resident slots
@@ -678,7 +624,6 @@ static int launch_afb_stream_t(AfbParams& p, int sms, cudaStream_t st) {
             while (R > rmin && (long long)p.planes * ceil_div(ceil_div(lv.Ho, R) * std::max(lv.ncpA, 1), kStreamNT) < slots)
                 R = std::max(rmin, R - 2);
         }
-        if (stream_rows_override() > 0) R = stream_rows_override();
         if (R > lv.Ho) R = lv.Ho;
         lv.R = R;
         const int nseg = ceil_div(lv.Ho, R);
@@ -696,28 +641,10 @@ static int launch_afb_stream_t(AfbParams& p, int sms, cudaStream_t st) {
         const int rc = zero_sync_words(p.ticket, (size_t)p.J * p.planes + 1, st);
         if (rc) return rc;
     }
-#ifdef B200W_TIMELINE
-    static unsigned long long* tl = nullptr;
-    const char* tl_path = getenv("B200W_TIMELINE_FILE");
-    if (tl_path) {
-        if (!tl) cudaMalloc(&tl, sizeof(unsigned long long) * 16 * 65536);
-        cudaMemsetAsync(tl, 0, sizeof(unsigned long long) * 16 * 65536, st);
-        cudaMemcpyToSymbolAsync(g_timeline, &tl, sizeof(tl), 0, cudaMemcpyHostToDevice, st);
-    }
-#endif
     afb_register_bounds(p, st);
     afb_stream_kernel<L, S><<<(unsigned)base, kStreamNT, C::smem, st>>>(p);
     note_launch("afb_stream_kernel");
     const cudaError_t e = cudaGetLastError();
-#ifdef B200W_TIMELINE
-    if (tl_path && base <= 65536) {
-        cudaStreamSynchronize(st);
-        static unsigned long long host[16 * 65536];
-        cudaMemcpy(host, tl, sizeof(unsigned long long) * 16 * (size_t)base, cudaMemcpyDeviceToHost);
-        FILE* f = fopen(tl_path, "wb");
-        if (f) { fwrite(host, sizeof(unsigned long long) * 16, (size_t)base, f); fclose(f); }
-    }
-#endif
     return e == cudaSuccess ? B200W_OK : set_last_cuda_error(e);
 }
 
@@ -727,39 +654,21 @@ static int launch_afb_stream_l(AfbParams& p, int sms, cudaStream_t st) {
     return launch_afb_stream_t<L, afb_shift(L, false)>(p, sms, st);
 }
 
-// interior / border split of the output columns of a level (the same for the stream and the owner kernel)
-template <int L, int S>
-static void afb_stream_columns(AfbLevel& lv) {
-    using C = AfbStreamCfg<L, S>;
-    lv.ncp = ceil_div(lv.Wo, 2);
-    lv.cp0A = (lv.offW + S) / 4;
-    int cpR = (lv.Wreal + lv.offW + S - C::NE) / 4 + 1;
-    if (lv.Wreal + lv.offW + S - C::NE < 0) cpR = 0;
-    if (cpR > lv.Wo / 2) cpR = lv.Wo / 2;
-    lv.ncpA = cpR - lv.cp0A;
-    if (lv.ncpA < kMinColPairs) lv.ncpA = 0;
-}
-
-constexpr size_t kOwnerSmemMax = 227 * 1024;
 // dynamic shared memory of the owner kernel: [rings | extension maps | low-pass images]
-
 template <int L, int S>
-static bool afb_owner_plan_t(const AfbParams& p, int sms, int j0_min, bool force, AfbOwnerParams& op) {
+static bool afb_owner_plan_t(const AfbParams& p, int sms, bool force, AfbOwnerParams& op) {
     using C = AfbStreamCfg<L, S>;
     constexpr int NT = AfbOwnerCfg<L>::NT, Q = AfbOwnerCfg<L>::Q;
     constexpr int H2 = L / 2;
     const int J = p.J;
-    if (J < 2 || j0_min > J - 2) return false;
+    if (J < 2) return false;
     const bool wraps = p.mode == B200W_MODE_PERIODIZATION || p.mode == B200W_MODE_PERIODIC;
     int parts = std::min(kMaxParts, std::max(1, sms / p.planes));
     if (wraps) parts = 1;   // a part would need rows from the far end of the image
     parts = std::min(parts, p.lv[J - 1].Ho);
-    if (!force) {
-        // one CTA per SM: a short last wave wastes up to half of the time (few CTAs are fine: small batches are
-        // latency-bound either way, and measured faster here than as ticketed chains, profiles/r01_smallbatch.log)
-        const long long ctas = (long long)p.planes * parts, waves = (ctas + sms - 1) / sms;
-        if (ctas * 4 < waves * sms * 3 && waves > 1) return false;
-    }
+    // one CTA per SM: a short last wave wastes up to half of the time (few CTAs are fine: small batches are
+    // latency-bound either way, and measured faster here than as ticketed chains, profiles/r01_smallbatch.log)
+    if (!force && short_last_wave((long long)p.planes * parts, sms)) return false;
     op.p = p;
     op.parts = parts;
     op.ring_floats = (int)((size_t)(NT / 32) * C::ring_float4_per_warp(Q) * 4);
@@ -792,119 +701,69 @@ static bool afb_owner_plan_t(const AfbParams& p, int sms, int j0_min, bool force
             op.ol[j].c1[q] = hi;
         }
     }
-    // start at the first level from which on the low-pass images fit next to the rings
-    for (int j0 = j0_min; j0 <= J - 2; ++j0) {
-        // Starting behind a chain launch of the first level(s) is only taken when asked for (B200W_OWNER=2 /
-        // B200W_OWNER_J0): with big first levels the dependent ones are a few percent of the work, and their parts
-        // recompute more rows than they own (16 x 2048^2, J = 5: 172 vs 164 us for the plain chain)
-        if (j0 > 0 && !force && j0_min == 0) return false;
-        size_t floats = 0;
-        for (int j = j0; j < J - 1; ++j) {
-            int rows = 0;
-            for (int q = 0; q < parts; ++q) rows = std::max(rows, op.ol[j].c1[q] - op.ol[j].c0[q]);
-            op.ol[j].pitch = (p.lv[j].Wo + 3) / 4 * 4;
-            op.ol[j].buf_off = (int)floats;
-            floats += (size_t)rows * op.ol[j].pitch;
-        }
-        int map_ints = 0;
-        for (int j = j0; j < J; ++j) {
-            int rows = 0;
-            for (int q = 0; q < parts; ++q) rows = std::max(rows, op.ol[j].c1[q] - op.ol[j].c0[q]);
-            op.ol[j].map_off = map_ints;
-            map_ints += 2 * rows + L + 2 * p.lv[j].Wo + L;
-        }
-        op.map_ints = (map_ints + 3) / 4 * 4;
-        if (((size_t)op.ring_floats + op.map_ints + floats) * 4 > kOwnerSmemMax) continue;
-        op.j0 = j0;
-        for (int j = j0; j < J; ++j) {
-            // segments sized so that one pass of the CTA's threads covers the part
-            int rows = 0;
-            for (int q = 0; q < parts; ++q) rows = std::max(rows, op.ol[j].c1[q] - op.ol[j].c0[q]);
-            const int ncpA = std::max(1, (op.p.lv[j].ncpA + Q - 1) / Q);   // lanes per row
-            const int rmin = std::max(2, H2 - 1);
-            // some warps are kept free for the border positions (about four rounds of them), which then run
-            // beside the interior segments instead of after them
-            const int itemsB = rows * (p.lv[j].Wo - 2 * op.p.lv[j].ncpA);
-            int spare = itemsB > 0 ? std::min(NT / 2, std::max(32, (ceil_div(itemsB, 4) + 31) & ~31)) : 0;
-            if ((NT - spare) / ncpA < 1) spare = 0;
-            const int rmax = std::max(16, 4 * (H2 - 1));
-            int R = std::max(rmin, ceil_div(rows, std::max(1, (NT - spare) / ncpA)));
-            if (R > rmax) {   // no room for spare warps: one class after the other
-                R = std::max(rmin, ceil_div(rows, std::max(1, NT / ncpA)));
-                // one pass of somewhat longer segments beats a second, mostly empty pass; far longer ones do not
-                if (R > 2 * rmax) R = rmax;
-            }
-            if (stream_rows_override() > 0) R = stream_rows_override();
-            op.ol[j].R = std::max(1, std::min(R, rows));
-        }
-        return true;
+    // the low-pass images of every level but the last must fit next to the rings
+    size_t floats = 0;
+    for (int j = 0; j < J - 1; ++j) {
+        int rows = 0;
+        for (int q = 0; q < parts; ++q) rows = std::max(rows, op.ol[j].c1[q] - op.ol[j].c0[q]);
+        op.ol[j].pitch = (p.lv[j].Wo + 3) / 4 * 4;
+        op.ol[j].buf_off = (int)floats;
+        floats += (size_t)rows * op.ol[j].pitch;
     }
-    return false;
+    int map_ints = 0;
+    for (int j = 0; j < J; ++j) {
+        int rows = 0;
+        for (int q = 0; q < parts; ++q) rows = std::max(rows, op.ol[j].c1[q] - op.ol[j].c0[q]);
+        op.ol[j].map_off = map_ints;
+        map_ints += 2 * rows + L + 2 * p.lv[j].Wo + L;
+    }
+    op.map_ints = (map_ints + 3) / 4 * 4;
+    if (((size_t)op.ring_floats + op.map_ints + floats) * 4 > kMaxDynSmem) return false;
+    for (int j = 0; j < J; ++j) {
+        // segments sized so that one pass of the CTA's threads covers the part
+        int rows = 0;
+        for (int q = 0; q < parts; ++q) rows = std::max(rows, op.ol[j].c1[q] - op.ol[j].c0[q]);
+        const int ncpA = std::max(1, (op.p.lv[j].ncpA + Q - 1) / Q);   // lanes per row
+        const int rmin = std::max(2, H2 - 1);
+        // some warps are kept free for the border positions (about four rounds of them), which then run
+        // beside the interior segments instead of after them
+        const int itemsB = rows * (p.lv[j].Wo - 2 * op.p.lv[j].ncpA);
+        int spare = itemsB > 0 ? std::min(NT / 2, std::max(32, (ceil_div(itemsB, 4) + 31) & ~31)) : 0;
+        if ((NT - spare) / ncpA < 1) spare = 0;
+        const int rmax = std::max(16, 4 * (H2 - 1));
+        int R = std::max(rmin, ceil_div(rows, std::max(1, (NT - spare) / ncpA)));
+        if (R > rmax) {   // no room for spare warps: one class after the other
+            R = std::max(rmin, ceil_div(rows, std::max(1, NT / ncpA)));
+            // one pass of somewhat longer segments beats a second, mostly empty pass; far longer ones do not
+            if (R > 2 * rmax) R = rmax;
+        }
+        op.ol[j].R = std::max(1, std::min(R, rows));
+    }
+    return true;
 }
 
 template <int L, int S>
 static int launch_afb_owner_t(const AfbOwnerParams& op, cudaStream_t st) {
     constexpr int NT = AfbOwnerCfg<L>::NT;
     size_t floats = (size_t)op.ring_floats + op.map_ints;
-    for (int j = op.j0; j < op.p.J - 1; ++j) {
+    for (int j = 0; j < op.p.J - 1; ++j) {
         int rows = 0;
         for (int q = 0; q < op.parts; ++q) rows = std::max(rows, op.ol[j].c1[q] - op.ol[j].c0[q]);
         floats = std::max(floats, (size_t)op.ring_floats + op.map_ints + op.ol[j].buf_off + (size_t)rows * op.ol[j].pitch);
     }
-    // the attribute is per device: a process may drive several GPUs
-    static bool attr_set[64] = {false};
-    int dev = 0;
-    cudaGetDevice(&dev);
-    if (dev < 0 || dev >= 64 || !attr_set[dev]) {
-        const cudaError_t e = cudaFuncSetAttribute(afb_owner_kernel<L, S>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                                   (int)kOwnerSmemMax);
-        if (e != cudaSuccess) return set_last_cuda_error(e);
-        if (dev >= 0 && dev < 64) attr_set[dev] = true;
-    }
-#ifdef B200W_TIMELINE
-    static unsigned long long* tl = nullptr;
-    const char* tl_path = getenv("B200W_TIMELINE_FILE");
-    const size_t ncta = (size_t)op.p.planes * op.parts;
-    if (tl_path && ncta <= 65536) {
-        if (!tl) cudaMalloc(&tl, sizeof(unsigned long long) * 16 * 65536);
-        cudaMemsetAsync(tl, 0, sizeof(unsigned long long) * 16 * 65536, st);
-        cudaMemcpyToSymbolAsync(g_timeline, &tl, sizeof(tl), 0, cudaMemcpyHostToDevice, st);
-    }
-#endif
+    if (const cudaError_t e = allow_max_dyn_smem<afb_owner_kernel<L, S>>()) return set_last_cuda_error(e);
     afb_register_bounds(op.p, st);
     const cudaError_t le = launch_pdl(afb_owner_kernel<L, S>, (unsigned)(op.p.planes * op.parts), NT, floats * 4, st, op);
     note_launch("afb_owner_kernel");
     const cudaError_t e = le != cudaSuccess ? le : cudaGetLastError();
-#ifdef B200W_TIMELINE
-    if (tl_path && ncta <= 65536) {
-        cudaStreamSynchronize(st);
-        static unsigned long long host[16 * 65536];
-        cudaMemcpy(host, tl, sizeof(unsigned long long) * 16 * ncta, cudaMemcpyDeviceToHost);
-        FILE* f = fopen(tl_path, "wb");
-        if (f) { fwrite(host, sizeof(unsigned long long) * 16, ncta, f); fclose(f); }
-    }
-#endif
     return e == cudaSuccess ? B200W_OK : set_last_cuda_error(e);
 }
 
-#define B200W_FOR_EACH_L(X) \
-    switch (L) {             \
-        case 2: X(2);        \
-        case 4: X(4);        \
-        case 6: X(6);        \
-        case 8: X(8);        \
-        case 10: X(10);      \
-        case 12: X(12);      \
-        case 14: X(14);      \
-        case 16: X(16);      \
-        default: break;      \
-    }
-
-bool afb_owner_plan(const AfbParams& p, int L, int sms, int j0_min, bool force, AfbOwnerParams& op) {
+bool afb_owner_plan(const AfbParams& p, int L, int sms, bool force, AfbOwnerParams& op) {
     if (!afb_stream_supported(p, L)) return false;
     const bool per = p.mode == B200W_MODE_PERIODIZATION;
-#define X(LL) return per ? afb_owner_plan_t<LL, afb_shift(LL, true)>(p, sms, j0_min, force, op) \
-                         : afb_owner_plan_t<LL, afb_shift(LL, false)>(p, sms, j0_min, force, op)
+#define X(LL) return per ? afb_owner_plan_t<LL, afb_shift(LL, true)>(p, sms, force, op) \
+                         : afb_owner_plan_t<LL, afb_shift(LL, false)>(p, sms, force, op)
     B200W_FOR_EACH_L(X)
 #undef X
     return false;
@@ -920,17 +779,10 @@ int launch_afb_owner(const AfbOwnerParams& op, int L, cudaStream_t st) {
 }
 
 int launch_afb_stream(AfbParams& p, int L, int sms, cudaStream_t st) {
-    switch (L) {
-        case 2: return launch_afb_stream_l<2>(p, sms, st);
-        case 4: return launch_afb_stream_l<4>(p, sms, st);
-        case 6: return launch_afb_stream_l<6>(p, sms, st);
-        case 8: return launch_afb_stream_l<8>(p, sms, st);
-        case 10: return launch_afb_stream_l<10>(p, sms, st);
-        case 12: return launch_afb_stream_l<12>(p, sms, st);
-        case 14: return launch_afb_stream_l<14>(p, sms, st);
-        case 16: return launch_afb_stream_l<16>(p, sms, st);
-        default: return B200W_ERR_BAD_TAPS;
-    }
+#define X(LL) return launch_afb_stream_l<LL>(p, sms, st)
+    B200W_FOR_EACH_L(X)
+#undef X
+    return B200W_ERR_BAD_TAPS;
 }
 
 }  // namespace b200w

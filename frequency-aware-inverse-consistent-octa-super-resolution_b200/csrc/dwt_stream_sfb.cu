@@ -22,7 +22,6 @@
 // the natural size crop.
 #include <algorithm>
 #include <cmath>
-#include <cstdio>
 #include "dwt_levels.cuh"
 
 namespace b200w {
@@ -427,23 +426,13 @@ __global__ void __launch_bounds__(kStreamNT, SfbStreamCfg<L, S2V>::MINB) sfb_str
     }
 }
 
-#ifdef B200W_TIMELINE
-// debug build only: per-CTA timestamps of the last owner launch (tools/timeline_owner.py)
-__device__ unsigned long long* g_sfb_timeline = nullptr;
-__device__ __forceinline__ unsigned long long sfb_gtime() {
-    unsigned long long t;
-    asm volatile("mov.u64 %0, %globaltimer;" : "=l"(t));
-    return t;
-}
-#endif
-
 // ---- owner kernel: every position of a synthesis chain for one (plane, part) in one CTA ------------------------
 // The coarsest position reads its low-pass input from global memory through the ring like the stream kernel; every
 // output but the last stays in shared memory, where the next position reads it as its low-pass input (SMEM_LOW),
 // the detail bands still streaming in through the ring.  One block barrier per position, no tickets or counters.
 template <int L>
 struct SfbOwnerCfg {
-    static constexpr int NT = L <= 8 ? B200W_OWNER_NT : 256;   // one CTA per SM; long filters need > 128 registers per thread
+    static constexpr int NT = L <= 8 ? kOwnerNT : 256;   // one CTA per SM; long filters need > 128 registers per thread
 };
 
 template <int L, int S2V>
@@ -457,16 +446,6 @@ __global__ void __launch_bounds__(SfbOwnerCfg<L>::NT, 1) sfb_owner_kernel(const 
     float* const y_area = reinterpret_cast<float*>(sfb_ring_all) + op.ring_floats;
     pdl_trigger();   // see afb_owner_kernel
     pdl_wait();
-#ifdef B200W_TIMELINE
-    // slot 0 / 14: %globaltimer at start / end; slot 15: clock at start; slots 1 + 3*c + {0,1,2}: clock after the
-    // set-up, the interior passes and the border passes of chain position c
-#define SFB_OWN_MARK(slot, v) do { if (g_sfb_timeline && tid == 0) g_sfb_timeline[(size_t)blockIdx.x * 16 + (slot)] = (v); } while (0)
-    SFB_OWN_MARK(0, sfb_gtime());
-    SFB_OWN_MARK(15, (unsigned long long)clock64());
-    SFB_OWN_MARK(13, (unsigned long long)clock64());
-#else
-#define SFB_OWN_MARK(slot, v) do { } while (0)
-#endif
 #pragma unroll 1
     for (int c = 0; c < p.J; ++c) {
         SfbLevel lv = p.lv[c];
@@ -494,7 +473,6 @@ __global__ void __launch_bounds__(SfbOwnerCfg<L>::NT, 1) sfb_owner_kernel(const 
         lv.Rp = ol.R;
         const int npairs = ((lv.offH + own.n1 - 1) >> 1) + 1 - ((own.n0 + lv.offH) >> 1);
         own.itemsA = ((npairs + lv.Rp - 1) / lv.Rp) * lv.ntA;
-        SFB_OWN_MARK(1 + 3 * c, (unsigned long long)clock64());
         for (int base = 0; base < own.itemsA; base += NT) {
             __syncwarp();   // the warp's ring is reused from pass to pass
             const int it = base + tid;
@@ -508,30 +486,12 @@ __global__ void __launch_bounds__(SfbOwnerCfg<L>::NT, 1) sfb_owner_kernel(const 
                 else sfb_ring_cta<L, 1, 0, true, false>(p, lv, plane, it, sfb_ring_all, nullptr, 0u, own);
             }
         }
-#ifdef B200W_TIMELINE
-        __syncthreads();
-        SFB_OWN_MARK(2 + 3 * c, (unsigned long long)clock64());
-#endif
         // border columns go to the last threads first: warps with no or short segments start them early
         const int itemsB = (own.n1 - own.n0) * (lv.nA0 + lv.out_w - lv.nA1);
         for (int it = NT - 1 - tid; it < itemsB; it += NT)
             sfb_border_item<L, true>(p, lv, plane, it, true, nullptr, 0u, own);
         __syncthreads();   // this position's output is complete before the next one reads it
-        SFB_OWN_MARK(3 + 3 * c, (unsigned long long)clock64());
     }
-    SFB_OWN_MARK(14, sfb_gtime());
-}
-
-static int sfb_env_int(const char* name, int dflt) {
-    const char* e = getenv(name);
-    if (!e || !*e) return dflt;
-    const int v = atoi(e);
-    return v > 0 ? v : dflt;
-}
-static int stream_pairs_override() {
-    static int v = -1;
-    if (v < 0) v = sfb_env_int("B200W_STREAM_ROWS", 0);
-    return v;
 }
 
 bool sfb_stream_supported(const SfbParams& p, int L) {
@@ -570,8 +530,6 @@ static void sfb_stream_columns(SfbLevel& lv) {
     if (lv.y_vec == 2 && !(lv.y_rs & 3) && !(lv.y_ps & 3) && aligned_to(lv.y, 16)) lv.y_vec = 4;
 }
 
-constexpr size_t kSfbOwnerSmemMax = 227 * 1024;
-
 template <int L, bool PER>
 static bool sfb_owner_plan_t(const SfbParams& p, int sms, bool force, SfbOwnerParams& op) {
     constexpr int NT = SfbOwnerCfg<L>::NT;
@@ -581,12 +539,9 @@ static bool sfb_owner_plan_t(const SfbParams& p, int sms, bool force, SfbOwnerPa
     int parts = std::min(kMaxParts, std::max(1, sms / p.planes));
     if (PER) parts = 1;   // the coefficient rows wrap around: a part would need rows from the far end
     parts = std::min(parts, p.lv[J - 1].out_h);
-    if (!force) {
-        // one CTA per SM: a short last wave wastes up to half of the time (few CTAs are fine: small batches are
-        // latency-bound either way, and measured faster here than as ticketed chains, profiles/r01_smallbatch.log)
-        const long long ctas = (long long)p.planes * parts, waves = (ctas + sms - 1) / sms;
-        if (ctas * 4 < waves * sms * 3 && waves > 1) return false;
-    }
+    // one CTA per SM: a short last wave wastes up to half of the time (few CTAs are fine: small batches are
+    // latency-bound either way, and measured faster here than as ticketed chains, profiles/r01_smallbatch.log)
+    if (!force && short_last_wave((long long)p.planes * parts, sms)) return false;
     op.p = p;
     op.parts = parts;
     // ring of the staging variants this launch can use (64-bit copies with the mode's shift, or 32-bit copies)
@@ -654,78 +609,36 @@ static bool sfb_owner_plan_t(const SfbParams& p, int sms, bool force, SfbOwnerPa
         int Rp = std::max(std::max(2, H2 - 1), ceil_div(npairs, std::max(1, NT / ntA)));
         // one pass of somewhat longer segments beats a second, mostly empty pass; far longer ones do not
         if (Rp > 2 * std::max(16, 4 * (H2 - 1))) Rp = std::max(16, 4 * (H2 - 1));
-        if (stream_pairs_override() > 0) Rp = stream_pairs_override();
         ol.R = std::max(1, Rp);
     }
     op.y_floats = (int)floats;
-    return ((size_t)op.ring_floats + floats) * 4 <= kSfbOwnerSmemMax;
+    return ((size_t)op.ring_floats + floats) * 4 <= kMaxDynSmem;
 }
 
 template <int L, bool PER>
 static int launch_sfb_owner_t(const SfbOwnerParams& op, cudaStream_t st) {
     constexpr int NT = SfbOwnerCfg<L>::NT;
     constexpr int S2V = sfb_shift2(L, PER);
-    // the attribute is per device: a process may drive several GPUs
-    static bool attr_set[64] = {false};
-    int dev = 0;
-    cudaGetDevice(&dev);
-    if (dev < 0 || dev >= 64 || !attr_set[dev]) {
-        const cudaError_t e = cudaFuncSetAttribute(sfb_owner_kernel<L, S2V>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                                   (int)kSfbOwnerSmemMax);
-        if (e != cudaSuccess) return set_last_cuda_error(e);
-        if (dev >= 0 && dev < 64) attr_set[dev] = true;
-    }
+    if (const cudaError_t e = allow_max_dyn_smem<sfb_owner_kernel<L, S2V>>()) return set_last_cuda_error(e);
     const size_t smem = ((size_t)op.ring_floats + op.y_floats) * 4;
-#ifdef B200W_TIMELINE
-    static unsigned long long* tl = nullptr;
-    const char* tl_path = getenv("B200W_TIMELINE_FILE_SFB");
-    const size_t ncta = (size_t)op.p.planes * op.parts;
-    if (tl_path && ncta <= 65536) {
-        if (!tl) cudaMalloc(&tl, sizeof(unsigned long long) * 16 * 65536);
-        cudaMemsetAsync(tl, 0, sizeof(unsigned long long) * 16 * 65536, st);
-        cudaMemcpyToSymbolAsync(g_sfb_timeline, &tl, sizeof(tl), 0, cudaMemcpyHostToDevice, st);
-    }
-#endif
     sfb_register_bounds(op.p, st);
     const cudaError_t le = launch_pdl(sfb_owner_kernel<L, S2V>, (unsigned)(op.p.planes * op.parts), NT, smem, st, op);
     note_launch("sfb_owner_kernel");
     const cudaError_t e = le != cudaSuccess ? le : cudaGetLastError();
-#ifdef B200W_TIMELINE
-    if (tl_path && ncta <= 65536) {
-        cudaStreamSynchronize(st);
-        static unsigned long long host[16 * 65536];
-        cudaMemcpy(host, tl, sizeof(unsigned long long) * 16 * ncta, cudaMemcpyDeviceToHost);
-        FILE* f = fopen(tl_path, "wb");
-        if (f) { fwrite(host, sizeof(unsigned long long) * 16, ncta, f); fclose(f); }
-    }
-#endif
     return e == cudaSuccess ? B200W_OK : set_last_cuda_error(e);
 }
-
-#define B200W_SFB_FOR_EACH_L(X) \
-    switch (L) {                 \
-        case 2: X(2);            \
-        case 4: X(4);            \
-        case 6: X(6);            \
-        case 8: X(8);            \
-        case 10: X(10);          \
-        case 12: X(12);          \
-        case 14: X(14);          \
-        case 16: X(16);          \
-        default: break;          \
-    }
 
 bool sfb_owner_plan(const SfbParams& p, int L, int sms, bool force, SfbOwnerParams& op) {
     if (!sfb_stream_supported(p, L)) return false;
 #define X(LL) return p.periodic ? sfb_owner_plan_t<LL, true>(p, sms, force, op) : sfb_owner_plan_t<LL, false>(p, sms, force, op)
-    B200W_SFB_FOR_EACH_L(X)
+    B200W_FOR_EACH_L(X)
 #undef X
     return false;
 }
 
 int launch_sfb_owner(const SfbOwnerParams& op, int L, cudaStream_t st) {
 #define X(LL) return op.p.periodic ? launch_sfb_owner_t<LL, true>(op, st) : launch_sfb_owner_t<LL, false>(op, st)
-    B200W_SFB_FOR_EACH_L(X)
+    B200W_FOR_EACH_L(X)
 #undef X
     return B200W_ERR_BAD_TAPS;
 }
@@ -751,7 +664,6 @@ static int launch_sfb_stream_t(SfbParams& p, int sms, cudaStream_t st) {
             while (Rp > rmin && (long long)p.planes * ceil_div(ceil_div(npairs, Rp) * std::max(lv.ntA, 1), kStreamNT) < slots)
                 Rp = std::max(rmin, Rp - 2);
         }
-        if (stream_pairs_override() > 0) Rp = stream_pairs_override();
         if (Rp > npairs) Rp = npairs;
         lv.Rp = Rp;
         lv.itemsA = ceil_div(npairs, Rp) * lv.ntA;
@@ -781,17 +693,10 @@ static int launch_sfb_stream_l(SfbParams& p, int sms, cudaStream_t st) {
 }
 
 int launch_sfb_stream(SfbParams& p, int L, int sms, cudaStream_t st) {
-    switch (L) {
-        case 2: return launch_sfb_stream_l<2>(p, sms, st);
-        case 4: return launch_sfb_stream_l<4>(p, sms, st);
-        case 6: return launch_sfb_stream_l<6>(p, sms, st);
-        case 8: return launch_sfb_stream_l<8>(p, sms, st);
-        case 10: return launch_sfb_stream_l<10>(p, sms, st);
-        case 12: return launch_sfb_stream_l<12>(p, sms, st);
-        case 14: return launch_sfb_stream_l<14>(p, sms, st);
-        case 16: return launch_sfb_stream_l<16>(p, sms, st);
-        default: return B200W_ERR_BAD_TAPS;
-    }
+#define X(LL) return launch_sfb_stream_l<LL>(p, sms, st)
+    B200W_FOR_EACH_L(X)
+#undef X
+    return B200W_ERR_BAD_TAPS;
 }
 
 }  // namespace b200w

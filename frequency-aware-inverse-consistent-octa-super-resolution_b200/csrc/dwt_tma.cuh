@@ -52,8 +52,6 @@ struct AfbTmaParams {
     int rp0_off, rp0_stride;   // per-pair row-address table of the first level: int offset, int2 entries per stream
     int fix0_off, fix0_n;      // int offset of the ring's column-patch table (int2 per stage row x extension column) and
                                // the extension columns per stage row
-    int dbg;                   // debug (B200W_TMA_DBG): 1 = consumers do not wait for the data, 2 = consumers skip the arithmetic
-    unsigned long long* timeline;   // debug (B200W_TMA_TIMELINE=file): per-CTA clock stamps, else null
     int bar_off, tab_off, zrow_off, ring_off;   // shared-memory layout (bytes from the dynamic base)
     int zrow_floats, tab_ints;
     int smem_bytes;
@@ -93,17 +91,17 @@ struct SfbTmaParams {
     int low_off;                      // resident yl rows (first position)
     int bar_off, ring_off;
     int smem_bytes;
-    int dbg;
-    unsigned long long* timeline;
 };
 static_assert(sizeof(SfbTmaParams) <= 4096, "kernel parameter block");
 
-bool sfb_tma_plan(const SfbParams& p, int L, int sms, bool force, SfbTmaParams& tp);
+// G / D > 0 replace the plan's row streams of the last position / ring stages (DwtPolicy::tma_G / tma_D)
+bool sfb_tma_plan(const SfbParams& p, int L, int sms, bool force, int G, int D, SfbTmaParams& tp);
 int launch_sfb_tma(const SfbTmaParams& tp, int L, cudaStream_t st);
 
 // planning + launch (dwt_tma_afb.cu).  afb_tma_plan returns false when the shapes do not qualify (unaligned rows, the
 // low-pass images do not fit, the driver has no tensor-map entry point, ...): the caller then takes the other kernels.
-bool afb_tma_plan(const AfbParams& p, int L, int sms, bool force, AfbTmaParams& tp);
+// G / D > 0 replace the plan's row streams / ring stages; `noboxes` fetches every extension row from its source row.
+bool afb_tma_plan(const AfbParams& p, int L, int sms, bool force, int G, int D, bool noboxes, AfbTmaParams& tp);
 int launch_afb_tma(const AfbTmaParams& tp, int L, cudaStream_t st);
 
 }  // namespace b200w

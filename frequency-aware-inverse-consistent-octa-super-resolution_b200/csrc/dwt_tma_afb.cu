@@ -29,13 +29,8 @@
 // The later levels read their input rows from the low-pass image of the level before (rows through a table of row
 // addresses, so the row extension costs nothing; extension columns written once per level by all threads).
 #include <algorithm>
-#include <cstdio>
-#include <cstdlib>
 #include <type_traits>
 #include "dwt_tma.cuh"
-#ifndef B200W_EXP_PFD
-#define B200W_EXP_PFD 1      // prefetch distance of the level-0 consumer loop (experiments: -DB200W_EXP_PFD=n)
-#endif
 
 namespace b200w {
 
@@ -168,13 +163,6 @@ __device__ __forceinline__ void afbt_pair(const T& t, const float (&v)[2][AfbT<L
         const float2 a = t.h_lo2[2 * u], b = t.h_hi2[2 * u];
         const float2 c = t.h_lo2[2 * u + 1], d = t.h_hi2[2 * u + 1];
         float2* s = acc[sl];
-#ifdef B200W_TMA_SCALAR_COL
-        // experiment: the column pass on scalar FFMA instead of the packed FFMA2
-#define SC_FMA(dst, tap, src, first) do { if (first) { dst.x = tap.x * src.x; dst.y = tap.x * src.y; } else { dst.x = fmaf(tap.x, src.x, dst.x); dst.y = fmaf(tap.x, src.y, dst.y); } } while (0)
-        SC_FMA(s[0], a, rl[0], u == 0); SC_FMA(s[1], b, rl[0], u == 0); SC_FMA(s[2], a, rh[0], u == 0); SC_FMA(s[3], b, rh[0], u == 0);
-        SC_FMA(s[0], c, rl[1], false); SC_FMA(s[1], d, rl[1], false); SC_FMA(s[2], c, rh[1], false); SC_FMA(s[3], d, rh[1], false);
-        continue;
-#endif
         if (u == 0) {   // first contribution: start the accumulators
             s[0] = fmul2(a, rl[0]);   // LL: W-lo, H-lo
             s[1] = fmul2(b, rl[0]);   // LH: W-lo, H-hi
@@ -202,7 +190,6 @@ struct ConstTaps {   // long filters: the taps stay in the constant bank
 
 // where a lane's completed output rows go
 struct AfbtOut {
-    int dbg;
     unsigned ll_s;         // shared address of the low-pass pair in the next level's input image (row of `orow`)
     unsigned ll_pitch_b;   // its row pitch in bytes
     float* low;            // last level: global address of the low-pass pair (row of `orow`)
@@ -220,7 +207,7 @@ __device__ __forceinline__ void afbt_store(const float2* s, AfbtOut& o) {
     if ((unsigned)(o.orow - o.i0) < (unsigned)o.nout) {
         const bool g = (unsigned)(o.orow - o.hlo) < (unsigned)o.hn;
         if (!LAST) {
-            if (!(o.dbg & 32)) sts64t(o.ll_s, s[0]);
+            sts64t(o.ll_s, s[0]);
         } else if (g) {
             B200W_CHK(o.low, o.c1ok ? 8 : 4);
             if (o.low_vec2) {
@@ -230,7 +217,7 @@ __device__ __forceinline__ void afbt_store(const float2* s, AfbtOut& o) {
                 if (o.c1ok) o.low[1] = s[0].y;
             }
         }
-        if (g && !(o.dbg & 16)) {
+        if (g) {
             B200W_CHK(o.hi, o.c1ok ? 8 : 4); B200W_CHK(o.hi + o.band, o.c1ok ? 8 : 4); B200W_CHK(o.hi + 2 * o.band, o.c1ok ? 8 : 4);
             if (o.vec2) {
                 *reinterpret_cast<float2*>(o.hi) = s[1];
@@ -272,16 +259,6 @@ __global__ void __launch_bounds__(AfbT<L, OFF>::NT, 1) afb_tma_kernel(const __gr
     constexpr int off = OFF;
     constexpr int hl = OFF + S;                  // columns left of the image in every staged / stored row
     pdl_trigger();   // the next kernel in the stream may be scheduled as SMs free up (it waits before touching memory)
-    // the stamp is made to depend on a shared-memory load: a warp runs on past a block barrier until it touches
-    // barrier-protected state, so a bare clock read would record when thread 0 ARRIVED at the barrier
-#define TMA_MARK(slot) do { if (p.timeline && tid == 0) { unsigned long long t_; const float z_ = lds32t(sbase + p.zrow_off); \
-        asm volatile("mov.u64 %0, %%clock64;" : "=l"(t_) : "f"(z_) : "memory"); p.timeline[(size_t)blockIdx.x * 64 + (slot)] = t_; } } while (0)
-    if (p.timeline && tid == 0) {
-        unsigned long long gt;
-        asm volatile("mov.u64 %0, %globaltimer;" : "=l"(gt));
-        p.timeline[(size_t)blockIdx.x * 64] = gt;
-    }
-    TMA_MARK(1);
     // every 64-byte line of the parameter block is touched by a different thread first: the constant-cache misses of a
     // freshly scheduled CTA then overlap instead of queueing up behind each other in the set-up code below
     if (tid < (int)((sizeof(AfbTmaParams) - sizeof(int) * kAfbTabMax) / 64)) {
@@ -314,7 +291,7 @@ __global__ void __launch_bounds__(AfbT<L, OFF>::NT, 1) afb_tma_kernel(const __gr
         tma_prefetch_map(&p.map_row);
     }
     __syncthreads();
-    const int early = (p.boxes != 0 && !(p.dbg & 8)) ? 2 : 0;   // stages issued here (0: the service warps issue them all)
+    const int early = p.boxes ? 2 : 0;   // stages issued here (0: the service warps issue them all)
     if (early && warp >= kProducerWarp && lane == 0 && warp - kProducerWarp < nseg0) {
         const int g = warp - kProducerWarp;
         const int i0 = c0_0 + g * l0.R;
@@ -345,7 +322,6 @@ __global__ void __launch_bounds__(AfbT<L, OFF>::NT, 1) afb_tma_kernel(const __gr
     for (int i = tid; i < p.zrow_floats; i += NT) reinterpret_cast<float*>(smem + p.zrow_off)[i] = 0.f;
     pdl_wait();      // everything above used only the parameter block; from here on global memory is touched
     __syncthreads();
-    TMA_MARK(2);
 
     const bool use_ready = mode != B200W_MODE_ZERO && nfix0 > 0;
     const int* const rt0 = tabs + l0.rtab_off;
@@ -358,7 +334,7 @@ __global__ void __launch_bounds__(AfbT<L, OFF>::NT, 1) afb_tma_kernel(const __gr
         // all lanes write the extension columns of a landed stage and release it to the consumers.  The patches run
         // one stage ahead of the consumers, the copies D stages ahead. ----
         const int g = warp - kProducerWarp;
-        if (g < nseg0 && !(p.dbg & 8)) {
+        if (g < nseg0) {
             const int i0 = c0_0 + g * l0.R;
             const int npairs = min(l0.R, c1_0 - i0) + H2 - 1;
             const int nst = (npairs + PS - 1) / PS;
@@ -372,7 +348,6 @@ __global__ void __launch_bounds__(AfbT<L, OFF>::NT, 1) afb_tma_kernel(const __gr
             // row table points at those rows instead.  Otherwise (wrapping modes) such stages are fetched row by row
             // from their source rows.
             const bool boxes = p.boxes != 0;
-#define SVC_MARK(slot, k) do { if (p.timeline && g == 0 && lane == 0 && (k) < 8) p.timeline[(size_t)blockIdx.x * 64 + (slot) + (k)] = (unsigned long long)clock64(); } while (0)
             auto issue = [&](int k) {
                 const int st = k % D;
                 const unsigned full = bar_full + 8u * (g * D + st);
@@ -407,11 +382,8 @@ __global__ void __launch_bounds__(AfbT<L, OFF>::NT, 1) afb_tma_kernel(const __gr
             };
             auto patch = [&](int k) {
                 const int st = k % D;
-                if (k == 0) SVC_MARK(8, 0);
                 mbar_wait(bar_full + 8u * (g * D + st), (unsigned)((k / D) & 1));
-                if (k == 0) SVC_MARK(8, 1);
                 const unsigned base = ring + (unsigned)st * stage_b;
-                if (k == 0) SVC_MARK(8, 2);
 #pragma unroll 2
                 for (int it = lane; it < npatch; it += 32) {
                     B200W_CHK(cf + 2 * it, 8);
@@ -419,26 +391,22 @@ __global__ void __launch_bounds__(AfbT<L, OFF>::NT, 1) afb_tma_kernel(const __gr
                     if (ds.y >= 0) sts32t(base + (unsigned)ds.x, lds32t(base + (unsigned)ds.y));
                 }
                 mbar_arrive(bar_ready + 8u * (g * D + st));
-                if (k == 0) SVC_MARK(8, 3);
             };
             // the first two stages go out first, so that the consumers can start while the rest of the ring is filled
-            SVC_MARK(48, 0);
             if (lane == 0)
-                for (int k = early; k < min(2, nst); ++k) { issue(k); SVC_MARK(48, 1 + k); }
+                for (int k = early; k < min(2, nst); ++k) issue(k);
             __syncwarp();
-            if (use_ready) { patch(0); SVC_MARK(24, 0); }
+            if (use_ready) patch(0);
             if (lane == 0)
                 for (int k = 2; k < min(D, nst); ++k) issue(k);
             __syncwarp();
 #pragma unroll 1
             for (int k = 0; k < nst; ++k) {
-                if (use_ready && k + 1 < nst) { patch(k + 1); SVC_MARK(24, k + 1); }
+                if (use_ready && k + 1 < nst) patch(k + 1);
                 if (k + D < nst) {
                     mbar_wait(bar_empty + 8u * (g * D + k % D), (unsigned)((k / D) & 1));
-                    SVC_MARK(32, k);
                     if (lane == 0) issue(k + D);
                     __syncwarp();
-                    SVC_MARK(40, k);
                 }
             }
         }
@@ -461,7 +429,6 @@ __global__ void __launch_bounds__(AfbT<L, OFF>::NT, 1) afb_tma_kernel(const __gr
             const unsigned bar_rel = bar_empty + 8u * (g * D);
             const AfbTmaLevel& l1 = p.lv[1];
             AfbtOut o;
-            o.dbg = p.dbg;
             o.orow = i0 - (H2 - 1);
             o.i0 = i0; o.nout = nout;
             o.hlo = max(i0, l0.h0[part]);
@@ -480,11 +447,9 @@ __global__ void __launch_bounds__(AfbT<L, OFF>::NT, 1) afb_tma_kernel(const __gr
             unsigned ph = 0;
 #pragma unroll 1
             for (int k = 0; k < nst; ++k) {
-                if (!(p.dbg & 1)) mbar_wait(bar_wait + 8u * st, ph);
-                if (p.timeline && tid == 0 && k < 8) p.timeline[(size_t)blockIdx.x * 64 + 16 + k] = (unsigned long long)clock64();
-                if (!(p.dbg & 2))
+                mbar_wait(bar_wait + 8u * st, ph);
                 if (C::kPrefetch) {   // the windows of row pair u + PFD are requested before row pair u is filtered
-                    constexpr int PFD = B200W_EXP_PFD < PS ? B200W_EXP_PFD : PS - 1;
+                    constexpr int PFD = 1;
                     float v[PFD + 1][2][NE];
 #pragma unroll
                     for (int u = 0; u < PFD; ++u) {
@@ -514,7 +479,7 @@ __global__ void __launch_bounds__(AfbT<L, OFF>::NT, 1) afb_tma_kernel(const __gr
                     afbt_store<L, OFF, false>(acc[kRotate ? 0 : (u + 1) % H2], o);
                     afbt_rotate<L, OFF>(acc);
                 }
-                if (!(p.dbg & 8)) mbar_arrive(bar_rel + 8u * st);
+                mbar_arrive(bar_rel + 8u * st);
                 if (++st == D) { st = 0; ph ^= 1u; }
             }
         }
@@ -526,7 +491,6 @@ __global__ void __launch_bounds__(AfbT<L, OFF>::NT, 1) afb_tma_kernel(const __gr
         const AfbTmaLevel& lv = p.lv[j];
         const bool last = j + 1 == p.J;
         __syncthreads();   // the previous level's low-pass rows are complete
-        TMA_MARK(1 + 2 * j);
         {   // extension columns of the input image, all rows of the part
             const int* const cf = tabs + lv.cfix_off;
             const int n = lv.in_pitch - lv.Wreal;
@@ -541,7 +505,6 @@ __global__ void __launch_bounds__(AfbT<L, OFF>::NT, 1) afb_tma_kernel(const __gr
             }
         }
         __syncthreads();
-        TMA_MARK(2 + 2 * j);
         if (warp >= kProducerWarp) continue;
         const int ct = tid;
         const int c0 = lv.c0[part], c1 = lv.c1[part];
@@ -554,7 +517,6 @@ __global__ void __launch_bounds__(AfbT<L, OFF>::NT, 1) afb_tma_kernel(const __gr
         const int* const rt = tabs + lv.rtab_off + 2 * (i0 - c0);
         const unsigned lane_b = sbase + (unsigned)cp * 16u;   // + table entry = the window of this lane in that row
         AfbtOut o;
-        o.dbg = p.dbg;
         o.orow = i0 - (H2 - 1);
         o.i0 = i0; o.nout = nout;
         o.hlo = max(i0, lv.h0[part]);
@@ -591,27 +553,11 @@ __global__ void __launch_bounds__(AfbT<L, OFF>::NT, 1) afb_tma_kernel(const __gr
             }
         }
     }
-    if (p.timeline) {   // debug only: the end of the last level
-        __syncthreads();
-        TMA_MARK(1 + 2 * p.J);
-    }
-#undef TMA_MARK
 }
 
 // ---- host: plan + launch ------------------------------------------------------------------------------------------
-static int tma_env() {
-    static int v = -1;
-    if (v < 0) {
-        const char* e = getenv("B200W_TMA");
-        v = (e && e[0] >= '0' && e[0] <= '2') ? e[0] - '0' : 1;
-    }
-    return v;
-}
-
-constexpr size_t kTmaSmemMax = 227 * 1024;
-
 template <int L, int OFF>
-static bool afb_tma_plan_t(const AfbParams& p, int sms, bool force, AfbTmaParams& tp) {
+static bool afb_tma_plan_t(const AfbParams& p, int sms, bool force, int G_req, int D_req, bool noboxes, AfbTmaParams& tp) {
     using C = AfbT<L, OFF>;
     constexpr int NE = C::NE, SR = C::SR, NTC = C::NTC;
     const int J = p.J;
@@ -632,14 +578,9 @@ static bool afb_tma_plan_t(const AfbParams& p, int sms, bool force, AfbTmaParams
     int parts = std::min(kMaxParts, std::max(1, sms / p.planes));
     if (wraps) parts = 1;   // a part would need rows from the far end of the image
     parts = std::min(parts, p.lv[J - 1].Ho);
-    if (!force) {
-        const long long ctas = (long long)p.planes * parts, waves = (ctas + sms - 1) / sms;
-        if (ctas * 4 < waves * sms * 3 && waves > 1) return false;   // a short last wave wastes too much of the device
-    }
+    if (!force && short_last_wave((long long)p.planes * parts, sms)) return false;
     AfbTmaParams& t = tp;
     t.J = J; t.planes = p.planes; t.parts = parts; t.mode = p.mode;
-    t.timeline = nullptr;
-    t.dbg = getenv("B200W_TMA_DBG") ? atoi(getenv("B200W_TMA_DBG")) : 0;
     for (int i = 0; i < kMaxTemplTaps; ++i) {
         t.t.w_lo[i] = p.t.w_lo[i]; t.t.w_hi[i] = p.t.w_hi[i];
         t.t.h_lo2[i] = p.t.h_lo2[i]; t.t.h_hi2[i] = p.t.h_hi2[i];
@@ -701,7 +642,7 @@ static bool afb_tma_plan_t(const AfbParams& p, int sms, bool force, AfbTmaParams
             const long long cost = (long long)ceil_div(warps, 4) * (ceil_div(maxrows[0], g) + C::H2 - 1);
             if (best < 0 || cost < best) { best = cost; G = g; }
         }
-        if (const char* e = getenv("B200W_TMA_G")) G = std::max(1, std::min(gmax, atoi(e)));
+        if (G_req > 0) G = std::min(gmax, G_req);
         lv.R = ceil_div(maxrows[0], G);
         lv.nseg = ceil_div(maxrows[0], lv.R);
     }
@@ -780,10 +721,10 @@ static bool afb_tma_plan_t(const AfbParams& p, int sms, bool force, AfbTmaParams
         later += ((size_t)t.lv[j].in_rows * t.lv[j].in_pitch * 4 + 127) & ~(size_t)127;
     }
     const size_t stage_b = (size_t)t.nstrips * SR * t.BW * 4;
-    if (o + std::max(later, 2 * stage_b * t.lv[0].nseg) > kTmaSmemMax) return false;
-    int D = (int)((kTmaSmemMax - o) / (stage_b * t.lv[0].nseg));
+    if (o + std::max(later, 2 * stage_b * t.lv[0].nseg) > kMaxDynSmem) return false;
+    int D = (int)((kMaxDynSmem - o) / (stage_b * t.lv[0].nseg));
     D = std::min(D, 8);
-    if (const char* e = getenv("B200W_TMA_D")) D = std::max(2, std::min(D, atoi(e)));
+    if (D_req > 0) D = std::max(2, std::min(D, D_req));
     if (D < 2) return false;
     t.D = D;
     t.smem_bytes = (int)(o + std::max(later, (size_t)D * stage_b * t.lv[0].nseg));
@@ -803,7 +744,7 @@ static bool afb_tma_plan_t(const AfbParams& p, int sms, bool force, AfbTmaParams
         // extension row finds its image row in a ring slot that is still valid when it is read: the same stage, or an
         // earlier stage of the stream that is never refilled (one of the last D stages).
         bool boxes = p.mode == B200W_MODE_ZERO || p.mode == B200W_MODE_SYMMETRIC || p.mode == B200W_MODE_REFLECT;
-        if (getenv("B200W_TMA_NOBOXES") && p.mode != B200W_MODE_ZERO) boxes = false;
+        if (noboxes && p.mode != B200W_MODE_ZERO) boxes = false;
         for (int pass = 0; pass < 2; ++pass) {   // pass 0: decide `boxes`; pass 1: fill the tables
         for (int q = 0; q < parts; ++q) {
             int* const tb = t.tab + q * t.tab_ints;
@@ -902,26 +843,7 @@ static bool afb_tma_plan_t(const AfbParams& p, int sms, bool force, AfbTmaParams
 template <int L, int OFF>
 static int launch_afb_tma_t(const AfbTmaParams& tp, cudaStream_t st) {
     using C = AfbT<L, OFF>;
-    static bool attr_set[64] = {false};
-    int dev = 0;
-    cudaGetDevice(&dev);
-    if (dev < 0 || dev >= 64 || !attr_set[dev]) {
-        const cudaError_t e = cudaFuncSetAttribute(afb_tma_kernel<L, OFF>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                                   (int)kTmaSmemMax);
-        if (e != cudaSuccess) return set_last_cuda_error(e);
-        if (dev >= 0 && dev < 64) attr_set[dev] = true;
-    }
-    // debug: B200W_TMA_TIMELINE=file dumps 32 clock stamps per CTA of every launch (synchronises: not for timing runs)
-    static unsigned long long* tl = nullptr;
-    const char* tl_path = getenv("B200W_TMA_TIMELINE");
-    const size_t ncta = (size_t)tp.planes * tp.parts;
-    AfbTmaParams tpl = tp;
-    tpl.timeline = nullptr;
-    if (tl_path && ncta <= 65536) {
-        if (!tl) cudaMalloc(&tl, sizeof(unsigned long long) * 64 * 65536);
-        cudaMemsetAsync(tl, 0, sizeof(unsigned long long) * 64 * ncta, st);
-        tpl.timeline = tl;
-    }
+    if (const cudaError_t e = allow_max_dyn_smem<afb_tma_kernel<L, OFF>>()) return set_last_cuda_error(e);
 #ifdef B200W_BOUNDS
     {
         BoundsList b;
@@ -933,40 +855,19 @@ static int launch_afb_tma_t(const AfbTmaParams& tp, cudaStream_t st) {
         bounds_set(b, st);
     }
 #endif
-    const cudaError_t le = launch_pdl(afb_tma_kernel<L, OFF>, (unsigned)ncta, C::NT, (size_t)tp.smem_bytes, st, tpl);
+    const cudaError_t le = launch_pdl(afb_tma_kernel<L, OFF>, (unsigned)(tp.planes * tp.parts), C::NT, (size_t)tp.smem_bytes,
+                                      st, tp);
     note_launch("afb_tma_kernel");
     const cudaError_t e = le != cudaSuccess ? le : cudaGetLastError();
-    if (tpl.timeline && e == cudaSuccess) {
-        cudaStreamSynchronize(st);
-        unsigned long long* host = (unsigned long long*)malloc(sizeof(unsigned long long) * 64 * ncta);
-        cudaMemcpy(host, tl, sizeof(unsigned long long) * 64 * ncta, cudaMemcpyDeviceToHost);
-        FILE* f = fopen(tl_path, "wb");
-        if (f) { fwrite(host, sizeof(unsigned long long) * 64, ncta, f); fclose(f); }
-        free(host);
-    }
     return e == cudaSuccess ? B200W_OK : set_last_cuda_error(e);
 }
 
-#define B200W_TMA_FOR_EACH_L(X) \
-    switch (L) {                 \
-        case 2: X(2);            \
-        case 4: X(4);            \
-        case 6: X(6);            \
-        case 8: X(8);            \
-        case 10: X(10);          \
-        case 12: X(12);          \
-        case 14: X(14);          \
-        case 16: X(16);          \
-        default: break;          \
-    }
-
-bool afb_tma_plan(const AfbParams& p, int L, int sms, bool force, AfbTmaParams& tp) {
-    if (tma_env() == 0 || !tma_encode_fn()) return false;
-    if (tma_env() == 2) force = true;
+bool afb_tma_plan(const AfbParams& p, int L, int sms, bool force, int G, int D, bool noboxes, AfbTmaParams& tp) {
+    if (!tma_encode_fn()) return false;
     const bool per = p.mode == B200W_MODE_PERIODIZATION;
-#define X(LL) return per ? afb_tma_plan_t<LL, afbt_off(LL, true)>(p, sms, force, tp) \
-                         : afb_tma_plan_t<LL, afbt_off(LL, false)>(p, sms, force, tp)
-    B200W_TMA_FOR_EACH_L(X)
+#define X(LL) return per ? afb_tma_plan_t<LL, afbt_off(LL, true)>(p, sms, force, G, D, noboxes, tp) \
+                         : afb_tma_plan_t<LL, afbt_off(LL, false)>(p, sms, force, G, D, noboxes, tp)
+    B200W_FOR_EACH_L(X)
 #undef X
     return false;
 }
@@ -975,7 +876,7 @@ int launch_afb_tma(const AfbTmaParams& tp, int L, cudaStream_t st) {
     const bool per = tp.mode == B200W_MODE_PERIODIZATION;
 #define X(LL) return per ? launch_afb_tma_t<LL, afbt_off(LL, true)>(tp, st) \
                          : launch_afb_tma_t<LL, afbt_off(LL, false)>(tp, st)
-    B200W_TMA_FOR_EACH_L(X)
+    B200W_FOR_EACH_L(X)
 #undef X
     return B200W_ERR_BAD_TAPS;
 }

@@ -23,8 +23,6 @@
 // of the four sub-bands in registers (taps in registers), H synthesis scattered into a ring of L/2 pending output row
 // pairs (packed FFMA2), completed pairs written with 128-bit stores.
 #include <algorithm>
-#include <cstdio>
-#include <cstdlib>
 #include <type_traits>
 #include "dwt_tma.cuh"
 
@@ -220,13 +218,6 @@ __global__ void __launch_bounds__(SfbT<L>::NT, 1) sfb_tma_kernel(const __grid_co
     const int part = blockIdx.x - plane * p.parts;
     const int J = p.J;
     pdl_trigger();
-#define SFB_MARK(slot) do { if (p.timeline && tid == 0) p.timeline[(size_t)blockIdx.x * 64 + (slot)] = (unsigned long long)clock64(); } while (0)
-    if (p.timeline && tid == 0) {
-        unsigned long long gt;
-        asm volatile("mov.u64 %0, %globaltimer;" : "=l"(gt));
-        p.timeline[(size_t)blockIdx.x * 64] = gt;
-    }
-    SFB_MARK(1);
     // every 64-byte line of the parameter block is touched by a different thread first (overlapping constant-cache misses)
     if (tid < (int)(sizeof(SfbTmaParams) / 64)) {
         const int v = reinterpret_cast<const int*>(&p)[tid * 16];
@@ -247,7 +238,6 @@ __global__ void __launch_bounds__(SfbT<L>::NT, 1) sfb_tma_kernel(const __grid_co
     if (tid == 0) *reinterpret_cast<float*>(smem + p.bar_off + 8 * (J - 1 + 2 * G * D)) = 0.f;   // the zero the taps are made opaque with
     pdl_wait();      // everything above used only the parameter block; from here on global memory is touched
     __syncthreads();
-    SFB_MARK(2);
 
     // ---- resident positions: one bulk copy per band (and one for yl); position c is issued by warp c ----
     if (warp < J - 1) {
@@ -285,7 +275,7 @@ __global__ void __launch_bounds__(SfbT<L>::NT, 1) sfb_tma_kernel(const __grid_co
         // ---- service warp of ring stream g (last position): lanes 0..2 issue the three band copies of a stage into a free
         // ring slot ----
         const int g = warp - kServiceWarp;
-        if (g < nsegL && !(p.dbg & 8)) {
+        if (g < nsegL) {
             const int m0 = lm_lo + g * pl.Rp;
             const int nm = min(pl.Rp, lm_hi - m0);
             const int kr0 = m0 - (H2 - 1);
@@ -330,7 +320,6 @@ __global__ void __launch_bounds__(SfbT<L>::NT, 1) sfb_tma_kernel(const __grid_co
                                              // waited for between positions
         // the previous position's output image is complete: barrier among the consumer warps only
         if (c > 0) asm volatile("bar.sync 1, %0;" ::"r"(NTC) : "memory");
-        SFB_MARK(2 + c + 1);
         const int n0 = ps.n0[part], n1 = ps.n1[part];
         const int m_lo = (n0 + off) >> 1, m_hi = ((n1 - 1 + off) >> 1) + 1;
         const int ct = tid;
@@ -423,7 +412,7 @@ __global__ void __launch_bounds__(SfbT<L>::NT, 1) sfb_tma_kernel(const __grid_co
                         if (qb + u < nrows_u) {
                             const bool live = qb + u < nrows;      // this lane's stream still has rows
                             if (fresh) {
-                                if (live && !(p.dbg & 1)) mbar_wait(bw + 8u * st, ph);
+                                if (live) mbar_wait(bw + 8u * st, ph);
                                 fresh = false;
 #pragma unroll
                                 for (int b = 0; b < 3; ++b)
@@ -435,7 +424,7 @@ __global__ void __launch_bounds__(SfbT<L>::NT, 1) sfb_tma_kernel(const __grid_co
                             a_low += low_pitch_b;
                             aH[0] += w_b; aH[1] += w_b; aH[2] += w_b;
                             if (++jr == SR || qb + u + 1 == nrows) {   // done with this stage
-                                if (live && !(p.dbg & 8)) mbar_arrive(be + 8u * st);
+                                if (live) mbar_arrive(be + 8u * st);
                                 jr = 0;
                                 r0 += SR;
                                 fresh = true;
@@ -449,28 +438,13 @@ __global__ void __launch_bounds__(SfbT<L>::NT, 1) sfb_tma_kernel(const __grid_co
             else run(std::integral_constant<int, 1>{});
         }
     }
-    if (p.timeline) {   // debug only: the end of the last position
-        __syncthreads();
-        SFB_MARK(3 + J);
-    }
-#undef SFB_MARK
 }
 
 // ---- host: plan + launch ------------------------------------------------------------------------------------------
-static int sfb_tma_env() {
-    static int v = -1;
-    if (v < 0) {
-        const char* e = getenv("B200W_TMA");
-        v = (e && e[0] >= '0' && e[0] <= '2') ? e[0] - '0' : 1;
-    }
-    return v;
-}
-
-constexpr size_t kSfbTmaSmemMax = 227 * 1024;
 static size_t up128(size_t n) { return (n + 127) & ~(size_t)127; }
 
 template <int L>
-static bool sfb_tma_plan_t(const SfbParams& p, int sms, bool force, SfbTmaParams& t) {
+static bool sfb_tma_plan_t(const SfbParams& p, int sms, bool force, int G_req, int D_req, SfbTmaParams& t) {
     using C = SfbT<L>;
     constexpr int H2 = C::H2, NTC = C::NTC, NCF = C::NCF;
     constexpr int off = L - 2;
@@ -491,13 +465,8 @@ static bool sfb_tma_plan_t(const SfbParams& p, int sms, bool force, SfbTmaParams
     if (!p.lv[J - 1].y) return false;
     int parts = std::min(kMaxParts, std::max(1, sms / p.planes));
     parts = std::min(parts, std::max(1, p.lv[J - 1].out_h / 2));
-    if (!force) {
-        const long long ctas = (long long)p.planes * parts, waves = (ctas + sms - 1) / sms;
-        if (ctas * 4 < waves * sms * 3 && waves > 1) return false;   // a short last wave wastes too much of the device
-    }
+    if (!force && short_last_wave((long long)p.planes * parts, sms)) return false;
     t.J = J; t.planes = p.planes; t.parts = parts;
-    t.timeline = nullptr;
-    t.dbg = getenv("B200W_TMA_DBG") ? atoi(getenv("B200W_TMA_DBG")) : 0;
     for (int i = 0; i < kMaxTemplTaps; ++i) {
         t.t.w_lo[i] = p.t.w_lo[i]; t.t.w_hi[i] = p.t.w_hi[i];
         t.t.h_lo2[i] = p.t.h_lo2[i]; t.t.h_hi2[i] = p.t.h_hi2[i];
@@ -543,7 +512,7 @@ static bool sfb_tma_plan_t(const SfbParams& p, int sms, bool force, SfbTmaParams
         int G = std::min(std::max(1, NTC / ps.nq), npairs);
         if (c == J - 1) {
             G = std::min(G, C::MAXG);
-            if (const char* e = getenv("B200W_TMA_G")) G = std::max(1, std::min(G, atoi(e)));
+            if (G_req > 0) G = std::min(G, G_req);
         }
         ps.Rp = ceil_div(npairs, G);
         ps.nseg = ceil_div(npairs, ps.Rp);
@@ -591,13 +560,13 @@ static bool sfb_tma_plan_t(const SfbParams& p, int sms, bool force, SfbTmaParams
     int SRb = 0, Db = 0;
     for (int SR : {8, 6, 4, 2}) {
         const size_t stage = 3 * chunk_bytes(SR, t.pos[J - 1].w);
-        if (o + 64 + 2 * stage * G > kSfbTmaSmemMax) continue;
-        int D = (int)((kSfbTmaSmemMax - o - 64) / (stage * G));
+        if (o + 64 + 2 * stage * G > kMaxDynSmem) continue;
+        int D = (int)((kMaxDynSmem - o - 64) / (stage * G));
         D = std::min(D, 8);
         if (SRb == 0 || (D - 1) * SR > (Db - 1) * SRb) { SRb = SR; Db = D; }
     }
     if (SRb == 0) return false;
-    if (const char* e = getenv("B200W_TMA_D")) Db = std::max(2, std::min(Db, atoi(e)));
+    if (D_req > 0) Db = std::max(2, std::min(Db, D_req));
     t.SR = SRb;
     t.D = Db;
     t.ring_band = (int)chunk_bytes(SRb, t.pos[J - 1].w);
@@ -609,26 +578,7 @@ static bool sfb_tma_plan_t(const SfbParams& p, int sms, bool force, SfbTmaParams
 template <int L>
 static int launch_sfb_tma_t(const SfbTmaParams& tp, cudaStream_t st) {
     using C = SfbT<L>;
-    static bool attr_set[64] = {false};
-    int dev = 0;
-    cudaGetDevice(&dev);
-    if (dev < 0 || dev >= 64 || !attr_set[dev]) {
-        const cudaError_t e = cudaFuncSetAttribute(sfb_tma_kernel<L>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                                   (int)kSfbTmaSmemMax);
-        if (e != cudaSuccess) return set_last_cuda_error(e);
-        if (dev >= 0 && dev < 64) attr_set[dev] = true;
-    }
-    // debug: B200W_TMA_TIMELINE_SFB=file dumps 64 clock stamps per CTA of every launch (synchronises: not for timing runs)
-    static unsigned long long* tl = nullptr;
-    const char* tl_path = getenv("B200W_TMA_TIMELINE_SFB");
-    const size_t ncta = (size_t)tp.planes * tp.parts;
-    SfbTmaParams tpl = tp;
-    tpl.timeline = nullptr;
-    if (tl_path && ncta <= 65536) {
-        if (!tl) cudaMalloc(&tl, sizeof(unsigned long long) * 64 * 65536);
-        cudaMemsetAsync(tl, 0, sizeof(unsigned long long) * 64 * ncta, st);
-        tpl.timeline = tl;
-    }
+    if (const cudaError_t e = allow_max_dyn_smem<sfb_tma_kernel<L>>()) return set_last_cuda_error(e);
 #ifdef B200W_BOUNDS
     {
         BoundsList b;
@@ -641,45 +591,23 @@ static int launch_sfb_tma_t(const SfbTmaParams& tp, cudaStream_t st) {
         bounds_set(b, st);
     }
 #endif
-    const cudaError_t le = launch_pdl(sfb_tma_kernel<L>, (unsigned)ncta, C::NT, (size_t)tp.smem_bytes, st, tpl);
+    const cudaError_t le = launch_pdl(sfb_tma_kernel<L>, (unsigned)(tp.planes * tp.parts), C::NT, (size_t)tp.smem_bytes, st, tp);
     note_launch("sfb_tma_kernel");
     const cudaError_t e = le != cudaSuccess ? le : cudaGetLastError();
-    if (tpl.timeline && e == cudaSuccess) {
-        cudaStreamSynchronize(st);
-        unsigned long long* host = (unsigned long long*)malloc(sizeof(unsigned long long) * 64 * ncta);
-        cudaMemcpy(host, tl, sizeof(unsigned long long) * 64 * ncta, cudaMemcpyDeviceToHost);
-        FILE* f = fopen(tl_path, "wb");
-        if (f) { fwrite(host, sizeof(unsigned long long) * 64, ncta, f); fclose(f); }
-        free(host);
-    }
     return e == cudaSuccess ? B200W_OK : set_last_cuda_error(e);
 }
 
-#define B200W_TMA_SFB_FOR_EACH_L(X) \
-    switch (L) {                     \
-        case 2: X(2);                \
-        case 4: X(4);                \
-        case 6: X(6);                \
-        case 8: X(8);                \
-        case 10: X(10);              \
-        case 12: X(12);              \
-        case 14: X(14);              \
-        case 16: X(16);              \
-        default: break;              \
-    }
-
-bool sfb_tma_plan(const SfbParams& p, int L, int sms, bool force, SfbTmaParams& tp) {
-    if (sfb_tma_env() == 0 || !tma_encode_fn()) return false;
-    if (sfb_tma_env() == 2) force = true;
-#define X(LL) return sfb_tma_plan_t<LL>(p, sms, force, tp)
-    B200W_TMA_SFB_FOR_EACH_L(X)
+bool sfb_tma_plan(const SfbParams& p, int L, int sms, bool force, int G, int D, SfbTmaParams& tp) {
+    if (!tma_encode_fn()) return false;
+#define X(LL) return sfb_tma_plan_t<LL>(p, sms, force, G, D, tp)
+    B200W_FOR_EACH_L(X)
 #undef X
     return false;
 }
 
 int launch_sfb_tma(const SfbTmaParams& tp, int L, cudaStream_t st) {
 #define X(LL) return launch_sfb_tma_t<LL>(tp, st)
-    B200W_TMA_SFB_FOR_EACH_L(X)
+    B200W_FOR_EACH_L(X)
 #undef X
     return B200W_ERR_BAD_TAPS;
 }
