@@ -1,18 +1,24 @@
-// 2-D DWT analysis / synthesis filter banks for sm_100a: one persistent kernel per multi-level transform.
+// 2-D DWT analysis / synthesis filter banks for sm_100a: kernel selection, the C entry points, the analysis tile
+// chain and the direct kernels.
 //
 // What it replaces.  Per level the reference runs pad-gather + 2x F.conv2d + reshape + 2x .contiguous()
 // (AFB2D, pw/dwt/lowlevel.py:336-347) resp. 6x F.conv_transpose2d + 3 adds (SFB2D, :671-680), and
 // DWTForward / DWTInverse loop over the J levels in Python (pw/dwt/transform2d.py:66-74, 134-148).
-// Here a J-level transform is ONE launch: a persistent grid walks an ordered list of tiles (all tiles of the
-// first level, then the next level, ...); a tile of level j+1 of image plane p starts as soon as every tile of
-// level j of that plane has been written (per-plane completion counters, release/acquire), so levels overlap,
-// there are no launch gaps between the small coarse levels, and the LL intermediates are consumed out of L2.
+// Here a J-level transform of up to 16 taps is ONE launch: an owner kernel for chains of small planes
+// (dwt_tma_*.cu, dwt_stream_*.cu), otherwise the ticketed stream chain (dwt_stream_*.cu).
 //
-// Per tile, analysis: the input patch (+halo) is staged in shared memory with cp.async -- the padding mode is
-// an index map applied to the source address -- double buffered so the next tile's fetch overlaps this tile's
-// arithmetic; row (W) pass with stride-2 decimation into shared memory; column (H) pass; LL goes to `low`,
-// LH/HL/HH straight into `highs[:, :, 0..2]`.  Synthesis is the polyphase mirror image (upsample + filter +
-// accumulate of all four sub-bands fused).
+// Analysis tile chain (inputs whose rows are not 16-byte aligned, and B200W_FORCE_TILED): a persistent grid walks an
+// ordered list of tiles (all tiles of the first level, then the next level, ...); a tile of level j+1 of image plane
+// p starts as soon as every tile of level j of that plane has been written (per-plane completion counters,
+// release/acquire), so levels overlap, there are no launch gaps between the small coarse levels, and the LL
+// intermediates are consumed out of L2.
+//
+// Per tile: the input patch (+halo) is staged in shared memory with cp.async -- the padding mode is an index map
+// applied to the source address -- double buffered so the next tile's fetch overlaps this tile's arithmetic; row (W)
+// pass with stride-2 decimation into shared memory; column (H) pass; LL goes to `low`, LH/HL/HH straight into
+// `highs[:, :, 0..2]`.
+//
+// Direct kernels: one thread per output of one level, any tap count, in fp32 and in fp64.
 //
 // Closed forms (SURVEY.md 8a, validated against the reference to 1e-15 by oracle/dwt_oracle.py):
 //   analysis   y_c[k] = sum_j w_c[j] * x_ext[2k + j - off],  off = p//2 with p = 2(M-1) - N + L,
@@ -24,6 +30,7 @@
 // These are HBM-bound stencils (8 B of traffic per pixel for 2L FMAs): the code keeps the instruction count
 // per pixel low -- 128-bit shared loads feeding register-blocked FMAs whose coefficients come from the
 // constant bank, 64-bit coalesced global stores, staging loops whose addresses advance by constants.
+#include <type_traits>
 #include "dwt_levels.cuh"
 #include "dwt_tma.cuh"
 
@@ -45,8 +52,7 @@ struct TileRef {
     int level, plane, th, tw;
 };
 
-template <class P>
-__device__ __forceinline__ TileRef decode_tile(const P& p, long long tile) {
+__device__ __forceinline__ TileRef decode_tile(const AfbParams& p, long long tile) {
     int level = 0;
     for (int j = 1; j < p.J; ++j)
         if (tile >= p.lv[j].tile_base) level = j;
@@ -63,8 +69,7 @@ __device__ __forceinline__ TileRef decode_tile(const P& p, long long tile) {
 }
 
 // has every tile of the previous level of this plane been written?
-template <class P>
-__device__ __forceinline__ bool tile_ready(const P& p, const TileRef& t) {
+__device__ __forceinline__ bool tile_ready(const AfbParams& p, const TileRef& t) {
     if (t.level == 0) return true;
     const unsigned need = (unsigned)(p.lv[t.level - 1].tiles_w * p.lv[t.level - 1].tiles_h);
     return ld_acquire_u32(p.done + (size_t)(t.level - 1) * p.planes + t.plane) >= need;
@@ -336,302 +341,115 @@ struct AfbOp {
     }
 };
 
-// analysis, direct (any tap counts up to kMaxTaps, odd or mixed lengths): one thread per output position of
-// ONE level, no staging.  Fallback and on-device cross-check of the tiled kernel.
+// ------------------------------------------------------------------------------------------------
+// direct kernels: one thread per output position of ONE level, no staging, any tap count up to kMaxTaps (odd or
+// mixed lengths).  In fp32 they serve the tap counts the templated kernels are not instantiated for (and
+// B200W_FORCE_DIRECT); in fp64 they are the whole path -- precision, not speed, is the point there.
+// ------------------------------------------------------------------------------------------------
+struct Taps64 {
+    double w_lo[kMaxTaps], w_hi[kMaxTaps], h_lo[kMaxTaps], h_hi[kMaxTaps];
+};
+template <class T>
+using DirectTaps = std::conditional_t<std::is_same<T, float>::value, Taps, Taps64>;
+
+// The fp32 chain runners fill these from AfbLevel / SfbLevel, the fp64 entry points directly.
+template <class T>
 struct AfbDirectParams {
-    AfbLevel lv;
+    const T* x;
+    T* low;
+    T* highs;                  // dense (planes,3,Ho,Wo)
+    long long x_ps, x_rs, low_ps, low_rs;
+    int H, W, Hreal, Wreal;    // as in AfbLevel
+    int Ho, Wo, offH, offW;
+    int st_low, st_hi;         // store epilogue of AfbLevel
+    T hi_scale, hi_shift;
     int planes, mode, Lw, Lh;
-    Taps t;
+    DirectTaps<T> t;
 };
 
-__global__ void __launch_bounds__(kThreads) afb2d_direct_kernel(const __grid_constant__ AfbDirectParams p) {
-    const AfbLevel& lv = p.lv;
-    const size_t band = (size_t)lv.Ho * lv.Wo;
+template <class T>
+__global__ void __launch_bounds__(kThreads) afb2d_direct_kernel(const __grid_constant__ AfbDirectParams<T> p) {
+    const size_t band = (size_t)p.Ho * p.Wo;
     const size_t total = band * p.planes;
     for (size_t idx = (size_t)blockIdx.x * blockDim.x + threadIdx.x; idx < total;
          idx += (size_t)gridDim.x * blockDim.x) {
-        const int k = (int)(idx % lv.Wo);
-        const int i = (int)((idx / lv.Wo) % lv.Ho);
+        const int k = (int)(idx % p.Wo);
+        const int i = (int)((idx / p.Wo) % p.Ho);
         const int plane = (int)(idx / band);
-        const float* __restrict__ xp = lv.x + (long long)plane * lv.x_ps;
-        float ll = 0.f, lh = 0.f, hl = 0.f, hh = 0.f;
+        const T* __restrict__ xp = p.x + (long long)plane * p.x_ps;
+        T ll = 0, lh = 0, hl = 0, hh = 0;
         for (int jh = 0; jh < p.Lh; ++jh) {
-            const int sr = ext_index(2 * i + jh - lv.offH, lv.H, p.mode);
-            if (sr < 0 || sr >= lv.Hreal) continue;
-            float lo = 0.f, hi = 0.f;
+            const int sr = ext_index(2 * i + jh - p.offH, p.H, p.mode);
+            if (sr < 0 || sr >= p.Hreal) continue;
+            T lo = 0, hi = 0;
             for (int jw = 0; jw < p.Lw; ++jw) {
-                const int sc = ext_index(2 * k + jw - lv.offW, lv.W, p.mode);
-                if (sc < 0 || sc >= lv.Wreal) continue;
-                const float v = __ldg(xp + (long long)sr * lv.x_rs + sc);
-                lo = fmaf(p.t.w_lo[jw], v, lo);
-                hi = fmaf(p.t.w_hi[jw], v, hi);
+                const int sc = ext_index(2 * k + jw - p.offW, p.W, p.mode);
+                if (sc < 0 || sc >= p.Wreal) continue;
+                const T v = __ldg(xp + (long long)sr * p.x_rs + sc);
+                lo = fma(p.t.w_lo[jw], v, lo);
+                hi = fma(p.t.w_hi[jw], v, hi);
             }
-            ll = fmaf(p.t.h_lo[jh], lo, ll);
-            lh = fmaf(p.t.h_hi[jh], lo, lh);
-            hl = fmaf(p.t.h_lo[jh], hi, hl);
-            hh = fmaf(p.t.h_hi[jh], hi, hh);
+            ll = fma(p.t.h_lo[jh], lo, ll);
+            lh = fma(p.t.h_hi[jh], lo, lh);
+            hl = fma(p.t.h_lo[jh], hi, hl);
+            hh = fma(p.t.h_hi[jh], hi, hh);
         }
-        const size_t o = (size_t)i * lv.Wo + k;
-        if (lv.st_low) lv.low[(long long)plane * lv.low_ps + (long long)i * lv.low_rs + k] = ll;
-        if (lv.st_hi) {
-            float* hip = lv.highs + (size_t)plane * 3 * band + o;
-            hip[0] = fmaf(lh, lv.hi_scale, lv.hi_shift);
-            hip[band] = fmaf(hl, lv.hi_scale, lv.hi_shift);
-            hip[2 * band] = fmaf(hh, lv.hi_scale, lv.hi_shift);
+        const size_t o = (size_t)i * p.Wo + k;
+        if (p.st_low) p.low[(long long)plane * p.low_ps + (long long)i * p.low_rs + k] = ll;
+        if (p.st_hi) {
+            T* hip = p.highs + (size_t)plane * 3 * band + o;
+            hip[0] = fma(lh, p.hi_scale, p.hi_shift);
+            hip[band] = fma(hl, p.hi_scale, p.hi_shift);
+            hip[2 * band] = fma(hh, p.hi_scale, p.hi_shift);
         }
     }
 }
 
-// ------------------------------------------------------------------------------------------------
-// synthesis tile.  Works in "A-space": a = n + off, so that the polyphase split (which taps an output uses)
-// depends only on the parity of the tile-local coordinate.  Output tile TH x TW.  W synthesis first (on the KH
-// coefficient rows), then H synthesis; by separability this equals the reference's H-then-W order
-// (pw/dwt/lowlevel.py:677-679) up to fp32 rounding.
-// ------------------------------------------------------------------------------------------------
-// Stage the 4 sub-band patches [4][KH][KWP] asynchronously; thread = one vector column, walking down the rows.
-// Coefficients outside the arrays are zero (or wrap for periodization); missing `highs` = zeros.
-template <int V, int KH, int KWP, int NT>
-__device__ __forceinline__ void stage_synthesis(unsigned sub_s, const float* __restrict__ lowp, long long low_rs,
-                                                const float* __restrict__ hip, size_t band, int kH0, int kW0, int h,
-                                                int w, bool periodic, int nrows, int ncols, int tid) {
-    constexpr int NVC = KWP / V;
-    constexpr int NRG = NT / NVC;
-    constexpr unsigned PBB = KH * KWP * 4;  // bytes of one band's patch
-    if (tid >= NVC * NRG) return;
-    const int cv = tid % NVC;
-    const int rg = tid / NVC;
-    if (V * cv >= ncols) return;
-    const int kc0 = kW0 + V * cv;
-    const bool col_in = kc0 >= 0 && kc0 + V <= w;
-    unsigned dst = sub_s + (unsigned)((rg * KWP + V * cv) * 4);
-    if (col_in && kH0 >= 0 && kH0 + nrows <= h && hip != nullptr) {
-        const float* lp = lowp + (long long)(kH0 + rg) * low_rs + kc0;
-        const float* hp = hip + (size_t)(kH0 + rg) * w + kc0;
-        const long long lstep = (long long)NRG * low_rs;
-        const size_t hstep = (size_t)NRG * w;
-#pragma unroll 2
-        for (int r = rg; r < nrows; r += NRG) {
-            cp_async<V>(dst, lp);
-            cp_async<V>(dst + PBB, hp);
-            cp_async<V>(dst + 2 * PBB, hp + band);
-            cp_async<V>(dst + 3 * PBB, hp + 2 * band);
-            dst += NRG * KWP * 4;
-            lp += lstep;
-            hp += hstep;
-        }
-        return;
-    }
-    int ci[V];
-#pragma unroll
-    for (int e = 0; e < V; ++e) ci[e] = coef_index(kc0 + e, w, periodic);
-    for (int r = rg; r < nrows; r += NRG, dst += NRG * KWP * 4) {
-        const int kr = coef_index(kH0 + r, h, periodic);
-        if (kr < 0) {
-#pragma unroll
-            for (int b = 0; b < 4; ++b) cp_async_zero<V>(dst + b * PBB, lowp);
-            continue;
-        }
-        const float* lp = lowp + (long long)kr * low_rs;
-        const float* hp = hip ? hip + (size_t)kr * w : nullptr;
-        if (col_in) {
-            cp_async<V>(dst, lp + kc0);
-            if (hp) {
-                cp_async<V>(dst + PBB, hp + kc0);
-                cp_async<V>(dst + 2 * PBB, hp + band + kc0);
-                cp_async<V>(dst + 3 * PBB, hp + 2 * band + kc0);
-            } else {
-#pragma unroll
-                for (int b = 1; b < 4; ++b) cp_async_zero<V>(dst + b * PBB, lowp);
-            }
-        } else {
-#pragma unroll
-            for (int e = 0; e < V; ++e) {
-                const bool ok = ci[e] >= 0;
-                const int k = ok ? ci[e] : 0;
-                cp_async4_if(dst + 4 * e, lp + k, ok);
-                cp_async4_if(dst + PBB + 4 * e, hp ? hp + k : lowp, ok && hp);
-                cp_async4_if(dst + 2 * PBB + 4 * e, hp ? hp + band + k : lowp, ok && hp);
-                cp_async4_if(dst + 3 * PBB + 4 * e, hp ? hp + 2 * band + k : lowp, ok && hp);
-            }
-        }
-    }
-}
-
-template <int L_, int TW_, int TH_, int NT_>
-struct SfbOp {
-    using Params = SfbParams;
-    static constexpr const char* name = "chain_kernel<SfbOp>";
-    static constexpr int L = L_, TW = TW_, TH = TH_, NT = NT_;
-    static constexpr int H2 = L / 2;
-    static constexpr int NV2 = (H2 + 2) / 2;            // float2 loads per band per W-synthesis item
-    static constexpr int KWP = TW / 2 - 2 + 2 * NV2;    // staged coefficient columns (even, >= TW/2 + H2 - 1)
-    static constexpr int KH = TH / 2 + H2 - 1;          // staged coefficient rows
-    static constexpr int PB = KH * KWP;                 // one band's patch
-    static constexpr int BUF = 4 * PB;                  // floats per staging buffer (LL, LH, HL, HH)
-    static constexpr int NQ = TW / 4;                   // W-synthesis items per coefficient row (4 outputs each)
-    static constexpr int QSTEP = NT / NQ;               // coefficient rows advanced per W-synthesis iteration
-    static constexpr int CP = TW / 2;                   // output column pairs (H pass)
-    static constexpr int NS = NT / CP;
-    static constexpr int RS = TH / NS;                  // output rows per thread in the H pass (even)
-    static constexpr int NR = RS / 2 + H2 - 1;          // coefficient rows feeding RS outputs
-    static constexpr size_t smem = sizeof(float) * (size_t)(2 * BUF + 2 * KH * TW);  // 2 x 4 patches + u_lo/u_hi
-    static_assert(L % 2 == 0 && TW % 4 == 0 && NT % CP == 0 && TH % NS == 0 && RS % 2 == 0 && NT % NQ == 0, "bad tile");
-    static_assert(KWP >= TW / 2 + H2 - 1 && KWP % 2 == 0 && KWP <= NT, "bad KWP");
-
-    static __device__ __forceinline__ void issue(const SfbParams& p, const TileRef& t, unsigned sub_s, int tid) {
-        const SfbLevel& lv = p.lv[t.level];
-        const int aW = lv.a0W + t.tw * TW, aH = lv.a0H + t.th * TH;
-        const int kW0 = aW / 2 - (H2 - 1);
-        const int kH0 = aH / 2 - (H2 - 1);
-        const size_t band = (size_t)lv.h * lv.w;
-        const float* lowp = lv.low + (long long)t.plane * lv.low_ps;
-        const float* hip = lv.highs ? lv.highs + (size_t)t.plane * 3 * band : nullptr;
-        // coefficient rows / columns feeding the valid outputs of an edge tile: a <= a_max -> k_local <= a_max/2 + H2-1
-        const int amax_h = min(TH - 1, lv.offH + lv.out_h - 1 - aH);
-        const int amax_w = min(TW - 1, lv.offW + lv.out_w - 1 - aW);
-        const int nrows = min(KH, amax_h / 2 + H2);
-        const int ncols = min(KWP, amax_w / 2 + H2);
-        // kW0 is even whenever in_vec2 is set (checked on the host)
-        if (lv.in_vec2)
-            stage_synthesis<2, KH, KWP, NT>(sub_s, lowp, lv.low_rs, hip, band, kH0, kW0, lv.h, lv.w, p.periodic, nrows, ncols, tid);
-        else
-            stage_synthesis<1, KH, KWP, NT>(sub_s, lowp, lv.low_rs, hip, band, kH0, kW0, lv.h, lv.w, p.periodic, nrows, ncols, tid);
-    }
-
-    // W synthesis: each item makes four consecutive outputs (a = 4qq .. 4qq+3) of one coefficient row, for both
-    // the h_lo branch (LL, HL) and the h_hi branch (LH, HH)
-    static __device__ __forceinline__ void pass1(const SfbParams& p, const TileRef&, const float* sub, float* u, int tid) {
-        const int qq = tid % NQ;
-        int r = tid / NQ;
-        const float* s0 = sub + r * KWP + 2 * qq;
-        float* d = u + r * TW + 4 * qq;
-        for (; r < KH; r += QSTEP, s0 += QSTEP * KWP, d += QSTEP * TW) {
-            float c[4][2 * NV2];  // local coefficients 2qq .. 2qq+2NV2-1 of LL, LH, HL, HH
-#pragma unroll
-            for (int b = 0; b < 4; ++b)
-#pragma unroll
-                for (int q = 0; q < NV2; ++q) {
-                    const float2 t = reinterpret_cast<const float2*>(s0 + b * PB)[q];
-                    c[b][2 * q] = t.x;
-                    c[b][2 * q + 1] = t.y;
-                }
-            float lo[4], hi[4];
-#pragma unroll
-            for (int e = 0; e < 4; ++e) {
-                const int qo = e >> 1, par = e & 1;  // output a = 2(2qq+qo) + par uses k_local = qo + H2-1-u
-                float a = 0.f, b = 0.f;
-#pragma unroll
-                for (int uu = 0; uu < H2; ++uu) {
-                    const int k = qo + H2 - 1 - uu;
-                    a = fmaf(c[0][k], p.t.w_lo[par + 2 * uu], a);
-                    a = fmaf(c[2][k], p.t.w_hi[par + 2 * uu], a);
-                    b = fmaf(c[1][k], p.t.w_lo[par + 2 * uu], b);
-                    b = fmaf(c[3][k], p.t.w_hi[par + 2 * uu], b);
-                }
-                lo[e] = a;
-                hi[e] = b;
-            }
-            *reinterpret_cast<float4*>(d) = make_float4(lo[0], lo[1], lo[2], lo[3]);
-            *reinterpret_cast<float4*>(d + KH * TW) = make_float4(hi[0], hi[1], hi[2], hi[3]);
-        }
-    }
-
-    // H synthesis: thread = two adjacent output columns, RS consecutive output rows
-    static __device__ __forceinline__ void pass2(const SfbParams& p, const TileRef& t, const float* u, int tid) {
-        const SfbLevel& lv = p.lv[t.level];
-        const int cp = tid % CP;
-        const int s = tid / CP;
-        float2 vlo[NR], vhi[NR];
-        const float2* plo = reinterpret_cast<const float2*>(u + (s * (RS / 2)) * TW + 2 * cp);
-        const float2* phi = reinterpret_cast<const float2*>(u + KH * TW + (s * (RS / 2)) * TW + 2 * cp);
-#pragma unroll
-        for (int r = 0; r < NR; ++r) {
-            vlo[r] = plo[r * (TW / 2)];
-            vhi[r] = phi[r * (TW / 2)];
-        }
-        float2 y[RS];
-#pragma unroll
-        for (int i = 0; i < RS / 2; ++i) {
-            float2 ye = make_float2(0.f, 0.f), yo = ye;
-#pragma unroll
-            for (int uu = 0; uu < H2; ++uu) {
-                const int r = i - uu + H2 - 1;  // local coefficient row
-                const float a0 = p.t.h_lo[2 * uu], b0 = p.t.h_hi[2 * uu], a1 = p.t.h_lo[2 * uu + 1], b1 = p.t.h_hi[2 * uu + 1];
-                ye.x = fmaf(vlo[r].x, a0, ye.x); ye.y = fmaf(vlo[r].y, a0, ye.y);
-                ye.x = fmaf(vhi[r].x, b0, ye.x); ye.y = fmaf(vhi[r].y, b0, ye.y);
-                yo.x = fmaf(vlo[r].x, a1, yo.x); yo.y = fmaf(vlo[r].y, a1, yo.y);
-                yo.x = fmaf(vhi[r].x, b1, yo.x); yo.y = fmaf(vhi[r].y, b1, yo.y);
-            }
-            y[2 * i] = ye;
-            y[2 * i + 1] = yo;
-        }
-        const int out_h = lv.out_h, out_w = lv.out_w;
-        const int nW = lv.a0W + t.tw * TW + 2 * cp - lv.offW;
-        const int nH = lv.a0H + t.th * TH + s * RS - lv.offH;
-        const long long yrs = lv.y_rs;
-        float* q = lv.y + (long long)t.plane * lv.y_ps + (long long)nH * yrs + nW;  // only dereferenced where valid
-        if (lv.out_vec2 && nH >= 0 && nH + RS <= out_h && nW >= 0 && nW + 1 < out_w) {
-#pragma unroll
-            for (int i = 0; i < RS; ++i) {
-                *reinterpret_cast<float2*>(q) = y[i];
-                q += yrs;
-            }
-        } else {
-            const bool ok0 = nW >= 0 && nW < out_w;
-            const bool ok1 = nW + 1 >= 0 && nW + 1 < out_w;
-#pragma unroll
-            for (int i = 0; i < RS; ++i) {
-                const int row = nH + i;
-                if (row >= 0 && row < out_h) {
-                    if (ok0) q[0] = y[i].x;
-                    if (ok1) q[1] = y[i].y;
-                }
-                q += yrs;
-            }
-        }
-    }
-};
-
-// synthesis, direct: one thread per output sample of ONE level; any tap count.
+template <class T>
 struct SfbDirectParams {
-    SfbLevel lv;
+    const T* low;
+    const T* highs;            // dense (planes,3,h,w); may be null (= zeros)
+    T* y;
+    long long low_ps, low_rs, y_ps, y_rs;
+    int h, w, out_h, out_w, offH, offW;
     int planes, periodic, Lw, Lh;
-    Taps t;
+    DirectTaps<T> t;
 };
 
-__global__ void __launch_bounds__(kThreads) sfb2d_direct_kernel(const __grid_constant__ SfbDirectParams p) {
-    const SfbLevel& lv = p.lv;
-    const size_t total = (size_t)p.planes * lv.out_h * lv.out_w;
-    const size_t band = (size_t)lv.h * lv.w;
+// "A-space" as in the other synthesis kernels: a = n + off; output a uses the taps of parity a & 1
+template <class T>
+__global__ void __launch_bounds__(kThreads) sfb2d_direct_kernel(const __grid_constant__ SfbDirectParams<T> p) {
+    const size_t total = (size_t)p.planes * p.out_h * p.out_w;
+    const size_t band = (size_t)p.h * p.w;
     for (size_t idx = (size_t)blockIdx.x * blockDim.x + threadIdx.x; idx < total;
          idx += (size_t)gridDim.x * blockDim.x) {
-        const int nW = (int)(idx % lv.out_w);
-        const int nH = (int)((idx / lv.out_w) % lv.out_h);
-        const int plane = (int)(idx / ((size_t)lv.out_h * lv.out_w));
-        const float* __restrict__ lowp = lv.low + (long long)plane * lv.low_ps;
-        const float* __restrict__ hip = lv.highs ? lv.highs + (size_t)plane * 3 * band : nullptr;
-        const int AH = nH + lv.offH, AW = nW + lv.offW;
-        float y = 0.f;
+        const int nW = (int)(idx % p.out_w);
+        const int nH = (int)((idx / p.out_w) % p.out_h);
+        const int plane = (int)(idx / ((size_t)p.out_h * p.out_w));
+        const T* __restrict__ lowp = p.low + (long long)plane * p.low_ps;
+        const T* __restrict__ hip = p.highs ? p.highs + (size_t)plane * 3 * band : nullptr;
+        const int AH = nH + p.offH, AW = nW + p.offW;
+        T y = 0;
         for (int tH = AH & 1; tH < p.Lh; tH += 2) {
-            const int kr = coef_index((AH - tH) / 2, lv.h, p.periodic);
+            const int kr = coef_index((AH - tH) / 2, p.h, p.periodic);
             if (kr < 0) continue;
-            float lo = 0.f, hi = 0.f;  // W-synthesised values to be combined with h_lo / h_hi
+            T lo = 0, hi = 0;  // W-synthesised values to be combined with h_lo / h_hi
             for (int tW = AW & 1; tW < p.Lw; tW += 2) {
-                const int kc = coef_index((AW - tW) / 2, lv.w, p.periodic);
+                const int kc = coef_index((AW - tW) / 2, p.w, p.periodic);
                 if (kc < 0) continue;
-                const float ll = __ldg(lowp + (long long)kr * lv.low_rs + kc);
-                lo = fmaf(ll, p.t.w_lo[tW], lo);
+                const T ll = __ldg(lowp + (long long)kr * p.low_rs + kc);
+                lo = fma(ll, p.t.w_lo[tW], lo);
                 if (hip) {
-                    const float* q = hip + (size_t)kr * lv.w + kc;
-                    hi = fmaf(__ldg(q), p.t.w_lo[tW], hi);               // LH
-                    lo = fmaf(__ldg(q + band), p.t.w_hi[tW], lo);        // HL
-                    hi = fmaf(__ldg(q + 2 * band), p.t.w_hi[tW], hi);    // HH
+                    const T* q = hip + (size_t)kr * p.w + kc;
+                    hi = fma(__ldg(q), p.t.w_lo[tW], hi);               // LH
+                    lo = fma(__ldg(q + band), p.t.w_hi[tW], lo);        // HL
+                    hi = fma(__ldg(q + 2 * band), p.t.w_hi[tW], hi);    // HH
                 }
             }
-            y = fmaf(lo, p.t.h_lo[tH], y);
-            y = fmaf(hi, p.t.h_hi[tH], y);
+            y = fma(lo, p.t.h_lo[tH], y);
+            y = fma(hi, p.t.h_hi[tH], y);
         }
-        lv.y[(long long)plane * lv.y_ps + (long long)nH * lv.y_rs + nW] = y;
+        p.y[(long long)plane * p.y_ps + (long long)nH * p.y_rs + nW] = y;
     }
 }
 
@@ -643,19 +461,22 @@ static bool mode_supported(int mode) {
            mode == B200W_MODE_REFLECT || mode == B200W_MODE_PERIODIC;
 }
 
-static int fill_taps(Taps& t, const float* w_lo, const float* w_hi, int Lw, const float* h_lo, const float* h_hi,
-                     int Lh) {
+// copies the taps into a kernel's tap block, zero beyond Lw / Lh
+template <class T>
+static int fill_taps(DirectTaps<T>& t, const T* w_lo, const T* w_hi, int Lw, const T* h_lo, const T* h_hi, int Lh) {
     if (Lw < 1 || Lw > kMaxTaps || Lh < 1 || Lh > kMaxTaps || !w_lo || !w_hi || !h_lo || !h_hi)
         return B200W_ERR_BAD_TAPS;
     for (int i = 0; i < kMaxTaps; ++i) {
-        t.w_lo[i] = i < Lw ? w_lo[i] : 0.f;
-        t.w_hi[i] = i < Lw ? w_hi[i] : 0.f;
-        t.h_lo[i] = i < Lh ? h_lo[i] : 0.f;
-        t.h_hi[i] = i < Lh ? h_hi[i] : 0.f;
+        t.w_lo[i] = i < Lw ? w_lo[i] : T(0);
+        t.w_hi[i] = i < Lw ? w_hi[i] : T(0);
+        t.h_lo[i] = i < Lh ? h_lo[i] : T(0);
+        t.h_hi[i] = i < Lh ? h_hi[i] : T(0);
     }
-    for (int i = 0; i < kMaxTemplTaps; ++i) {
-        t.h_lo2[i] = make_float2(t.h_lo[i], t.h_lo[i]);
-        t.h_hi2[i] = make_float2(t.h_hi[i], t.h_hi[i]);
+    if constexpr (std::is_same<T, float>::value) {
+        for (int i = 0; i < kMaxTemplTaps; ++i) {
+            t.h_lo2[i] = make_float2(t.h_lo[i], t.h_lo[i]);
+            t.h_hi2[i] = make_float2(t.h_hi[i], t.h_hi[i]);
+        }
     }
     return B200W_OK;
 }
@@ -676,6 +497,9 @@ static int analysis_offset(int n, int l, int mode, int* off) {
     *off = p / 2;
     return B200W_OK;
 }
+
+// A-space offset of the synthesis bank along one axis
+static int synthesis_offset(int l, int mode) { return mode == B200W_MODE_PERIODIZATION ? l / 2 - 1 : l - 2; }
 
 constexpr int kMaxDevices = 64;
 
@@ -776,32 +600,19 @@ static int launch_afb_chain(AfbParams& p, cudaStream_t st) {
     return launch_chain<Op>(p, occ, st);
 }
 
-template <int L>
-static int launch_sfb_chain(SfbParams& p, cudaStream_t st) {
-    using Op = SfbOp<L, 64, 64, 256>;
-    static int occ[kMaxDevices] = {0};
-    long long base = 0;
-    for (int j = 0; j < p.J; ++j) {
-        SfbLevel& lv = p.lv[j];
-        lv.a0W = lv.offW & ~1;
-        lv.a0H = lv.offH & ~1;
-        lv.tiles_w = ceil_div(lv.offW + lv.out_w - lv.a0W, Op::TW);
-        lv.tiles_h = ceil_div(lv.offH + lv.out_h - lv.a0H, Op::TH);
-        // tile 0 starts at coefficient column a0W/2 - (L/2-1): even for every non-periodization mode
-        const int kW0 = lv.a0W / 2 - (L / 2 - 1);
-        if ((kW0 & 1) != 0) lv.in_vec2 = 0;
-        if ((lv.offW & 1) != 0) lv.out_vec2 = 0;
-        lv.tile_base = base;
-        base += (long long)lv.tiles_w * lv.tiles_h * p.planes;
-    }
-    p.total = base;
-    return launch_chain<Op>(p, occ, st);
-}
-
 static size_t direct_grid(size_t total) {
     size_t g = (total + kThreads - 1) / kThreads;
     const size_t cap = 148 * 16;
     return g < 1 ? 1 : (g > cap ? cap : g);
+}
+
+// one launch of a direct kernel; `outputs` = output positions over all planes
+template <class Params>
+static int launch_direct(void (*kernel)(Params), const Params& d, size_t outputs, const char* name, cudaStream_t st) {
+    kernel<<<(unsigned)direct_grid(outputs), kThreads, 0, st>>>(d);
+    note_launch(name);
+    const cudaError_t e = cudaGetLastError();
+    return e == cudaSuccess ? B200W_OK : set_last_cuda_error(e);
 }
 
 static bool templated_taps(int Lw, int Lh) {
@@ -935,30 +746,17 @@ static int run_afb_chain(const float* x, int64_t x_ps, int64_t x_rs, int planes,
         return run_afb_big_levels(p, Lw, st);
     }
     for (int j = 0; j < J; ++j) {  // level by level with the direct kernel
-        AfbDirectParams d;
-        d.lv = p.lv[j];
-        d.planes = planes;
-        d.mode = mode;
-        d.Lw = Lw;
-        d.Lh = Lh;
-        d.t = p.t;
-        afb2d_direct_kernel<<<(unsigned)direct_grid((size_t)planes * d.lv.Ho * d.lv.Wo), kThreads, 0, st>>>(d);
-        note_launch("afb2d_direct_kernel");
-        cudaError_t e = cudaGetLastError();
-        if (e != cudaSuccess) return set_last_cuda_error(e);
+        const AfbLevel& lv = p.lv[j];
+        const AfbDirectParams<float> d = {lv.x, lv.low, lv.highs, lv.x_ps, lv.x_rs, lv.low_ps, lv.low_rs, lv.H, lv.W,
+                                          lv.Hreal, lv.Wreal, lv.Ho, lv.Wo, lv.offH, lv.offW, lv.st_low, lv.st_hi,
+                                          lv.hi_scale, lv.hi_shift, planes, mode, Lw, Lh, p.t};
+        if ((rc = launch_direct(afb2d_direct_kernel<float>, d, (size_t)planes * lv.Ho * lv.Wo, "afb2d_direct_kernel", st)))
+            return rc;
     }
     return B200W_OK;
 }
 
 // ---- synthesis chain -------------------------------------------------------------------------------
-static int run_sfb_big_levels(SfbParams& p, int L, cudaStream_t st) {
-    if (!dwt_policy().force_tiled && sfb_stream_supported(p, L)) return launch_sfb_stream(p, L, device_info().sms, st);
-#define X(LL) return launch_sfb_chain<LL>(p, st)
-    B200W_FOR_EACH_L(X)
-#undef X
-    return B200W_ERR_BAD_TAPS;
-}
-
 static int sfb_check_dims(int planes, const int* hs, const int* ws, int Lw, int Lh, int mode, int J, const int* out_hs,
                           const int* out_ws) {
     if (!mode_supported(mode)) return B200W_ERR_BAD_MODE;
@@ -1030,20 +828,18 @@ static int run_sfb_chain(const float* yl, int64_t yl_ps, int64_t yl_rs, const fl
             lv.y_ps = (long long)lv.out_h * lv.y_rs;
             scratch += scratch_bytes(planes, lv.out_h, lv.out_w);
         }
-        lv.offW = per ? Lw / 2 - 1 : Lw - 2;
-        lv.offH = per ? Lh / 2 - 1 : Lh - 2;
-        lv.a0W = lv.a0H = 0;
-        lv.in_vec2 = ((lv.w % 2) == 0 && (lv.low_rs % 2) == 0 && (lv.low_ps % 2) == 0 && aligned_to(lv.low, 8) &&
-                      (!lv.highs || aligned_to(lv.highs, 8))) ? 1 : 0;
-        lv.out_vec2 = ((lv.y_rs % 2) == 0 && (lv.y_ps % 2) == 0 && aligned_to(lv.y, 8)) ? 1 : 0;
-        lv.tile_base = lv.cta_base = 0;
-        lv.tiles_h = lv.tiles_w = lv.Rp = lv.cpp = lv.tA0 = lv.ntA = lv.itemsA = lv.cppA = 0;
+        lv.offW = synthesis_offset(Lw, mode);
+        lv.offH = synthesis_offset(Lh, mode);
+        lv.cta_base = 0;
+        lv.Rp = lv.cpp = lv.tA0 = lv.ntA = lv.itemsA = lv.cppA = 0;
         lv.nA0 = lv.nA1 = lv.itemsB = lv.n0_off = lv.kb_off = lv.m_lo = lv.vec2 = 0;
         lv.y_vec = 1;
     }
     if (templated_taps(Lw, Lh)) {
+        // chains of small planes: one CTA owns a part of a plane for all positions (TMA-staged owner kernel first, the
+        // cp.async owner kernel for the shapes it declines); everything else goes through the ticketed stream chain
         const DwtPolicy& pol = dwt_policy();
-        const bool owner = J > 1 && !pol.force_tiled && pol.owner != 0, force = pol.owner == 2;
+        const bool owner = J > 1 && pol.owner != 0, force = pol.owner == 2;
         if (owner && pol.tma) {
             SfbTmaParams tp;
             if (sfb_tma_plan(p, Lw, device_info().sms, force, pol.tma_G, pol.tma_D, tp)) return launch_sfb_tma(tp, Lw, st);
@@ -1052,20 +848,15 @@ static int run_sfb_chain(const float* yl, int64_t yl_ps, int64_t yl_rs, const fl
             SfbOwnerParams op;
             if (sfb_owner_plan(p, Lw, device_info().sms, force, op)) return launch_sfb_owner(op, Lw, st);
         }
-        return run_sfb_big_levels(p, Lw, st);
+        return launch_sfb_stream(p, Lw, device_info().sms, st);
     }
     for (int c = 0; c < J; ++c) {
-        SfbDirectParams d;
-        d.lv = p.lv[c];
-        d.planes = planes;
-        d.periodic = p.periodic;
-        d.Lw = Lw;
-        d.Lh = Lh;
-        d.t = p.t;
-        sfb2d_direct_kernel<<<(unsigned)direct_grid((size_t)planes * d.lv.out_h * d.lv.out_w), kThreads, 0, st>>>(d);
-        note_launch("sfb2d_direct_kernel");
-        cudaError_t e = cudaGetLastError();
-        if (e != cudaSuccess) return set_last_cuda_error(e);
+        const SfbLevel& lv = p.lv[c];
+        const SfbDirectParams<float> d = {lv.low, lv.highs, lv.y, lv.low_ps, lv.low_rs, lv.y_ps, lv.y_rs, lv.h, lv.w,
+                                          lv.out_h, lv.out_w, lv.offH, lv.offW, planes, p.periodic, Lw, Lh, p.t};
+        if ((rc = launch_direct(sfb2d_direct_kernel<float>, d, (size_t)planes * lv.out_h * lv.out_w, "sfb2d_direct_kernel",
+                                st)))
+            return rc;
     }
     return B200W_OK;
 }
@@ -1136,6 +927,78 @@ extern "C" int b200w_sfb2d_f32(const float* low, int64_t low_plane_stride, int64
     const float* his[1] = {highs};
     return run_sfb_chain(low, low_plane_stride, low_row_stride, his, planes, &h, &w, w_lo, w_hi, Lw, h_lo, h_hi, Lh,
                          mode, 1, &out_h, &out_w, y, nullptr, 0, (cudaStream_t)stream);
+}
+
+// The reference's fp64 mode (modules built under torch.set_default_dtype(torch.float64)): one level through the direct
+// kernels.  Unlike the fp32 entry points these check the data pointers before the mode, report null taps as
+// B200W_ERR_NULL_POINTER and reject outputs of more than 2^31-1 pixels per plane (ABI status codes).  The detail bands
+// pass the store epilogue with scale 1 and shift 0, which stores a -0 as +0.
+extern "C" int b200w_afb2d_f64(const double* x, int64_t x_ps, int64_t x_rs, int planes, int H, int W, const double* w_lo,
+                               const double* w_hi, int Lw, const double* h_lo, const double* h_hi, int Lh, int mode,
+                               double* low, double* highs, void* stream) {
+    if (!x || !low || !highs) return B200W_ERR_NULL_POINTER;
+    if (!mode_supported(mode)) return B200W_ERR_BAD_MODE;
+    if (planes < 1 || H < 1 || W < 1) return B200W_ERR_BAD_SHAPE;
+    if (!w_lo || !w_hi || !h_lo || !h_hi) return B200W_ERR_NULL_POINTER;
+    AfbDirectParams<double> d = {};
+    int rc = fill_taps(d.t, w_lo, w_hi, Lw, h_lo, h_hi, Lh);
+    if (rc || (rc = analysis_offset(H, Lh, mode, &d.offH)) || (rc = analysis_offset(W, Lw, mode, &d.offW))) return rc;
+    d.Ho = coeff_len(H, Lh, mode);
+    d.Wo = coeff_len(W, Lw, mode);
+    if (d.Ho < 1 || d.Wo < 1 || (long long)d.Ho * d.Wo > 0x7fffffffLL) return B200W_ERR_BAD_SHAPE;
+    d.x = x;
+    d.x_ps = x_ps;
+    d.x_rs = x_rs;
+    d.low = low;
+    d.low_rs = d.Wo;
+    d.low_ps = (long long)d.Ho * d.Wo;
+    d.highs = highs;
+    d.H = d.Hreal = H;
+    d.W = d.Wreal = W;
+    d.st_low = d.st_hi = 1;
+    d.hi_scale = 1.0;
+    d.hi_shift = 0.0;
+    d.planes = planes;
+    d.mode = mode;
+    d.Lw = Lw;
+    d.Lh = Lh;
+    return launch_direct(afb2d_direct_kernel<double>, d, (size_t)planes * d.Ho * d.Wo, "afb2d_f64_kernel",
+                         (cudaStream_t)stream);
+}
+
+extern "C" int b200w_sfb2d_f64(const double* low, int64_t low_ps, int64_t low_rs, const double* highs, int planes, int h,
+                               int w, const double* w_lo, const double* w_hi, int Lw, const double* h_lo,
+                               const double* h_hi, int Lh, int mode, double* y, int out_h, int out_w, void* stream) {
+    if (!low || !y) return B200W_ERR_NULL_POINTER;
+    if (!mode_supported(mode)) return B200W_ERR_BAD_MODE;
+    if (planes < 1 || h < 1 || w < 1 || out_h < 1 || out_w < 1) return B200W_ERR_BAD_SHAPE;
+    if (!w_lo || !w_hi || !h_lo || !h_hi) return B200W_ERR_NULL_POINTER;
+    SfbDirectParams<double> d = {};
+    const int rc = fill_taps(d.t, w_lo, w_hi, Lw, h_lo, h_hi, Lh);
+    if (rc) return rc;
+    const bool per = mode == B200W_MODE_PERIODIZATION;
+    if (per && (2 * h < Lh || 2 * w < Lw)) return B200W_ERR_PER_TOO_SHORT;
+    if (out_h > idwt_len(h, Lh, mode) || out_w > idwt_len(w, Lw, mode) || (long long)out_h * out_w > 0x7fffffffLL)
+        return B200W_ERR_BAD_SHAPE;
+    d.low = low;
+    d.low_ps = low_ps;
+    d.low_rs = low_rs;
+    d.highs = highs;
+    d.y = y;
+    d.y_rs = out_w;
+    d.y_ps = (long long)out_h * out_w;
+    d.h = h;
+    d.w = w;
+    d.out_h = out_h;
+    d.out_w = out_w;
+    d.offH = synthesis_offset(Lh, mode);
+    d.offW = synthesis_offset(Lw, mode);
+    d.planes = planes;
+    d.periodic = per;
+    d.Lw = Lw;
+    d.Lh = Lh;
+    return launch_direct(sfb2d_direct_kernel<double>, d, (size_t)planes * out_h * out_w, "sfb2d_f64_kernel",
+                         (cudaStream_t)stream);
 }
 
 extern "C" int b200w_idwt2_f32(const float* yl, int64_t yl_plane_stride, int64_t yl_row_stride,

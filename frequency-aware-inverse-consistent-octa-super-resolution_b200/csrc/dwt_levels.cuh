@@ -1,4 +1,4 @@
-// Level geometry and chain bookkeeping shared by the DWT kernels (tile, stream and direct variants).
+// Level geometry and chain bookkeeping shared by the DWT chain kernels (tile, stream, owner and TMA variants).
 //
 // A multi-level transform is ONE launch: the work items of all levels form one ordered list (all items of the
 // first level, then the next level, ...).  An item of level j+1 of image plane p may start once every item of
@@ -99,12 +99,6 @@ struct SfbLevel {
     long long y_ps, y_rs;  // output strides: dense for the last level, padded scratch for intermediates
     int h, w, out_h, out_w;
     int offH, offW;
-    // tile kernels
-    long long tile_base;
-    int a0H, a0W;          // first A-space coordinate (even) covered by tile 0
-    int tiles_h, tiles_w;
-    int in_vec2;           // 64-bit staging copies allowed
-    int out_vec2;          // 64-bit stores allowed
     // stream kernels: a thread owns four adjacent output columns over Rp output row pairs.  Threads whose
     // coefficient window and outputs lie inside the arrays ("interior", tA0 <= t < tA0 + ntA) stage through the
     // per-warp ring; the few border output columns are evaluated one thread per output position.
@@ -194,7 +188,7 @@ static inline bool aligned_to(const void* p, size_t a) { return (reinterpret_cas
 // written kernel families against each other on the same inputs; the defaults are what every other run takes.
 struct DwtPolicy {
     bool force_direct;   // B200W_FORCE_DIRECT=1: one-thread-per-output kernels only
-    bool force_tiled;    // B200W_FORCE_TILED=1: shared-memory tile kernels instead of the stream and owner kernels
+    bool force_tiled;    // B200W_FORCE_TILED=1: analysis tile kernels instead of the stream and owner kernels
     int owner;           // B200W_OWNER: 0 = no owner kernels (ticketed chains), 1 = where they pay off, 2 = whenever they fit
     bool tma;            // B200W_TMA=0: cp.async owner kernels instead of the TMA-staged ones
     bool tma_noboxes;    // B200W_TMA_NOBOXES: TMA analysis ring fetches every extension row from its source row

@@ -3,8 +3,8 @@ under ``torch.set_default_dtype(torch.float64)``, ``tests/test_dwt.py:132-160``)
 
 Same contract as the fp32 ops in ``ops.py`` -- outputs allocated by torch, launch on the current stream, CUDA-only, the
 reference's hand-written backward (``afb2d`` backward = ``sfb2d`` with the analysis taps + crop, ``sfb2d`` backward =
-``afb2d`` with the synthesis taps) -- on double tensors with double taps, through the simple one-thread-per-output
-kernels of ``csrc/dwt_f64.cu``.  ``DWTForward`` / ``DWTInverse`` run fp64 transforms level by level through these ops
+``afb2d`` with the synthesis taps) -- on double tensors with double taps, through the one-thread-per-output direct
+kernels of ``csrc/dwt.cu``, instantiated for ``double``.  ``DWTForward`` / ``DWTInverse`` run fp64 transforms level by level through these ops
 (precision, not speed, is the point of this path).
 """
 import torch

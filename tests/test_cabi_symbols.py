@@ -91,6 +91,66 @@ def test_argument_validation_happens_before_any_launch(lib):
         _cabi.check(_cabi.ERR_BAD_SHAPE)
 
 
+def test_f64_argument_validation_happens_before_any_launch(lib):
+    """b200w_afb2d_f64 / b200w_sfb2d_f64: bad arguments come back as status codes without touching the (absent) GPU.
+    Unlike the fp32 entry points they check the data pointers before the mode and report null taps as
+    ERR_NULL_POINTER; outputs of more than 2^31-1 pixels per plane are ERR_BAD_SHAPE."""
+    t2, n2 = _cabi.taps_array_f64([0.5, 0.5])
+    t6, n6 = _cabi.taps_array_f64([0.1] * 6)
+    t1, n1 = _cabi.taps_array_f64([1.0])
+    bogus = ctypes.c_void_p(256)
+
+    def taps(w=(t2, n2), h=(t2, n2)):   # (w_lo, w_hi, Lw, h_lo, h_hi, Lh)
+        return (w[0], w[0], w[1], h[0], h[0], h[1])
+
+    def afb(x=bogus, planes=1, H=8, W=8, tp=taps(), mode=0, low=bogus, highs=bogus):
+        return lib.b200w_afb2d_f64(x, H * W, W, planes, H, W, *tp, mode, low, highs, None)
+
+    assert afb(x=None, mode=3) == _cabi.ERR_NULL_POINTER                  # pointers before the mode
+    assert afb(low=None) == _cabi.ERR_NULL_POINTER
+    assert afb(highs=None) == _cabi.ERR_NULL_POINTER
+    assert afb(mode=3, planes=0) == _cabi.ERR_BAD_MODE                    # mode before the shape
+    assert afb(mode=5) == _cabi.ERR_BAD_MODE
+    assert afb(planes=0, tp=taps(w=(None, n2))) == _cabi.ERR_BAD_SHAPE    # shape before the taps
+    assert afb(H=0) == _cabi.ERR_BAD_SHAPE
+    assert afb(tp=taps(w=(None, 0))) == _cabi.ERR_NULL_POINTER            # null taps before the tap count
+    assert afb(tp=(t2, t2, n2, t2, None, n2)) == _cabi.ERR_NULL_POINTER
+    assert afb(tp=taps(w=(t2, 0))) == _cabi.ERR_BAD_TAPS
+    assert afb(tp=taps(h=(t2, _cabi.MAX_TAPS + 1))) == _cabi.ERR_BAD_TAPS
+    # reflect padding needs pad < dimension: 4-sample axis, 6 taps -> pad 4; the taps are checked first
+    assert afb(H=4, W=4, tp=taps((t6, n6), (t6, n6)), mode=4) == _cabi.ERR_REFLECT_PAD
+    assert afb(H=16, W=4, tp=taps((t6, n6), (t6, n6)), mode=4) == _cabi.ERR_REFLECT_PAD
+    assert afb(H=4, W=4, tp=taps((t6, 0), (t6, n6)), mode=4) == _cabi.ERR_BAD_TAPS
+    assert afb(H=4, W=4, tp=taps((t6, n6), (t6, n6)), mode=2) == _cabi.ERR_PER_TOO_SHORT
+    assert afb(H=4, W=16, tp=taps((t2, n2), (t6, n6)), mode=2) == _cabi.ERR_PER_TOO_SHORT
+    assert afb(H=1, W=8, tp=taps(h=(t1, n1))) == _cabi.ERR_BAD_SHAPE        # zero output rows
+    assert afb(H=100000, W=100000) == _cabi.ERR_BAD_SHAPE                   # 50000^2 output pixels
+
+    def sfb(low=bogus, planes=1, h=4, w=4, tp=taps(), mode=0, y=bogus, out_h=8, out_w=8):
+        return lib.b200w_sfb2d_f64(low, h * w, w, None, planes, h, w, *tp, mode, y, out_h, out_w, None)
+
+    assert sfb(low=None, mode=3) == _cabi.ERR_NULL_POINTER
+    assert sfb(y=None) == _cabi.ERR_NULL_POINTER
+    assert sfb(mode=3, planes=0) == _cabi.ERR_BAD_MODE
+    assert sfb(planes=0, tp=taps(w=(None, n2))) == _cabi.ERR_BAD_SHAPE
+    assert sfb(w=0) == _cabi.ERR_BAD_SHAPE
+    assert sfb(out_w=0) == _cabi.ERR_BAD_SHAPE
+    assert sfb(tp=taps(w=(None, 0))) == _cabi.ERR_NULL_POINTER
+    assert sfb(tp=(t2, t2, n2, t2, None, n2)) == _cabi.ERR_NULL_POINTER
+    assert sfb(tp=taps(w=(t2, 0))) == _cabi.ERR_BAD_TAPS
+    assert sfb(tp=taps(h=(t2, _cabi.MAX_TAPS + 1))) == _cabi.ERR_BAD_TAPS
+    assert sfb(h=2, w=2, tp=taps((t6, n6), (t6, n6)), mode=2, out_h=4, out_w=4) == _cabi.ERR_PER_TOO_SHORT
+    assert sfb(h=8, w=2, tp=taps((t6, n6), (t6, n6)), mode=2, out_h=4, out_w=4) == _cabi.ERR_PER_TOO_SHORT
+    assert sfb(h=2, w=8, tp=taps((t6, 0), (t6, n6)), mode=2, out_h=4, out_w=4) == _cabi.ERR_BAD_TAPS
+    assert sfb(h=2, w=2, tp=taps((t6, n6), (t6, n6)), mode=2, out_h=99) == _cabi.ERR_PER_TOO_SHORT
+    # synthesis: out larger than the natural output (idwt_len)
+    assert sfb(out_h=9) == _cabi.ERR_BAD_SHAPE
+    assert sfb(out_w=9, mode=1) == _cabi.ERR_BAD_SHAPE
+    assert sfb(out_h=9, mode=2) == _cabi.ERR_BAD_SHAPE
+    assert sfb(tp=taps((t6, n6), (t6, n6)), out_h=5, out_w=4) == _cabi.ERR_BAD_SHAPE
+    assert sfb(h=50000, w=50000, out_h=100000, out_w=100000) == _cabi.ERR_BAD_SHAPE   # 10^10 output pixels
+
+
 def test_multilevel_entry_points_validate_before_any_launch(lib):
     """b200w_dwt2_f32 / b200w_idwt2_f32: workspace sizing is host arithmetic and bad arguments come back as status
     codes without touching the (absent) GPU."""

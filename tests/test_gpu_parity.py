@@ -489,7 +489,7 @@ def test_host_pipeline_matches_direct_call():
                                  "B200W_TMA_NOBOXES=1 B200W_OWNER=2", "B200W_TMA_G=2 B200W_TMA_D=2 B200W_OWNER=2"])
 def test_alternative_kernel_paths(env):
     """The same golden / oracle cases through the other implementations of the path (the env switches are read
-    once per process, hence a child pytest): shared-memory tile kernels, direct kernels, the owner kernels forced
+    once per process, hence a child pytest): analysis tile kernels, direct kernels, the owner kernels forced
     onto every multi-level shape that fits (TMA-staged ones first; B200W_TMA=0: the cp.async ones), the ticketed
     chain kernels alone, the TMA kernels with row-by-row staging of the extension rows / with few streams and the
     shallowest ring."""
