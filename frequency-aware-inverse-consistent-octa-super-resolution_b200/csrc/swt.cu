@@ -16,59 +16,62 @@
 
 namespace b200w {
 
+// T = float, or double for the reference's fp64 mode
+template <typename T>
 struct SwtParams {
-    const float* in;     // forward: x (planes, H, W) ; backward: dy (planes, 4, H, W)
-    float* out;          // forward: y (planes, 4, H, W) ; backward: dx (planes, H, W)
+    const T* in;         // forward: x (planes, H, W) ; backward: dy (planes, 4, H, W)
+    T* out;              // forward: y (planes, 4, H, W) ; backward: dx (planes, H, W)
     int planes, H, W, L, d, pl, pr, mode;
-    float w_lo[kMaxTaps], w_hi[kMaxTaps], h_lo[kMaxTaps], h_hi[kMaxTaps];
+    T w_lo[kMaxTaps], w_hi[kMaxTaps], h_lo[kMaxTaps], h_hi[kMaxTaps];
 };
 
-__global__ void __launch_bounds__(kThreads) swt2d_fwd_kernel(const __grid_constant__ SwtParams p) {
+template <typename T>
+__global__ void __launch_bounds__(kThreads) swt2d_fwd_kernel(const __grid_constant__ SwtParams<T> p) {
     const size_t plane_px = (size_t)p.H * p.W;
     // planes on grid.y, pixels of a plane on grid.x with 32-bit index arithmetic (H * W < 2^31 is checked by the host)
     for (int plane = blockIdx.y; plane < p.planes; plane += gridDim.y)
     for (unsigned px = blockIdx.x * blockDim.x + threadIdx.x; px < (unsigned)plane_px; px += gridDim.x * blockDim.x) {
         const int i = (int)(px / (unsigned)p.W);
         const int k = (int)(px - (unsigned)i * (unsigned)p.W);
-        const float* __restrict__ xp = p.in + plane * plane_px;
-        float ll = 0.f, lh = 0.f, hl = 0.f, hh = 0.f;   // (row lo, col lo), (row lo, col hi), (row hi, col lo), (row hi, col hi)
+        const T* __restrict__ xp = p.in + plane * plane_px;
+        T ll = 0, lh = 0, hl = 0, hh = 0;   // (row lo, col lo), (row lo, col hi), (row hi, col lo), (row hi, col hi)
         const int r0 = i - p.pl, c0 = k - p.pl, span = p.d * (p.L - 1);
         if (r0 >= 0 && r0 + span < p.H && c0 >= 0 && c0 + span < p.W) {      // interior window: no index maps
-            const float* __restrict__ xw = xp + (size_t)r0 * p.W + c0;
+            const T* __restrict__ xw = xp + (size_t)r0 * p.W + c0;
             for (int jh = 0; jh < p.L; ++jh) {
-                const float* __restrict__ xr = xw + (size_t)(p.d * jh) * p.W;
-                float lo = 0.f, hi = 0.f;
+                const T* __restrict__ xr = xw + (size_t)(p.d * jh) * p.W;
+                T lo = 0, hi = 0;
 #pragma unroll 4
                 for (int jw = 0; jw < p.L; ++jw) {
-                    const float v = __ldg(xr + p.d * jw);
-                    lo = fmaf(p.w_lo[jw], v, lo);
-                    hi = fmaf(p.w_hi[jw], v, hi);
+                    const T v = __ldg(xr + p.d * jw);
+                    lo = fma(p.w_lo[jw], v, lo);
+                    hi = fma(p.w_hi[jw], v, hi);
                 }
-                ll = fmaf(p.h_lo[jh], lo, ll);
-                lh = fmaf(p.h_hi[jh], lo, lh);
-                hl = fmaf(p.h_lo[jh], hi, hl);
-                hh = fmaf(p.h_hi[jh], hi, hh);
+                ll = fma(p.h_lo[jh], lo, ll);
+                lh = fma(p.h_hi[jh], lo, lh);
+                hl = fma(p.h_lo[jh], hi, hl);
+                hh = fma(p.h_hi[jh], hi, hh);
             }
         } else {
             for (int jh = 0; jh < p.L; ++jh) {
                 const int r = ext_index(r0 + p.d * jh, p.H, p.mode);
                 if (r < 0) continue;
-                const float* __restrict__ xr = xp + (size_t)r * p.W;
-                float lo = 0.f, hi = 0.f;
+                const T* __restrict__ xr = xp + (size_t)r * p.W;
+                T lo = 0, hi = 0;
                 for (int jw = 0; jw < p.L; ++jw) {
                     const int c = ext_index(c0 + p.d * jw, p.W, p.mode);
                     if (c < 0) continue;
-                    const float v = __ldg(xr + c);
-                    lo = fmaf(p.w_lo[jw], v, lo);
-                    hi = fmaf(p.w_hi[jw], v, hi);
+                    const T v = __ldg(xr + c);
+                    lo = fma(p.w_lo[jw], v, lo);
+                    hi = fma(p.w_hi[jw], v, hi);
                 }
-                ll = fmaf(p.h_lo[jh], lo, ll);
-                lh = fmaf(p.h_hi[jh], lo, lh);
-                hl = fmaf(p.h_lo[jh], hi, hl);
-                hh = fmaf(p.h_hi[jh], hi, hh);
+                ll = fma(p.h_lo[jh], lo, ll);
+                lh = fma(p.h_hi[jh], lo, lh);
+                hl = fma(p.h_lo[jh], hi, hl);
+                hh = fma(p.h_hi[jh], hi, hh);
             }
         }
-        float* o = p.out + plane * 4 * plane_px + (size_t)i * p.W + k;
+        T* o = p.out + plane * 4 * plane_px + (size_t)i * p.W + k;
         o[0] = ll;
         o[plane_px] = lh;
         o[2 * plane_px] = hl;
@@ -104,37 +107,38 @@ __device__ __forceinline__ int preimages(int s, int n, int pl, int pr, int mode,
     return cnt;
 }
 
-__global__ void __launch_bounds__(kThreads) swt2d_bwd_kernel(const __grid_constant__ SwtParams p) {
+template <typename T>
+__global__ void __launch_bounds__(kThreads) swt2d_bwd_kernel(const __grid_constant__ SwtParams<T> p) {
     const size_t plane_px = (size_t)p.H * p.W;
     for (int plane = blockIdx.y; plane < p.planes; plane += gridDim.y)
     for (unsigned px = blockIdx.x * blockDim.x + threadIdx.x; px < (unsigned)plane_px; px += gridDim.x * blockDim.x) {
         const int r = (int)(px / (unsigned)p.W);
         const int c = (int)(px - (unsigned)r * (unsigned)p.W);
-        const float* __restrict__ g = p.in + plane * 4 * plane_px;
+        const T* __restrict__ g = p.in + plane * 4 * plane_px;
         int tr[kMaxPre], tc[kMaxPre];
         const int nr = preimages(r, p.H, p.pl, p.pr, p.mode, tr);
         const int nc = preimages(c, p.W, p.pl, p.pr, p.mode, tc);
-        float acc = 0.f;
+        T acc = 0;
         for (int a = 0; a < nr; ++a) {
             for (int jh = 0; jh < p.L; ++jh) {
                 const int i = tr[a] + p.pl - p.d * jh;
                 if (i < 0 || i >= p.H) continue;
-                float s_lo = 0.f, s_hi = 0.f;   // sums over the W taps of (h_lo-weighted, h_hi-weighted) band gradients
+                T s_lo = 0, s_hi = 0;   // sums over the W taps of (h_lo-weighted, h_hi-weighted) band gradients
                 for (int b = 0; b < nc; ++b) {
                     for (int jw = 0; jw < p.L; ++jw) {
                         const int k = tc[b] + p.pl - p.d * jw;
                         if (k < 0 || k >= p.W) continue;
-                        const float* q = g + (size_t)i * p.W + k;
-                        const float gll = __ldg(q), glh = __ldg(q + plane_px), ghl = __ldg(q + 2 * plane_px),
+                        const T* q = g + (size_t)i * p.W + k;
+                        const T gll = __ldg(q), glh = __ldg(q + plane_px), ghl = __ldg(q + 2 * plane_px),
                                     ghh = __ldg(q + 3 * plane_px);
-                        s_lo = fmaf(p.w_lo[jw], gll, s_lo);
-                        s_lo = fmaf(p.w_hi[jw], ghl, s_lo);
-                        s_hi = fmaf(p.w_lo[jw], glh, s_hi);
-                        s_hi = fmaf(p.w_hi[jw], ghh, s_hi);
+                        s_lo = fma(p.w_lo[jw], gll, s_lo);
+                        s_lo = fma(p.w_hi[jw], ghl, s_lo);
+                        s_hi = fma(p.w_lo[jw], glh, s_hi);
+                        s_hi = fma(p.w_hi[jw], ghh, s_hi);
                     }
                 }
-                acc = fmaf(p.h_lo[jh], s_lo, acc);
-                acc = fmaf(p.h_hi[jh], s_hi, acc);
+                acc = fma(p.h_lo[jh], s_lo, acc);
+                acc = fma(p.h_hi[jh], s_hi, acc);
             }
         }
         p.out[plane * plane_px + px] = acc;
@@ -148,8 +152,9 @@ static dim3 swt_grid(int planes, size_t plane_px) {
     return dim3(gx < 1 ? 1 : gx, gy, 1);
 }
 
-static int swt_fill(SwtParams& p, int planes, int H, int W, const float* w_lo, const float* w_hi, const float* h_lo,
-                    const float* h_hi, int L, int dilation, int mode) {
+template <typename T>
+static int swt_fill(SwtParams<T>& p, int planes, int H, int W, const T* w_lo, const T* w_hi, const T* h_lo,
+                    const T* h_hi, int L, int dilation, int mode) {
     if (!w_lo || !w_hi || !h_lo || !h_hi) return B200W_ERR_NULL_POINTER;
     if (!(mode == B200W_MODE_ZERO || mode == B200W_MODE_SYMMETRIC || mode == B200W_MODE_REFLECT ||
           mode == B200W_MODE_PERIODIC))
@@ -172,6 +177,29 @@ static int swt_fill(SwtParams& p, int planes, int H, int W, const float* w_lo, c
     return B200W_OK;
 }
 
+// the fp32 and fp64 entry points share their checks (same codes, same order) and their launch
+template <typename T>
+static int swt2d_run(bool fwd, const T* in, int planes, int H, int W, const T* w_lo, const T* w_hi, const T* h_lo,
+                     const T* h_hi, int L, int dilation, int mode, T* out, void* stream) {
+    if (!in || !out) return B200W_ERR_NULL_POINTER;
+    SwtParams<T> p = {};
+    const int rc = swt_fill(p, planes, H, W, w_lo, w_hi, h_lo, h_hi, L, dilation, mode);
+    if (rc) return rc;
+    p.in = in;
+    p.out = out;
+    const dim3 grid = swt_grid(planes, (size_t)H * W);
+    const bool f64 = sizeof(T) == 8;
+    if (fwd) {
+        swt2d_fwd_kernel<T><<<grid, kThreads, 0, (cudaStream_t)stream>>>(p);
+        note_launch(f64 ? "swt2d_fwd_kernel<double>" : "swt2d_fwd_kernel");
+    } else {
+        swt2d_bwd_kernel<T><<<grid, kThreads, 0, (cudaStream_t)stream>>>(p);
+        note_launch(f64 ? "swt2d_bwd_kernel<double>" : "swt2d_bwd_kernel");
+    }
+    const cudaError_t e = cudaGetLastError();
+    return e == cudaSuccess ? B200W_OK : set_last_cuda_error(e);
+}
+
 }  // namespace b200w
 
 using namespace b200w;
@@ -179,29 +207,23 @@ using namespace b200w;
 extern "C" int b200w_swt2d_fwd_f32(const float* x, int planes, int H, int W, const float* w_lo, const float* w_hi,
                                    const float* h_lo, const float* h_hi, int L, int dilation, int mode, float* y,
                                    void* stream) {
-    if (!x || !y) return B200W_ERR_NULL_POINTER;
-    SwtParams p = {};
-    const int rc = swt_fill(p, planes, H, W, w_lo, w_hi, h_lo, h_hi, L, dilation, mode);
-    if (rc) return rc;
-    p.in = x;
-    p.out = y;
-    swt2d_fwd_kernel<<<swt_grid(planes, (size_t)H * W), kThreads, 0, (cudaStream_t)stream>>>(p);
-    note_launch("swt2d_fwd_kernel");
-    const cudaError_t e = cudaGetLastError();
-    return e == cudaSuccess ? B200W_OK : set_last_cuda_error(e);
+    return swt2d_run(true, x, planes, H, W, w_lo, w_hi, h_lo, h_hi, L, dilation, mode, y, stream);
 }
 
 extern "C" int b200w_swt2d_bwd_f32(const float* dy, int planes, int H, int W, const float* w_lo, const float* w_hi,
                                    const float* h_lo, const float* h_hi, int L, int dilation, int mode, float* dx,
                                    void* stream) {
-    if (!dy || !dx) return B200W_ERR_NULL_POINTER;
-    SwtParams p = {};
-    const int rc = swt_fill(p, planes, H, W, w_lo, w_hi, h_lo, h_hi, L, dilation, mode);
-    if (rc) return rc;
-    p.in = dy;
-    p.out = dx;
-    swt2d_bwd_kernel<<<swt_grid(planes, (size_t)H * W), kThreads, 0, (cudaStream_t)stream>>>(p);
-    note_launch("swt2d_bwd_kernel");
-    const cudaError_t e = cudaGetLastError();
-    return e == cudaSuccess ? B200W_OK : set_last_cuda_error(e);
+    return swt2d_run(false, dy, planes, H, W, w_lo, w_hi, h_lo, h_hi, L, dilation, mode, dx, stream);
+}
+
+extern "C" int b200w_swt2d_fwd_f64(const double* x, int planes, int H, int W, const double* w_lo, const double* w_hi,
+                                   const double* h_lo, const double* h_hi, int L, int dilation, int mode, double* y,
+                                   void* stream) {
+    return swt2d_run(true, x, planes, H, W, w_lo, w_hi, h_lo, h_hi, L, dilation, mode, y, stream);
+}
+
+extern "C" int b200w_swt2d_bwd_f64(const double* dy, int planes, int H, int W, const double* w_lo, const double* w_hi,
+                                   const double* h_lo, const double* h_hi, int L, int dilation, int mode, double* dx,
+                                   void* stream) {
+    return swt2d_run(false, dy, planes, H, W, w_lo, w_hi, h_lo, h_hi, L, dilation, mode, dx, stream);
 }

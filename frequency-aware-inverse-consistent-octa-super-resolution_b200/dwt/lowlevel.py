@@ -63,6 +63,20 @@ def host_taps(f):
     return tuple(float(v) for v in np.asarray(f, dtype=np.float64).ravel())
 
 
+def _is_f64(x, filt):
+    """Double inputs are served when the module's filters are double too (built under
+    ``torch.set_default_dtype(torch.float64)``, as the reference requires: with fp32 filters its conv raises)."""
+    if x.dtype != torch.float64:
+        if x.dtype == torch.float32 and filt.dtype == torch.float64:
+            raise RuntimeError("expected scalar type Double but found Float: the module holds float64 filters (built "
+                               "under torch.set_default_dtype(torch.float64)); pass double inputs, as with the reference")
+        return False
+    if filt.dtype != torch.float64:
+        raise RuntimeError("expected scalar type Float but found Double: the module holds float32 filters; build it "
+                           "under torch.set_default_dtype(torch.float64) for double inputs (as with the reference)")
+    return True
+
+
 def _as_taps(f, reverse):
     """Non-tensor filters are converted like afb1d/sfb1d do (lowlevel.py:120-125, 232-237)."""
     if isinstance(f, torch.Tensor):
@@ -107,7 +121,8 @@ class AFB1D(object):
     @staticmethod
     def apply(x, h0, h1, mode):
         int_to_mode(mode)
-        return ops.afb1d(x, _as_taps(h0, True), _as_taps(h1, True), int(mode))
+        op = ops64.afb1d if x.dtype == torch.float64 else ops.afb1d
+        return op(x, _as_taps(h0, True), _as_taps(h1, True), int(mode))
 
 
 class SFB1D(object):
@@ -117,7 +132,8 @@ class SFB1D(object):
     @staticmethod
     def apply(low, high, g0, g1, mode):
         int_to_mode(mode)
-        return ops.sfb1d(low, high, _as_taps(g0, False), _as_taps(g1, False), int(mode), -1)
+        op = ops64.sfb1d if low.dtype == torch.float64 else ops.sfb1d
+        return op(low, high, _as_taps(g0, False), _as_taps(g1, False), int(mode), -1)
 
 
 def afb2d_atrous(x, filts, mode="periodization", dilation=1):
@@ -133,8 +149,9 @@ def afb2d_atrous(x, filts, mode="periodization", dilation=1):
     h0_col, h1_col, h0_row, h1_row = filts
     if mode in ("per", "periodization") or mode not in _MODES:
         raise ValueError("Unkown pad type: {}".format(mode))
-    return ops.swt2d(x, _as_taps(h0_row, True), _as_taps(h1_row, True), _as_taps(h0_col, True), _as_taps(h1_col, True),
-                     mode_to_int(mode), int(dilation))
+    op = ops64.swt2d if x.dtype == torch.float64 else ops.swt2d
+    return op(x, _as_taps(h0_row, True), _as_taps(h1_row, True), _as_taps(h0_col, True), _as_taps(h1_col, True),
+              mode_to_int(mode), int(dilation))
 
 
 def _four_filters(filts, prep, device=None):

@@ -35,6 +35,7 @@ class DWT1DForward(nn.Module):
         highs = []
         x0 = x
         mode = lowlevel.mode_to_int(self.mode)
+        lowlevel._is_f64(x, self.h0)   # double input needs double filters and vice versa
         for _ in range(self.J):
             x0, x1 = lowlevel.AFB1D.apply(x0, self.h0, self.h1, mode)
             highs.append(x1)
@@ -56,6 +57,7 @@ class DWT1DInverse(nn.Module):
         x0, highs = coeffs
         assert x0.ndim == 3, "Can only handle 3d inputs (N, C, L)"
         mode = lowlevel.mode_to_int(self.mode)
+        lowlevel._is_f64(x0, self.g0)
         for x1 in highs[::-1]:
             # 'unpad' (transform1d.py:110-112) as a view: the kernel takes the row stride
             if x1 is not None and x0.shape[-1] > x1.shape[-1]:

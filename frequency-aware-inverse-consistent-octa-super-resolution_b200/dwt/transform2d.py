@@ -6,7 +6,6 @@ Same constructor arguments and defaults, same registered buffer names and shapes
 stay loadable, same ``(yl, [yh_1 (finest) .. yh_J])`` output structure
 (``pw/dwt/transform2d.py:7-148``).  Every level is one fused sm_100a kernel.
 """
-import torch
 import torch.nn as nn
 
 from . import lowlevel
@@ -26,20 +25,6 @@ def _filters_from(wave, attrs):
     if len(wave) == 4:
         return wave[0], wave[1], wave[2], wave[3]
     raise ValueError("wave must be a name, a Wavelet, or a tuple of 2 or 4 filters")
-
-
-def _is_f64(x, filt):
-    """Double inputs are served when the module's filters are double too (built under
-    ``torch.set_default_dtype(torch.float64)``, as the reference requires: with fp32 filters its conv raises)."""
-    if x.dtype != torch.float64:
-        if x.dtype == torch.float32 and filt.dtype == torch.float64:
-            raise RuntimeError("expected scalar type Double but found Float: the module holds float64 filters (built "
-                               "under torch.set_default_dtype(torch.float64)); pass double inputs, as with the reference")
-        return False
-    if filt.dtype != torch.float64:
-        raise RuntimeError("expected scalar type Float but found Double: the module holds float32 filters; build it "
-                           "under torch.set_default_dtype(torch.float64) for double inputs (as with the reference)")
-    return True
 
 
 class DWTForward(nn.Module):
@@ -71,7 +56,7 @@ class DWTForward(nn.Module):
         yh = []
         ll = x
         J = int(self.J)
-        if _is_f64(x, self.h0_col):   # the reference's double mode: level by level through the fp64 kernels
+        if lowlevel._is_f64(x, self.h0_col):   # the reference's double mode: level by level through the fp64 kernels
             for _ in range(J):
                 ll, high = ops64.afb2d(ll, taps[0], taps[1], taps[2], taps[3], mode)
                 yh.append(high)
@@ -103,7 +88,7 @@ class DWTInverse(nn.Module):
         taps = [lowlevel.host_taps(f) for f in (self.g0_col, self.g1_col, self.g0_row, self.g1_row)]
         yh = list(yh)
         ll = yl
-        if _is_f64(yl, self.g0_col):   # double mode: pw/dwt/transform2d.py:134-148 level by level
+        if lowlevel._is_f64(yl, self.g0_col):   # double mode: pw/dwt/transform2d.py:134-148 level by level
             for h in yh[::-1]:
                 if h is not None:
                     if ll.shape[-2] > h.shape[-2]:
@@ -148,6 +133,7 @@ class SWTForward(nn.Module):
         ll = x
         coeffs = []
         filts = (self.h0_col, self.h1_col, self.h0_row, self.h1_row)
+        lowlevel._is_f64(x, self.h0_col)   # double input needs double filters and vice versa
         for j in range(self.J):
             y = lowlevel.afb2d_atrous(ll, filts, self.mode, 2 ** j)
             coeffs.append(y)

@@ -4,6 +4,8 @@
 ``TVLoss_weight * 2 * (h_tv / count_h + w_tv / count_w) / batch_size``.  The reference slices ``x`` four times,
 subtracts, squares and reduces (about ten elementwise passes and as many again in autograd's backward); here the two
 sums come out of one pass over ``x`` (``b200w_tv_fwd_f32``) and the gradient out of one more (``b200w_tv_bwd_f32``).
+Double images run through the same kernels instantiated for double (``b200w_tv_fwd_f64`` / ``b200w_tv_bwd_f64``), as
+the reference computes in the images' dtype.
 
 ``phase_consistency_loss`` -- drop-in for ``model.py:36-58`` (constructed at ``train.py:94``): minus the cosine
 similarity of the masked log-amplitude spectra of ``x[0]`` and ``y[0]``.  The reference rebuilds the rows x cols mask
@@ -19,7 +21,7 @@ import torch
 from torch.autograd.function import once_differentiable
 import torch.nn as nn
 
-from . import _cabi
+from . import _cabi, ops64
 
 _LIB = torch.library.Library("b200wave_losses", "DEF")
 _LIB.define("tv_sums(Tensor x) -> Tensor")
@@ -147,8 +149,10 @@ class _TV(torch.autograd.Function):
         n, c, h, w = x.shape
         count_h = c * (h - 1) * w          # model.py:26-27 via _tensor_size
         count_w = c * h * (w - 1)
-        sums = torch.ops.b200wave_losses.tv_sums(x)
+        f64 = x.dtype == torch.float64
+        sums = ops64.tv_sums(x) if f64 else torch.ops.b200wave_losses.tv_sums(x)
         ctx.save_for_backward(x)
+        ctx.f64 = f64
         ctx.scales = (weight, n, count_h, count_w)
         # the same arithmetic as model.py:30 (a zero count divides by zero exactly as the reference does)
         return weight * 2 * (sums[0] / count_h + sums[1] / count_w) / n
@@ -160,7 +164,8 @@ class _TV(torch.autograd.Function):
         weight, n, count_h, count_w = ctx.scales
         ch = weight * 2.0 / (n * count_h) if count_h else float("nan")
         cw = weight * 2.0 / (n * count_w) if count_w else float("nan")
-        return torch.ops.b200wave_losses.tv_grad(x, g, ch, cw), None
+        grad = ops64.tv_grad if ctx.f64 else torch.ops.b200wave_losses.tv_grad
+        return grad(x, g, ch, cw), None
 
 
 class TVLoss(nn.Module):

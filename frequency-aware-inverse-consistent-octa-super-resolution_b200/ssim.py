@@ -5,12 +5,18 @@
 signatures (``ssim.py:39-73``); ``gaussian`` / ``create_window`` build the same
 fp32 window (``ssim.py:7-15``).  The five blurs, the SSIM map, its reduction
 and the backward run in two fused sm_100a kernels (``csrc/ssim.cu``).
+
+Double images run through the fp64 kernels (``csrc/ssim_f64.cu``), which apply
+the dense 2-D window the reference applies in double: built in the default
+dtype current when it is (re)built, rounded with ``.float()``, cast to the
+images' dtype (``ssim.py:7-15, 50-73``).
 """
 from math import exp
 
 import torch
 
-from . import ops
+from . import ops, ops64
+from .dwt.lowlevel import host_taps
 
 
 def gaussian(window_size, sigma):
@@ -48,23 +54,56 @@ def _win_taps(window_size):
     return taps
 
 
+def _reference_window(window_size, channel):
+    """The window as ssim.py:7-15 builds it: 1-D Gaussian and outer product in the CURRENT default dtype (the
+    reference's ``torch.Tensor([...])``), rounded with ``.float()``.  Under a float64 default it is not the outer
+    product of an fp32 Gaussian, and not separable."""
+    dt = torch.get_default_dtype()
+    gauss = torch.tensor([exp(-(x - window_size // 2) ** 2 / float(2 * 1.5 ** 2)) for x in range(window_size)],
+                         dtype=dt)
+    w1 = (gauss / gauss.sum()).unsqueeze(1)
+    w2 = w1.mm(w1.t()).float().unsqueeze(0).unsqueeze(0)
+    return w2.expand(channel, 1, window_size, window_size).contiguous()
+
+
+_win2d_cache = {}
+
+
+def _win2d_taps(window_size):
+    """ssim() rebuilds the window on every call (ssim.py:65-73): the same taps, cached by the default dtype."""
+    _check_window(window_size)
+    key = (window_size, torch.get_default_dtype())
+    taps = _win2d_cache.get(key)
+    if taps is None:
+        taps = tuple(float(v) for v in _reference_window(window_size, 1).double().reshape(-1).tolist())
+        _win2d_cache[key] = taps
+    return taps
+
+
 def _ssim(img1, img2, window, window_size, channel, size_average=True):
-    """ssim.py:17-37.  ``window`` is accepted for signature compatibility; the kernel applies the
-    separable form of the same Gaussian (the 2-D window is its outer product)."""
+    """ssim.py:17-37.  For fp32 images ``window`` is accepted for signature compatibility; the kernel applies the
+    separable form of the same Gaussian (the 2-D window is its outer product).  For double images the kernel applies
+    ``window`` tap by tap (``None``: the window ``ssim()`` builds)."""
     if img1.dim() != 4 or img1.shape != img2.shape:
         raise RuntimeError("ssim expects two (N, C, H, W) tensors of equal shape, got %s and %s"
                            % (tuple(img1.shape), tuple(img2.shape)))
-    win = _win_taps(window_size)
+    if img1.dtype == torch.float64:
+        fwd = ops64.ssim_fwd
+        ws2 = window_size * window_size
+        win = _win2d_taps(window_size) if window is None else host_taps(window)[:ws2]
+    else:
+        fwd = ops.ssim_fwd
+        win = _win_taps(window_size)
     grad = torch.is_grad_enabled()
     need1 = grad and img1.requires_grad
     need2 = grad and img2.requires_grad
     if need2 and not need1:
         # SSIM is symmetric in its arguments: put the tensor that needs the gradient first so the
         # forward stores 3 derivative maps instead of 4
-        val, _ = ops.ssim_fwd(img2, img1, win, bool(size_average), 3)
+        val, _ = fwd(img2, img1, win, bool(size_average), 3)
         return val
     n_maps = 4 if need2 else (3 if need1 else 0)
-    val, _ = ops.ssim_fwd(img1, img2, win, bool(size_average), n_maps)
+    val, _ = fwd(img1, img2, win, bool(size_average), n_maps)
     return val
 
 
@@ -80,8 +119,9 @@ class SSIM(torch.nn.Module):
     def forward(self, img1, img2):
         channel = img1.size(1)
         if channel != self.channel or self.window.dtype != img1.dtype or self.window.device != img1.device:
-            # kept as a plain attribute, lazily re-created like ssim.py:50-60
-            self.window = create_window(self.window_size, channel).to(device=img1.device, dtype=img1.dtype)
+            # kept as a plain attribute, lazily re-created like ssim.py:50-60; in double the kernel applies these taps
+            build = _reference_window if img1.dtype == torch.float64 else create_window
+            self.window = build(self.window_size, channel).to(device=img1.device, dtype=img1.dtype)
             self.channel = channel
         return _ssim(img1, img2, self.window, self.window_size, channel, self.size_average)
 

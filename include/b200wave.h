@@ -26,6 +26,8 @@
  *   b200w_swt2d_fwd_f32 / b200w_swt2d_bwd_f32     pw/dwt/lowlevel.py:175-223, 475-521  afb2d_atrous / SWTForward (8f row 3)
  *   b200w_tv_fwd_f32 / b200w_tv_bwd_f32           model.py:17-33  TVLoss (SURVEY.md 8f row 4)
  *   b200w_phase_sums_c64 / b200w_phase_grad_c64   model.py:36-58  phase_consistency_loss (SURVEY.md 8f row 4)
+ *   b200w_*_f64         the same bodies on double tensors (the reference's double mode): afb2d / sfb2d, afb1d / sfb1d,
+ *                       swt2d, tv, and ssim (ssim.py:17-37 with the dense window of ssim.py:7-15, see below)
  *
  * Conventions
  *   - every image pointer is DEVICE memory owned by the caller (torch); the library never
@@ -261,6 +263,50 @@ int b200w_swt2d_fwd_f32(const float* x, int planes, int H, int W, const float* w
                         const float* h_lo, const float* h_hi, int L, int dilation, int mode, float* y, void* stream);
 int b200w_swt2d_bwd_f32(const float* dy, int planes, int H, int W, const float* w_lo, const float* w_hi,
                         const float* h_lo, const float* h_hi, int L, int dilation, int mode, float* dx, void* stream);
+
+/*
+ * Double twins of the 1-D, a trous and TV entry points above (the reference's double mode: modules built under
+ * torch.set_default_dtype(torch.float64), or double images for TVLoss): the same arguments, status codes and order of
+ * the checks, on double data with double taps; the kernels are the fp32 ones instantiated for double.
+ * b200w_afb1d_f64 / b200w_sfb1d_f64       pw/dwt/lowlevel.py:368-424, 697-743  AFB1D / SFB1D
+ * b200w_swt2d_fwd_f64 / b200w_swt2d_bwd_f64 pw/dwt/lowlevel.py:175-223, 475-521 afb2d_atrous / SWTForward
+ * b200w_tv_fwd_f64 / b200w_tv_bwd_f64     model.py:17-33  TVLoss; out2, grad_out (device), ch and cw are double, the
+ *   workspace is b200w_tv_workspace_bytes_f64(planes, H) bytes (double partials).
+ */
+int b200w_afb1d_f64(const double* x, int64_t x_rs, int rows, int n, const double* h0, const double* h1, int L, int mode,
+                    double* lo, double* hi, void* stream);
+int b200w_sfb1d_f64(const double* lo, int64_t lo_rs, const double* hi, int rows, int m, const double* g0,
+                    const double* g1, int L, int mode, int out_len, double* y, void* stream);
+int b200w_swt2d_fwd_f64(const double* x, int planes, int H, int W, const double* w_lo, const double* w_hi,
+                        const double* h_lo, const double* h_hi, int L, int dilation, int mode, double* y, void* stream);
+int b200w_swt2d_bwd_f64(const double* dy, int planes, int H, int W, const double* w_lo, const double* w_hi,
+                        const double* h_lo, const double* h_hi, int L, int dilation, int mode, double* dx, void* stream);
+size_t b200w_tv_workspace_bytes_f64(int planes, int H);
+int b200w_tv_fwd_f64(const double* x, int planes, int H, int W, void* workspace, size_t workspace_bytes,
+                     double* out2, void* stream);
+int b200w_tv_bwd_f64(const double* x, const double* grad_out, double ch, double cw, int planes, int H, int W,
+                     double* dx, void* stream);
+
+/*
+ * SSIM in double precision, ssim.py:17-37 on double images (b200w_ssim_fwd_f64) and the closed form of autograd
+ * through it (b200w_ssim_bwd_f64).  The arguments, status codes and order of the checks are those of
+ * b200w_ssim_fwd_f32 / b200w_ssim_bwd_f32 except:
+ *   - win2d: ws x ws HOST doubles, row-major, the DENSE 2-D window.  In double the reference applies the fp32 rounding
+ *     of the outer product of the 1-D Gaussian (ssim.py:11-15: .float(), then type_as), which is not separable; the
+ *     kernels apply the taps they are given.  They are copied into the parameter block.
+ *   - img1, img2, maps, out, grad_out, d1, d2 are double; out is 1 or N doubles.
+ *   - workspace: DEVICE scratch of at least b200w_ssim_workspace_bytes_f64() bytes (double per-CTA partials, reduced
+ *     in a fixed order: bit-reproducible).
+ */
+size_t b200w_ssim_workspace_bytes_f64(int N, int C, int H, int W);
+int b200w_ssim_fwd_f64(const double* img1, const double* img2, int N, int C, int H, int W,
+                       const double* win2d, int ws, int size_average,
+                       int n_maps, double* maps, double* out,
+                       void* workspace, size_t workspace_bytes, void* stream);
+int b200w_ssim_bwd_f64(const double* img1, const double* img2, const double* maps, int n_maps,
+                       const double* grad_out, int N, int C, int H, int W,
+                       const double* win2d, int ws, int size_average,
+                       double* d1, double* d2, void* stream);
 
 /*
  * phase_consistency_loss, model.py:36-58 (constructed at train.py:94), SURVEY.md 8f row 4: minus the cosine
