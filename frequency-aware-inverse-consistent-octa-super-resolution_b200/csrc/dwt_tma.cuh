@@ -41,7 +41,7 @@ struct AfbTmaLevel {
     int h0[kMaxParts], h1[kMaxParts];   // output rows a part stores to global memory (a partition of [0, Ho))
 };
 
-struct AfbTmaParams {
+struct AfbTmaHead {   // everything of the analysis kernel's parameter block but the tables
     CUtensorMap map_full;  // level-0 input (W, H, planes), box {BW, SR, 1}
     CUtensorMap map_row;   // the same tensor, box {BW, 1, 1}: rows the padding mode maps somewhere else
     AfbTmaLevel lv[kMaxLevels];
@@ -55,10 +55,18 @@ struct AfbTmaParams {
     int bar_off, tab_off, zrow_off, ring_off;   // shared-memory layout (bytes from the dynamic base)
     int zrow_floats, tab_ints;
     int smem_bytes;
-    // the row / patch tables of every part, built on the host (part q's tab_ints entries start at q * tab_ints): a CTA
-    // only copies its part's share into shared memory instead of spending ~2 us of set-up on index arithmetic
-    int tab[kAfbTabMax];
 };
+// the row / patch tables of every part, built on the host (part q's tab_ints entries start at q * tab_ints): a CTA
+// only copies its part's share into shared memory instead of spending ~2 us of set-up on index arithmetic.
+// The whole parameter block travels with every launch, and its size shows up between kernels: at cfg2 (1444 table
+// ints) a 10.6 KB block instead of 22.9 KB makes the four-launch step 2.4 us shorter.  So the kernel is built for two
+// table capacities and the launch picks the smaller one the plan fits in.
+template <int N>
+struct AfbTmaParamsN : AfbTmaHead {
+    int tab[N];
+};
+constexpr int kAfbTabSmall = 2048;
+using AfbTmaParams = AfbTmaParamsN<kAfbTabMax>;   // what the plan fills
 static_assert(sizeof(AfbTmaParams) <= 32764, "kernel parameter block (CUDA 12.1+: 32764 bytes)");
 
 // ---- synthesis ---------------------------------------------------------------------------------------------------

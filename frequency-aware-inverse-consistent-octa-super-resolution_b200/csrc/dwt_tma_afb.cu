@@ -245,8 +245,8 @@ __device__ __forceinline__ void afbt_rotate(float2 (&acc)[L / 2][4]) {
     }
 }
 
-template <int L, int OFF>
-__global__ void __launch_bounds__(AfbT<L, OFF>::NT, 1) afb_tma_kernel(const __grid_constant__ AfbTmaParams p) {
+template <int L, int OFF, int NTAB>
+__global__ void __launch_bounds__(AfbT<L, OFF>::NT, 1) afb_tma_kernel(const __grid_constant__ AfbTmaParamsN<NTAB> p) {
     using C = AfbT<L, OFF>;
     constexpr int H2 = C::H2, NE = C::NE, PS = C::PS, SR = C::SR, NT = C::NT, NTC = C::NTC, S = C::S;
     constexpr bool kRotate = C::kRotate;
@@ -261,7 +261,7 @@ __global__ void __launch_bounds__(AfbT<L, OFF>::NT, 1) afb_tma_kernel(const __gr
     pdl_trigger();   // the next kernel in the stream may be scheduled as SMs free up (it waits before touching memory)
     // every 64-byte line of the parameter block is touched by a different thread first: the constant-cache misses of a
     // freshly scheduled CTA then overlap instead of queueing up behind each other in the set-up code below
-    if (tid < (int)((sizeof(AfbTmaParams) - sizeof(int) * kAfbTabMax) / 64)) {
+    if (tid < (int)(sizeof(AfbTmaHead) / 64)) {
         const int v = reinterpret_cast<const int*>(&p)[tid * 16];
         asm volatile("" ::"r"(v));
     }
@@ -840,10 +840,10 @@ static bool afb_tma_plan_t(const AfbParams& p, int sms, bool force, int G_req, i
     return true;
 }
 
-template <int L, int OFF>
-static int launch_afb_tma_t(const AfbTmaParams& tp, cudaStream_t st) {
+template <int L, int OFF, int NTAB>
+static int launch_afb_tma_n(const AfbTmaParamsN<NTAB>& tp, cudaStream_t st) {
     using C = AfbT<L, OFF>;
-    if (const cudaError_t e = allow_max_dyn_smem<afb_tma_kernel<L, OFF>>()) return set_last_cuda_error(e);
+    if (const cudaError_t e = allow_max_dyn_smem<afb_tma_kernel<L, OFF, NTAB>>()) return set_last_cuda_error(e);
 #ifdef B200W_BOUNDS
     {
         BoundsList b;
@@ -855,11 +855,23 @@ static int launch_afb_tma_t(const AfbTmaParams& tp, cudaStream_t st) {
         bounds_set(b, st);
     }
 #endif
-    const cudaError_t le = launch_pdl(afb_tma_kernel<L, OFF>, (unsigned)(tp.planes * tp.parts), C::NT, (size_t)tp.smem_bytes,
-                                      st, tp);
+    const cudaError_t le = launch_pdl(afb_tma_kernel<L, OFF, NTAB>, (unsigned)(tp.planes * tp.parts), C::NT,
+                                      (size_t)tp.smem_bytes, st, tp);
     note_launch("afb_tma_kernel");
     const cudaError_t e = le != cudaSuccess ? le : cudaGetLastError();
     return e == cudaSuccess ? B200W_OK : set_last_cuda_error(e);
+}
+
+// the smaller parameter block when the tables fit in it (see AfbTmaParamsN)
+template <int L, int OFF>
+static int launch_afb_tma_t(const AfbTmaParams& tp, cudaStream_t st) {
+    const int n = tp.tab_ints * tp.parts;
+    if (n > kAfbTabSmall) return launch_afb_tma_n<L, OFF, kAfbTabMax>(tp, st);
+    AfbTmaParamsN<kAfbTabSmall> sp;
+    static_cast<AfbTmaHead&>(sp) = tp;
+    std::copy(tp.tab, tp.tab + n, sp.tab);
+    std::fill(sp.tab + n, sp.tab + kAfbTabSmall, 0);
+    return launch_afb_tma_n<L, OFF, kAfbTabSmall>(sp, st);
 }
 
 bool afb_tma_plan(const AfbParams& p, int L, int sms, bool force, int G, int D, bool noboxes, AfbTmaParams& tp) {
