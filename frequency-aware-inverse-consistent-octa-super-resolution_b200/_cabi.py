@@ -91,6 +91,11 @@ SYMBOLS = {
     "b200w_ssim_workspace_bytes_f64": (_sz, [_i, _i, _i, _i]),
     "b200w_ssim_fwd_f64": (_i, [_vp, _vp, _i, _i, _i, _i, _c_double_p, _i, _i, _i, _vp, _vp, _vp, _sz, _vp]),
     "b200w_ssim_bwd_f64": (_i, [_vp, _vp, _vp, _i, _vp, _i, _i, _i, _i, _c_double_p, _i, _i, _vp, _vp, _vp]),
+    "b200w_afb2d_ex_f64": (_i, [_vp, _i64, _i64, _i, _i, _i, _c_double_p, _c_double_p, _i, _c_double_p, _c_double_p, _i,
+                                _i, _vp, _vp, ctypes.c_double, ctypes.c_double, _vp]),
+    "b200w_freq_mask_c128": (_i, [_vp, _i, _i, _i, ctypes.c_double, _i, _vp]),
+    "b200w_abs_sign_f64": (_i, [_vp, _vp, _sz, ctypes.c_double, _vp]),
+    "b200w_sign_mul_f64": (_i, [_vp, _vp, _vp, _sz, ctypes.c_double, _vp]),
 }
 
 _lock = threading.Lock()

@@ -68,12 +68,11 @@ def patch_model(model_module):
     discriminators' constructors, state dicts and ``forward`` are untouched.  ``model.TVLoss`` and
     ``model.phase_consistency_loss`` (``model.py:17-58``) are replaced by the fused versions in ``b200wave.losses``."""
     from b200wave import fsd
-    from b200wave.dwt import lowlevel
 
     def make(variant):
         def filter_wavelet(self, x, norm=True):
             d = self.DWT2
-            taps = tuple(lowlevel.host_taps(f) for f in (d.h0_col, d.h1_col, d.h0_row, d.h1_row))
+            taps = fsd.module_taps(x, (d.h0_col, d.h1_col, d.h0_row, d.h1_row))
             return fsd.filter_wavelet(x, self.cs, norm, variant, taps, d.mode)
         return filter_wavelet
 

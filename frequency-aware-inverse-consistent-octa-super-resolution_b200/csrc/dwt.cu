@@ -861,6 +861,31 @@ static int run_sfb_chain(const float* yl, int64_t yl_ps, int64_t yl_rs, const fl
     return B200W_OK;
 }
 
+// one fp64 analysis level through the direct kernel; the caller has validated the arguments and set d.t, d.offH, d.offW,
+// d.Ho and d.Wo
+static int launch_afb2d_f64(AfbDirectParams<double>& d, const double* x, int64_t x_ps, int64_t x_rs, int planes, int H,
+                            int W, int Lw, int Lh, int mode, double* low, double* highs, double hi_scale,
+                            double hi_shift, cudaStream_t st) {
+    d.x = x;
+    d.x_ps = x_ps;
+    d.x_rs = x_rs;
+    d.low = low;
+    d.low_rs = d.Wo;
+    d.low_ps = (long long)d.Ho * d.Wo;
+    d.highs = highs;
+    d.H = d.Hreal = H;
+    d.W = d.Wreal = W;
+    d.st_low = low != nullptr;
+    d.st_hi = highs != nullptr;
+    d.hi_scale = hi_scale;
+    d.hi_shift = hi_shift;
+    d.planes = planes;
+    d.mode = mode;
+    d.Lw = Lw;
+    d.Lh = Lh;
+    return launch_direct(afb2d_direct_kernel<double>, d, (size_t)planes * d.Ho * d.Wo, "afb2d_f64_kernel", st);
+}
+
 }  // namespace b200w
 
 using namespace b200w;
@@ -946,24 +971,24 @@ extern "C" int b200w_afb2d_f64(const double* x, int64_t x_ps, int64_t x_rs, int 
     d.Ho = coeff_len(H, Lh, mode);
     d.Wo = coeff_len(W, Lw, mode);
     if (d.Ho < 1 || d.Wo < 1 || (long long)d.Ho * d.Wo > 0x7fffffffLL) return B200W_ERR_BAD_SHAPE;
-    d.x = x;
-    d.x_ps = x_ps;
-    d.x_rs = x_rs;
-    d.low = low;
-    d.low_rs = d.Wo;
-    d.low_ps = (long long)d.Ho * d.Wo;
-    d.highs = highs;
-    d.H = d.Hreal = H;
-    d.W = d.Wreal = W;
-    d.st_low = d.st_hi = 1;
-    d.hi_scale = 1.0;
-    d.hi_shift = 0.0;
-    d.planes = planes;
-    d.mode = mode;
-    d.Lw = Lw;
-    d.Lh = Lh;
-    return launch_direct(afb2d_direct_kernel<double>, d, (size_t)planes * d.Ho * d.Wo, "afb2d_f64_kernel",
-                         (cudaStream_t)stream);
+    return launch_afb2d_f64(d, x, x_ps, x_rs, planes, H, W, Lw, Lh, mode, low, highs, 1.0, 0.0, (cudaStream_t)stream);
+}
+
+// FS_Discriminator.filter_wavelet in double: the checks of b200w_afb2d_ex_f32, in its order, then the direct kernel with
+// the same store epilogue (a NULL output is not written; detail bands stored as hi_scale * v + hi_shift).
+extern "C" int b200w_afb2d_ex_f64(const double* x, int64_t x_ps, int64_t x_rs, int planes, int H, int W,
+                                  const double* w_lo, const double* w_hi, int Lw, const double* h_lo, const double* h_hi,
+                                  int Lh, int mode, double* low, double* highs, double hi_scale, double hi_shift,
+                                  void* stream) {
+    if (!mode_supported(mode)) return B200W_ERR_BAD_MODE;
+    if (!x || (!low && !highs)) return B200W_ERR_NULL_POINTER;
+    if (planes < 1 || H < 1 || W < 1) return B200W_ERR_BAD_SHAPE;
+    AfbDirectParams<double> d = {};
+    int rc = fill_taps(d.t, w_lo, w_hi, Lw, h_lo, h_hi, Lh);
+    if (rc || (rc = afb_dims(H, W, Lw, Lh, mode, 1, nullptr, &d.Ho, &d.Wo))) return rc;
+    if ((rc = analysis_offset(W, Lw, mode, &d.offW)) || (rc = analysis_offset(H, Lh, mode, &d.offH))) return rc;
+    return launch_afb2d_f64(d, x, x_ps, x_rs, planes, H, W, Lw, Lh, mode, low, highs, hi_scale, hi_shift,
+                            (cudaStream_t)stream);
 }
 
 extern "C" int b200w_sfb2d_f64(const double* low, int64_t low_ps, int64_t low_rs, const double* highs, int planes, int h,

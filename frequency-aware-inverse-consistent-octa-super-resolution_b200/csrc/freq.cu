@@ -11,15 +11,32 @@
 //   freq_mask   in place on the (planes, rows, cols/2+1) complex half spectrum: 16 B of traffic per bin
 //   abs_sign    y = sign * |x| (low_pass returns -|.|, utils.py:117), optionally keeping sgn(x) for backward
 //   sign_mul    backward of abs_sign: g * sign * sgn(x)
+// The three are instantiated for float and, for the reference's double mode (complex128 spectra), for double.
+#include <type_traits>
+
 #include "common.cuh"
 
 namespace b200w {
 
-// flat grid-stride loop over the bins of all planes; the mask costs one expf and two small integer divisions per
+// The mask of one bin.  fp32: the fast exponential with 0.5 / r^2 folded into one factor.  fp64 (the reference's
+// double mode): the mask is what utils.py stores -- built in numpy float64 as exp(-0.5 d^2 / r^2), 1 - that for the
+// high pass, then rounded once to fp32 by torch.from_numpy(mask).float() -- and the complex128 spectrum is multiplied
+// by that fp32 value in double.  `rp` is 0.5 / r^2 in fp32 and r^2 in fp64 (numpy divides by r^2).
+__device__ __forceinline__ float gauss_mask(int du, int dv, float rp, int highpass) {
+    const float m = __expf(-(float)(du * du + dv * dv) * rp);
+    return highpass ? 1.f - m : m;
+}
+__device__ __forceinline__ double gauss_mask(int du, int dv, double rp, int highpass) {
+    const double e = exp(-0.5 * ((double)du * du + (double)dv * dv) / rp);
+    return (double)(float)(highpass ? 1.0 - e : e);
+}
+
+// flat grid-stride loop over the bins of all planes; the mask costs one exp and two small integer divisions per
 // bin (an (u, v)-outer / plane-inner variant that evaluates the mask once per bin was slower: its plane-strided
-// accesses and 129-bin rows used the memory system worse -- profiles/r01_notes.md)
-__global__ void __launch_bounds__(256) freq_mask_kernel(float2* __restrict__ spec, int planes, int rows, int cols, int wh,
-                                                        float inv2r2, int highpass) {
+// accesses and 129-bin rows used the memory system worse -- profiles/r01_notes.md).  Z = float2 / double2 bins.
+template <class Z, class S>
+__global__ void __launch_bounds__(256) freq_mask_kernel(Z* __restrict__ spec, int planes, int rows, int cols, int wh,
+                                                        S rp, int highpass) {
     const unsigned per_plane = (unsigned)rows * (unsigned)wh;
     const size_t total = (size_t)per_plane * planes;
     for (size_t idx = (size_t)blockIdx.x * blockDim.x + threadIdx.x; idx < total; idx += (size_t)gridDim.x * blockDim.x) {
@@ -27,31 +44,52 @@ __global__ void __launch_bounds__(256) freq_mask_kernel(float2* __restrict__ spe
         const int u = (int)(rem / (unsigned)wh), v = (int)(rem - (unsigned)u * (unsigned)wh);
         const int du = u < rows - rows / 2 ? u : u - rows;
         const int dv = v < cols - cols / 2 ? v : v - cols;
-        float m = __expf(-(float)(du * du + dv * dv) * inv2r2);
-        if (highpass) m = 1.f - m;
-        float2 z = spec[idx];
+        const S m = gauss_mask(du, dv, rp, highpass);
+        Z z = spec[idx];
         z.x *= m;
         z.y *= m;
         spec[idx] = z;
     }
 }
 
-__global__ void __launch_bounds__(256) abs_sign_kernel(const float4* __restrict__ x, float4* __restrict__ y, size_t n4,
-                                                       const float* __restrict__ xt, float* __restrict__ yt, size_t n,
-                                                       float sign) {
-    for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < n4; i += (size_t)gridDim.x * blockDim.x) {
-        const float4 a = x[i];
-        y[i] = make_float4(sign * fabsf(a.x), sign * fabsf(a.y), sign * fabsf(a.z), sign * fabsf(a.w));
-    }
+// 16-byte vectors of the abs pass: float4 / double2
+template <class T>
+using Vec16 = std::conditional_t<std::is_same<T, float>::value, float4, double2>;
+__device__ __forceinline__ float4 scaled_abs(float4 a, float s) {
+    return make_float4(s * fabsf(a.x), s * fabsf(a.y), s * fabsf(a.z), s * fabsf(a.w));
+}
+__device__ __forceinline__ double2 scaled_abs(double2 a, double s) { return make_double2(s * fabs(a.x), s * fabs(a.y)); }
+
+template <class T>
+__global__ void __launch_bounds__(256) abs_sign_kernel(const Vec16<T>* __restrict__ x, Vec16<T>* __restrict__ y,
+                                                       size_t nv, const T* __restrict__ xt, T* __restrict__ yt, size_t n,
+                                                       T sign) {
+    for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < nv; i += (size_t)gridDim.x * blockDim.x)
+        y[i] = scaled_abs(x[i], sign);
     if (blockIdx.x == 0)
-        for (size_t i = 4 * n4 + threadIdx.x; i < n; i += blockDim.x) yt[i] = sign * fabsf(xt[i]);
+        for (size_t i = (16 / sizeof(T)) * nv + threadIdx.x; i < n; i += blockDim.x) yt[i] = sign * fabs(xt[i]);
 }
 
-__global__ void __launch_bounds__(256) sign_mul_kernel(const float* __restrict__ g, const float* __restrict__ x,
-                                                       float* __restrict__ out, size_t n, float sign) {
-    for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (size_t)gridDim.x * blockDim.x) {
-        const float v = x[i];
-        out[i] = v > 0.f ? sign * g[i] : (v < 0.f ? -sign * g[i] : 0.f);
+// fp32 reads scalars; fp64 reads double2 pairs when all three pointers are 16-byte aligned, and the odd last element
+// (or every element of a misaligned call) in the scalar loop
+template <class T>
+__global__ void __launch_bounds__(256) sign_mul_kernel(const T* __restrict__ g, const T* __restrict__ x,
+                                                       T* __restrict__ out, size_t n, T sign) {
+    size_t i0 = 0;
+    if constexpr (std::is_same<T, double>::value) {
+        if ((((uintptr_t)g | (uintptr_t)x | (uintptr_t)out) & 15) == 0) {
+            const size_t n2 = n / 2;
+            for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < n2; i += (size_t)gridDim.x * blockDim.x) {
+                const double2 a = ((const double2*)g)[i], v = ((const double2*)x)[i];
+                ((double2*)out)[i] = make_double2(v.x > 0.0 ? sign * a.x : (v.x < 0.0 ? -sign * a.x : 0.0),
+                                                  v.y > 0.0 ? sign * a.y : (v.y < 0.0 ? -sign * a.y : 0.0));
+            }
+            i0 = 2 * n2;
+        }
+    }
+    for (size_t i = i0 + (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (size_t)gridDim.x * blockDim.x) {
+        const T v = x[i];
+        out[i] = v > T(0) ? sign * g[i] : (v < T(0) ? -sign * g[i] : T(0));
     }
 }
 
@@ -139,42 +177,73 @@ static unsigned pointwise_grid(size_t n) {
     return (unsigned)(g < 1 ? 1 : (g > cap ? cap : g));
 }
 
+// the fp32 and fp64 entry points: the same checks in the same order
+template <class T>
+static int freq_mask_run(void* spec, int planes, int rows, int cols, T radius, int highpass, cudaStream_t st) {
+    constexpr bool f64 = std::is_same<T, double>::value;
+    if (!spec) return B200W_ERR_NULL_POINTER;
+    if (planes < 1 || rows < 1 || cols < 1 || !(radius > T(0))) return B200W_ERR_BAD_SHAPE;
+    const int wh = cols / 2 + 1;
+    if ((long long)rows * wh > 0x7fffffffLL) return B200W_ERR_BAD_SHAPE;
+    const size_t total = (size_t)planes * rows * wh;
+    using Z = std::conditional_t<f64, double2, float2>;
+    freq_mask_kernel<<<pointwise_grid(total), 256, 0, st>>>((Z*)spec, planes, rows, cols, wh,
+                                                            f64 ? radius * radius : T(0.5) / (radius * radius),
+                                                            highpass ? 1 : 0);
+    b200w::note_launch(f64 ? "freq_mask_kernel<double2>" : "freq_mask_kernel");
+    const cudaError_t e = cudaGetLastError();
+    return e == cudaSuccess ? B200W_OK : set_last_cuda_error(e);
+}
+
+template <class T>
+static int abs_sign_run(const T* x, T* y, size_t n, T sign, cudaStream_t st) {
+    if (!x || !y) return B200W_ERR_NULL_POINTER;
+    if (n == 0) return B200W_OK;
+    const bool vec = ((reinterpret_cast<uintptr_t>(x) | reinterpret_cast<uintptr_t>(y)) & 15) == 0;
+    const size_t nv = vec ? n / (16 / sizeof(T)) : 0;
+    abs_sign_kernel<T><<<pointwise_grid(nv ? nv : n), 256, 0, st>>>((const Vec16<T>*)x, (Vec16<T>*)y, nv, x, y, n, sign);
+    b200w::note_launch(sizeof(T) == 8 ? "abs_sign_kernel<double>" : "abs_sign_kernel");
+    const cudaError_t e = cudaGetLastError();
+    return e == cudaSuccess ? B200W_OK : set_last_cuda_error(e);
+}
+
+template <class T>
+static int sign_mul_run(const T* g, const T* x, T* out, size_t n, T sign, cudaStream_t st) {
+    if (!g || !x || !out) return B200W_ERR_NULL_POINTER;
+    if (n == 0) return B200W_OK;
+    sign_mul_kernel<T><<<pointwise_grid(sizeof(T) == 8 ? (n + 1) / 2 : n), 256, 0, st>>>(g, x, out, n, sign);
+    b200w::note_launch(sizeof(T) == 8 ? "sign_mul_kernel<double>" : "sign_mul_kernel");
+    const cudaError_t e = cudaGetLastError();
+    return e == cudaSuccess ? B200W_OK : set_last_cuda_error(e);
+}
+
 }  // namespace b200w
 
 using namespace b200w;
 
 extern "C" int b200w_freq_mask_c64(void* spec, int planes, int rows, int cols, float radius, int highpass, void* stream) {
-    if (!spec) return B200W_ERR_NULL_POINTER;
-    if (planes < 1 || rows < 1 || cols < 1 || !(radius > 0.f)) return B200W_ERR_BAD_SHAPE;
-    const int wh = cols / 2 + 1;
-    if ((long long)rows * wh > 0x7fffffffLL) return B200W_ERR_BAD_SHAPE;
-    const size_t total = (size_t)planes * rows * wh;
-    freq_mask_kernel<<<pointwise_grid(total), 256, 0, (cudaStream_t)stream>>>((float2*)spec, planes, rows, cols, wh,
-                                                                              0.5f / (radius * radius), highpass ? 1 : 0);
-    b200w::note_launch("freq_mask_kernel");
-    const cudaError_t e = cudaGetLastError();
-    return e == cudaSuccess ? B200W_OK : set_last_cuda_error(e);
+    return freq_mask_run(spec, planes, rows, cols, radius, highpass, (cudaStream_t)stream);
 }
 
 extern "C" int b200w_abs_sign_f32(const float* x, float* y, size_t n, float sign, void* stream) {
-    if (!x || !y) return B200W_ERR_NULL_POINTER;
-    if (n == 0) return B200W_OK;
-    const bool vec = ((reinterpret_cast<uintptr_t>(x) | reinterpret_cast<uintptr_t>(y)) & 15) == 0;
-    const size_t n4 = vec ? n / 4 : 0;
-    abs_sign_kernel<<<pointwise_grid(n4 ? n4 : n), 256, 0, (cudaStream_t)stream>>>((const float4*)x, (float4*)y, n4, x, y, n,
-                                                                                  sign);
-    b200w::note_launch("abs_sign_kernel");
-    const cudaError_t e = cudaGetLastError();
-    return e == cudaSuccess ? B200W_OK : set_last_cuda_error(e);
+    return abs_sign_run(x, y, n, sign, (cudaStream_t)stream);
 }
 
 extern "C" int b200w_sign_mul_f32(const float* g, const float* x, float* out, size_t n, float sign, void* stream) {
-    if (!g || !x || !out) return B200W_ERR_NULL_POINTER;
-    if (n == 0) return B200W_OK;
-    sign_mul_kernel<<<pointwise_grid(n), 256, 0, (cudaStream_t)stream>>>(g, x, out, n, sign);
-    b200w::note_launch("sign_mul_kernel");
-    const cudaError_t e = cudaGetLastError();
-    return e == cudaSuccess ? B200W_OK : set_last_cuda_error(e);
+    return sign_mul_run(g, x, out, n, sign, (cudaStream_t)stream);
+}
+
+extern "C" int b200w_freq_mask_c128(void* spec, int planes, int rows, int cols, double radius, int highpass,
+                                    void* stream) {
+    return freq_mask_run(spec, planes, rows, cols, radius, highpass, (cudaStream_t)stream);
+}
+
+extern "C" int b200w_abs_sign_f64(const double* x, double* y, size_t n, double sign, void* stream) {
+    return abs_sign_run(x, y, n, sign, (cudaStream_t)stream);
+}
+
+extern "C" int b200w_sign_mul_f64(const double* g, const double* x, double* out, size_t n, double sign, void* stream) {
+    return sign_mul_run(g, x, out, n, sign, (cudaStream_t)stream);
 }
 
 extern "C" size_t b200w_phase_workspace_bytes(int planes, int rows, int cols) {

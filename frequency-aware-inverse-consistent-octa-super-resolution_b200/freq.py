@@ -10,13 +10,15 @@ the mask is evaluated inside the pointwise kernel (``csrc/freq.cu``) -- no mask 
   ``(1, H, W)``; the result is ``(H, W)``; ``low_pass`` returns ``-|.|`` exactly like ``utils.py:117``).
 * ``gaussian_split(x, radius, highpass, sign)``: the batched form for ``(..., H, W)`` tensors.
 Differentiable: the filter is linear and self-adjoint (real, even mask), ``abs`` back-propagates ``sgn``.
+float32 and float64 images are served; float64 is the reference's double mode (complex128 FFTs, the mask evaluated in
+double and rounded to fp32 as ``torch.from_numpy(mask).float()`` stores it), through the ``ops64`` twins of the ops.
 """
 import ctypes
 
 import torch
 from torch.autograd.function import once_differentiable
 
-from . import _cabi
+from . import _cabi, ops64
 
 _LIB = torch.library.Library("b200wave_freq", "DEF")
 _LIB.define("mask_(Tensor(a!) spec, int rows, int cols, float radius, bool highpass) -> Tensor(a!)")
@@ -85,11 +87,17 @@ for _name in ("mask_", "abs_sign", "sign_mul"):
     _LIB.impl(_name, _cpu_refuse(_name), "CPU")
 
 
+# (mask_, abs_sign, sign_mul) by dtype: fp32 here, float64 / complex128 in ops64 (the reference's double mode)
+_OPS = {torch.float32: (torch.ops.b200wave_freq.mask_, torch.ops.b200wave_freq.abs_sign,
+                        torch.ops.b200wave_freq.sign_mul),
+        torch.float64: (ops64.freq_mask_, ops64.abs_sign, ops64.sign_mul)}
+
+
 def _filter(x, radius, highpass):
     """irfft2(mask * rfft2(x)) over the last two dims (cuFFT + the in-place mask kernel)."""
     rows, cols = x.shape[-2:]
     spec = torch.fft.rfft2(x).contiguous()
-    torch.ops.b200wave_freq.mask_(spec, rows, cols, float(radius), bool(highpass))
+    _OPS[x.dtype][0](spec, rows, cols, float(radius), bool(highpass))
     return torch.fft.irfft2(spec, s=(rows, cols))
 
 
@@ -99,22 +107,23 @@ class _GaussianSplit(torch.autograd.Function):
         y = _filter(x, radius, highpass)
         ctx.save_for_backward(y)
         ctx.args = (radius, highpass, sign)
-        return torch.ops.b200wave_freq.abs_sign(y, float(sign))
+        return _OPS[y.dtype][1](y, float(sign))
 
     @staticmethod
     @once_differentiable   # the backward kernels have no autograd formula of their own: double backward raises
     def backward(ctx, g):
         (y,) = ctx.saved_tensors
         radius, highpass, sign = ctx.args
-        t = torch.ops.b200wave_freq.sign_mul(g, y, float(sign))
+        t = _OPS[y.dtype][2](g, y, float(sign))
         return _filter(t, radius, highpass), None, None, None   # the filter is self-adjoint
 
 
 def gaussian_split(x, radius, highpass, sign=1.0):
-    """``sign * |ifft2(mask_r * fft2(x))|`` over the last two dims of a real fp32 CUDA tensor, batched over the rest."""
+    """``sign * |ifft2(mask_r * fft2(x))|`` over the last two dims of a real fp32 or float64 CUDA tensor, batched over
+    the rest.  float64 follows the reference's double mode: complex128 FFTs, the mask rounded to fp32."""
     if not x.is_cuda:
         raise RuntimeError("b200wave.freq is CUDA-only (sm_100a); there is no CPU fallback -- got a %s tensor" % x.device)
-    if x.dtype != torch.float32:
+    if x.dtype not in _OPS:
         raise RuntimeError("b200wave.freq: expected scalar type Float but found %s" % x.dtype)
     if x.dim() < 2:
         raise ValueError("b200wave.freq expects (..., H, W)")

@@ -13,6 +13,10 @@ stream, CUDA-only, the same backward structure -- on double tensors with double 
   ``tv_sums`` through ``tv_grad`` (once differentiable).
 * ``ssim_fwd`` / ``ssim_bwd`` (``csrc/ssim_f64.cu``): ``win`` is the DENSE ws x ws window, row-major (in double the
   reference's window is the fp32 rounding of an outer product, which is not separable).
+* ``afb2d_select`` (``b200w_afb2d_ex_f64``): the discriminators' ``filter_wavelet`` level (``fsd.py``) on the direct
+  kernel; backward = ``sfb2d`` of ``(dlow, hi_scale * dhighs)``, as ``ops.afb2d_select``.
+* ``freq_mask_`` / ``abs_sign`` / ``sign_mul`` (``csrc/freq.cu``): the pointwise passes of ``freq.gaussian_split`` on
+  complex128 / double tensors; the mask is rounded to fp32 as the reference stores it.
 """
 import torch
 
@@ -33,6 +37,11 @@ _LIB.define("ssim_bwd(Tensor img1, Tensor img2, Tensor maps, Tensor grad_out, fl
             "bool need_d2) -> (Tensor, Tensor)")
 _LIB.define("tv_sums(Tensor x) -> Tensor")
 _LIB.define("tv_grad(Tensor x, Tensor grad_out, float ch, float cw) -> Tensor")
+_LIB.define("afb2d_select(Tensor x, float[] w_lo, float[] w_hi, float[] h_lo, float[] h_hi, int mode, bool want_low, "
+            "bool want_highs, float hi_scale, float hi_shift) -> (Tensor, Tensor)")
+_LIB.define("freq_mask_(Tensor(a!) spec, int rows, int cols, float radius, bool highpass) -> Tensor(a!)")
+_LIB.define("abs_sign(Tensor x, float sign) -> Tensor")
+_LIB.define("sign_mul(Tensor g, Tensor x, float sign) -> Tensor")
 
 
 def _require_cuda_f64(t, name):
@@ -153,6 +162,72 @@ def _sfb2d_backward(ctx, dy):
         if not need_high:
             dhighs = None
     return dlow, dhighs, None, None, None, None, None, None, None
+
+
+# ------------------------------------------------------------------------------------------- afb2d_select
+def _afb2d_select_cuda(x, w_lo, w_hi, h_lo, h_hi, mode, want_low, want_highs, hi_scale, hi_shift):
+    """One analysis level that writes only the sub-bands asked for, the detail bands as hi_scale*v + hi_shift; an
+    output that is not wanted comes back with 0 elements."""
+    _check_mode(mode)
+    _require_cuda_f64(x, "afb2d_select")
+    if x.dim() != 4:
+        raise IndexError("b200wave64::afb2d_select expects a 4-D (N, C, H, W) tensor, got %d-D" % x.dim())
+    if not (want_low or want_highs):
+        raise ValueError("afb2d_select: at least one of the low-pass / detail outputs must be requested")
+    lib = _cabi.load()
+    N, C, H, W = x.shape
+    Lw, Lh = len(w_lo), len(h_lo)
+    if len(w_hi) != Lw or len(h_hi) != Lh:
+        raise RuntimeError("low- and high-pass filters must have the same length along an axis")
+    Ho, Wo = coeff_len(H, Lh, mode), coeff_len(W, Lw, mode)
+    low = torch.empty((N, C, Ho, Wo) if want_low else (0,), device=x.device, dtype=torch.float64)
+    highs = torch.empty((N, C, 3, Ho, Wo) if want_highs else (0,), device=x.device, dtype=torch.float64)
+    if N * C * Ho * Wo == 0:
+        return low, highs
+    xk, ps, rs = _planes_view(x)
+    a = _taps(w_lo, w_hi, h_lo, h_hi)
+    with torch.cuda.device(x.device):
+        rc = lib.b200w_afb2d_ex_f64(xk.data_ptr(), ps, rs, N * C, H, W, a[0], a[1], Lw, a[2], a[3], Lh, int(mode),
+                                    low.data_ptr() if want_low else None, highs.data_ptr() if want_highs else None,
+                                    float(hi_scale), float(hi_shift), _stream())
+    _cabi.check(rc, _mode_name(mode))
+    return low, highs
+
+
+def _afb2d_select_fake(x, w_lo, w_hi, h_lo, h_hi, mode, want_low, want_highs, hi_scale, hi_shift):
+    N, C, H, W = x.shape
+    Ho, Wo = coeff_len(H, len(h_lo), mode), coeff_len(W, len(w_lo), mode)
+    return (x.new_empty((N, C, Ho, Wo) if want_low else (0,)),
+            x.new_empty((N, C, 3, Ho, Wo) if want_highs else (0,)))
+
+
+def _afb2d_select_setup(ctx, inputs, output):
+    x, w_lo, w_hi, h_lo, h_hi, mode, want_low, want_highs, hi_scale, _ = inputs
+    ctx.taps = (w_lo, w_hi, h_lo, h_hi)
+    ctx.mode = mode
+    ctx.in_shape = tuple(x.shape)
+    ctx.want = (want_low, want_highs)
+    ctx.hi_scale = hi_scale
+    ctx.set_materialize_grads(False)
+
+
+def _afb2d_select_backward(ctx, dlow, dhighs):
+    none = (None,) * 10
+    if not ctx.needs_input_grad[0]:
+        return none
+    want_low, want_highs = ctx.want
+    dlow = dlow if want_low else None
+    dhighs = dhighs if want_highs else None
+    if dlow is None and dhighs is None:
+        return none
+    N, C, H, W = ctx.in_shape
+    if dlow is None:
+        dlow = dhighs.new_zeros((N, C) + tuple(dhighs.shape[-2:]))
+    if dhighs is not None and ctx.hi_scale != 1.0:
+        dhighs = dhighs * ctx.hi_scale   # d(hi_scale * v + hi_shift) / dv
+    # AFB2D.backward's pseudo-adjoint (lowlevel.py:356-364); a missing detail gradient is never materialised
+    dx = torch.ops.b200wave64.sfb2d(dlow, dhighs, *ctx.taps, ctx.mode, H, W)
+    return (dx,) + none[1:]
 
 
 # ------------------------------------------------------------------------------------------- 1-D banks
@@ -431,6 +506,52 @@ def _tv_grad_cuda(x, grad_out, ch, cw):
     return dx
 
 
+# ------------------------------------------------------------------------------------------- frequency split
+def _require_freq(t, name, dtype):
+    if not t.is_cuda:
+        raise RuntimeError("b200wave64::%s is CUDA-only (sm_100a); there is no CPU fallback -- got a %s tensor"
+                           % (name, t.device))
+    if t.dtype != dtype:
+        raise RuntimeError("b200wave64::%s: expected %s but found %s" % (name, dtype, t.dtype))
+
+
+def _freq_mask_cuda(spec, rows, cols, radius, highpass):
+    _require_freq(spec, "freq_mask_", torch.complex128)
+    if not spec.is_contiguous() or spec.shape[-2] != rows or spec.shape[-1] != cols // 2 + 1:
+        raise RuntimeError("b200wave64::freq_mask_ expects the contiguous half spectrum (..., %d, %d), got %s"
+                           % (rows, cols // 2 + 1, tuple(spec.shape)))
+    if spec.numel() == 0:
+        return spec
+    planes = spec.numel() // (rows * (cols // 2 + 1))
+    with torch.cuda.device(spec.device):
+        rc = _cabi.load().b200w_freq_mask_c128(spec.data_ptr(), planes, rows, cols, float(radius),
+                                               int(bool(highpass)), _stream())
+    _cabi.check(rc)
+    return spec
+
+
+def _abs_sign_cuda(x, sign):
+    _require_freq(x, "abs_sign", torch.float64)
+    x = x.contiguous()
+    y = torch.empty_like(x)
+    with torch.cuda.device(x.device):
+        rc = _cabi.load().b200w_abs_sign_f64(x.data_ptr(), y.data_ptr(), x.numel(), float(sign), _stream())
+    _cabi.check(rc)
+    return y
+
+
+def _sign_mul_cuda(g, x, sign):
+    _require_freq(g, "sign_mul", torch.float64)
+    _require_freq(x, "sign_mul", torch.float64)
+    g, x = g.contiguous(), x.contiguous()
+    out = torch.empty_like(x)
+    with torch.cuda.device(x.device):
+        rc = _cabi.load().b200w_sign_mul_f64(g.data_ptr(), x.data_ptr(), out.data_ptr(), x.numel(), float(sign),
+                                             _stream())
+    _cabi.check(rc)
+    return out
+
+
 def _cpu_refuse(name):
     def impl(*args, **kwargs):
         raise RuntimeError("b200wave64::%s is CUDA-only (sm_100a): there is no CPU fallback. Move the tensors to "
@@ -448,8 +569,12 @@ _LIB.impl("ssim_fwd", _ssim_fwd_cuda, "CUDA")
 _LIB.impl("ssim_bwd", _ssim_bwd_cuda, "CUDA")
 _LIB.impl("tv_sums", _tv_sums_cuda, "CUDA")
 _LIB.impl("tv_grad", _tv_grad_cuda, "CUDA")
+_LIB.impl("afb2d_select", _afb2d_select_cuda, "CUDA")
+_LIB.impl("freq_mask_", _freq_mask_cuda, "CUDA")
+_LIB.impl("abs_sign", _abs_sign_cuda, "CUDA")
+_LIB.impl("sign_mul", _sign_mul_cuda, "CUDA")
 for _name in ("afb2d", "sfb2d", "afb1d", "sfb1d", "swt2d", "swt2d_adjoint", "ssim_fwd", "ssim_bwd", "tv_sums",
-              "tv_grad"):
+              "tv_grad", "afb2d_select", "freq_mask_", "abs_sign", "sign_mul"):
     _LIB.impl(_name, _cpu_refuse(_name), "CPU")
 torch.library.register_fake("b200wave64::afb2d", _afb2d_fake, lib=_LIB)
 torch.library.register_fake("b200wave64::sfb2d", _sfb2d_fake, lib=_LIB)
@@ -469,6 +594,9 @@ torch.library.register_autograd("b200wave64::afb1d", _afb1d_backward, setup_cont
 torch.library.register_autograd("b200wave64::sfb1d", _sfb1d_backward, setup_context=_sfb1d_setup, lib=_LIB)
 torch.library.register_autograd("b200wave64::swt2d", _swt2d_backward, setup_context=_swt2d_setup, lib=_LIB)
 torch.library.register_autograd("b200wave64::ssim_fwd", _ssim_backward, setup_context=_ssim_setup, lib=_LIB)
+torch.library.register_fake("b200wave64::afb2d_select", _afb2d_select_fake, lib=_LIB)
+torch.library.register_autograd("b200wave64::afb2d_select", _afb2d_select_backward, setup_context=_afb2d_select_setup,
+                                lib=_LIB)
 
 afb2d = torch.ops.b200wave64.afb2d
 sfb2d = torch.ops.b200wave64.sfb2d
@@ -480,3 +608,7 @@ ssim_fwd = torch.ops.b200wave64.ssim_fwd
 ssim_bwd = torch.ops.b200wave64.ssim_bwd
 tv_sums = torch.ops.b200wave64.tv_sums
 tv_grad = torch.ops.b200wave64.tv_grad
+afb2d_select = torch.ops.b200wave64.afb2d_select
+freq_mask_ = torch.ops.b200wave64.freq_mask_
+abs_sign = torch.ops.b200wave64.abs_sign
+sign_mul = torch.ops.b200wave64.sign_mul

@@ -26,8 +26,9 @@
  *   b200w_swt2d_fwd_f32 / b200w_swt2d_bwd_f32     pw/dwt/lowlevel.py:175-223, 475-521  afb2d_atrous / SWTForward (8f row 3)
  *   b200w_tv_fwd_f32 / b200w_tv_bwd_f32           model.py:17-33  TVLoss (SURVEY.md 8f row 4)
  *   b200w_phase_sums_c64 / b200w_phase_grad_c64   model.py:36-58  phase_consistency_loss (SURVEY.md 8f row 4)
- *   b200w_*_f64         the same bodies on double tensors (the reference's double mode): afb2d / sfb2d, afb1d / sfb1d,
- *                       swt2d, tv, and ssim (ssim.py:17-37 with the dense window of ssim.py:7-15, see below)
+ *   b200w_*_f64         the same bodies on double tensors (the reference's double mode): afb2d / sfb2d, afb2d_ex,
+ *                       afb1d / sfb1d, swt2d, tv, abs_sign / sign_mul, and ssim (ssim.py:17-37 with the dense window of
+ *                       ssim.py:7-15, see below); b200w_freq_mask_c128 on complex128 spectra
  *
  * Conventions
  *   - every image pointer is DEVICE memory owned by the caller (torch); the library never
@@ -234,6 +235,23 @@ int b200w_afb2d_f64(const double* x, int64_t x_plane_stride, int64_t x_row_strid
 int b200w_sfb2d_f64(const double* low, int64_t low_plane_stride, int64_t low_row_stride, const double* highs, int planes,
                     int h, int w, const double* w_lo, const double* w_hi, int Lw, const double* h_lo, const double* h_hi,
                     int Lh, int mode, double* y, int out_h, int out_w, void* stream);
+
+/*
+ * Double twins of b200w_afb2d_ex_f32 and of the frequency-split passes (the reference's double mode: discriminators
+ * built under torch.set_default_dtype(torch.float64), double images into utils.high_pass / low_pass): the same
+ * arguments, status codes and order of the checks, on double data.
+ * b200w_afb2d_ex_f64     model.py:166-179, 222-235  filter_wavelet; double taps, hi_scale and hi_shift (direct kernel)
+ * b200w_freq_mask_c128   utils.py:71-91  in place on the complex128 half spectrum.  As in the reference, the mask is
+ *   exp(-0.5 (du^2+dv^2) / radius^2) (1 - that when highpass) evaluated in double and rounded once to float
+ *   (torch.from_numpy(mask).float()); each bin is multiplied by that float value in double.
+ * b200w_abs_sign_f64 / b200w_sign_mul_f64   utils.py:103, 117  y = sign * |x| and its backward, on doubles.
+ */
+int b200w_afb2d_ex_f64(const double* x, int64_t x_plane_stride, int64_t x_row_stride, int planes, int H, int W,
+                       const double* w_lo, const double* w_hi, int Lw, const double* h_lo, const double* h_hi, int Lh,
+                       int mode, double* low, double* highs, double hi_scale, double hi_shift, void* stream);
+int b200w_freq_mask_c128(void* spec, int planes, int rows, int cols, double radius, int highpass, void* stream);
+int b200w_abs_sign_f64(const double* x, double* y, size_t n, double sign, void* stream);
+int b200w_sign_mul_f64(const double* g, const double* x, double* out, size_t n, double sign, void* stream);
 
 /*
  * 1-D analysis / synthesis banks, SURVEY.md 8f row 3: the bodies of AFB1D.forward / SFB1D.forward

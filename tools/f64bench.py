@@ -1,7 +1,8 @@
 """Double-precision paths on the B200: fp64 SSIM forward (+3 derivative maps) and backward at the cfg3 shape
 (256 x 1 x 400 x 400, 328 MB per double image, larger than L2), against the incumbent for this mode -- a torch
 restatement of the reference's _ssim (ssim.py:17-37: five dense grouped F.conv2d + pointwise, autograd backward) in
-double on the same card -- and the 1-D / a trous kernels in double against fp32.  Times are CUDA events around
+double on the same card -- the 1-D / a trous kernels in double against fp32, and the frequency split's pointwise
+kernels and filter_wavelet in double against fp32 (achieved GB/s against the HBM peak).  Times are CUDA events around
 `--iters` launches after `--warmup`.  Prints one JSON line with the card name and power limit read in the same run.
 
     python tools/f64bench.py [--iters 20] [--warmup 3] [--dfma-per-s X]
@@ -17,7 +18,8 @@ import sys
 import torch
 import torch.nn.functional as F
 
-sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path.insert(0, ROOT)
 import b200wave  # noqa: E402
 from b200wave import ops, ops64  # noqa: E402
 
@@ -132,7 +134,55 @@ def main():
         swt[name + "_fwd_ms"] = timed(lambda: fwd(s, a0, a1, a0, a1, 0, 1), it, wu)
         swt[name + "_adjoint_ms"] = timed(lambda: adj(yy, a0, a1, a0, a1, 0, 1), it, wu)
     res["swt_64x304^2_db2"] = swt
+    res.update(freq_and_fsd(it, wu))
     print(json.dumps(res))
+
+
+def hbm_peak_gbs():
+    try:
+        with open(os.path.join(ROOT, "MEASURED_PEAKS.json")) as fh:
+            return float(json.load(fh)["hbm_gbs"]), "MEASURED_PEAKS.json"
+    except (OSError, KeyError, ValueError):
+        return 7700.0, "data sheet (MEASURED_PEAKS.json absent)"
+
+
+def freq_and_fsd(it, wu):
+    """Double frequency split (mask kernel on the complex128 half spectrum, abs kernel) and double filter_wavelet at
+    64 x 256^2 (the spectrum and the image fit the 126 MB L2) and 64 x 1024^2 (they do not), with the fp32 kernels
+    beside them.  Algorithmic bytes per call: mask 2 x the bin (16 B/bin fp32 complex64 -> 32 B/bin complex128), abs
+    2 x the pixel; filter_wavelet reads the image once and writes LL (cs='sum', A) or the three detail bands
+    (cs='cat', B) at a quarter of the pixels: fp64 8 B/px in + 2 or 6 B/px out (fp32 half of that, DESIGN K6)."""
+    from b200wave import freq, fsd
+    peak, src = hbm_peak_gbs()
+    dev = "cuda"
+    out = {"hbm_peak_gbs": peak, "hbm_peak_source": src}
+    for side in (256, 1024):
+        key = "64x%d^2" % side
+        r = {}
+        for name, dt in (("f64", torch.float64), ("f32", torch.float32)):
+            mask_, abs_sign = freq._OPS[dt][0], freq._OPS[dt][1]
+            es = torch.finfo(dt).bits // 8
+            x = torch.rand((64, 1, side, side), device=dev, dtype=dt)
+            spec = torch.fft.rfft2(x).contiguous()
+            bins, px = spec.numel(), x.numel()
+            t_mask = timed(lambda: mask_(spec, side, side, 10.0, True), it, wu)
+            t_abs = timed(lambda: abs_sign(x, 1.0), it, wu)
+            t_split = timed(lambda: freq.gaussian_split(x, 10, True), it, wu)
+            r[name + "_mask_ms"] = t_mask
+            r[name + "_mask_gbs"] = 4 * es * bins / (t_mask * 1e6)
+            r[name + "_abs_ms"] = t_abs
+            r[name + "_abs_gbs"] = 2 * es * px / (t_abs * 1e6)
+            r[name + "_split_fwd_ms"] = t_split
+            for cs, variant, out_b in (("sum", "A", 1), ("cat", "B", 3)):
+                t = timed(lambda: fsd.filter_wavelet(x, cs, True, variant), it, wu)
+                r["%s_fsd_%s%s_ms" % (name, cs, variant)] = t
+                r["%s_fsd_%s%s_gbs" % (name, cs, variant)] = (es + out_b * es / 4) * px / (t * 1e6)
+            for k in [k for k in r if k.startswith(name) and k.endswith("_gbs")]:
+                r[k[:-4] + "_share_of_hbm_peak"] = r[k] / peak
+            del x, spec
+            torch.cuda.empty_cache()
+        out["freq_fsd_" + key] = r
+    return out
 
 
 if __name__ == "__main__":
