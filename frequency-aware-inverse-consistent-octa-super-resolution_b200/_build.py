@@ -72,7 +72,7 @@ def build_bounds(verbose=False):
     want = _source_hash() + "+bounds"
     if os.path.exists(BOUNDS_LIB_PATH) and os.path.exists(stamp) and open(stamp).read().strip() == want:
         return BOUNDS_LIB_PATH
-    build()   # the sources without checks (api, tile / direct kernels, SSIM, ...) come from the regular build
+    build()   # the sources without checks (api, direct kernels, SSIM, ...) come from the regular build
     import fcntl
     with open(os.path.join(LIB_DIR, ".build.lock"), "w") as lock:
         fcntl.flock(lock, fcntl.LOCK_EX)

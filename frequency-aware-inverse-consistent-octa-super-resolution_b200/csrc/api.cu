@@ -21,7 +21,6 @@ const DwtPolicy& dwt_policy() {
         const char* tma = getenv("B200W_TMA");
         DwtPolicy p;
         p.force_direct = flag("B200W_FORCE_DIRECT");
-        p.force_tiled = flag("B200W_FORCE_TILED");
         p.owner = (owner && owner[0] >= '0' && owner[0] <= '2') ? owner[0] - '0' : 1;
         p.tma = !(tma && tma[0] == '0');
         p.tma_noboxes = getenv("B200W_TMA_NOBOXES") != nullptr;

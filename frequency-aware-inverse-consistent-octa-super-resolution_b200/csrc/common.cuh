@@ -183,12 +183,6 @@ __device__ __forceinline__ void cp_async_zero(unsigned dst, const float* src) {
     else if (V == 2) asm volatile("cp.async.ca.shared.global [%0], [%1], 8, %2;" ::"r"(dst), "l"(src), "r"(z) : "memory");
     else asm volatile("cp.async.ca.shared.global [%0], [%1], 4, %2;" ::"r"(dst), "l"(src), "r"(z) : "memory");
 }
-__device__ __forceinline__ void cp_async4_if(unsigned dst, const float* src, bool valid) {
-    B200W_CHK_S(dst, 4);
-    if (valid) B200W_CHK(src, 4);
-    const int n = valid ? 4 : 0;
-    asm volatile("cp.async.ca.shared.global [%0], [%1], 4, %2;" ::"r"(dst), "l"(src), "r"(n) : "memory");
-}
 __device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
 template <int N>
 __device__ __forceinline__ void cp_async_wait() { asm volatile("cp.async.wait_group %0;" ::"n"(N) : "memory"); }

@@ -1,22 +1,11 @@
-// 2-D DWT analysis / synthesis filter banks for sm_100a: kernel selection, the C entry points, the analysis tile
-// chain and the direct kernels.
+// 2-D DWT analysis / synthesis filter banks for sm_100a: kernel selection, the C entry points and the direct kernels.
 //
 // What it replaces.  Per level the reference runs pad-gather + 2x F.conv2d + reshape + 2x .contiguous()
 // (AFB2D, pw/dwt/lowlevel.py:336-347) resp. 6x F.conv_transpose2d + 3 adds (SFB2D, :671-680), and
 // DWTForward / DWTInverse loop over the J levels in Python (pw/dwt/transform2d.py:66-74, 134-148).
 // Here a J-level transform of up to 16 taps is ONE launch: an owner kernel for chains of small planes
-// (dwt_tma_*.cu, dwt_stream_*.cu), otherwise the ticketed stream chain (dwt_stream_*.cu).
-//
-// Analysis tile chain (inputs whose rows are not 16-byte aligned, and B200W_FORCE_TILED): a persistent grid walks an
-// ordered list of tiles (all tiles of the first level, then the next level, ...); a tile of level j+1 of image plane
-// p starts as soon as every tile of level j of that plane has been written (per-plane completion counters,
-// release/acquire), so levels overlap, there are no launch gaps between the small coarse levels, and the LL
-// intermediates are consumed out of L2.
-//
-// Per tile: the input patch (+halo) is staged in shared memory with cp.async -- the padding mode is an index map
-// applied to the source address -- double buffered so the next tile's fetch overlaps this tile's arithmetic; row (W)
-// pass with stride-2 decimation into shared memory; column (H) pass; LL goes to `low`, LH/HL/HH straight into
-// `highs[:, :, 0..2]`.
+// (dwt_tma_*.cu, dwt_stream_*.cu; analysis: 16-byte aligned rows), otherwise the ticketed stream chain
+// (dwt_stream_*.cu), which takes rows of any alignment.
 //
 // Direct kernels: one thread per output of one level, any tap count, in fp32 and in fp64.
 //
@@ -47,299 +36,6 @@ int zero_sync_words(unsigned* words, size_t n, cudaStream_t st) {
     const cudaError_t e = cudaGetLastError();
     return e == cudaSuccess ? B200W_OK : set_last_cuda_error(e);
 }
-
-struct TileRef {
-    int level, plane, th, tw;
-};
-
-__device__ __forceinline__ TileRef decode_tile(const AfbParams& p, long long tile) {
-    int level = 0;
-    for (int j = 1; j < p.J; ++j)
-        if (tile >= p.lv[j].tile_base) level = j;
-    const unsigned local = (unsigned)(tile - p.lv[level].tile_base);
-    const unsigned ntw = (unsigned)p.lv[level].tiles_w;
-    const unsigned tpp = ntw * (unsigned)p.lv[level].tiles_h;
-    TileRef t;
-    t.level = level;
-    t.plane = (int)(local / tpp);
-    const unsigned rem = local - (unsigned)t.plane * tpp;
-    t.th = (int)(rem / ntw);
-    t.tw = (int)(rem - (unsigned)t.th * ntw);
-    return t;
-}
-
-// has every tile of the previous level of this plane been written?
-__device__ __forceinline__ bool tile_ready(const AfbParams& p, const TileRef& t) {
-    if (t.level == 0) return true;
-    const unsigned need = (unsigned)(p.lv[t.level - 1].tiles_w * p.lv[t.level - 1].tiles_h);
-    return ld_acquire_u32(p.done + (size_t)(t.level - 1) * p.planes + t.plane) >= need;
-}
-
-// Persistent, double-buffered walk over the tile list.  Op provides the tile body:
-//   issue(p, tile, shared-window address of the staging buffer, tid)   cp.async the tile's inputs
-//   pass1(p, tile, staging buffer, scratch, tid)                        first 1-D pass, shared -> shared
-//   pass2(p, tile, scratch, tid)                                        second 1-D pass + global stores
-template <class Op>
-__global__ void __launch_bounds__(Op::NT) chain_kernel(const __grid_constant__ typename Op::Params p) {
-    extern __shared__ __align__(16) float smem[];
-    __shared__ int s_pf_ok;
-    float* scratch = smem + 2 * Op::BUF;   // two staging buffers come first
-    const unsigned smem_s = (unsigned)__cvta_generic_to_shared(smem);
-    const int tid = threadIdx.x;
-    const long long G = gridDim.x;
-
-    long long tile = blockIdx.x;
-    if (tile >= p.total) return;
-    TileRef cur = decode_tile(p, tile), nxt = cur;
-    if (cur.level > 0) {   // only when the grid is larger than the first level
-        if (tid == 0)
-            while (!tile_ready(p, cur)) __nanosleep(64);
-        __syncthreads();
-    }
-    Op::issue(p, cur, smem_s, tid);
-    cp_async_commit();
-    // prefetch decision for the following tile; later ones are made by thread 0 inside the loop
-    int pf_ok = (tile + G < p.total) && (tile + G < (p.J > 1 ? p.lv[1].tile_base : p.total));
-    int pend_level = -1, pend_plane = 0;   // tile whose completion still has to be published
-
-    for (int buf = 0;; buf ^= 1) {
-        cp_async_wait<0>();   // this thread's copies of the current tile have landed ...
-        __syncthreads();      // ... and everybody else's; the previous tile's stores are ordered before this barrier
-        // publish the previous tile BEFORE this thread has copies in flight again (the fence waits for them)
-        if (tid == 0 && pend_level >= 0) signal_done(p.done + (size_t)pend_level * p.planes + pend_plane);
-        const long long ntile = tile + G;
-        const bool have_next = ntile < p.total;
-        bool prefetched = false;
-        if (have_next) {
-            nxt = decode_tile(p, ntile);
-            if (pf_ok) {   // the next tile's inputs are complete: fetch them while this tile is processed
-                Op::issue(p, nxt, smem_s + (unsigned)((buf ^ 1) * Op::BUF * 4), tid);
-                prefetched = true;
-            }
-        }
-        cp_async_commit();
-        // thread 0 probes whether the tile after next will be fetchable; the load stays in flight across pass1
-        unsigned dep_have = 1, dep_need = 0;
-        if (tid == 0) {
-            const long long nn = ntile + G;
-            if (nn >= p.total) {
-                dep_have = 0;
-                dep_need = 1;
-            } else {
-                const TileRef t2 = decode_tile(p, nn);
-                if (t2.level > 0) {
-                    dep_need = (unsigned)(p.lv[t2.level - 1].tiles_w * p.lv[t2.level - 1].tiles_h);
-                    dep_have = ld_acquire_u32(p.done + (size_t)(t2.level - 1) * p.planes + t2.plane);
-                }
-            }
-        }
-        Op::pass1(p, cur, smem + buf * Op::BUF, scratch, tid);
-        if (tid == 0) s_pf_ok = dep_have >= dep_need ? 1 : 0;
-        __syncthreads();
-        Op::pass2(p, cur, scratch, tid);
-        pf_ok = s_pf_ok;
-        const bool has_consumer = cur.level + 1 < p.J;
-        pend_level = has_consumer ? cur.level : -1;
-        pend_plane = cur.plane;
-        if (!have_next) break;
-        if (!prefetched) {
-            // the next tile's inputs were not complete when we looked: publish our own result first (it may be
-            // the missing piece), then wait for the producers -- all of them own earlier tiles and are resident
-            __syncthreads();
-            if (tid == 0) {
-                if (pend_level >= 0) signal_done(p.done + (size_t)pend_level * p.planes + pend_plane);
-                while (!tile_ready(p, nxt)) __nanosleep(64);
-            }
-            pend_level = -1;
-            __syncthreads();
-            Op::issue(p, nxt, smem_s + (unsigned)((buf ^ 1) * Op::BUF * 4), tid);
-            cp_async_commit();
-        }
-        tile = ntile;
-        cur = nxt;
-    }
-    if (pend_level >= 0) {
-        __syncthreads();
-        if (tid == 0) signal_done(p.done + (size_t)pend_level * p.planes + pend_plane);
-    }
-}
-
-// ------------------------------------------------------------------------------------------------
-// analysis tile.  Output tile TH x TW (x4 sub-bands), NT threads.
-// ------------------------------------------------------------------------------------------------
-// Stage ROWS x PITCH floats asynchronously.  Every thread owns one vector column (V floats) and walks down
-// the rows, so both addresses advance by constants.  (r0, c0) = source coordinates of patch element (0,0);
-// the padding mode is applied as an index map, "zero" = zero fill (cp.async with src-size 0).
-template <int V, int ROWS, int PITCH, int NT>
-__device__ __forceinline__ void stage_analysis(unsigned patch_s, const float* __restrict__ xp, long long rs, int r0,
-                                               int c0, int H, int W, int Hreal, int Wreal, int mode, int nrows,
-                                               int ncols, int tid) {
-    constexpr int NVC = PITCH / V;   // vector columns per row
-    constexpr int NRG = NT / NVC;    // row groups
-    if (tid >= NVC * NRG) return;
-    const int cv = tid % NVC;
-    const int rg = tid / NVC;
-    if (V * cv >= ncols) return;     // columns that feed no valid output of an edge tile are not staged
-    const int sc0 = c0 + V * cv;
-    const bool col_in = sc0 >= 0 && sc0 + V <= Wreal;
-    unsigned dst = patch_s + (unsigned)((rg * PITCH + V * cv) * 4);
-    if (col_in && r0 >= 0 && r0 + nrows <= Hreal) {
-        const float* src = xp + (long long)(r0 + rg) * rs + sc0;
-        const long long step = (long long)NRG * rs;
-#pragma unroll 4
-        for (int r = rg; r < nrows; r += NRG) {
-            cp_async<V>(dst, src);
-            dst += NRG * PITCH * 4;
-            src += step;
-        }
-        return;
-    }
-    int ci[V];
-#pragma unroll
-    for (int e = 0; e < V; ++e) {
-        ci[e] = ext_index(sc0 + e, W, mode);
-        if (ci[e] >= Wreal) ci[e] = -1;
-    }
-    for (int r = rg; r < nrows; r += NRG, dst += NRG * PITCH * 4) {
-        const int sr = ext_index(r0 + r, H, mode);
-        if (sr < 0 || sr >= Hreal) {
-            cp_async_zero<V>(dst, xp);
-            continue;
-        }
-        const float* rowp = xp + (long long)sr * rs;
-        if (col_in) {
-            cp_async<V>(dst, rowp + sc0);
-        } else {
-#pragma unroll
-            for (int e = 0; e < V; ++e) cp_async4_if(dst + 4 * e, ci[e] >= 0 ? rowp + ci[e] : xp, ci[e] >= 0);
-        }
-    }
-}
-
-template <int L_, int TW_, int TH_, int NT_>
-struct AfbOp {
-    using Params = AfbParams;
-    static constexpr const char* name = "chain_kernel<AfbOp>";
-    static constexpr int L = L_, TW = TW_, TH = TH_, NT = NT_;
-    static constexpr int PC = 2 * TW + L - 2;     // staged patch columns actually needed
-    static constexpr int PCP = (PC + 3) & ~3;     // row pitch (multiple of 4 floats: 128-bit LDS)
-    static constexpr int PR = 2 * TH + L - 2;     // staged patch rows
-    static constexpr int BUF = PR * PCP;          // floats per staging buffer
-    static constexpr int NP = TW / 2;             // output pairs per row (row pass)
-    static constexpr int RSTEP = NT / NP;         // patch rows advanced per row-pass iteration
-    static constexpr int NV = (L + 2 + 3) / 4;    // float4 loads per row-pass item
-    static constexpr int CP = TW / 2;             // column pairs (column pass)
-    static constexpr int NS = NT / CP;            // row strips in the column pass
-    static constexpr int RS = TH / NS;            // output rows per thread in the column pass
-    static constexpr size_t smem = sizeof(float) * (size_t)(2 * BUF + 2 * PR * TW);  // 2 patches + mid_lo/mid_hi
-    static_assert(L % 2 == 0 && TW % 4 == 0 && NT % CP == 0 && TH % NS == 0 && NT % NP == 0, "bad tile");
-    static_assert(2 * TW - 4 + 4 * NV <= PCP, "row pass would read past the patch row");
-    static_assert(PCP <= NT, "staging needs one thread per scalar column");
-
-    static __device__ __forceinline__ void issue(const AfbParams& p, const TileRef& t, unsigned patch_s, int tid) {
-        const AfbLevel& lv = p.lv[t.level];
-        const int r0 = 2 * t.th * TH - lv.offH;  // source row of patch row 0
-        const int c0 = 2 * t.tw * TW - lv.offW;
-        const float* xp = lv.x + (long long)t.plane * lv.x_ps;
-        // an edge tile only needs the rows / columns its valid outputs read: 2*(n_valid-1) + L of them
-        const int nrows = min(PR, 2 * (min(TH, lv.Ho - t.th * TH) - 1) + L);
-        const int ncols = min(PCP, 2 * (min(TW, lv.Wo - t.tw * TW) - 1) + L);
-        if (lv.in_vec == 4)
-            stage_analysis<4, PR, PCP, NT>(patch_s, xp, lv.x_rs, r0, c0, lv.H, lv.W, lv.Hreal, lv.Wreal, p.mode, nrows, ncols, tid);
-        else if (lv.in_vec == 2)
-            stage_analysis<2, PR, PCP, NT>(patch_s, xp, lv.x_rs, r0, c0, lv.H, lv.W, lv.Hreal, lv.Wreal, p.mode, nrows, ncols, tid);
-        else
-            stage_analysis<1, PR, PCP, NT>(patch_s, xp, lv.x_rs, r0, c0, lv.H, lv.W, lv.Hreal, lv.Wreal, p.mode, nrows, ncols, tid);
-    }
-
-    // row pass (along W), decimate by 2: each item makes two adjacent outputs of one patch row from NV 128-bit
-    // shared loads (conflict free: consecutive lanes read consecutive float4)
-    static __device__ __forceinline__ void pass1(const AfbParams& p, const TileRef&, const float* patch, float* mid,
-                                                 int tid) {
-        const int kk = tid % NP;
-        int r = tid / NP;
-        const float* src = patch + r * PCP + 4 * kk;
-        float* dlo = mid + r * TW + 2 * kk;
-#pragma unroll 2
-        for (; r < PR; r += RSTEP, src += RSTEP * PCP, dlo += RSTEP * TW) {
-            float v[4 * NV];
-#pragma unroll
-            for (int q = 0; q < NV; ++q) {
-                const float4 t = reinterpret_cast<const float4*>(src)[q];
-                v[4 * q] = t.x; v[4 * q + 1] = t.y; v[4 * q + 2] = t.z; v[4 * q + 3] = t.w;
-            }
-            float lo0 = 0.f, hi0 = 0.f, lo1 = 0.f, hi1 = 0.f;
-#pragma unroll
-            for (int j = 0; j < L; ++j) {
-                lo0 = fmaf(p.t.w_lo[j], v[j], lo0);
-                hi0 = fmaf(p.t.w_hi[j], v[j], hi0);
-                lo1 = fmaf(p.t.w_lo[j], v[j + 2], lo1);
-                hi1 = fmaf(p.t.w_hi[j], v[j + 2], hi1);
-            }
-            *reinterpret_cast<float2*>(dlo) = make_float2(lo0, lo1);
-            *reinterpret_cast<float2*>(dlo + PR * TW) = make_float2(hi0, hi1);
-        }
-    }
-
-    // column pass (along H), decimate by 2; each thread owns RS output rows of two adjacent columns
-    static __device__ __forceinline__ void pass2(const AfbParams& p, const TileRef& t, const float* mid, int tid) {
-        const AfbLevel& lv = p.lv[t.level];
-        const int cp = tid % CP;
-        const int s = tid / CP;
-        float2 acc[RS][4];
-#pragma unroll
-        for (int i = 0; i < RS; ++i)
-#pragma unroll
-            for (int b = 0; b < 4; ++b) acc[i][b] = make_float2(0.f, 0.f);
-        const float2* plo = reinterpret_cast<const float2*>(mid + (2 * s * RS) * TW + 2 * cp);
-        const float2* phi = reinterpret_cast<const float2*>(mid + PR * TW + (2 * s * RS) * TW + 2 * cp);
-#pragma unroll
-        for (int rr = 0; rr < 2 * RS + L - 2; ++rr) {
-            const float2 vlo = plo[rr * (TW / 2)];
-            const float2 vhi = phi[rr * (TW / 2)];
-#pragma unroll
-            for (int i = 0; i < RS; ++i) {
-                const int j = rr - 2 * i;
-                if (j >= 0 && j < L) {
-                    const float a = p.t.h_lo[j], b = p.t.h_hi[j];
-                    acc[i][0].x = fmaf(a, vlo.x, acc[i][0].x); acc[i][0].y = fmaf(a, vlo.y, acc[i][0].y);  // LL
-                    acc[i][1].x = fmaf(b, vlo.x, acc[i][1].x); acc[i][1].y = fmaf(b, vlo.y, acc[i][1].y);  // LH: W-lo, H-hi
-                    acc[i][2].x = fmaf(a, vhi.x, acc[i][2].x); acc[i][2].y = fmaf(a, vhi.y, acc[i][2].y);  // HL: W-hi, H-lo
-                    acc[i][3].x = fmaf(b, vhi.x, acc[i][3].x); acc[i][3].y = fmaf(b, vhi.y, acc[i][3].y);  // HH
-                }
-            }
-        }
-        const int Ho = lv.Ho, Wo = lv.Wo;
-        const int kk = t.tw * TW + 2 * cp;
-        const int row0 = t.th * TH + s * RS;
-        const size_t band = (size_t)Ho * Wo;
-        const long long lrs = lv.low_rs;
-        float* q0 = lv.low + (long long)t.plane * lv.low_ps + (long long)row0 * lrs + kk;
-        float* q1 = lv.highs + (size_t)t.plane * 3 * band + (size_t)row0 * Wo + kk;
-        float* q2 = q1 + band;
-        float* q3 = q2 + band;
-        if (lv.out_vec2 && lv.low_vec2 && row0 + RS <= Ho && kk + 1 < Wo) {  // whole strip inside: 64-bit stores
-#pragma unroll
-            for (int i = 0; i < RS; ++i) {
-                *reinterpret_cast<float2*>(q0) = acc[i][0];
-                *reinterpret_cast<float2*>(q1) = acc[i][1];
-                *reinterpret_cast<float2*>(q2) = acc[i][2];
-                *reinterpret_cast<float2*>(q3) = acc[i][3];
-                q0 += lrs; q1 += Wo; q2 += Wo; q3 += Wo;
-            }
-        } else if (kk < Wo) {
-            const bool second = kk + 1 < Wo;
-#pragma unroll
-            for (int i = 0; i < RS; ++i) {
-                if (row0 + i < Ho) {
-                    q0[0] = acc[i][0].x; q1[0] = acc[i][1].x; q2[0] = acc[i][2].x; q3[0] = acc[i][3].x;
-                    if (second) { q0[1] = acc[i][0].y; q1[1] = acc[i][1].y; q2[1] = acc[i][2].y; q3[1] = acc[i][3].y; }
-                }
-                q0 += lrs; q1 += Wo; q2 += Wo; q3 += Wo;
-            }
-        }
-    }
-};
 
 // ------------------------------------------------------------------------------------------------
 // direct kernels: one thread per output position of ONE level, no staging, any tap count up to kMaxTaps (odd or
@@ -503,25 +199,17 @@ static int synthesis_offset(int l, int mode) { return mode == B200W_MODE_PERIODI
 
 constexpr int kMaxDevices = 64;
 
-struct DeviceInfo {
-    int dev;
-    int sms;
-};
-
-static DeviceInfo device_info() {
+// SM count of the current device, queried once per device
+static int device_sms() {
     static int sms[kMaxDevices] = {0};
-    DeviceInfo d{0, 148};
-    if (cudaGetDevice(&d.dev) != cudaSuccess || d.dev < 0 || d.dev >= kMaxDevices) {
-        d.dev = 0;
-        return d;
-    }
-    if (sms[d.dev] == 0) {
+    int dev = 0;
+    if (cudaGetDevice(&dev) != cudaSuccess || dev < 0 || dev >= kMaxDevices) return 148;
+    if (sms[dev] == 0) {
         int n = 0;
-        if (cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, d.dev) != cudaSuccess || n <= 0) n = 148;
-        sms[d.dev] = n;
+        if (cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess || n <= 0) n = 148;
+        sms[dev] = n;
     }
-    d.sms = sms[d.dev];
-    return d;
+    return sms[dev];
 }
 
 // Workspace layout of a J-level chain: [ticket, done[J][planes]] (u32), then the intermediate low-pass images
@@ -532,72 +220,6 @@ static size_t sync_bytes(int planes, int J) { return J > 1 ? round256(sizeof(uns
 static int pitch4(int w) { return (w + 3) & ~3; }
 static size_t scratch_bytes(int planes, int rows, int cols) {
     return round256(sizeof(float) * (size_t)planes * rows * pitch4(cols));
-}
-
-// Persistent launch of a tile chain: grid = min(tiles, SMs x occupancy).  A multi-level chain spins on completion
-// counters, so its CTAs must all be resident: it is launched cooperatively (the runtime refuses the launch
-// otherwise) and the counters are cleared on the stream first.  `occ_cache` is the caller's per-kernel,
-// per-device cache of the occupancy (0 = not queried yet; the query also raises the kernel's dynamic
-// shared-memory limit).  Both are immutable facts about (kernel, device), so caching them keeps the library
-// re-entrant.
-template <class Op>
-static int launch_chain(typename Op::Params& p, int* occ_cache, cudaStream_t st) {
-    auto kernel = chain_kernel<Op>;
-    const DeviceInfo di = device_info();
-    int& occ = occ_cache[di.dev];
-    if (occ == 0) {
-        cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Op::smem);
-        if (e != cudaSuccess) return set_last_cuda_error(e);
-        int o = 0;
-        e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&o, kernel, Op::NT, Op::smem);
-        if (e != cudaSuccess) return set_last_cuda_error(e);
-        occ = o > 0 ? o : 1;
-    }
-    long long grid = (long long)di.sms * occ;
-    if (grid > p.total) grid = p.total;
-    cudaError_t e;
-    if (p.J > 1) {
-        const int rc = zero_sync_words(p.ticket, (size_t)p.J * p.planes + 1, st);
-        if (rc) return rc;
-        void* args[] = {(void*)&p};
-        e = cudaLaunchCooperativeKernel((const void*)kernel, dim3((unsigned)grid), dim3(Op::NT), args, Op::smem, st);
-    } else {
-        kernel<<<(unsigned)grid, Op::NT, Op::smem, st>>>(p);
-        e = cudaGetLastError();
-    }
-    note_launch(Op::name);
-    return e == cudaSuccess ? B200W_OK : set_last_cuda_error(e);
-}
-
-template <int TW, int TH>
-static void afb_layout(AfbParams& p) {
-    long long base = 0;
-    for (int j = 0; j < p.J; ++j) {
-        p.lv[j].tiles_w = ceil_div(p.lv[j].Wo, TW);
-        p.lv[j].tiles_h = ceil_div(p.lv[j].Ho, TH);
-        p.lv[j].tile_base = base;
-        base += (long long)p.lv[j].tiles_w * p.lv[j].tiles_h * p.planes;
-    }
-    p.total = base;
-}
-
-template <int L>
-static int launch_afb_chain(AfbParams& p, cudaStream_t st) {
-    // two tile shapes: 32x32 outputs / 128 threads, or 64 wide x 32 / 256 threads (less halo); take the wide
-    // one for wide single-level problems unless it wastes noticeably more of the padded output area
-    const int Wo = p.lv[0].Wo;
-    const long long a32 = (long long)ceil_div(Wo, 32) * 32;
-    const long long a64 = (long long)ceil_div(Wo, 64) * 64;
-    if (p.J == 1 && Wo >= 128 && a64 * 100 <= a32 * 103) {
-        using Op = AfbOp<L, 64, 32, 256>;
-        static int occ[kMaxDevices] = {0};
-        afb_layout<Op::TW, Op::TH>(p);
-        return launch_chain<Op>(p, occ, st);
-    }
-    using Op = AfbOp<L, 32, 32, 128>;
-    static int occ[kMaxDevices] = {0};
-    afb_layout<Op::TW, Op::TH>(p);
-    return launch_chain<Op>(p, occ, st);
 }
 
 static size_t direct_grid(size_t total) {
@@ -617,15 +239,6 @@ static int launch_direct(void (*kernel)(Params), const Params& d, size_t outputs
 
 static bool templated_taps(int Lw, int Lh) {
     return Lw == Lh && (Lw % 2) == 0 && Lw >= 2 && Lw <= 16 && !dwt_policy().force_direct;
-}
-
-// ---- analysis chain --------------------------------------------------------------------------------
-static int run_afb_big_levels(AfbParams& p, int L, cudaStream_t st) {
-    if (!dwt_policy().force_tiled && afb_stream_supported(p, L)) return launch_afb_stream(p, L, device_info().sms, st);
-#define X(LL) return launch_afb_chain<LL>(p, st)
-    B200W_FOR_EACH_L(X)
-#undef X
-    return B200W_ERR_BAD_TAPS;
 }
 
 // level sizes of the analysis chain; returns a status
@@ -660,7 +273,6 @@ static int run_afb_chain(const float* x, int64_t x_ps, int64_t x_rs, int planes,
     if (J < 1 || J > kMaxLevels) return B200W_ERR_BAD_SHAPE;
     // the filter_wavelet entry point (single level) may leave out the low-pass or the detail output
     if (!x || !highs || (!allow_skip && !yl) || (allow_skip && !yl && !highs[0])) return B200W_ERR_NULL_POINTER;
-    const bool plain = !allow_skip && hi_scale == 1.f && hi_shift == 0.f;
     if (planes < 1 || H < 1 || W < 1) return B200W_ERR_BAD_SHAPE;
     AfbParams p;
     int rc = fill_taps(p.t, w_lo, w_hi, Lw, h_lo, h_hi, Lh);
@@ -715,37 +327,31 @@ static int run_afb_chain(const float* x, int64_t x_ps, int64_t x_rs, int planes,
             scratch += scratch_bytes(planes, lv.Ho, lv.Wo);
         }
         lv.highs = highs[j];
-        // staging vector width of the tile kernel: the first staged column of every tile is 2*TW*tw - offW
-        lv.in_vec = 1;
-        if ((lv.offW % 2) == 0 && (lv.x_rs % 2) == 0 && (lv.x_ps % 2) == 0 && aligned_to(lv.x, 8)) lv.in_vec = 2;
-        if (lv.in_vec == 2 && (lv.offW % 4) == 0 && (lv.x_rs % 4) == 0 && (lv.x_ps % 4) == 0 && aligned_to(lv.x, 16))
-            lv.in_vec = 4;
         lv.out_vec2 = ((lv.Wo % 2) == 0 && lv.highs && aligned_to(lv.highs, 8)) ? 1 : 0;
         lv.low_vec2 = ((lv.low_rs % 2) == 0 && (lv.low_ps % 2) == 0 && lv.low && aligned_to(lv.low, 8)) ? 1 : 0;
-        lv.tile_base = lv.cta_base = 0;
-        lv.tiles_h = lv.tiles_w = lv.R = lv.ncp = lv.cpp = lv.cp0A = lv.ncpA = lv.itemsA = lv.cppA = lv.RB = lv.itemsB = 0;
+        lv.cta_base = 0;
+        lv.R = lv.ncp = lv.cpp = lv.cp0A = lv.ncpA = lv.itemsA = lv.cppA = lv.RB = lv.itemsB = 0;
         h = lv.Ho;
         w = lv.Wo;
     }
-    // the store epilogue lives in the stream and the direct kernels: other inputs (unaligned rows) take the direct one
-    const DwtPolicy& pol = dwt_policy();
-    if (templated_taps(Lw, Lh) && (plain || (!pol.force_tiled && afb_stream_supported(p, Lw)))) {
+    if (templated_taps(Lw, Lh) && afb_stream_supported(p, Lw)) {
         // chains of small planes: one CTA owns a part of a plane for all levels (TMA-staged owner kernel first, the
-        // cp.async owner kernel for the shapes it declines); everything else goes through the ticketed stream chain
-        // (or the tile chain when rows are unaligned)
-        const bool owner = J > 1 && !pol.force_tiled && pol.owner != 0, force = pol.owner == 2;
-        if (owner && plain && pol.tma) {
+        // cp.async owner kernel for the shapes it declines; both need 16-byte aligned rows); everything else goes
+        // through the ticketed stream chain
+        const DwtPolicy& pol = dwt_policy();
+        const bool owner = J > 1 && pol.owner != 0, force = pol.owner == 2;
+        if (owner && pol.tma) {
             AfbTmaParams tp;
-            if (afb_tma_plan(p, Lw, device_info().sms, force, pol.tma_G, pol.tma_D, pol.tma_noboxes, tp))
+            if (afb_tma_plan(p, Lw, device_sms(), force, pol.tma_G, pol.tma_D, pol.tma_noboxes, tp))
                 return launch_afb_tma(tp, Lw, st);
         }
         if (owner) {
             AfbOwnerParams op;
-            if (afb_owner_plan(p, Lw, device_info().sms, force, op)) return launch_afb_owner(op, Lw, st);
+            if (afb_owner_plan(p, Lw, device_sms(), force, op)) return launch_afb_owner(op, Lw, st);
         }
-        return run_afb_big_levels(p, Lw, st);
+        return launch_afb_stream(p, Lw, device_sms(), st);
     }
-    for (int j = 0; j < J; ++j) {  // level by level with the direct kernel
+    for (int j = 0; j < J; ++j) {  // other taps and row strides: level by level with the direct kernel
         const AfbLevel& lv = p.lv[j];
         const AfbDirectParams<float> d = {lv.x, lv.low, lv.highs, lv.x_ps, lv.x_rs, lv.low_ps, lv.low_rs, lv.H, lv.W,
                                           lv.Hreal, lv.Wreal, lv.Ho, lv.Wo, lv.offH, lv.offW, lv.st_low, lv.st_hi,
@@ -842,13 +448,13 @@ static int run_sfb_chain(const float* yl, int64_t yl_ps, int64_t yl_rs, const fl
         const bool owner = J > 1 && pol.owner != 0, force = pol.owner == 2;
         if (owner && pol.tma) {
             SfbTmaParams tp;
-            if (sfb_tma_plan(p, Lw, device_info().sms, force, pol.tma_G, pol.tma_D, tp)) return launch_sfb_tma(tp, Lw, st);
+            if (sfb_tma_plan(p, Lw, device_sms(), force, pol.tma_G, pol.tma_D, tp)) return launch_sfb_tma(tp, Lw, st);
         }
         if (owner) {
             SfbOwnerParams op;
-            if (sfb_owner_plan(p, Lw, device_info().sms, force, op)) return launch_sfb_owner(op, Lw, st);
+            if (sfb_owner_plan(p, Lw, device_sms(), force, op)) return launch_sfb_owner(op, Lw, st);
         }
-        return launch_sfb_stream(p, Lw, device_info().sms, st);
+        return launch_sfb_stream(p, Lw, device_sms(), st);
     }
     for (int c = 0; c < J; ++c) {
         const SfbLevel& lv = p.lv[c];

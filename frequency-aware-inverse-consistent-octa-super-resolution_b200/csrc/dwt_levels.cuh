@@ -1,12 +1,11 @@
-// Level geometry and chain bookkeeping shared by the DWT chain kernels (tile, stream, owner and TMA variants).
+// Level geometry and chain bookkeeping shared by the DWT chain kernels (stream, owner and TMA variants).
 //
-// A multi-level transform is ONE launch: the work items of all levels form one ordered list (all items of the
-// first level, then the next level, ...).  An item of level j+1 of image plane p may start once every item of
-// level j of that plane has been written: per-(level, plane) completion counters, published with a gpu-scope
-// release (fence + atomic) and consumed with ld.acquire.  Work items are handed out in list order -- by a
-// persistent grid (tile kernels, cooperative launch) or by an atomic ticket taken when a CTA starts (stream
-// kernels) -- so an item only ever waits for items that are already running or done: no deadlock, no launch
-// gaps between the small coarse levels, and the LL intermediates are consumed out of L2.
+// A multi-level transform is ONE launch.  In the stream kernels the work items of all levels form one ordered list
+// (all items of the first level, then the next level, ...).  An item of level j+1 of image plane p may start once
+// every item of level j of that plane has been written: per-(level, plane) completion counters, published with a
+// gpu-scope release (fence + atomic) and consumed with ld.acquire.  Work items are handed out in list order by an
+// atomic ticket taken when a CTA starts, so an item only ever waits for items that are already running or done: no
+// deadlock, no launch gaps between the small coarse levels, and the LL intermediates are consumed out of L2.
 #pragma once
 #include "common.cuh"
 
@@ -44,10 +43,6 @@ struct AfbLevel {
     // written, and the three detail bands are stored as hi_scale * v + hi_shift (1, 0 = plain DWT)
     int st_low, st_hi;
     float hi_scale, hi_shift;
-    // tile kernels
-    long long tile_base;   // index of this level's first tile in the global tile order
-    int tiles_h, tiles_w;
-    int in_vec;            // widest aligned vector (1, 2 or 4 floats) usable for staging copies
     // stream kernels: a thread owns one pair of output columns over R output rows.  Column pairs whose input
     // window lies inside the image ("interior", cp0A <= cp < cp0A + ncpA) are staged through the per-warp ring;
     // the few pairs at the left / right border go through the per-thread path with a column map.
@@ -138,8 +133,8 @@ bool sfb_stream_supported(const SfbParams& p, int L);
 int launch_sfb_stream(SfbParams& p, int L, int sms, cudaStream_t st);
 
 // owner kernel (dwt_stream_afb.cu): all levels of an analysis chain in one launch without grid-wide dependencies.
-// afb_owner_plan fills `op` and returns true when the shapes qualify (low-pass images fit in shared memory, enough
-// planes x parts to occupy the device -- unless `force`).
+// afb_owner_plan fills `op` and returns true when the shapes qualify (16-byte aligned rows, low-pass images fit in
+// shared memory, enough planes x parts to occupy the device -- unless `force`).
 bool afb_owner_plan(const AfbParams& p, int L, int sms, bool force, AfbOwnerParams& op);
 int launch_afb_owner(const AfbOwnerParams& op, int L, cudaStream_t st);
 
@@ -188,7 +183,6 @@ static inline bool aligned_to(const void* p, size_t a) { return (reinterpret_cas
 // written kernel families against each other on the same inputs; the defaults are what every other run takes.
 struct DwtPolicy {
     bool force_direct;   // B200W_FORCE_DIRECT=1: one-thread-per-output kernels only
-    bool force_tiled;    // B200W_FORCE_TILED=1: analysis tile kernels instead of the stream and owner kernels
     int owner;           // B200W_OWNER: 0 = no owner kernels (ticketed chains), 1 = where they pay off, 2 = whenever they fit
     bool tma;            // B200W_TMA=0: cp.async owner kernels instead of the TMA-staged ones
     bool tma_noboxes;    // B200W_TMA_NOBOXES: TMA analysis ring fetches every extension row from its source row

@@ -1,4 +1,4 @@
-// Analysis filter bank, streaming register-blocked kernel (the fast path for 16-byte aligned rows).
+// Analysis filter bank, streaming register-blocked kernel (every row alignment; the fast path of the templated taps).
 //
 // Replaces afb1d(dim=3) + afb1d(dim=2) + reshape + 2x .contiguous() of AFB2D.forward
 // (pw/dwt/lowlevel.py:336-347, 91-172) -- and the J-level loop around it (pw/dwt/transform2d.py:66-74).
@@ -18,6 +18,9 @@
 // warp are in flight without holding registers; a lane then reads its window (own float4 + the neighbours')
 // with NV 128-bit shared loads.  Only __syncwarp is needed.  Rows outside the image are remapped per row
 // (symmetric / reflect / periodic / periodization) or cleared with shared stores.
+// The window starts at a multiple of 4 columns of the row, so the 16 bytes a lane copies are 16-byte aligned in
+// global memory exactly when the rows are (V = 4: one copy); for other rows (odd widths, strided views) the same
+// 16 bytes are copied as four 4-byte cp.async (V = 1).  Ring, window reads and arithmetic do not depend on V.
 // The few border columns of each row run in separate CTAs, one thread per output position, through the row /
 // column maps of the padding mode.
 // Segments overlap by L-2 input rows (re-read through L2).
@@ -140,11 +143,24 @@ __device__ __forceinline__ float4 lds128(unsigned addr) {
     return v;
 }
 
+// one 16-byte ring slot from global memory: a single 16-byte cp.async (V = 4, `src` 16-byte aligned) or four 4-byte
+// ones (V = 1, `src` 4-byte aligned)
+template <int V>
+__device__ __forceinline__ void ring_copy16(unsigned dst, const float* src) {
+    static_assert(V == 4 || V == 1, "ring copy width");
+    if constexpr (V == 4) {
+        cp_async<4>(dst, src);
+    } else {
+#pragma unroll
+        for (int i = 0; i < 4; ++i) cp_async<1>(dst + 4u * i, src + i);
+    }
+}
+
 // ---- interior column pairs: per-warp cp.async ring ---------------------------------------------------
-// `it` = the thread's item (segment-major: segment * ncpA + interior column pair).  OWNER: the rows come from `own`
-// instead of the whole level; SMEM_SRC (owner kernel, dependent levels): the input image already lies in shared
-// memory, so a lane reads its window straight from there and the ring is not used.
-template <int L, int S, bool OWNER = false, bool SMEM_SRC = false, int Q = 1>
+// `it` = the thread's item (segment-major: segment * ncpA + interior column pair).  V = global copy width (above).
+// OWNER: the rows come from `own` instead of the whole level; SMEM_SRC (owner kernel, dependent levels): the input
+// image already lies in shared memory, so a lane reads its window straight from there and the ring is not used.
+template <int L, int S, int V, bool OWNER = false, bool SMEM_SRC = false, int Q = 1>
 __device__ __forceinline__ void afb_ring_cta(const AfbParams& p, const AfbLevel& lv, int plane, int it, float4* ring_all,
                                              const unsigned* wait_ctr, unsigned wait_need, const OwnRows& own) {
     using C = AfbStreamCfg<L, S>;
@@ -183,8 +199,8 @@ __device__ __forceinline__ void afb_ring_cta(const AfbParams& p, const AfbLevel&
     const unsigned ring_s = (unsigned)__cvta_generic_to_shared(ring) + (unsigned)slot * 16u;
 
     // stage one input row pair (pair index q of this lane's segment) into ring stage `st`.  Rows inside the image
-    // take the plain 16-byte cp.async (the zero-filling form costs three padding instructions each); zero rows
-    // are cleared with shared stores.
+    // take the plain cp.async (the zero-filling form costs three padding instructions each); zero rows are cleared
+    // with shared stores.
     auto issue = [&](int q, int st) {
         // nothing is staged beyond this lane's segment: the lanes that would read those slots (same run, same
         // segment) are past their last pair too, and an idle lane must not touch slots that belong to others
@@ -196,12 +212,12 @@ __device__ __forceinline__ void afb_ring_cta(const AfbParams& p, const AfbLevel&
                 if (sr >= 0) {
                     const float* src = reinterpret_cast<const float*>(reinterpret_cast<const char*>(xcol) +
                                                                       (unsigned long long)(unsigned)sr * rs_b);
-                    cp_async<4>(dst, src);
-                    if (Q == 2 && ncopy == 2) cp_async<4>(dst + 16u, src + 4);
+                    ring_copy16<V>(dst, src);
+                    if (Q == 2 && ncopy == 2) ring_copy16<V>(dst + 16u, src + 4);
                     if (run_last) {
 #pragma unroll
                         for (int k = 0; k < NV - 1; ++k)
-                            if (k < nextra) cp_async<4>(dst + 16u * (ncopy + k), src + 4 * (ncopy + k));
+                            if (k < nextra) ring_copy16<V>(dst + 16u * (ncopy + k), src + 4 * (ncopy + k));
                     }
                 } else {
                     float4* d = ring + (st * 2 + e) * RP + slot;
@@ -436,7 +452,7 @@ __device__ __forceinline__ void afb_border_item(const AfbParams& p, const AfbLev
     }
 }
 
-template <int L, int S>
+template <int L, int S, int V>
 __global__ void __launch_bounds__(kStreamNT, AfbStreamCfg<L, S>::MINB) afb_stream_kernel(const __grid_constant__ AfbParams p) {
     extern __shared__ float4 ring_all[];
     __shared__ unsigned s_item;
@@ -459,7 +475,7 @@ __global__ void __launch_bounds__(kStreamNT, AfbStreamCfg<L, S>::MINB) afb_strea
     const unsigned wait_need = level > 0 ? (unsigned)p.lv[level - 1].cpp : 0u;
     const OwnRows none{};
     if (cta < lv.cppA) {
-        afb_ring_cta<L, S>(p, lv, plane, cta * kStreamNT + tid, ring_all, wait_ctr, wait_need, none);
+        afb_ring_cta<L, S, V>(p, lv, plane, cta * kStreamNT + tid, ring_all, wait_ctr, wait_need, none);
     } else {
         const int it = (cta - lv.cppA) * kStreamNT + tid;
         afb_border_item<L, S>(p, lv, plane, it, it < lv.itemsB, wait_ctr, wait_need, none);
@@ -556,9 +572,9 @@ __global__ void __launch_bounds__(AfbOwnerCfg<L>::NT, 1) afb_owner_kernel(const 
             for (int base = 0; base < own.itemsA; base += ntA) {
                 __syncwarp();   // the warp's ring is reused from pass to pass
                 if (smem_src)
-                    afb_ring_cta<L, S, true, true, Q>(p, lv, plane, base + tid, ring_all, nullptr, 0u, own);
+                    afb_ring_cta<L, S, 4, true, true, Q>(p, lv, plane, base + tid, ring_all, nullptr, 0u, own);
                 else
-                    afb_ring_cta<L, S, true, false, Q>(p, lv, plane, base + tid, ring_all, nullptr, 0u, own);
+                    afb_ring_cta<L, S, 4, true, false, Q>(p, lv, plane, base + tid, ring_all, nullptr, 0u, own);
             }
         }
         if (!beside || tid >= padA) {
@@ -575,9 +591,18 @@ bool afb_stream_supported(const AfbParams& p, int L) {
     const bool per = p.mode == B200W_MODE_PERIODIZATION;
     for (int j = 0; j < p.J; ++j) {
         const AfbLevel& lv = p.lv[j];
-        if ((lv.x_rs & 3) || (lv.x_ps & 3) || !aligned_to(lv.x, 16)) return false;
         if (lv.x_rs < 0 || lv.x_rs >= (1LL << 30)) return false;   // the ring addresses rows with a 32-bit byte stride
         if (lv.offW != afb_off(L, per) || lv.offH != afb_off(L, per)) return false;
+    }
+    return true;
+}
+
+// every level's input rows start 16-byte aligned: the ring may copy with 16-byte cp.async (V = 4).  Only level 0 can
+// fail this; the intermediate low-pass images lie in the 256-byte aligned workspace with a pitch of 4 floats.
+static bool afb_rows_16b(const AfbParams& p) {
+    for (int j = 0; j < p.J; ++j) {
+        const AfbLevel& lv = p.lv[j];
+        if ((lv.x_rs & 3) || (lv.x_ps & 3) || !aligned_to(lv.x, 16)) return false;
     }
     return true;
 }
@@ -642,7 +667,10 @@ static int launch_afb_stream_t(AfbParams& p, int sms, cudaStream_t st) {
         if (rc) return rc;
     }
     afb_register_bounds(p, st);
-    afb_stream_kernel<L, S><<<(unsigned)base, kStreamNT, C::smem, st>>>(p);
+    if (afb_rows_16b(p))
+        afb_stream_kernel<L, S, 4><<<(unsigned)base, kStreamNT, C::smem, st>>>(p);
+    else
+        afb_stream_kernel<L, S, 1><<<(unsigned)base, kStreamNT, C::smem, st>>>(p);
     note_launch("afb_stream_kernel");
     const cudaError_t e = cudaGetLastError();
     return e == cudaSuccess ? B200W_OK : set_last_cuda_error(e);
@@ -760,7 +788,8 @@ static int launch_afb_owner_t(const AfbOwnerParams& op, cudaStream_t st) {
 }
 
 bool afb_owner_plan(const AfbParams& p, int L, int sms, bool force, AfbOwnerParams& op) {
-    if (!afb_stream_supported(p, L)) return false;
+    // the owner kernel's ring is instantiated with 16-byte copies only
+    if (!afb_stream_supported(p, L) || !afb_rows_16b(p)) return false;
     const bool per = p.mode == B200W_MODE_PERIODIZATION;
 #define X(LL) return per ? afb_owner_plan_t<LL, afb_shift(LL, true)>(p, sms, force, op) \
                          : afb_owner_plan_t<LL, afb_shift(LL, false)>(p, sms, force, op)

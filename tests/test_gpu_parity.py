@@ -236,9 +236,10 @@ def test_oracle_dwt_roundtrip_seeded(wave, J, mode, shape):
 
 # Full-plane oracle parity at the sizes of the cfg5 sweep (BASELINE configs[4]): here different code runs than on the
 # small golden images -- many ring segments per row, the ticketed multi-level chain over big planes, sub-band widths
-# 513 .. 519 with 4-byte aligned rows, the shifting accumulator ring of the long filters at scale.
+# 513 .. 519 with 4-byte aligned rows, the shifting accumulator ring of the long filters at scale; an odd size, whose
+# rows are not 16-byte aligned (the stream kernel's 4-byte copies) in the forward chain and the inverse's backward.
 _LARGE = [(size, wave, mode, J) for size in (1024, 2048) for wave in ("db1", "db4", "db8")
-          for mode in ("zero", "symmetric", "periodization") for J in (1, 5)]
+          for mode in ("zero", "symmetric", "periodization") for J in (1, 5)] + [(1023, "db4", "symmetric", 5)]
 
 
 @pytest.mark.parametrize("size,wave,mode,J", _LARGE, ids=["%d-%s-%s-J%d" % c for c in _LARGE])
@@ -349,6 +350,21 @@ def test_strided_and_noncontiguous_inputs():
         a_l, a_h = xfm(v)
         b_l, b_h = xfm(v.contiguous())
         assert torch.equal(a_l, b_l) and torch.equal(a_h[0], b_h[0])
+    # a three-level chain on rows that are not 16-byte aligned (the stream kernel with 4-byte copies) against the
+    # contiguous copy (16-byte copies): bit-identical, forward and backward
+    from b200wave import _cabi
+    big = torch.randn(2, 1, 1030, 1030, device=DEV)
+    xfm = b200wave.DWTForward(J=3, wave="db3", mode="symmetric").to(DEV)
+    xu = big.clone().requires_grad_()
+    xc = big[..., 3:1027, 5:1029].contiguous().requires_grad_()
+    a_l, a_h = xfm(xu[..., 3:1027, 5:1029])
+    assert _cabi.recent_kernels(1) == ["afb_stream_kernel"]
+    b_l, b_h = xfm(xc)
+    assert torch.equal(a_l, b_l) and all(torch.equal(a, b) for a, b in zip(a_h, b_h))
+    gl, gh = torch.randn_like(a_l), [torch.randn_like(h) for h in a_h]
+    (da,) = torch.autograd.grad([a_l] + a_h, xu, [gl] + gh)
+    (db,) = torch.autograd.grad([b_l] + b_h, xc, [gl] + gh)
+    assert torch.equal(da[..., 3:1027, 5:1029], db)
 
 
 def test_error_behaviour_on_gpu():
@@ -484,15 +500,15 @@ def test_host_pipeline_matches_direct_call():
         assert rel_err(dx, dx_ref.detach().cpu()) < 1e-6
 
 
-@pytest.mark.parametrize("env", ["B200W_FORCE_TILED=1", "B200W_FORCE_DIRECT=1", "B200W_OWNER=2",
-                                 "B200W_OWNER=0", "B200W_TMA=0", "B200W_TMA=0 B200W_OWNER=2",
+@pytest.mark.parametrize("env", ["B200W_FORCE_DIRECT=1", "B200W_OWNER=2", "B200W_OWNER=0", "B200W_TMA=0",
+                                 "B200W_TMA=0 B200W_OWNER=2",
                                  "B200W_TMA_NOBOXES=1 B200W_OWNER=2", "B200W_TMA_G=2 B200W_TMA_D=2 B200W_OWNER=2"])
 def test_alternative_kernel_paths(env):
     """The same golden / oracle cases through the other implementations of the path (the env switches are read
-    once per process, hence a child pytest): analysis tile kernels, direct kernels, the owner kernels forced
-    onto every multi-level shape that fits (TMA-staged ones first; B200W_TMA=0: the cp.async ones), the ticketed
-    chain kernels alone, the TMA kernels with row-by-row staging of the extension rows / with few streams and the
-    shallowest ring."""
+    once per process, hence a child pytest): direct kernels (with the store epilogue of filter_wavelet), the owner
+    kernels forced onto every multi-level shape that fits (TMA-staged ones first; B200W_TMA=0: the cp.async ones), the
+    ticketed chain kernels alone, the TMA kernels with row-by-row staging of the extension rows / with few streams and
+    the shallowest ring."""
     import subprocess
     root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
     child_env = dict(os.environ)
@@ -501,14 +517,14 @@ def test_alternative_kernel_paths(env):
         child_env[k] = v
     res = subprocess.run([sys.executable, "-m", "pytest", os.path.join(root, "tests", "test_gpu_parity.py"), "-q", "-x",
                           "-m", "gpu", "-k", "golden_dwt or golden_idwt or oracle_dwt_roundtrip or commutativity or "
-                          "owner_kernel",
+                          "owner_kernel or filter_wavelet",
                           "-p", "no:cacheprovider"],
                          cwd=root, env=child_env, stdout=subprocess.PIPE, stderr=subprocess.STDOUT, text=True,
                          timeout=1500)
     assert res.returncode == 0, res.stdout[-3000:]
 
 
-@pytest.mark.parametrize("env", ["B200W_OWNER=0", "B200W_OWNER=2", "B200W_TMA=0", "B200W_FORCE_TILED=1"])
+@pytest.mark.parametrize("env", ["B200W_OWNER=0", "B200W_OWNER=2", "B200W_TMA=0"])
 def test_large_planes_other_policies(env):
     """The large-plane oracle comparisons through the other kernel-selection policies (child pytest: the switches are
     read once per process)."""
@@ -667,7 +683,8 @@ def test_filter_wavelet_matches_unfused_path(shape):
 
 
 def test_filter_wavelet_other_filters_and_errors():
-    """Longer filters and other modes go through the same epilogue (stream ring, border items, direct kernel)."""
+    """Longer filters and other modes go through the same epilogue (stream ring with 16- and 4-byte copies, border
+    items)."""
     from b200wave import fsd, ops
     rng = np.random.default_rng(5)
     for wave, mode, shape in [("db2", "symmetric", (2, 1, 96, 200)), ("db4", "zero", (1, 2, 301, 77)),
@@ -681,7 +698,7 @@ def test_filter_wavelet_other_filters_and_errors():
             assert torch.equal(got[1 + b], hi[:, :, b] * 0.5 + 0.5)
         cat = fsd.WaveletFilter(cs="cat", variant="B", wave=wave, mode=mode).to(DEV)(x, False)[0]
         assert torch.equal(cat, torch.cat((hi[:, :, 0], hi[:, :, 1], hi[:, :, 2]), 1))
-        # a strided (non 16-byte-aligned) view takes the direct kernel
+        # a strided view: rows that are not 16-byte aligned (4-byte copies into the stream kernel's ring)
         xs = x[..., 1:]
         lls, (his,) = b200wave.DWTForward(J=1, wave=wave, mode=mode).to(DEV)(xs)
         gs = filt(xs)
