@@ -6,6 +6,8 @@ Drop-in surface (same names and signatures as the reference):
 * ``DWTForward``, ``DWTInverse`` and the aliases ``DWT``, ``IDWT``, ``DWT2D``, ``IDWT2D``
   (``pytorch_wavelets/__init__.py:24-33``), ``dwt.lowlevel.AFB2D`` / ``SFB2D`` / ``afb2d`` / ``sfb2d``
 * ``DWT1DForward``, ``DWT1DInverse`` (aliases ``DWT1D``, ``IDWT1D``), ``dwt.lowlevel.AFB1D`` / ``SFB1D``
+* ``SWTForward`` and its periodic inverse ``SWTInverse`` (the reference has no usable one), ``dwt.lowlevel.afb2d_atrous`` /
+  ``sfb2d_atrous``
 * ``SSIM``, ``ssim`` (``ssim.py``)
 * ``freq.high_pass``, ``freq.low_pass`` (``utils.py:93-117``) and the batched ``freq.gaussian_split``
 * ``HostPipeline``: host-buffer front end (chunked, stream-overlapped H2D | kernels | D2H)
@@ -16,7 +18,7 @@ there is no CPU path.
 from . import ops  # noqa: F401  (registers torch.ops.b200wave.*)
 from . import dwt  # noqa: F401
 from .dwt import lowlevel  # noqa: F401
-from .dwt.transform2d import DWTForward, DWTInverse, SWTForward
+from .dwt.transform2d import DWTForward, DWTInverse, SWTForward, SWTInverse
 from .dwt.transform1d import DWT1DForward, DWT1DInverse
 from .ssim import SSIM, ssim
 from .wavelets import Wavelet, wavelist  # noqa: F401
@@ -36,5 +38,5 @@ DWT1D = DWT1DForward
 IDWT1D = DWT1DInverse
 
 __all__ = ["DWTForward", "DWTInverse", "DWT", "IDWT", "DWT2D", "IDWT2D", "DWT1DForward", "DWT1DInverse", "DWT1D", "IDWT1D", "SWTForward",
-           "SSIM", "ssim", "lowlevel",
+           "SWTInverse",           "SSIM", "ssim", "lowlevel",
            "Wavelet", "wavelist", "HostPipeline", "TVLoss", "phase_consistency_loss", "__version__"]

@@ -21,7 +21,7 @@ LIB_DIR = os.path.join(PKG_DIR, "_lib")
 LIB_PATH = os.path.join(LIB_DIR, "libb200wave.so")
 STAMP = os.path.join(LIB_DIR, "libb200wave.stamp")
 
-SOURCES = ["api.cu", "dwt.cu", "dwt_stream_afb.cu", "dwt_stream_sfb.cu", "dwt_tma_afb.cu", "dwt_tma_sfb.cu", "dwt1d.cu", "swt.cu", "ssim.cu", "ssim_f64.cu", "freq.cu", "tv.cu"]
+SOURCES = ["api.cu", "dwt.cu", "dwt_stream_afb.cu", "dwt_stream_sfb.cu", "dwt_tma_afb.cu", "dwt_tma_sfb.cu", "dwt1d.cu", "swt.cu", "swt_inverse.cu", "ssim.cu", "ssim_f64.cu", "freq.cu", "tv.cu"]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a",
     "-O3", "-lineinfo", "-std=c++17",

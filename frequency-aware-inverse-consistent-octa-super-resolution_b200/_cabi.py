@@ -85,6 +85,10 @@ SYMBOLS = {
                                  _vp]),
     "b200w_swt2d_bwd_f64": (_i, [_vp, _i, _i, _i, _c_double_p, _c_double_p, _c_double_p, _c_double_p, _i, _i, _i, _vp,
                                  _vp]),
+    "b200w_iswt2d_f32": (_i, [_vp, _i64, _vp, _i, _i, _i, _c_float_p, _c_float_p, _c_float_p, _c_float_p, _i, _i, _vp,
+                              _vp]),
+    "b200w_iswt2d_f64": (_i, [_vp, _i64, _vp, _i, _i, _i, _c_double_p, _c_double_p, _c_double_p, _c_double_p, _i, _i,
+                              _vp, _vp]),
     "b200w_tv_workspace_bytes_f64": (_sz, [_i, _i]),
     "b200w_tv_fwd_f64": (_i, [_vp, _i, _i, _i, _vp, _sz, _vp, _vp]),
     "b200w_tv_bwd_f64": (_i, [_vp, _vp, ctypes.c_double, ctypes.c_double, _i, _i, _i, _vp, _vp]),

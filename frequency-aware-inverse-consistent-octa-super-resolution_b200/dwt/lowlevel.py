@@ -154,6 +154,28 @@ def afb2d_atrous(x, filts, mode="periodization", dilation=1):
               mode_to_int(mode), int(dilation))
 
 
+def sfb2d_atrous(y, filts, mode="periodic", dilation=1, ll=None):
+    """One undecimated 2-D synthesis level, the functional mirror of ``afb2d_atrous`` and the inverse of it in periodic
+    mode: y (N, 4C, H, W) as ``afb2d_atrous`` returns it -> (N, C, H, W).  ``ll`` (N, C, H, W) replaces band 0 of ``y``
+    (the low band reconstructed from the coarser levels; default: band 0 of ``y`` itself).  ``filts`` = (g0, g1) or
+    (g0_col, g1_col, g0_row, g1_row): synthesis taps, arrays or ``prep_filt_sfb2d`` tensors; ``*_row`` run along W,
+    ``*_col`` along H, as the analysis filters of ``afb2d_atrous`` do.  Only ``mode='periodic'`` has an exact
+    undecimated inverse; any other mode raises ``ValueError``."""
+    if len(filts) == 2:
+        filts = (filts[0], filts[1], filts[0], filts[1])
+    elif len(filts) != 4:
+        raise ValueError("Unknown form for input filts")
+    if mode != "periodic":
+        raise ValueError("sfb2d_atrous: only periodic extension ('periodic') has an exact undecimated inverse, got %r"
+                         % (mode,))
+    g0_col, g1_col, g0_row, g1_row = filts
+    if ll is None:
+        ll = y[:, 0::4]
+    op = ops64.iswt2d if y.dtype == torch.float64 else ops.iswt2d
+    return op(ll, y, _as_taps(g0_row, False), _as_taps(g1_row, False), _as_taps(g0_col, False),
+              _as_taps(g1_col, False), int(dilation))
+
+
 def _four_filters(filts, prep, device=None):
     """Normalise the ``filts`` argument of afb2d / sfb2d to (col_lo, col_hi, row_lo, row_hi) tensors.
     A pair means "same filters on both axes"; raw arrays go through ``prep``; prepared tensors are

@@ -140,3 +140,44 @@ class SWTForward(nn.Module):
             n, c4, h, w = y.shape
             ll = y.view(n, c4 // 4, 4, h, w)[:, :, 0]
         return coeffs
+
+
+class SWTInverse(nn.Module):
+    """Inverse of ``SWTForward`` with ``mode='periodic'``; ``forward(coeffs)`` takes the list ``SWTForward`` returns
+    (finest level first, each (N, 4C, H, W)) and gives back the (N, C, H, W) image.  Buffers ``g0_col, g1_col, g0_row,
+    g1_row`` as in ``DWTInverse``.  Each level is one launch of the a-trous synthesis kernel (``csrc/swt_inverse.cu``)
+    with dilation 2**j, coarsest first; it starts from band 0 of the coarsest level, read in place, and never reads band
+    0 of the finer levels.
+
+    The reference offers no usable inverse (its ``swt_inverse.py`` is unfinished and not exported), so the semantics
+    are defined here (DESIGN.md K12): each axis is undone by the synthesis pair of the wavelet, halved.  Only periodic
+    extension has an exact undecimated inverse; any other mode raises ``ValueError`` at construction.
+    """
+
+    def __init__(self, wave="db1", mode="periodic"):
+        super().__init__()
+        if mode != "periodic":
+            raise ValueError("SWTInverse: only periodic extension (mode='periodic') has an exact undecimated inverse; "
+                             "got mode %r" % (mode,))
+        filts = lowlevel.prep_filt_sfb2d(*_filters_from(wave, ("rec_lo", "rec_hi")))
+        for name, f in zip(("g0_col", "g1_col", "g0_row", "g1_row"), filts):
+            self.register_buffer(name, f)
+        self.mode = mode
+
+    def forward(self, coeffs):
+        coeffs = list(coeffs)
+        if not coeffs:
+            raise ValueError("SWTInverse: coeffs is empty; expected the list SWTForward returns")
+        shape = tuple(coeffs[0].shape)
+        if len(shape) != 4 or shape[1] % 4:
+            raise ValueError("SWTInverse: coefficients must be (N, 4C, H, W), got %s" % (shape,))
+        for j, c in enumerate(coeffs):
+            if tuple(c.shape) != shape:
+                raise ValueError("SWTInverse: coeffs[%d] has shape %s, coeffs[0] %s; every level must have the same "
+                                 "shape" % (j, tuple(c.shape), shape))
+            lowlevel._is_f64(c, self.g0_col)   # double coefficients need double filters and vice versa
+        filts = (self.g0_col, self.g1_col, self.g0_row, self.g1_row)
+        ll = coeffs[-1][:, 0::4]
+        for j in range(len(coeffs) - 1, -1, -1):
+            ll = lowlevel.sfb2d_atrous(coeffs[j], filts, self.mode, 2 ** j, ll=ll)
+        return ll

@@ -38,6 +38,7 @@ _LIB.define("sfb1d(Tensor low, Tensor? high, float[] g0, float[] g1, int mode, i
 _LIB.define("swt2d(Tensor x, float[] w_lo, float[] w_hi, float[] h_lo, float[] h_hi, int mode, int dilation) -> Tensor")
 _LIB.define("swt2d_adjoint(Tensor dy, float[] w_lo, float[] w_hi, float[] h_lo, float[] h_hi, int mode, int dilation) "
             "-> Tensor")
+_LIB.define("iswt2d(Tensor ll, Tensor y, float[] w_lo, float[] w_hi, float[] h_lo, float[] h_hi, int dilation) -> Tensor")
 _LIB.define("ssim_fwd(Tensor img1, Tensor img2, float[] win, bool size_average, int n_maps) -> (Tensor, Tensor)")
 _LIB.define("ssim_bwd(Tensor img1, Tensor img2, Tensor maps, Tensor grad_out, float[] win, bool size_average, "
             "bool need_d2) -> (Tensor, Tensor)")
@@ -668,6 +669,78 @@ def _swt2d_backward(ctx, dy):
     return dx, None, None, None, None, None, None
 
 
+# ------------------------------------------------------------------------------------------- inverse SWT
+PERIODIC = 6
+
+
+def iswt_layout(ll, y, name):
+    """Checks the shapes of one inverse-SWT level and returns (ll as (tensor, plane stride), dense y); copies only what
+    the kernel cannot read in place: ll needs unit column stride, row stride W and uniform plane spacing."""
+    if ll.dim() != 4 or y.dim() != 4:
+        raise IndexError("%s expects 4-D ll (N, C, H, W) and y (N, 4C, H, W), got %d-D and %d-D"
+                         % (name, ll.dim(), y.dim()))
+    N, C4, H, W = y.shape
+    if C4 % 4 or tuple(ll.shape) != (N, C4 // 4, H, W):
+        raise RuntimeError("%s: y must be (N, 4C, H, W) and ll (N, C, H, W), got %s and %s"
+                           % (name, tuple(y.shape), tuple(ll.shape)))
+    lk, ps, rs = _planes_view(ll)
+    if rs != W and H > 1:
+        lk = ll.contiguous()
+        ps = H * W
+    return lk, ps, y.contiguous()
+
+
+def iswt_adjoint_taps(w_lo, w_hi, h_lo, h_hi):
+    """The inverse level is (1/4) x the transpose of an analysis level with the synthesis taps: halved taps (exact)."""
+    return [[0.5 * float(v) for v in t] for t in (w_lo, w_hi, h_lo, h_hi)]
+
+
+def _iswt2d_cuda(ll, y, w_lo, w_hi, h_lo, h_hi, dilation):
+    _require_cuda_f32(ll, "iswt2d")
+    _require_cuda_f32(y, "iswt2d")
+    if not (len(w_lo) == len(w_hi) == len(h_lo) == len(h_hi)):
+        raise RuntimeError("b200wave::iswt2d: all four filters must have the same length")
+    lk, ps, yk = iswt_layout(ll, y, "b200wave::iswt2d")
+    N, C4, H, W = yk.shape
+    x = torch.empty((N, C4 // 4, H, W), device=y.device, dtype=torch.float32)
+    if x.numel() == 0:
+        return x
+    lib = _cabi.load()
+    a = [_cabi.taps_array(t)[0] for t in (w_lo, w_hi, h_lo, h_hi)]
+    with torch.cuda.device(y.device):
+        rc = lib.b200w_iswt2d_f32(lk.data_ptr(), ps, yk.data_ptr(), N * (C4 // 4), H, W, a[0], a[1], a[2], a[3],
+                                  len(w_lo), int(dilation), x.data_ptr(), _stream())
+    _cabi.check(rc)
+    return x
+
+
+def _iswt2d_setup(ctx, inputs, output):
+    ll, y, w_lo, w_hi, h_lo, h_hi, dilation = inputs
+    ctx.taps = iswt_adjoint_taps(w_lo, w_hi, h_lo, h_hi)
+    ctx.dilation = dilation
+
+
+def iswt2d_backward(swt2d_op, ctx, dx):
+    """Transpose of the level: the analysis kernel with the halved synthesis taps; band 0 of its output is the gradient
+    of ll, bands 1..3 that of y (whose band 0 the level never reads)."""
+    need_ll, need_y = ctx.needs_input_grad[0], ctx.needs_input_grad[1]
+    if dx is None or not (need_ll or need_y):
+        return (None,) * 7
+    g = swt2d_op(dx, *ctx.taps, PERIODIC, ctx.dilation)
+    N, C4, H, W = g.shape
+    g5 = g.view(N, C4 // 4, 4, H, W)
+    dll = g5[:, :, 0].clone() if need_ll else None
+    dy = None
+    if need_y:
+        g5[:, :, 0] = 0
+        dy = g
+    return (dll, dy) + (None,) * 5
+
+
+def _iswt2d_backward(ctx, dx):
+    return iswt2d_backward(torch.ops.b200wave.swt2d, ctx, dx)
+
+
 # ------------------------------------------------------------------------------------------- ssim
 def _ssim_common(img1, img2, win, name):
     _require_cuda_f32(img1, name)
@@ -763,6 +836,7 @@ _LIB.impl("afb1d", _afb1d_cuda, "CUDA")
 _LIB.impl("swt2d", _swt2d_cuda, "CUDA")
 _LIB.impl("swt2d_adjoint", _swt2d_adjoint_cuda, "CUDA")
 _LIB.impl("sfb1d", _sfb1d_cuda, "CUDA")
+_LIB.impl("iswt2d", _iswt2d_cuda, "CUDA")
 
 
 def _cpu_refuse(name):
@@ -773,7 +847,7 @@ def _cpu_refuse(name):
 
 
 for _name in ("afb2d", "afb2d_select", "sfb2d", "dwt2", "idwt2", "ssim_fwd", "ssim_bwd", "afb1d", "sfb1d", "swt2d",
-              "swt2d_adjoint"):
+              "swt2d_adjoint", "iswt2d"):
     _LIB.impl(_name, _cpu_refuse(_name), "CPU")
 
 torch.library.register_fake("b200wave::afb2d", _afb2d_fake, lib=_LIB)
@@ -789,6 +863,9 @@ torch.library.register_fake("b200wave::swt2d_adjoint", lambda dy, wl, wh, hl, hh
                             dy.new_empty((dy.shape[0], dy.shape[1] // 4, dy.shape[2], dy.shape[3])), lib=_LIB)
 torch.library.register_autograd("b200wave::swt2d", _swt2d_backward, setup_context=_swt2d_setup, lib=_LIB)
 torch.library.register_fake("b200wave::sfb1d", _sfb1d_fake, lib=_LIB)
+torch.library.register_fake("b200wave::iswt2d", lambda ll, y, wl, wh, hl, hh, d:
+                            y.new_empty((y.shape[0], y.shape[1] // 4, y.shape[2], y.shape[3])), lib=_LIB)
+torch.library.register_autograd("b200wave::iswt2d", _iswt2d_backward, setup_context=_iswt2d_setup, lib=_LIB)
 torch.library.register_autograd("b200wave::afb1d", _afb1d_backward, setup_context=_afb1d_setup, lib=_LIB)
 torch.library.register_autograd("b200wave::sfb1d", _sfb1d_backward, setup_context=_sfb1d_setup, lib=_LIB)
 torch.library.register_fake("b200wave::idwt2", _idwt2_fake, lib=_LIB)
@@ -807,6 +884,8 @@ ssim_fwd = torch.ops.b200wave.ssim_fwd
 ssim_bwd = torch.ops.b200wave.ssim_bwd
 afb1d = torch.ops.b200wave.afb1d
 swt2d = torch.ops.b200wave.swt2d
+swt2d_adjoint = torch.ops.b200wave.swt2d_adjoint
+iswt2d = torch.ops.b200wave.iswt2d
 sfb1d = torch.ops.b200wave.sfb1d
 
 

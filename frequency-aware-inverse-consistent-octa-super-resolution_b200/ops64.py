@@ -8,7 +8,8 @@ stream, CUDA-only, the same backward structure -- on double tensors with double 
   ``DWTForward`` / ``DWTInverse`` run fp64 transforms level by level through them (precision, not speed, is the point
   of this path).  ``afb2d`` backward = ``sfb2d`` with the analysis taps + crop, ``sfb2d`` backward = ``afb2d`` with the
   synthesis taps.
-* ``afb1d`` / ``sfb1d`` (``csrc/dwt1d.cu``), ``swt2d`` / ``swt2d_adjoint`` (``csrc/swt.cu``), ``tv_sums`` / ``tv_grad``
+* ``afb1d`` / ``sfb1d`` (``csrc/dwt1d.cu``), ``swt2d`` / ``swt2d_adjoint`` (``csrc/swt.cu``), ``iswt2d``
+  (``csrc/swt_inverse.cu``), ``tv_sums`` / ``tv_grad``
   (``csrc/tv.cu``): the fp32 kernels instantiated for ``double``.  As in fp32, ``losses.TVLoss`` differentiates
   ``tv_sums`` through ``tv_grad`` (once differentiable).
 * ``ssim_fwd`` / ``ssim_bwd`` (``csrc/ssim_f64.cu``): ``win`` is the DENSE ws x ws window, row-major (in double the
@@ -21,7 +22,8 @@ stream, CUDA-only, the same backward structure -- on double tensors with double 
 import torch
 
 from . import _cabi
-from .ops import _check_mode, _check_swt_mode, _mode_name, _planes_view, _rows_view, _stream, coeff_len, idwt_len
+from .ops import (_check_mode, _check_swt_mode, _mode_name, _planes_view, _rows_view, _stream, coeff_len, idwt_len,
+                  iswt2d_backward, iswt_adjoint_taps, iswt_layout)
 
 _LIB = torch.library.Library("b200wave64", "DEF")
 _LIB.define("afb2d(Tensor x, float[] w_lo, float[] w_hi, float[] h_lo, float[] h_hi, int mode) -> (Tensor, Tensor)")
@@ -32,6 +34,7 @@ _LIB.define("sfb1d(Tensor low, Tensor? high, float[] g0, float[] g1, int mode, i
 _LIB.define("swt2d(Tensor x, float[] w_lo, float[] w_hi, float[] h_lo, float[] h_hi, int mode, int dilation) -> Tensor")
 _LIB.define("swt2d_adjoint(Tensor dy, float[] w_lo, float[] w_hi, float[] h_lo, float[] h_hi, int mode, int dilation) "
             "-> Tensor")
+_LIB.define("iswt2d(Tensor ll, Tensor y, float[] w_lo, float[] w_hi, float[] h_lo, float[] h_hi, int dilation) -> Tensor")
 _LIB.define("ssim_fwd(Tensor img1, Tensor img2, float[] win, bool size_average, int n_maps) -> (Tensor, Tensor)")
 _LIB.define("ssim_bwd(Tensor img1, Tensor img2, Tensor maps, Tensor grad_out, float[] win, bool size_average, "
             "bool need_d2) -> (Tensor, Tensor)")
@@ -381,6 +384,36 @@ def _swt2d_backward(ctx, dy):
     return dx, None, None, None, None, None, None
 
 
+# ------------------------------------------------------------------------------------------- inverse SWT
+def _iswt2d_cuda(ll, y, w_lo, w_hi, h_lo, h_hi, dilation):
+    _require_cuda_f64(ll, "iswt2d")
+    _require_cuda_f64(y, "iswt2d")
+    if not (len(w_lo) == len(w_hi) == len(h_lo) == len(h_hi)):
+        raise RuntimeError("b200wave64::iswt2d: all four filters must have the same length")
+    lk, ps, yk = iswt_layout(ll, y, "b200wave64::iswt2d")
+    N, C4, H, W = yk.shape
+    x = torch.empty((N, C4 // 4, H, W), device=y.device, dtype=torch.float64)
+    if x.numel() == 0:
+        return x
+    lib = _cabi.load()
+    a = _taps(w_lo, w_hi, h_lo, h_hi)
+    with torch.cuda.device(y.device):
+        rc = lib.b200w_iswt2d_f64(lk.data_ptr(), ps, yk.data_ptr(), N * (C4 // 4), H, W, a[0], a[1], a[2], a[3],
+                                  len(w_lo), int(dilation), x.data_ptr(), _stream())
+    _cabi.check(rc)
+    return x
+
+
+def _iswt2d_setup(ctx, inputs, output):
+    ll, y, w_lo, w_hi, h_lo, h_hi, dilation = inputs
+    ctx.taps = iswt_adjoint_taps(w_lo, w_hi, h_lo, h_hi)
+    ctx.dilation = dilation
+
+
+def _iswt2d_backward(ctx, dx):
+    return iswt2d_backward(torch.ops.b200wave64.swt2d, ctx, dx)
+
+
 # ------------------------------------------------------------------------------------------- ssim
 def _ssim_common(img1, img2, win, name):
     _require_cuda_f64(img1, name)
@@ -565,6 +598,7 @@ _LIB.impl("afb1d", _afb1d_cuda, "CUDA")
 _LIB.impl("sfb1d", _sfb1d_cuda, "CUDA")
 _LIB.impl("swt2d", _swt2d_cuda, "CUDA")
 _LIB.impl("swt2d_adjoint", _swt2d_adjoint_cuda, "CUDA")
+_LIB.impl("iswt2d", _iswt2d_cuda, "CUDA")
 _LIB.impl("ssim_fwd", _ssim_fwd_cuda, "CUDA")
 _LIB.impl("ssim_bwd", _ssim_bwd_cuda, "CUDA")
 _LIB.impl("tv_sums", _tv_sums_cuda, "CUDA")
@@ -574,7 +608,7 @@ _LIB.impl("freq_mask_", _freq_mask_cuda, "CUDA")
 _LIB.impl("abs_sign", _abs_sign_cuda, "CUDA")
 _LIB.impl("sign_mul", _sign_mul_cuda, "CUDA")
 for _name in ("afb2d", "sfb2d", "afb1d", "sfb1d", "swt2d", "swt2d_adjoint", "ssim_fwd", "ssim_bwd", "tv_sums",
-              "tv_grad", "afb2d_select", "freq_mask_", "abs_sign", "sign_mul"):
+              "tv_grad", "afb2d_select", "freq_mask_", "abs_sign", "sign_mul", "iswt2d"):
     _LIB.impl(_name, _cpu_refuse(_name), "CPU")
 torch.library.register_fake("b200wave64::afb2d", _afb2d_fake, lib=_LIB)
 torch.library.register_fake("b200wave64::sfb2d", _sfb2d_fake, lib=_LIB)
@@ -593,6 +627,9 @@ torch.library.register_autograd("b200wave64::sfb2d", _sfb2d_backward, setup_cont
 torch.library.register_autograd("b200wave64::afb1d", _afb1d_backward, setup_context=_afb1d_setup, lib=_LIB)
 torch.library.register_autograd("b200wave64::sfb1d", _sfb1d_backward, setup_context=_sfb1d_setup, lib=_LIB)
 torch.library.register_autograd("b200wave64::swt2d", _swt2d_backward, setup_context=_swt2d_setup, lib=_LIB)
+torch.library.register_fake("b200wave64::iswt2d", lambda ll, y, wl, wh, hl, hh, d:
+                            y.new_empty((y.shape[0], y.shape[1] // 4, y.shape[2], y.shape[3])), lib=_LIB)
+torch.library.register_autograd("b200wave64::iswt2d", _iswt2d_backward, setup_context=_iswt2d_setup, lib=_LIB)
 torch.library.register_autograd("b200wave64::ssim_fwd", _ssim_backward, setup_context=_ssim_setup, lib=_LIB)
 torch.library.register_fake("b200wave64::afb2d_select", _afb2d_select_fake, lib=_LIB)
 torch.library.register_autograd("b200wave64::afb2d_select", _afb2d_select_backward, setup_context=_afb2d_select_setup,
@@ -604,6 +641,7 @@ afb1d = torch.ops.b200wave64.afb1d
 sfb1d = torch.ops.b200wave64.sfb1d
 swt2d = torch.ops.b200wave64.swt2d
 swt2d_adjoint = torch.ops.b200wave64.swt2d_adjoint
+iswt2d = torch.ops.b200wave64.iswt2d
 ssim_fwd = torch.ops.b200wave64.ssim_fwd
 ssim_bwd = torch.ops.b200wave64.ssim_bwd
 tv_sums = torch.ops.b200wave64.tv_sums

@@ -24,6 +24,8 @@
  *                       utils.py:71-117  Gaussian low / high pass in the Fourier domain (SURVEY.md 8f row 1)
  *   b200w_afb1d_f32 / b200w_sfb1d_f32             pw/dwt/lowlevel.py:368-424, 697-743  AFB1D / SFB1D (SURVEY.md 8f row 3)
  *   b200w_swt2d_fwd_f32 / b200w_swt2d_bwd_f32     pw/dwt/lowlevel.py:175-223, 475-521  afb2d_atrous / SWTForward (8f row 3)
+ *   b200w_iswt2d_f32 / b200w_iswt2d_f64           one level of SWTInverse, the periodic inverse of SWTForward (the
+ *                       reference's pw/dwt/swt_inverse.py is unfinished and not exported: semantics in DESIGN.md K12)
  *   b200w_tv_fwd_f32 / b200w_tv_bwd_f32           model.py:17-33  TVLoss (SURVEY.md 8f row 4)
  *   b200w_phase_sums_c64 / b200w_phase_grad_c64   model.py:36-58  phase_consistency_loss (SURVEY.md 8f row 4)
  *   b200w_*_f64         the same bodies on double tensors (the reference's double mode): afb2d / sfb2d, afb2d_ex,
@@ -281,6 +283,25 @@ int b200w_swt2d_fwd_f32(const float* x, int planes, int H, int W, const float* w
                         const float* h_lo, const float* h_hi, int L, int dilation, int mode, float* y, void* stream);
 int b200w_swt2d_bwd_f32(const float* dy, int planes, int H, int W, const float* w_lo, const float* w_hi,
                         const float* h_lo, const float* h_hi, int L, int dilation, int mode, float* dx, void* stream);
+
+/*
+ * Undecimated (a trous) 2-D synthesis, one level of SWTInverse (DESIGN.md K12): the exact inverse of SWTForward with
+ * mode 'periodic', the only extension for which an undecimated synthesis bank is exact (hence no mode argument).
+ * With pl = floor(L * dilation / 2) - dilation,
+ *   x[r][c] = sum_{a,e} sum_{jh,jw} (h_e[jh] / 2) (w_a[jw] / 2) y_{2a+e}[(r - d jh + pl) mod H][(c - d jw + pl) mod W]
+ * where y_0 = ll and y_1..y_3 = bands 1..3 of `y`.
+ *   ll: (planes, H, W), unit column stride, plane stride `ll_ps` elements (4 H W when ll is band 0 of the coarsest
+ *       level's coefficients, H W for a reconstructed level); `y`: dense (planes, 4, H, W), band 0 is not read;
+ *   x: dense (planes, H, W).  Taps: synthesis taps as prep_filt_sfb2d stores them (not reversed), `w_*` along W (g*_row),
+ *   `h_*` along H (g*_col); the factor 1/2 per axis is applied inside.  The shapes are those b200w_swt2d_fwd_* accepts:
+ *   2 <= L <= B200W_MAX_TAPS, dilation >= 1, H * W < 2^31, floor(L * dilation / 2) <= 3 * min(H, W).
+ *   Both return the same codes, in the same order, before any launch.
+ */
+int b200w_iswt2d_f32(const float* ll, int64_t ll_ps, const float* y, int planes, int H, int W, const float* w_lo,
+                     const float* w_hi, const float* h_lo, const float* h_hi, int L, int dilation, float* x, void* stream);
+int b200w_iswt2d_f64(const double* ll, int64_t ll_ps, const double* y, int planes, int H, int W, const double* w_lo,
+                     const double* w_hi, const double* h_lo, const double* h_hi, int L, int dilation, double* x,
+                     void* stream);
 
 /*
  * Double twins of the 1-D, a trous and TV entry points above (the reference's double mode: modules built under

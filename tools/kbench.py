@@ -1,7 +1,7 @@
 """Kernel micro-benchmark: per-launch duration of single levels / SSIM kernels (CUDA graph of back-to-back
 launches over rotating inputs larger than L2, CUDA events).
 
-    python tools/kbench.py [dwt|ssim|all]
+    python tools/kbench.py [dwt|ssim|swt|iswt|dwt1d|fsd|freq|tv|all]
 """
 import os
 import sys
@@ -158,7 +158,36 @@ def swt_case(n, h, w, wave, mode, dilation):
         wave, mode, dilation, n, h, w, t * 1e6, b / t / 1e9, b / t / 1e9 / PEAK * 100), flush=True)
 
 
+def iswt_case(n, h, w, wave, dilation):
+    """One level of SWTInverse (the a-trous synthesis kernel) and the same level through the adjoint route (the analysis
+    kernel's gather-form adjoint with the halved synthesis taps, swt2d_adjoint); ll is band 0 of the coefficients, as at
+    the top level.  Algorithmic bytes 20 B/px: 4 planes read, 1 written."""
+    nsets = max(2, int(2 * 126e6 * 1.05 / (16 * n * h * w)) + 1)
+    ys = [torch.randn(n, 4, h, w, device=dev) for _ in range(nsets)]
+    m = b200wave.SWTInverse(wave=wave).to(dev)
+    filts = (m.g0_col, m.g1_col, m.g0_row, m.g1_row)
+    half = ops.iswt_adjoint_taps(*[lowlevel.host_taps(f) for f in (m.g0_row, m.g1_row, m.g0_col, m.g1_col)])
+    with torch.no_grad():
+        ref = ops.swt2d_adjoint(ys[0], *half, ops.PERIODIC, dilation)
+        err = ((lowlevel.sfb2d_atrous(ys[0], filts, "periodic", dilation) - ref).abs().max() / ref.abs().max()).item()
+        tk = timeit(lambda i: lowlevel.sfb2d_atrous(ys[i % nsets], filts, "periodic", dilation), nsets)
+        ta = timeit(lambda i: ops.swt2d_adjoint(ys[i % nsets], *half, ops.PERIODIC, dilation), nsets, 10)
+    b = 20.0 * n * h * w
+    print("iswt  %-5s d=%-2d %4dx%4dx%4d  kernel %8.1f us %6.0f GB/s (%4.1f%%) | adjoint route %9.1f us %6.0f GB/s "
+          "(%4.1f%%) | x%.1f | rel diff %.1e" % (
+              wave, dilation, n, h, w, tk * 1e6, b / tk / 1e9, b / tk / 1e9 / PEAK * 100, ta * 1e6, b / ta / 1e9,
+              b / ta / 1e9 / PEAK * 100, ta / tk, err), flush=True)
+
+
 what = (sys.argv[1] if len(sys.argv) > 1 else "all") if __name__ == "__main__" else "none"
+if what in ("iswt", "all"):
+    import subprocess
+    print("device:", subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit,clocks.max.sm", "--format=csv,noheader",
+                                     "-i", "0"], capture_output=True, text=True).stdout.strip(), flush=True)
+    for wave in ("haar", "db2", "db8"):
+        iswt_case(64, 304, 304, wave, 1)
+        for d in (1, 4, 16):
+            iswt_case(64, 1024, 1024, wave, d)
 if what in ("dwt1d", "all"):
     dwt1d_case(64, 1 << 20, "db3", "symmetric")
     dwt1d_case(64, 1 << 20, "haar", "zero")
