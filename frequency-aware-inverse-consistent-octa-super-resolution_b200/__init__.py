@@ -8,7 +8,8 @@ Drop-in surface (same names and signatures as the reference):
 * ``DWT1DForward``, ``DWT1DInverse`` (aliases ``DWT1D``, ``IDWT1D``), ``dwt.lowlevel.AFB1D`` / ``SFB1D``
 * ``SWTForward`` and its periodic inverse ``SWTInverse`` (the reference has no usable one), ``dwt.lowlevel.afb2d_atrous`` /
   ``sfb2d_atrous``
-* ``SSIM``, ``ssim`` (``ssim.py``)
+* ``SSIM``, ``ssim`` (``ssim.py``), and the multi-scale ``MS_SSIM``, ``ms_ssim`` built on the same kernels (the
+  reference has no MS-SSIM; ``msssim.py`` defines it)
 * ``freq.high_pass``, ``freq.low_pass`` (``utils.py:93-117``) and the batched ``freq.gaussian_split``
 * ``HostPipeline``: host-buffer front end (chunked, stream-overlapped H2D | kernels | D2H)
 
@@ -21,6 +22,7 @@ from .dwt import lowlevel  # noqa: F401
 from .dwt.transform2d import DWTForward, DWTInverse, SWTForward, SWTInverse
 from .dwt.transform1d import DWT1DForward, DWT1DInverse
 from .ssim import SSIM, ssim
+from .msssim import MS_SSIM, ms_ssim
 from .wavelets import Wavelet, wavelist  # noqa: F401
 from .hostpipe import HostPipeline
 from . import freq  # noqa: F401  (utils.high_pass / low_pass, SURVEY 8f row 1)
@@ -38,5 +40,5 @@ DWT1D = DWT1DForward
 IDWT1D = DWT1DInverse
 
 __all__ = ["DWTForward", "DWTInverse", "DWT", "IDWT", "DWT2D", "IDWT2D", "DWT1DForward", "DWT1DInverse", "DWT1D", "IDWT1D", "SWTForward",
-           "SWTInverse",           "SSIM", "ssim", "lowlevel",
+           "SWTInverse",           "SSIM", "ssim", "MS_SSIM", "ms_ssim", "lowlevel",
            "Wavelet", "wavelist", "HostPipeline", "TVLoss", "phase_consistency_loss", "__version__"]

@@ -33,6 +33,12 @@ constexpr int kHR = kCR + 2 * kHalo;         // 42 horizontally-blurred rows res
 // backward: two (its 3-4 staged maps are loaded a whole chunk ahead)
 template <bool FWD> constexpr int kSsimStageBufs = FWD ? 1 : 2;
 
+// options of the MS-SSIM scale instantiations (0: the plain SSIM kernels)
+constexpr int kOptMs = 1;    // fwd: the map value by correctly rounded division, so identical images give exactly 1
+constexpr int kOptCs = 2;    // fwd: the contrast-structure map cs = A2/B2 and its derivative maps instead of S
+constexpr int kOptPool = 4;  // fwd: also write avg_pool2d(img1, 2) and avg_pool2d(img2, 2)
+constexpr int kOptUp = 8;    // bwd: add 0.25 up[r/2][c/2] (the transpose of that pooling) to d1 / d2
+
 struct SsimParams {
     const float* in[4];   // fwd: img1, img2 ; bwd: maps 0..3
     const float* img1;    // bwd epilogue
@@ -54,6 +60,12 @@ struct SsimParams {
     float2 wa[6];
     float2 wb[6];
     float2 w2[kWin];
+    // MS-SSIM scale fields, after the plain SSIM ones so that those keep their parameter offsets
+    float* pooled1;       // fwd (kOptPool): (planes, Hp, Wp)
+    float* pooled2;
+    const float* up1;     // bwd (kOptUp): (planes, Hp, Wp) or null
+    const float* up2;
+    int Hp, Wp;           // H / 2, W / 2
 };
 
 // Stage rows [row0, row0+nrows) x cols [C0-8, C0+72) of one plane into dst[nrows][kPW] with cp.async, zero
@@ -85,7 +97,7 @@ __device__ __forceinline__ int hbuf_col(int c) { return ((((c >> 1) ^ ((c >> 4) 
 
 // FWD: 4 channels (x1, x2, x1^2 + x2^2, x1 x2) from NI = 2 staged inputs.  BWD: NC = NI = 3 or 4 staged maps.
 // Either way the window holds 2 channel pairs (the fourth channel of the 3-map backward is a zero lane).
-template <bool FWD, int NC>
+template <bool FWD, int NC, int OPT = 0>
 __global__ void __launch_bounds__(kThreads, FWD ? 3 : 2) ssim_stream_kernel(const __grid_constant__ SsimParams p) {
     constexpr int NI = FWD ? 2 : NC;
     constexpr int NB = kSsimStageBufs<FWD>;    // staging buffers
@@ -133,6 +145,8 @@ __global__ void __launch_bounds__(kThreads, FWD ? 3 : 2) ssim_stream_kernel(cons
     // backward epilogue inputs x1, x2 of this thread's 8 output rows of a chunk (thread = (column, strip), as in the
     // vertical pass), loaded a whole chunk ahead so that their DRAM latency hides behind a chunk of filtering
     float x1n[8], x2n[8];
+    // kOptUp: 0.25 up of the 4 pooled rows under those 8 rows (row0 is even), fetched with them
+    float u1n[4], u2n[4];
     auto fetch_x = [&](int qn) {
         const int col = C0 + tid % kTW;
         const int row0 = S0 + kCR * qn + 8 * (tid / kTW);
@@ -142,6 +156,16 @@ __global__ void __launch_bounds__(kThreads, FWD ? 3 : 2) ssim_stream_kernel(cons
             const bool ok = col < W && row0 + i < S1;
             x1n[i] = ok ? __ldg(p.img1 + off + (long long)i * W) : 0.f;
             x2n[i] = ok ? __ldg(p.img2 + off + (long long)i * W) : 0.f;
+        }
+        if constexpr ((OPT & kOptUp) != 0) {
+            const int pr0 = row0 >> 1, pc = col >> 1;
+            const long long uoff = ((long long)plane * p.Hp + pr0) * p.Wp + pc;
+#pragma unroll
+            for (int k = 0; k < 4; ++k) {
+                const bool ok = pc < p.Wp && pr0 + k < p.Hp;
+                u1n[k] = ok && p.up1 ? 0.25f * __ldg(p.up1 + uoff + (long long)k * p.Wp) : 0.f;
+                u2n[k] = ok && p.up2 ? 0.25f * __ldg(p.up2 + uoff + (long long)k * p.Wp) : 0.f;
+            }
         }
     };
     if (!FWD) fetch_x(0);
@@ -221,6 +245,33 @@ __global__ void __launch_bounds__(kThreads, FWD ? 3 : 2) ssim_stream_kernel(cons
                 }
             }
         }
+        if constexpr (FWD && (OPT & kOptPool) != 0) {
+            // ---- 2x2 average pools of the staged rows, before the staging buffer is reused.  A chunk stages rows
+            //      [in_row0, in_row0 + nrows) with in_row0 odd (S0 is even) and nrows even: staged row r even is an odd
+            //      image row, the bottom of pooled row (in_row0 + r - 1) / 2, whose top is staged row r - 1 or, for
+            //      r = 0, the last row of the previous chunk, kept in a carry row (two of them, alternating by chunk)
+            float* carry = smem + NB * SB + 2 * 2 * kHR * kTW;   // [2][NI][kTW]
+            const float* cin = carry + (q & 1) * NI * kTW;
+            float* cout = carry + ((q + 1) & 1) * NI * kTW;
+            const int in_row0 = q < 0 ? S0 - kHalo : S0 + kCR * q + kHalo;
+            const long long pplane = (long long)plane * p.Hp * p.Wp;
+            for (int it = tid; it < (nrows / 2) * (kTW / 2); it += kThreads) {
+                const int r = 2 * (it / (kTW / 2)), pc = it % (kTW / 2);
+                const int gr = in_row0 + r;
+                if (gr - 1 < S0 || gr >= S1 || C0 + 2 * pc + 1 >= W) continue;
+                const long long o = pplane + (long long)((gr - 1) >> 1) * p.Wp + (C0 >> 1) + pc;
+#pragma unroll
+                for (int i = 0; i < NI; ++i) {
+                    const float* sp = stage + i * kCR * kPW + 2 * pc + 8;
+                    const float2 t = r == 0 ? *reinterpret_cast<const float2*>(cin + i * kTW + 2 * pc)
+                                            : *reinterpret_cast<const float2*>(sp + (r - 1) * kPW);
+                    const float2 b = *reinterpret_cast<const float2*>(sp + r * kPW);
+                    (i == 0 ? p.pooled1 : p.pooled2)[o] = (((t.x + t.y) + b.x) + b.y) * 0.25f;   // avg_pool2d's order
+                }
+            }
+            for (int it = tid; it < NI * kTW; it += kThreads)
+                cout[it] = stage[(it / kTW) * kCR * kPW + (nrows - 1) * kPW + it % kTW + 8];
+        }
         __syncthreads();
         if (NB == 1) {   // the one staging buffer is free again: the next chunk lands during the vertical pass
             if (q + 1 < niter) issue(q + 1, 0);
@@ -236,10 +287,14 @@ __global__ void __launch_bounds__(kThreads, FWD ? 3 : 2) ssim_stream_kernel(cons
             const int row0 = S0 + kCR * q + 8 * s;
             const bool live = col < W && row0 < S1;
             const long long off = (long long)plane * p.plane_elems + (long long)row0 * W + col;
-            float x1v[8], x2v[8];
+            float x1v[8], x2v[8], u1v[4], u2v[4];
             if (!FWD) {   // the epilogue's inputs were requested one chunk ago; request the next chunk's now
 #pragma unroll
                 for (int i = 0; i < 8; ++i) { x1v[i] = x1n[i]; x2v[i] = x2n[i]; }
+                if constexpr ((OPT & kOptUp) != 0) {
+#pragma unroll
+                    for (int k = 0; k < 4; ++k) { u1v[k] = u1n[k]; u2v[k] = u2n[k]; }
+                }
                 fetch_x(q + 1);
             }
             float2 acc[2][8];
@@ -274,8 +329,23 @@ __global__ void __launch_bounds__(kThreads, FWD ? 3 : 2) ssim_stream_kernel(cons
                             const float ssum = __fsub_rn(acc[1][i].x, msum);   // sigma1^2 + sigma2^2
                             const float A1 = __fmaf_rn(2.f, mu12, C1), A2 = __fmaf_rn(2.f, s12, C2);
                             const float B1 = __fadd_rn(msum, C1), B2 = __fadd_rn(ssum, C2);
+                            if constexpr ((OPT & kOptCs) != 0) {
+                                const float cs = __fdiv_rn(A2, B2);   // exactly 1 where A2 == B2
+                                local_sum += cs;
+                                if (p.n_maps) {
+                                    const float ib = __fdividef(1.f, B2);
+                                    m0[0] = 2.f * (mu1 * cs - mu2) * ib;                       // M0 = dcs/dmu1
+                                    m0[ms] = -cs * ib;                                         // M1 = -cs / B2
+                                    m0[2 * ms] = 2.f * ib;                                     // M2 = 2 / B2
+                                    if (p.n_maps == 4) m0[3 * ms] = 2.f * (mu2 * cs - mu1) * ib;   // M3 = dcs/dmu2
+                                }
+                                m0 += W;
+                                continue;
+                            }
                             const float inv = __fdividef(1.f, B1 * B2);   // B1, B2 >= ~1e-4: one MUFU.RCP, 2 ulp
-                            const float S = (A1 * A2) * inv;
+                            // kOptMs: correctly rounded, exactly 1 where A1 == B1 and A2 == B2
+                            const float S = (OPT & kOptMs) != 0 ? __fdiv_rn(__fmul_rn(A1, A2), __fmul_rn(B1, B2))
+                                                                : (A1 * A2) * inv;
                             local_sum += S;
                             if (p.n_maps) {
                                 const float k = 2.f * (A2 - A1) * inv;            // common factor of dS/dmu
@@ -296,8 +366,13 @@ __global__ void __launch_bounds__(kThreads, FWD ? 3 : 2) ssim_stream_kernel(cons
                         if (row0 + i < S1) {
                             const float x1 = x1v[i], x2 = x2v[i];
                             const float b0 = acc[0][i].x, b1 = acc[0][i].y, b2 = acc[1][i].x, b3 = acc[1][i].y;
-                            *d1 = g * (b0 + 2.f * x1 * b1 + x2 * b2);
-                            if (NC == 4 && d2) *d2 = g * (b3 + 2.f * x2 * b1 + x1 * b2);
+                            if constexpr ((OPT & kOptUp) != 0) {
+                                *d1 = g * (b0 + 2.f * x1 * b1 + x2 * b2) + u1v[i >> 1];
+                                if (NC == 4 && d2) *d2 = g * (b3 + 2.f * x2 * b1 + x1 * b2) + u2v[i >> 1];
+                            } else {
+                                *d1 = g * (b0 + 2.f * x1 * b1 + x2 * b2);
+                                if (NC == 4 && d2) *d2 = g * (b3 + 2.f * x2 * b1 + x1 * b2);
+                            }
                         }
                         d1 += W;
                         if (NC == 4 && d2) d2 += W;
@@ -365,11 +440,12 @@ static void plan_grid(int planes, int H, int W, int* strips, int* nseg, int* seg
     *nseg = (H + rows - 1) / rows;
 }
 
-template <bool FWD, int NC>
+template <bool FWD, int NC, int OPT = 0>
 static int launch_ssim(const SsimParams& p, cudaStream_t st) {
     constexpr int NI = FWD ? 2 : NC;
-    const size_t smem = sizeof(float) * (size_t)(kSsimStageBufs<FWD> * NI * kCR * kPW + 2 * 2 * kHR * kTW);
-    auto kern = ssim_stream_kernel<FWD, NC>;
+    constexpr int carry = (OPT & kOptPool) != 0 ? 2 * NI * kTW : 0;
+    const size_t smem = sizeof(float) * (size_t)(kSsimStageBufs<FWD> * NI * kCR * kPW + 2 * 2 * kHR * kTW + carry);
+    auto kern = ssim_stream_kernel<FWD, NC, OPT>;
     cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return set_last_cuda_error(e);
     const size_t grid = (size_t)p.planes * p.nseg * p.strips;
@@ -474,4 +550,88 @@ extern "C" int b200w_ssim_bwd_f32(const float* img1, const float* img2, const fl
     cudaStream_t st = (cudaStream_t)stream;
     if (d2) return launch_ssim<false, 4>(p, st);
     return launch_ssim<false, 3>(p, st);
+}
+
+// MS-SSIM, one scale: the SSIM kernels with the per-sample value of the SSIM map (cs == 0) or of the contrast-structure
+// map (cs != 0), optionally the 2x2 average pools of both images (forward) and the pooling's transpose (backward)
+extern "C" int b200w_msssim_scale_fwd_f32(const float* img1, const float* img2, int N, int C, int H, int W,
+                                          const float* win, int ws, int cs, int n_maps, float* maps, float* out,
+                                          float* pooled1, float* pooled2, void* workspace, size_t workspace_bytes,
+                                          void* stream) {
+    if (!img1 || !img2 || !out) return B200W_ERR_NULL_POINTER;
+    if (N < 1 || C < 1 || H < 1 || W < 1) return B200W_ERR_BAD_SHAPE;
+    if (!(n_maps == 0 || n_maps == 3 || n_maps == 4)) return B200W_ERR_BAD_SHAPE;
+    if (n_maps && !maps) return B200W_ERR_NULL_POINTER;
+    if (!pooled1 != !pooled2) return B200W_ERR_NULL_POINTER;
+    const bool pool = pooled1 != nullptr;
+    if (pool && (H < 2 || W < 2)) return B200W_ERR_BAD_SHAPE;
+    SsimParams p = {};
+    int rc = fill_window(p, win, ws);
+    if (rc) return rc;
+    p.planes = N * C;
+    p.C = C;
+    p.H = H;
+    p.W = W;
+    plan_grid(p.planes, H, W, &p.strips, &p.nseg, &p.seg_rows);
+    const size_t need = sizeof(float) * (size_t)p.planes * p.strips * p.nseg;
+    if (!workspace || workspace_bytes < need) return B200W_ERR_WORKSPACE;
+    p.in[0] = img1;
+    p.in[1] = img2;
+    p.out0 = maps;
+    p.partials = (float*)workspace;
+    p.plane_elems = (long long)H * W;
+    p.map_stride = (long long)p.planes * H * W;
+    p.n_maps = n_maps;
+    p.vec_ok = ((W % 4) == 0 && aligned16(img1) && aligned16(img2)) ? 1 : 0;
+    p.pooled1 = pooled1;
+    p.pooled2 = pooled2;
+    p.Hp = H / 2;
+    p.Wp = W / 2;
+    cudaStream_t st = (cudaStream_t)stream;
+    if (cs) rc = pool ? launch_ssim<true, 4, kOptMs | kOptCs | kOptPool>(p, st) : launch_ssim<true, 4, kOptMs | kOptCs>(p, st);
+    else rc = pool ? launch_ssim<true, 4, kOptMs | kOptPool>(p, st) : launch_ssim<true, 4, kOptMs>(p, st);
+    if (rc) return rc;
+    const int per_plane = p.strips * p.nseg;
+    ssim_finalize_kernel<<<N, kThreads, 0, st>>>(p.partials, C * per_plane, 1.0 / ((double)C * H * W), out);
+    note_launch("ssim_finalize_kernel");
+    cudaError_t e = cudaGetLastError();
+    return e == cudaSuccess ? B200W_OK : set_last_cuda_error(e);
+}
+
+extern "C" int b200w_msssim_scale_bwd_f32(const float* img1, const float* img2, const float* maps, int n_maps,
+                                          const float* grad_out, int N, int C, int H, int W, const float* win, int ws,
+                                          const float* up1, const float* up2, float* d1, float* d2, void* stream) {
+    if (!img1 || !img2 || !maps || !grad_out || !d1) return B200W_ERR_NULL_POINTER;
+    if (N < 1 || C < 1 || H < 1 || W < 1) return B200W_ERR_BAD_SHAPE;
+    if (!(n_maps == 3 || n_maps == 4) || (d2 && n_maps != 4)) return B200W_ERR_BAD_SHAPE;
+    if (up2 && !d2) return B200W_ERR_BAD_SHAPE;
+    const bool up = up1 || up2;
+    if (up && (H < 2 || W < 2)) return B200W_ERR_BAD_SHAPE;
+    SsimParams p = {};
+    int rc = fill_window(p, win, ws);
+    if (rc) return rc;
+    p.planes = N * C;
+    p.C = C;
+    p.H = H;
+    p.W = W;
+    plan_grid(p.planes, H, W, &p.strips, &p.nseg, &p.seg_rows);
+    p.plane_elems = (long long)H * W;
+    p.map_stride = (long long)p.planes * H * W;
+    for (int i = 0; i < n_maps; ++i) p.in[i] = maps + (size_t)i * p.map_stride;
+    p.img1 = img1;
+    p.img2 = img2;
+    p.grad_out = grad_out;
+    p.out0 = d1;
+    p.out1 = d2;
+    p.n_maps = n_maps;
+    p.size_average = 0;
+    p.inv_count = (float)(1.0 / ((double)C * H * W));
+    p.vec_ok = ((W % 4) == 0 && aligned16(maps)) ? 1 : 0;
+    p.up1 = up1;
+    p.up2 = up2;
+    p.Hp = H / 2;
+    p.Wp = W / 2;
+    cudaStream_t st = (cudaStream_t)stream;
+    if (d2) return up ? launch_ssim<false, 4, kOptUp>(p, st) : launch_ssim<false, 4>(p, st);
+    return up ? launch_ssim<false, 3, kOptUp>(p, st) : launch_ssim<false, 3>(p, st);
 }

@@ -33,6 +33,10 @@ constexpr int kTH = kR * (kThreads / kTW);    // 32 output rows per CTA tile
 constexpr int kSW = kTW + kWin - 1;           // 74 staged columns
 constexpr int kSH = kTH + kWin - 1;           // 42 staged rows
 constexpr int kPlaneS = kSW * kSH;            // doubles per staged channel
+// options of the MS-SSIM scale instantiations (0: the plain SSIM kernels)
+constexpr int kOptCs = 2;     // fwd: the contrast-structure map cs = A2/B2 and its derivative maps instead of S
+constexpr int kOptPool = 4;   // fwd: also write avg_pool2d(img1, 2) and avg_pool2d(img2, 2)
+constexpr int kOptUp = 8;     // bwd: add 0.25 up[r/2][c/2] (the transpose of that pooling) to d1 / d2
 }  // namespace f64ssim
 
 struct SsimF64Params {
@@ -49,6 +53,12 @@ struct SsimF64Params {
     int n_maps, size_average;
     double inv_count;        // bwd: 1/(N*C*H*W) or 1/(C*H*W)
     double win[f64ssim::kWin * f64ssim::kWin];   // [dy][dx], a smaller window centred with zero outer taps
+    // MS-SSIM scale fields, after the plain SSIM ones so that those keep their parameter offsets
+    double* pooled1;         // fwd (kOptPool): (planes, Hp, Wp)
+    double* pooled2;
+    const double* up1;       // bwd (kOptUp): (planes, Hp, Wp) or null
+    const double* up2;
+    int Hp, Wp;              // H / 2, W / 2
 };
 
 // stage rows [Y0-5, Y0+37) x cols [X0-5, X0+69) of one plane into dst[kSH][kSW], zero outside the image
@@ -105,6 +115,7 @@ __device__ __forceinline__ double block_sum_f64(double v, double* red) {
     return t;
 }
 
+template <int OPT = 0>
 __global__ void __launch_bounds__(kThreads, 2) ssim_f64_kernel(const __grid_constant__ SsimF64Params p) {
     using namespace f64ssim;
     extern __shared__ __align__(16) double sm[];   // [4][kSH][kSW]: x1, x2, x1^2 + x2^2, x1 x2
@@ -130,6 +141,21 @@ __global__ void __launch_bounds__(kThreads, 2) ssim_f64_kernel(const __grid_cons
         sm[2 * kPlaneS + idx] = __dadd_rn(__dmul_rn(a, a), __dmul_rn(b, b));
         sm[3 * kPlaneS + idx] = __dmul_rn(a, b);
     }
+    if constexpr ((OPT & kOptPool) != 0) {
+        // 2x2 average pools of the tile (Y0, X0 even): pooled (Y0/2 + k, X0/2 + pc) from staged rows 2k+5, 2k+6 and
+        // columns 2pc+5, 2pc+6, summed in avg_pool2d's order
+        const long long pplane = (long long)plane * p.Hp * p.Wp;
+        for (int it = tid; it < (kTH / 2) * (kTW / 2); it += kThreads) {
+            const int k = it / (kTW / 2), pc = it % (kTW / 2);
+            if (Y0 + 2 * k + 1 >= H || X0 + 2 * pc + 1 >= W) continue;
+            const long long o = pplane + (long long)(Y0 / 2 + k) * p.Wp + X0 / 2 + pc;
+#pragma unroll
+            for (int i = 0; i < 2; ++i) {
+                const double* t = sm + i * kPlaneS + (2 * k + kHalo) * kSW + 2 * pc + kHalo;
+                (i == 0 ? p.pooled1 : p.pooled2)[o] = (((t[0] + t[1]) + t[kSW]) + t[kSW + 1]) * 0.25;
+            }
+        }
+    }
     __syncthreads();
 
     const int c = tid % kTW, s = tid / kTW;
@@ -152,6 +178,19 @@ __global__ void __launch_bounds__(kThreads, 2) ssim_f64_kernel(const __grid_cons
                 const double ssum = __dsub_rn(acc[2][i], msum);   // sigma1^2 + sigma2^2
                 const double A1 = __fma_rn(2.0, mu12, C1), A2 = __fma_rn(2.0, s12, C2);
                 const double B1 = __dadd_rn(msum, C1), B2 = __dadd_rn(ssum, C2);
+                if constexpr ((OPT & kOptCs) != 0) {
+                    const double cs = __ddiv_rn(A2, B2);   // exactly 1 where A2 == B2
+                    local += cs;
+                    if (p.n_maps) {
+                        const double ib = 1.0 / B2;
+                        m0[0] = 2.0 * (mu1 * cs - mu2) * ib;                       // M0 = dcs/dmu1
+                        m0[ms] = -cs * ib;                                         // M1 = -cs / B2
+                        m0[2 * ms] = 2.0 * ib;                                     // M2 = 2 / B2
+                        if (p.n_maps == 4) m0[3 * ms] = 2.0 * (mu2 * cs - mu1) * ib;   // M3 = dcs/dmu2
+                    }
+                    if (m0) m0 += W;
+                    continue;
+                }
                 const double den = __dmul_rn(B1, B2);
                 const double S = __ddiv_rn(__dmul_rn(A1, A2), den);
                 local += S;
@@ -172,7 +211,7 @@ __global__ void __launch_bounds__(kThreads, 2) ssim_f64_kernel(const __grid_cons
     if (tid == 0) p.partials[blockIdx.x] = t;
 }
 
-template <int NC>
+template <int NC, int OPT = 0>
 __global__ void __launch_bounds__(kThreads, 2) ssim_f64_bwd_kernel(const __grid_constant__ SsimF64Params p) {
     using namespace f64ssim;
     extern __shared__ __align__(16) double sm[];   // [NC][kSH][kSW]: the saved maps
@@ -206,8 +245,18 @@ __global__ void __launch_bounds__(kThreads, 2) ssim_f64_bwd_kernel(const __grid_
         if (row0 + i < H) {
             const long long o = off + (long long)i * W;
             const double x1 = __ldg(p.img1 + o), x2 = __ldg(p.img2 + o);
-            p.out0[o] = g * (acc[0][i] + 2.0 * x1 * acc[1][i] + x2 * acc[2][i]);
-            if (NC == 4 && d2) d2[o] = g * (acc[NC - 1][i] + 2.0 * x2 * acc[1][i] + x1 * acc[2][i]);
+            if constexpr ((OPT & kOptUp) != 0) {
+                const int pr = (row0 + i) >> 1, pc = col >> 1;
+                const bool in = pr < p.Hp && pc < p.Wp;
+                const long long uo = ((long long)plane * p.Hp + pr) * p.Wp + pc;
+                const double u1 = in && p.up1 ? 0.25 * __ldg(p.up1 + uo) : 0.0;
+                const double u2 = in && p.up2 ? 0.25 * __ldg(p.up2 + uo) : 0.0;
+                p.out0[o] = g * (acc[0][i] + 2.0 * x1 * acc[1][i] + x2 * acc[2][i]) + u1;
+                if (NC == 4 && d2) d2[o] = g * (acc[NC - 1][i] + 2.0 * x2 * acc[1][i] + x1 * acc[2][i]) + u2;
+            } else {
+                p.out0[o] = g * (acc[0][i] + 2.0 * x1 * acc[1][i] + x2 * acc[2][i]);
+                if (NC == 4 && d2) d2[o] = g * (acc[NC - 1][i] + 2.0 * x2 * acc[1][i] + x1 * acc[2][i]);
+            }
         }
     }
 }
@@ -292,7 +341,7 @@ extern "C" int b200w_ssim_fwd_f64(const double* img1, const double* img2, int N,
     p.n_maps = n_maps;
     p.size_average = size_average ? 1 : 0;
     cudaStream_t st = (cudaStream_t)stream;
-    rc = launch_f64(ssim_f64_kernel, 4, p, planes, st, "ssim_f64_kernel");
+    rc = launch_f64(ssim_f64_kernel<>, 4, p, planes, st, "ssim_f64_kernel");
     if (rc) return rc;
     const int per_plane = p.tiles_x * p.tiles_y;
     const int nout = size_average ? 1 : N;
@@ -334,4 +383,93 @@ extern "C" int b200w_ssim_bwd_f64(const double* img1, const double* img2, const 
     cudaStream_t st = (cudaStream_t)stream;
     if (d2) return launch_f64(ssim_f64_bwd_kernel<4>, 4, p, planes, st, "ssim_f64_bwd_kernel<4>");
     return launch_f64(ssim_f64_bwd_kernel<3>, 3, p, planes, st, "ssim_f64_bwd_kernel<3>");
+}
+
+// MS-SSIM, one scale (see b200w_msssim_scale_fwd_f32): the same checks in the same order
+extern "C" int b200w_msssim_scale_fwd_f64(const double* img1, const double* img2, int N, int C, int H, int W,
+                                          const double* win2d, int ws, int cs, int n_maps, double* maps, double* out,
+                                          double* pooled1, double* pooled2, void* workspace, size_t workspace_bytes,
+                                          void* stream) {
+    if (!img1 || !img2 || !out) return B200W_ERR_NULL_POINTER;
+    if (N < 1 || C < 1 || H < 1 || W < 1) return B200W_ERR_BAD_SHAPE;
+    if (!(n_maps == 0 || n_maps == 3 || n_maps == 4)) return B200W_ERR_BAD_SHAPE;
+    if (n_maps && !maps) return B200W_ERR_NULL_POINTER;
+    if (!pooled1 != !pooled2) return B200W_ERR_NULL_POINTER;
+    const bool pool = pooled1 != nullptr;
+    if (pool && (H < 2 || W < 2)) return B200W_ERR_BAD_SHAPE;
+    SsimF64Params p = {};
+    int rc = fill_window_f64(p, win2d, ws, false);
+    if (rc) return rc;
+    const int planes = N * C;
+    p.C = C;
+    p.H = H;
+    p.W = W;
+    tiles_f64(H, W, &p.tiles_x, &p.tiles_y);
+    const size_t need = b200w_ssim_workspace_bytes_f64(N, C, H, W);
+    if (!workspace || workspace_bytes < need) return B200W_ERR_WORKSPACE;
+    p.in[0] = img1;
+    p.in[1] = img2;
+    p.out0 = n_maps ? maps : nullptr;
+    p.partials = (double*)workspace;
+    p.plane_elems = (long long)H * W;
+    p.map_stride = (long long)planes * H * W;
+    p.n_maps = n_maps;
+    p.pooled1 = pooled1;
+    p.pooled2 = pooled2;
+    p.Hp = H / 2;
+    p.Wp = W / 2;
+    cudaStream_t st = (cudaStream_t)stream;
+    using namespace f64ssim;
+    if (cs) rc = pool ? launch_f64(ssim_f64_kernel<kOptCs | kOptPool>, 4, p, planes, st, "ssim_f64_kernel<cs,pool>")
+                      : launch_f64(ssim_f64_kernel<kOptCs>, 4, p, planes, st, "ssim_f64_kernel<cs>");
+    else rc = pool ? launch_f64(ssim_f64_kernel<kOptPool>, 4, p, planes, st, "ssim_f64_kernel<pool>")
+                   : launch_f64(ssim_f64_kernel<>, 4, p, planes, st, "ssim_f64_kernel");
+    if (rc) return rc;
+    ssim_f64_finalize_kernel<<<N, kThreads, 0, st>>>(p.partials, C * p.tiles_x * p.tiles_y, 1.0 / ((double)C * H * W),
+                                                      out);
+    note_launch("ssim_f64_finalize_kernel");
+    cudaError_t e = cudaGetLastError();
+    return e == cudaSuccess ? B200W_OK : set_last_cuda_error(e);
+}
+
+extern "C" int b200w_msssim_scale_bwd_f64(const double* img1, const double* img2, const double* maps, int n_maps,
+                                          const double* grad_out, int N, int C, int H, int W, const double* win2d,
+                                          int ws, const double* up1, const double* up2, double* d1, double* d2,
+                                          void* stream) {
+    if (!img1 || !img2 || !maps || !grad_out || !d1) return B200W_ERR_NULL_POINTER;
+    if (N < 1 || C < 1 || H < 1 || W < 1) return B200W_ERR_BAD_SHAPE;
+    if (!(n_maps == 3 || n_maps == 4) || (d2 && n_maps != 4)) return B200W_ERR_BAD_SHAPE;
+    if (up2 && !d2) return B200W_ERR_BAD_SHAPE;
+    const bool up = up1 || up2;
+    if (up && (H < 2 || W < 2)) return B200W_ERR_BAD_SHAPE;
+    SsimF64Params p = {};
+    int rc = fill_window_f64(p, win2d, ws, true);
+    if (rc) return rc;
+    const int planes = N * C;
+    p.C = C;
+    p.H = H;
+    p.W = W;
+    tiles_f64(H, W, &p.tiles_x, &p.tiles_y);
+    p.plane_elems = (long long)H * W;
+    p.map_stride = (long long)planes * H * W;
+    const int nc = d2 ? 4 : 3;
+    for (int i = 0; i < nc; ++i) p.in[i] = maps + (size_t)i * p.map_stride;
+    p.img1 = img1;
+    p.img2 = img2;
+    p.grad_out = grad_out;
+    p.out0 = d1;
+    p.out1 = d2;
+    p.n_maps = n_maps;
+    p.size_average = 0;
+    p.inv_count = 1.0 / ((double)C * H * W);
+    p.up1 = up1;
+    p.up2 = up2;
+    p.Hp = H / 2;
+    p.Wp = W / 2;
+    cudaStream_t st = (cudaStream_t)stream;
+    using namespace f64ssim;
+    if (d2) return up ? launch_f64(ssim_f64_bwd_kernel<4, kOptUp>, 4, p, planes, st, "ssim_f64_bwd_kernel<4,up>")
+                      : launch_f64(ssim_f64_bwd_kernel<4>, 4, p, planes, st, "ssim_f64_bwd_kernel<4>");
+    return up ? launch_f64(ssim_f64_bwd_kernel<3, kOptUp>, 3, p, planes, st, "ssim_f64_bwd_kernel<3,up>")
+              : launch_f64(ssim_f64_bwd_kernel<3>, 3, p, planes, st, "ssim_f64_bwd_kernel<3>");
 }

@@ -14,6 +14,8 @@ mathematical adjoint (SURVEY.md 8a-Q1):
 * ``sfb2d`` backward  = ``afb2d`` of ``dy`` with the synthesis taps as
   correlation kernels                     (pw/dwt/lowlevel.py:682-694)
 * ``ssim_fwd`` backward = ``ssim_bwd`` (closed form of autograd through ssim.py:17-37)
+* ``msssim_scale`` backward = ``msssim_scale_bwd``: the same closed form for the SSIM or the contrast-structure map,
+  plus the transpose of the 2x2 pooling applied to the gradients of the pooled outputs
 """
 import ctypes
 
@@ -42,6 +44,10 @@ _LIB.define("iswt2d(Tensor ll, Tensor y, float[] w_lo, float[] w_hi, float[] h_l
 _LIB.define("ssim_fwd(Tensor img1, Tensor img2, float[] win, bool size_average, int n_maps) -> (Tensor, Tensor)")
 _LIB.define("ssim_bwd(Tensor img1, Tensor img2, Tensor maps, Tensor grad_out, float[] win, bool size_average, "
             "bool need_d2) -> (Tensor, Tensor)")
+_LIB.define("msssim_scale(Tensor img1, Tensor img2, float[] win, bool cs, bool pool, int n_maps) "
+            "-> (Tensor, Tensor, Tensor, Tensor)")
+_LIB.define("msssim_scale_bwd(Tensor img1, Tensor img2, Tensor maps, Tensor grad_out, float[] win, Tensor? up1, "
+            "Tensor? up2, bool need_d2) -> (Tensor, Tensor)")
 
 MAX_LEVELS = _cabi.MAX_LEVELS
 
@@ -825,6 +831,101 @@ def _ssim_backward(ctx, dval, dmaps):
     return (d1 if need1 else None), (d2 if need2 else None), None, None, None
 
 
+# ------------------------------------------------------------------------------------------- MS-SSIM scale
+def pooled_shape(img, pool):
+    N, C, H, W = img.shape
+    return (N, C, H // 2, W // 2) if pool else (0,)
+
+
+def msssim_up(t, img, name):
+    """The gradient of a pooled output as the backward kernel reads it (or None)."""
+    if t is None:
+        return None
+    if tuple(t.shape) != pooled_shape(img, True):
+        raise RuntimeError("b200wave::%s: the gradient of a pooled image has shape %s, expected %s"
+                           % (name, tuple(t.shape), pooled_shape(img, True)))
+    return t.to(dtype=img.dtype).contiguous()
+
+
+def _msssim_scale_cuda(img1, img2, win, cs, pool, n_maps):
+    _ssim_common(img1, img2, win, "msssim_scale")
+    lib = _cabi.load()
+    img1, img2 = img1.contiguous(), img2.contiguous()
+    N, C, H, W = img1.shape
+    out = torch.empty((N,), device=img1.device, dtype=torch.float32)
+    maps = torch.empty((n_maps, N, C, H, W), device=img1.device, dtype=torch.float32)
+    p1 = torch.empty(pooled_shape(img1, pool), device=img1.device, dtype=torch.float32)
+    p2 = torch.empty_like(p1)
+    ws_bytes = lib.b200w_ssim_workspace_bytes(N, C, H, W)
+    work = torch.empty((max(ws_bytes, 4) // 4,), device=img1.device, dtype=torch.float32)
+    a_win, nwin = _cabi.taps_array(win)
+    with torch.cuda.device(img1.device):
+        rc = lib.b200w_msssim_scale_fwd_f32(img1.data_ptr(), img2.data_ptr(), N, C, H, W, a_win, nwin, int(cs),
+                                            int(n_maps), maps.data_ptr() if n_maps else None, out.data_ptr(),
+                                            p1.data_ptr() if pool else None, p2.data_ptr() if pool else None,
+                                            work.data_ptr(), ws_bytes, _stream())
+    _cabi.check(rc)
+    return out, maps, p1, p2
+
+
+def msssim_scale_fake(img1, img2, win, cs, pool, n_maps):
+    N, C, H, W = img1.shape
+    p = img1.new_empty(pooled_shape(img1, pool))
+    return img1.new_empty((N,)), img1.new_empty((n_maps, N, C, H, W)), p, torch.empty_like(p)
+
+
+def _msssim_scale_bwd_cuda(img1, img2, maps, grad_out, win, up1, up2, need_d2):
+    _ssim_common(img1, img2, win, "msssim_scale_bwd")
+    lib = _cabi.load()
+    img1, img2, maps = img1.contiguous(), img2.contiguous(), maps.contiguous()
+    N, C, H, W = img1.shape
+    n_maps = maps.shape[0]
+    if n_maps not in (3, 4) or (need_d2 and n_maps != 4):
+        raise RuntimeError("b200wave::msssim_scale_bwd: forward saved %d derivative maps, not enough for this backward"
+                           % n_maps)
+    g = grad_out.to(device=img1.device, dtype=torch.float32).contiguous()
+    if g.numel() != N:
+        raise RuntimeError("b200wave::msssim_scale_bwd: grad_out has %d elements" % g.numel())
+    up1, up2 = msssim_up(up1, img1, "msssim_scale_bwd"), msssim_up(up2, img1, "msssim_scale_bwd")
+    d1 = torch.empty_like(img1)
+    d2 = torch.empty_like(img2) if need_d2 else torch.empty((0,), device=img1.device, dtype=torch.float32)
+    a_win, nwin = _cabi.taps_array(win)
+    with torch.cuda.device(img1.device):
+        rc = lib.b200w_msssim_scale_bwd_f32(img1.data_ptr(), img2.data_ptr(), maps.data_ptr(), n_maps, g.data_ptr(),
+                                            N, C, H, W, a_win, nwin, None if up1 is None else up1.data_ptr(),
+                                            None if up2 is None else up2.data_ptr(), d1.data_ptr(),
+                                            d2.data_ptr() if need_d2 else None, _stream())
+    _cabi.check(rc)
+    return d1, d2
+
+
+def msssim_scale_setup(ctx, inputs, output):
+    img1, img2, win, cs, pool, n_maps = inputs
+    ctx.save_for_backward(img1, img2, output[1])
+    ctx.win = win
+    ctx.n_maps = n_maps
+    ctx.set_materialize_grads(False)
+
+
+def msssim_scale_backward(bwd_op, ctx, dval, dmaps, dp1, dp2):
+    """One backward launch: the closed form for ``dval`` plus 0.25 ``dp`` spread over each 2x2 block."""
+    need1, need2 = ctx.needs_input_grad[0], ctx.needs_input_grad[1]
+    if not (need1 or need2):
+        return (None,) * 6
+    if ctx.n_maps < 3 or (need2 and ctx.n_maps < 4):
+        raise RuntimeError("msssim_scale was called with n_maps=%d, which does not support the requested gradient "
+                           "(use 3 for d/dimg1, 4 for both)" % ctx.n_maps)
+    img1, img2, maps = ctx.saved_tensors
+    if dval is None:
+        dval = img1.new_zeros((img1.shape[0],))
+    d1, d2 = bwd_op(img1, img2, maps, dval, ctx.win, dp1 if need1 else None, dp2 if need2 else None, bool(need2))
+    return (d1 if need1 else None), (d2 if need2 else None), None, None, None, None
+
+
+def _msssim_scale_backward(ctx, dval, dmaps, dp1, dp2):
+    return msssim_scale_backward(torch.ops.b200wave.msssim_scale_bwd, ctx, dval, dmaps, dp1, dp2)
+
+
 _LIB.impl("afb2d", _afb2d_cuda, "CUDA")
 _LIB.impl("sfb2d", _sfb2d_cuda, "CUDA")
 _LIB.impl("dwt2", _dwt2_cuda, "CUDA")
@@ -837,6 +938,8 @@ _LIB.impl("swt2d", _swt2d_cuda, "CUDA")
 _LIB.impl("swt2d_adjoint", _swt2d_adjoint_cuda, "CUDA")
 _LIB.impl("sfb1d", _sfb1d_cuda, "CUDA")
 _LIB.impl("iswt2d", _iswt2d_cuda, "CUDA")
+_LIB.impl("msssim_scale", _msssim_scale_cuda, "CUDA")
+_LIB.impl("msssim_scale_bwd", _msssim_scale_bwd_cuda, "CUDA")
 
 
 def _cpu_refuse(name):
@@ -847,7 +950,7 @@ def _cpu_refuse(name):
 
 
 for _name in ("afb2d", "afb2d_select", "sfb2d", "dwt2", "idwt2", "ssim_fwd", "ssim_bwd", "afb1d", "sfb1d", "swt2d",
-              "swt2d_adjoint", "iswt2d"):
+              "swt2d_adjoint", "iswt2d", "msssim_scale", "msssim_scale_bwd"):
     _LIB.impl(_name, _cpu_refuse(_name), "CPU")
 
 torch.library.register_fake("b200wave::afb2d", _afb2d_fake, lib=_LIB)
@@ -874,6 +977,11 @@ torch.library.register_fake("b200wave::ssim_bwd", _ssim_bwd_fake, lib=_LIB)
 torch.library.register_autograd("b200wave::afb2d", _afb2d_backward, setup_context=_afb2d_setup, lib=_LIB)
 torch.library.register_autograd("b200wave::sfb2d", _sfb2d_backward, setup_context=_sfb2d_setup, lib=_LIB)
 torch.library.register_autograd("b200wave::ssim_fwd", _ssim_backward, setup_context=_ssim_setup, lib=_LIB)
+torch.library.register_fake("b200wave::msssim_scale", msssim_scale_fake, lib=_LIB)
+torch.library.register_fake("b200wave::msssim_scale_bwd", lambda img1, img2, maps, g, win, up1, up2, need_d2:
+                            _ssim_bwd_fake(img1, img2, maps, g, win, False, need_d2), lib=_LIB)
+torch.library.register_autograd("b200wave::msssim_scale", _msssim_scale_backward, setup_context=msssim_scale_setup,
+                                lib=_LIB)
 
 afb2d = torch.ops.b200wave.afb2d
 afb2d_select = torch.ops.b200wave.afb2d_select
@@ -887,6 +995,8 @@ swt2d = torch.ops.b200wave.swt2d
 swt2d_adjoint = torch.ops.b200wave.swt2d_adjoint
 iswt2d = torch.ops.b200wave.iswt2d
 sfb1d = torch.ops.b200wave.sfb1d
+msssim_scale = torch.ops.b200wave.msssim_scale
+msssim_scale_bwd = torch.ops.b200wave.msssim_scale_bwd
 
 
 def ssim_bench_kernels(sets, win):

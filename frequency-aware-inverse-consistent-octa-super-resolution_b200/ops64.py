@@ -13,7 +13,8 @@ stream, CUDA-only, the same backward structure -- on double tensors with double 
   (``csrc/tv.cu``): the fp32 kernels instantiated for ``double``.  As in fp32, ``losses.TVLoss`` differentiates
   ``tv_sums`` through ``tv_grad`` (once differentiable).
 * ``ssim_fwd`` / ``ssim_bwd`` (``csrc/ssim_f64.cu``): ``win`` is the DENSE ws x ws window, row-major (in double the
-  reference's window is the fp32 rounding of an outer product, which is not separable).
+  reference's window is the fp32 rounding of an outer product, which is not separable).  ``msssim_scale`` /
+  ``msssim_scale_bwd``: one MS-SSIM scale on the same kernels, as ``ops.msssim_scale``.
 * ``afb2d_select`` (``b200w_afb2d_ex_f64``): the discriminators' ``filter_wavelet`` level (``fsd.py``) on the direct
   kernel; backward = ``sfb2d`` of ``(dlow, hi_scale * dhighs)``, as ``ops.afb2d_select``.
 * ``freq_mask_`` / ``abs_sign`` / ``sign_mul`` (``csrc/freq.cu``): the pointwise passes of ``freq.gaussian_split`` on
@@ -23,7 +24,8 @@ import torch
 
 from . import _cabi
 from .ops import (_check_mode, _check_swt_mode, _mode_name, _planes_view, _rows_view, _stream, coeff_len, idwt_len,
-                  iswt2d_backward, iswt_adjoint_taps, iswt_layout)
+                  iswt2d_backward, iswt_adjoint_taps, iswt_layout, msssim_scale_backward, msssim_scale_fake,
+                  msssim_scale_setup, msssim_up, pooled_shape)
 
 _LIB = torch.library.Library("b200wave64", "DEF")
 _LIB.define("afb2d(Tensor x, float[] w_lo, float[] w_hi, float[] h_lo, float[] h_hi, int mode) -> (Tensor, Tensor)")
@@ -38,6 +40,10 @@ _LIB.define("iswt2d(Tensor ll, Tensor y, float[] w_lo, float[] w_hi, float[] h_l
 _LIB.define("ssim_fwd(Tensor img1, Tensor img2, float[] win, bool size_average, int n_maps) -> (Tensor, Tensor)")
 _LIB.define("ssim_bwd(Tensor img1, Tensor img2, Tensor maps, Tensor grad_out, float[] win, bool size_average, "
             "bool need_d2) -> (Tensor, Tensor)")
+_LIB.define("msssim_scale(Tensor img1, Tensor img2, float[] win, bool cs, bool pool, int n_maps) "
+            "-> (Tensor, Tensor, Tensor, Tensor)")
+_LIB.define("msssim_scale_bwd(Tensor img1, Tensor img2, Tensor maps, Tensor grad_out, float[] win, Tensor? up1, "
+            "Tensor? up2, bool need_d2) -> (Tensor, Tensor)")
 _LIB.define("tv_sums(Tensor x) -> Tensor")
 _LIB.define("tv_grad(Tensor x, Tensor grad_out, float ch, float cw) -> Tensor")
 _LIB.define("afb2d_select(Tensor x, float[] w_lo, float[] w_hi, float[] h_lo, float[] h_hi, int mode, bool want_low, "
@@ -500,6 +506,57 @@ def _ssim_backward(ctx, dval, dmaps):
     return (d1 if need1 else None), (d2 if need2 else None), None, None, None
 
 
+# ------------------------------------------------------------------------------------------- MS-SSIM scale
+def _msssim_scale_cuda(img1, img2, win, cs, pool, n_maps):
+    ws = _ssim_common(img1, img2, win, "msssim_scale")
+    lib = _cabi.load()
+    img1, img2 = img1.contiguous(), img2.contiguous()
+    N, C, H, W = img1.shape
+    out = torch.empty((N,), device=img1.device, dtype=torch.float64)
+    maps = torch.empty((n_maps, N, C, H, W), device=img1.device, dtype=torch.float64)
+    p1 = torch.empty(pooled_shape(img1, pool), device=img1.device, dtype=torch.float64)
+    p2 = torch.empty_like(p1)
+    ws_bytes = lib.b200w_ssim_workspace_bytes_f64(N, C, H, W)
+    work = torch.empty((max(ws_bytes, 8) // 8,), device=img1.device, dtype=torch.float64)
+    a_win, _ = _cabi.taps_array_f64(win)
+    with torch.cuda.device(img1.device):
+        rc = lib.b200w_msssim_scale_fwd_f64(img1.data_ptr(), img2.data_ptr(), N, C, H, W, a_win, ws, int(cs),
+                                            int(n_maps), maps.data_ptr() if n_maps else None, out.data_ptr(),
+                                            p1.data_ptr() if pool else None, p2.data_ptr() if pool else None,
+                                            work.data_ptr(), ws_bytes, _stream())
+    _cabi.check(rc)
+    return out, maps, p1, p2
+
+
+def _msssim_scale_bwd_cuda(img1, img2, maps, grad_out, win, up1, up2, need_d2):
+    ws = _ssim_common(img1, img2, win, "msssim_scale_bwd")
+    lib = _cabi.load()
+    img1, img2, maps = img1.contiguous(), img2.contiguous(), maps.contiguous()
+    N, C, H, W = img1.shape
+    n_maps = maps.shape[0]
+    if n_maps not in (3, 4) or (need_d2 and n_maps != 4):
+        raise RuntimeError("b200wave64::msssim_scale_bwd: forward saved %d derivative maps, not enough for this "
+                           "backward" % n_maps)
+    g = grad_out.to(device=img1.device, dtype=torch.float64).contiguous()
+    if g.numel() != N:
+        raise RuntimeError("b200wave64::msssim_scale_bwd: grad_out has %d elements" % g.numel())
+    up1, up2 = msssim_up(up1, img1, "msssim_scale_bwd"), msssim_up(up2, img1, "msssim_scale_bwd")
+    d1 = torch.empty_like(img1)
+    d2 = torch.empty_like(img2) if need_d2 else torch.empty((0,), device=img1.device, dtype=torch.float64)
+    a_win, _ = _cabi.taps_array_f64(win)
+    with torch.cuda.device(img1.device):
+        rc = lib.b200w_msssim_scale_bwd_f64(img1.data_ptr(), img2.data_ptr(), maps.data_ptr(), n_maps, g.data_ptr(),
+                                            N, C, H, W, a_win, ws, None if up1 is None else up1.data_ptr(),
+                                            None if up2 is None else up2.data_ptr(), d1.data_ptr(),
+                                            d2.data_ptr() if need_d2 else None, _stream())
+    _cabi.check(rc)
+    return d1, d2
+
+
+def _msssim_scale_backward(ctx, dval, dmaps, dp1, dp2):
+    return msssim_scale_backward(torch.ops.b200wave64.msssim_scale_bwd, ctx, dval, dmaps, dp1, dp2)
+
+
 # ------------------------------------------------------------------------------------------- TV
 def _check_tv(x, name):
     _require_cuda_f64(x, name)
@@ -601,6 +658,8 @@ _LIB.impl("swt2d_adjoint", _swt2d_adjoint_cuda, "CUDA")
 _LIB.impl("iswt2d", _iswt2d_cuda, "CUDA")
 _LIB.impl("ssim_fwd", _ssim_fwd_cuda, "CUDA")
 _LIB.impl("ssim_bwd", _ssim_bwd_cuda, "CUDA")
+_LIB.impl("msssim_scale", _msssim_scale_cuda, "CUDA")
+_LIB.impl("msssim_scale_bwd", _msssim_scale_bwd_cuda, "CUDA")
 _LIB.impl("tv_sums", _tv_sums_cuda, "CUDA")
 _LIB.impl("tv_grad", _tv_grad_cuda, "CUDA")
 _LIB.impl("afb2d_select", _afb2d_select_cuda, "CUDA")
@@ -608,7 +667,8 @@ _LIB.impl("freq_mask_", _freq_mask_cuda, "CUDA")
 _LIB.impl("abs_sign", _abs_sign_cuda, "CUDA")
 _LIB.impl("sign_mul", _sign_mul_cuda, "CUDA")
 for _name in ("afb2d", "sfb2d", "afb1d", "sfb1d", "swt2d", "swt2d_adjoint", "ssim_fwd", "ssim_bwd", "tv_sums",
-              "tv_grad", "afb2d_select", "freq_mask_", "abs_sign", "sign_mul", "iswt2d"):
+              "tv_grad", "afb2d_select", "freq_mask_", "abs_sign", "sign_mul", "iswt2d", "msssim_scale",
+              "msssim_scale_bwd"):
     _LIB.impl(_name, _cpu_refuse(_name), "CPU")
 torch.library.register_fake("b200wave64::afb2d", _afb2d_fake, lib=_LIB)
 torch.library.register_fake("b200wave64::sfb2d", _sfb2d_fake, lib=_LIB)
@@ -631,6 +691,11 @@ torch.library.register_fake("b200wave64::iswt2d", lambda ll, y, wl, wh, hl, hh, 
                             y.new_empty((y.shape[0], y.shape[1] // 4, y.shape[2], y.shape[3])), lib=_LIB)
 torch.library.register_autograd("b200wave64::iswt2d", _iswt2d_backward, setup_context=_iswt2d_setup, lib=_LIB)
 torch.library.register_autograd("b200wave64::ssim_fwd", _ssim_backward, setup_context=_ssim_setup, lib=_LIB)
+torch.library.register_fake("b200wave64::msssim_scale", msssim_scale_fake, lib=_LIB)
+torch.library.register_fake("b200wave64::msssim_scale_bwd", lambda img1, img2, maps, g, win, up1, up2, need_d2:
+                            _ssim_bwd_fake(img1, img2, maps, g, win, False, need_d2), lib=_LIB)
+torch.library.register_autograd("b200wave64::msssim_scale", _msssim_scale_backward, setup_context=msssim_scale_setup,
+                                lib=_LIB)
 torch.library.register_fake("b200wave64::afb2d_select", _afb2d_select_fake, lib=_LIB)
 torch.library.register_autograd("b200wave64::afb2d_select", _afb2d_select_backward, setup_context=_afb2d_select_setup,
                                 lib=_LIB)
@@ -644,6 +709,8 @@ swt2d_adjoint = torch.ops.b200wave64.swt2d_adjoint
 iswt2d = torch.ops.b200wave64.iswt2d
 ssim_fwd = torch.ops.b200wave64.ssim_fwd
 ssim_bwd = torch.ops.b200wave64.ssim_bwd
+msssim_scale = torch.ops.b200wave64.msssim_scale
+msssim_scale_bwd = torch.ops.b200wave64.msssim_scale_bwd
 tv_sums = torch.ops.b200wave64.tv_sums
 tv_grad = torch.ops.b200wave64.tv_grad
 afb2d_select = torch.ops.b200wave64.afb2d_select

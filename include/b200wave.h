@@ -13,6 +13,7 @@
  *                       pw/dwt/lowlevel.py:349-365  AFB2D.backward (same arithmetic + crop to the input H, W)
  *   b200w_ssim_fwd_f32  ssim.py:17-37               _ssim (five 11x11 Gaussian blurs, SSIM map, mean)
  *   b200w_ssim_bwd_f32  autograd through ssim.py:17-37 (closed form, SURVEY.md 8a-a10)
+ *   b200w_msssim_scale_fwd_f32 / _bwd_f32 (and _f64)  one scale of MS-SSIM (no counterpart in the reference)
  *   b200w_dwt2_f32      pw/dwt/transform2d.py:66-74    the J-level loop of DWTForward.forward over AFB2D.apply,
  *                       and the backward of DWTInverse (J x SFB2D.backward through the 'unpad' crops) -- ONE launch
  *   b200w_idwt2_f32     pw/dwt/transform2d.py:134-148  the J-level loop of DWTInverse.forward over SFB2D.apply incl.
@@ -346,6 +347,36 @@ int b200w_ssim_bwd_f64(const double* img1, const double* img2, const double* map
                        const double* grad_out, int N, int C, int H, int W,
                        const double* win2d, int ws, int size_average,
                        double* d1, double* d2, void* stream);
+
+/*
+ * MS-SSIM, one scale (b200wave.ms_ssim chains them).  The arguments, status codes and order of the checks are those of
+ * b200w_ssim_fwd_f32 / b200w_ssim_bwd_f32 (and _f64, with the dense window), except:
+ *   - out / grad_out: always N per-sample values (means over C, H, W); there is no size_average.
+ *   - cs != 0: the value is the mean of the contrast-structure map cs = A2/B2 (= (2 sigma12 + C2) /
+ *     (sigma1^2 + sigma2^2 + C2)) and maps hold its derivatives, in the same order (d/dmu1, d/dE[x^2], d/dE[x1x2],
+ *     d/dmu2).  cs == 0: the SSIM map.  Either value is formed by correctly rounded division, so identical images
+ *     give exactly 1.
+ *   - pooled1, pooled2: DEVICE (N,C,H/2,W/2), written with avg_pool2d(img, 2) of img1 and img2 (an odd last row or
+ *     column is dropped), or both NULL (no pooling).  One NULL and one not: B200W_ERR_NULL_POINTER; pooling with
+ *     H < 2 or W < 2: B200W_ERR_BAD_SHAPE.
+ *   - up1, up2: DEVICE (N,C,H/2,W/2) gradients of the pooled images, or NULL; the backward adds
+ *     0.25 up[r/2][c/2] to d1 (d2) for r < 2 (H/2), c < 2 (W/2).  up2 without d2, or either with H < 2 or W < 2:
+ *     B200W_ERR_BAD_SHAPE.
+ * The workspace is that of b200w_ssim_fwd_f32 / _f64 (b200w_ssim_workspace_bytes / _f64).
+ */
+int b200w_msssim_scale_fwd_f32(const float* img1, const float* img2, int N, int C, int H, int W,
+                               const float* win, int ws, int cs, int n_maps, float* maps, float* out,
+                               float* pooled1, float* pooled2, void* workspace, size_t workspace_bytes, void* stream);
+int b200w_msssim_scale_bwd_f32(const float* img1, const float* img2, const float* maps, int n_maps,
+                               const float* grad_out, int N, int C, int H, int W, const float* win, int ws,
+                               const float* up1, const float* up2, float* d1, float* d2, void* stream);
+int b200w_msssim_scale_fwd_f64(const double* img1, const double* img2, int N, int C, int H, int W,
+                               const double* win2d, int ws, int cs, int n_maps, double* maps, double* out,
+                               double* pooled1, double* pooled2, void* workspace, size_t workspace_bytes,
+                               void* stream);
+int b200w_msssim_scale_bwd_f64(const double* img1, const double* img2, const double* maps, int n_maps,
+                               const double* grad_out, int N, int C, int H, int W, const double* win2d, int ws,
+                               const double* up1, const double* up2, double* d1, double* d2, void* stream);
 
 /*
  * phase_consistency_loss, model.py:36-58 (constructed at train.py:94), SURVEY.md 8f row 4: minus the cosine

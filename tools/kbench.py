@@ -1,7 +1,7 @@
 """Kernel micro-benchmark: per-launch duration of single levels / SSIM kernels (CUDA graph of back-to-back
 launches over rotating inputs larger than L2, CUDA events).
 
-    python tools/kbench.py [dwt|ssim|swt|iswt|dwt1d|fsd|freq|tv|all]
+    python tools/kbench.py [dwt|ssim|msssim|swt|iswt|dwt1d|fsd|freq|tv|all]
 """
 import os
 import sys
@@ -252,3 +252,61 @@ if what in ("tv", "all"):
     tv_case(8, 256, 256)
     tv_case(64, 304, 304)
     tv_case(64, 1024, 1024)
+
+
+def msssim_case(n, h, w, M=5):
+    """MS-SSIM (M scales, gradient of img1): the scale ops against the same formula written in torch ops (dense 11x11
+    F.conv2d, avg_pool2d, autograd).  Algorithmic bytes per pixel of scale j: forward 8 in + 2 pooled (not at the last
+    scale) + 12 saved maps; backward 20 in + 1 for the coarser scale's gradient (not at the last scale) + 4 out."""
+    import torch.nn.functional as F
+    from b200wave.ssim import create_window
+    nsets = max(2, int(2 * 126e6 / (8 * n * h * w)) + 1)
+    a = [torch.rand(n, 1, h, w, device=dev).requires_grad_(True) for _ in range(nsets)]
+    b = [(t.detach() + 0.1 * torch.randn_like(t)).clamp_(0, 1) for t in a]
+    weights = b200wave.msssim.WEIGHTS
+    win2d = create_window(11, 1).to(dev)
+
+    def torch_ms(x, y):
+        vals = []
+        for j in range(M):
+            if j:
+                x, y = F.avg_pool2d(x, 2), F.avg_pool2d(y, 2)
+            mu1, mu2 = F.conv2d(x, win2d, padding=5), F.conv2d(y, win2d, padding=5)
+            s11 = F.conv2d(x * x, win2d, padding=5) - mu1 * mu1
+            s22 = F.conv2d(y * y, win2d, padding=5) - mu2 * mu2
+            s12 = F.conv2d(x * y, win2d, padding=5) - mu1 * mu2
+            cs = (2 * s12 + 0.03 ** 2) / (s11 + s22 + 0.03 ** 2)
+            if j == M - 1:
+                cs = (2 * mu1 * mu2 + 0.01 ** 2) / (mu1 * mu1 + mu2 * mu2 + 0.01 ** 2) * cs
+            vals.append(cs.mean(dim=(1, 2, 3)))
+        ms = 1.0
+        for v, wj in zip(vals, weights):
+            ms = ms * torch.relu(v) ** wj
+        return ms.mean()
+
+    ours = lambda i: b200wave.ms_ssim(a[i % nsets], b[i % nsets])
+    ref = lambda i: torch_ms(a[i % nsets], b[i % nsets])
+    t_f = timeit(ours, nsets, 20)
+    t_fb = timeit(lambda i: torch.autograd.grad(ours(i), a[i % nsets]), nsets, 20)
+    r_f = timeit(ref, nsets, 20)
+    r_fb = timeit(lambda i: torch.autograd.grad(ref(i), a[i % nsets]), nsets, 20)
+    err = (b200wave.ms_ssim(a[0], b[0]) - torch_ms(a[0], b[0])).abs().item()
+    px = [n * (h >> j) * (w >> j) for j in range(M)]
+    by_f = sum(p * (20 + (2 if j < M - 1 else 0)) for j, p in enumerate(px))
+    by_b = sum(p * (24 + (1 if j < M - 1 else 0)) for j, p in enumerate(px))
+    t_b = t_fb - t_f
+    print("msssim M=%d %4dx%4dx%4d  fwd %7.1f us %6.1f Gpx/s %5.0f GB/s (%4.1f%%) | bwd %7.1f us %5.0f GB/s (%4.1f%%) | "
+          "fwd+bwd %7.1f us | torch ops fwd %8.1f us fwd+bwd %8.1f us (x%.1f) | |ours - torch| %.1e" % (
+              M, n, h, w, t_f * 1e6, px[0] / t_f / 1e9, by_f / t_f / 1e9, by_f / t_f / 1e9 / PEAK * 100, t_b * 1e6,
+              by_b / t_b / 1e9, by_b / t_b / 1e9 / PEAK * 100, t_fb * 1e6, r_f * 1e6, r_fb * 1e6, r_fb / t_fb, err),
+          flush=True)
+
+
+if what in ("msssim", "all"):
+    import subprocess
+    q = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit,clocks.max.sm", "--format=csv,noheader"],
+                       capture_output=True, text=True).stdout.strip().splitlines()
+    print("device: %s | nvidia-smi: %s" % (torch.cuda.get_device_name(), q[0] if q else "n/a"), flush=True)
+    msssim_case(8, 256, 256)
+    msssim_case(64, 256, 256)
+    msssim_case(256, 400, 400)
