@@ -13,91 +13,84 @@ Differentiable: the filter is linear and self-adjoint (real, even mask), ``abs``
 float32 and float64 images are served; float64 is the reference's double mode (complex128 FFTs, the mask evaluated in
 double and rounded to fp32 as ``torch.from_numpy(mask).float()`` stores it), through the ``ops64`` twins of the ops.
 """
-import ctypes
+import functools
 
 import torch
 from torch.autograd.function import once_differentiable
 
-from . import _cabi, ops64
+from . import _cabi
+from .ops import F32, _cpu_refuse, _require, _stream
 
 _LIB = torch.library.Library("b200wave_freq", "DEF")
 _LIB.define("mask_(Tensor(a!) spec, int rows, int cols, float radius, bool highpass) -> Tensor(a!)")
 _LIB.define("abs_sign(Tensor x, float sign) -> Tensor")
 _LIB.define("sign_mul(Tensor g, Tensor x, float sign) -> Tensor")
 
-
-def _stream():
-    return ctypes.c_void_p(torch.cuda.current_stream().cuda_stream)
-
-
-def _require(t, name, dtype):
-    if not t.is_cuda:
-        raise RuntimeError("b200wave_freq::%s is CUDA-only (sm_100a); there is no CPU fallback -- got a %s tensor"
-                           % (name, t.device))
-    if t.dtype != dtype:
-        raise RuntimeError("b200wave_freq::%s: expected %s but found %s" % (name, dtype, t.dtype))
+# the fp32 ops live in this namespace; their float64 / complex128 twins, b200wave64::freq_mask_ / abs_sign / sign_mul,
+# are registered by ops64 from the same bodies (the reference's double mode)
+_F32 = F32._replace(ns="b200wave_freq")
 
 
-def _mask_cuda(spec, rows, cols, radius, highpass):
-    _require(spec, "mask_", torch.complex64)
+def _mask_cuda(p, spec, rows, cols, radius, highpass):
+    f64 = p.dtype == torch.float64
+    name = "freq_mask_" if f64 else "mask_"
+    _require(p, spec, name, p.dtype.to_complex())
     if not spec.is_contiguous() or spec.shape[-2] != rows or spec.shape[-1] != cols // 2 + 1:
-        raise RuntimeError("b200wave_freq::mask_ expects the contiguous half spectrum (..., %d, %d), got %s"
-                           % (rows, cols // 2 + 1, tuple(spec.shape)))
+        raise RuntimeError("%s::%s expects the contiguous half spectrum (..., %d, %d), got %s"
+                           % (p.ns, name, rows, cols // 2 + 1, tuple(spec.shape)))
     if spec.numel() == 0:
         return spec
     planes = spec.numel() // (rows * (cols // 2 + 1))
+    lib = _cabi.load()
+    mask = lib.b200w_freq_mask_c128 if f64 else lib.b200w_freq_mask_c64
     with torch.cuda.device(spec.device):
-        rc = _cabi.load().b200w_freq_mask_c64(spec.data_ptr(), planes, rows, cols, float(radius), int(bool(highpass)),
-                                              _stream())
+        rc = mask(spec.data_ptr(), planes, rows, cols, float(radius), int(bool(highpass)), _stream())
     _cabi.check(rc)
     return spec
 
 
-def _abs_sign_cuda(x, sign):
-    _require(x, "abs_sign", torch.float32)
+def _abs_sign_cuda(p, x, sign):
+    _require(p, x, "abs_sign")
     x = x.contiguous()
     y = torch.empty_like(x)
     with torch.cuda.device(x.device):
-        rc = _cabi.load().b200w_abs_sign_f32(x.data_ptr(), y.data_ptr(), x.numel(), float(sign), _stream())
+        rc = p.lib.b200w_abs_sign(x.data_ptr(), y.data_ptr(), x.numel(), float(sign), _stream())
     _cabi.check(rc)
     return y
 
 
-def _sign_mul_cuda(g, x, sign):
-    _require(g, "sign_mul", torch.float32)
-    _require(x, "sign_mul", torch.float32)
+def _sign_mul_cuda(p, g, x, sign):
+    _require(p, g, "sign_mul")
+    _require(p, x, "sign_mul")
     g, x = g.contiguous(), x.contiguous()
     out = torch.empty_like(x)
     with torch.cuda.device(x.device):
-        rc = _cabi.load().b200w_sign_mul_f32(g.data_ptr(), x.data_ptr(), out.data_ptr(), x.numel(), float(sign), _stream())
+        rc = p.lib.b200w_sign_mul(g.data_ptr(), x.data_ptr(), out.data_ptr(), x.numel(), float(sign), _stream())
     _cabi.check(rc)
     return out
 
 
-def _cpu_refuse(name):
-    def impl(*args, **kwargs):
-        raise RuntimeError("b200wave_freq::%s is CUDA-only (sm_100a): there is no CPU fallback." % name)
-    return impl
-
-
-_LIB.impl("mask_", _mask_cuda, "CUDA")
-_LIB.impl("abs_sign", _abs_sign_cuda, "CUDA")
-_LIB.impl("sign_mul", _sign_mul_cuda, "CUDA")
+_LIB.impl("mask_", functools.partial(_mask_cuda, _F32), "CUDA")
+_LIB.impl("abs_sign", functools.partial(_abs_sign_cuda, _F32), "CUDA")
+_LIB.impl("sign_mul", functools.partial(_sign_mul_cuda, _F32), "CUDA")
 for _name in ("mask_", "abs_sign", "sign_mul"):
-    _LIB.impl(_name, _cpu_refuse(_name), "CPU")
+    _LIB.impl(_name, _cpu_refuse(_F32.ns, _name), "CPU")
 
 
-# (mask_, abs_sign, sign_mul) by dtype: fp32 here, float64 / complex128 in ops64 (the reference's double mode)
-_OPS = {torch.float32: (torch.ops.b200wave_freq.mask_, torch.ops.b200wave_freq.abs_sign,
-                        torch.ops.b200wave_freq.sign_mul),
-        torch.float64: (ops64.freq_mask_, ops64.abs_sign, ops64.sign_mul)}
+@functools.cache
+def _ops(dtype):
+    """(mask_, abs_sign, sign_mul) of the dtype, looked up on first use: the float64 / complex128 ones are registered by
+    ops64, which imports this module."""
+    if dtype == torch.float64:
+        return torch.ops.b200wave64.freq_mask_, torch.ops.b200wave64.abs_sign, torch.ops.b200wave64.sign_mul
+    return torch.ops.b200wave_freq.mask_, torch.ops.b200wave_freq.abs_sign, torch.ops.b200wave_freq.sign_mul
 
 
 def _filter(x, radius, highpass):
     """irfft2(mask * rfft2(x)) over the last two dims (cuFFT + the in-place mask kernel)."""
     rows, cols = x.shape[-2:]
     spec = torch.fft.rfft2(x).contiguous()
-    _OPS[x.dtype][0](spec, rows, cols, float(radius), bool(highpass))
+    _ops(x.dtype)[0](spec, rows, cols, float(radius), bool(highpass))
     return torch.fft.irfft2(spec, s=(rows, cols))
 
 
@@ -107,14 +100,14 @@ class _GaussianSplit(torch.autograd.Function):
         y = _filter(x, radius, highpass)
         ctx.save_for_backward(y)
         ctx.args = (radius, highpass, sign)
-        return _OPS[y.dtype][1](y, float(sign))
+        return _ops(y.dtype)[1](y, float(sign))
 
     @staticmethod
     @once_differentiable   # the backward kernels have no autograd formula of their own: double backward raises
     def backward(ctx, g):
         (y,) = ctx.saved_tensors
         radius, highpass, sign = ctx.args
-        t = _OPS[y.dtype][2](g, y, float(sign))
+        t = _ops(y.dtype)[2](g, y, float(sign))
         return _filter(t, radius, highpass), None, None, None   # the filter is self-adjoint
 
 
@@ -123,7 +116,7 @@ def gaussian_split(x, radius, highpass, sign=1.0):
     the rest.  float64 follows the reference's double mode: complex128 FFTs, the mask rounded to fp32."""
     if not x.is_cuda:
         raise RuntimeError("b200wave.freq is CUDA-only (sm_100a); there is no CPU fallback -- got a %s tensor" % x.device)
-    if x.dtype not in _OPS:
+    if x.dtype not in (torch.float32, torch.float64):
         raise RuntimeError("b200wave.freq: expected scalar type Float but found %s" % x.dtype)
     if x.dim() < 2:
         raise ValueError("b200wave.freq expects (..., H, W)")

@@ -15,13 +15,14 @@ evaluated in place (``b200w_phase_sums_c64``), one kernel for the gradient w.r.t
 (``b200w_phase_grad_c64``); autograd's own ``rfft2`` backward carries it to the images.
 CUDA-only, like the rest of the package.
 """
-import ctypes
+import functools
 
 import torch
 from torch.autograd.function import once_differentiable
 import torch.nn as nn
 
-from . import _cabi, ops64
+from . import _cabi
+from .ops import F32, _cpu_refuse, _require, _stream
 
 _LIB = torch.library.Library("b200wave_losses", "DEF")
 _LIB.define("tv_sums(Tensor x) -> Tensor")
@@ -30,58 +31,60 @@ _LIB.define("phase_sums(Tensor fx, Tensor fy, int cols, float radius) -> Tensor"
 _LIB.define("phase_grad(Tensor fx, Tensor fy, int cols, float radius, Tensor sums, Tensor grad_out, float eps) "
             "-> (Tensor, Tensor)")
 
+# the fp32 TV ops live in this namespace; their float64 twins, b200wave64::tv_*, are registered by ops64 from the
+# same bodies
+_F32 = F32._replace(ns="b200wave_losses")
 
-def _stream():
-    return ctypes.c_void_p(torch.cuda.current_stream().cuda_stream)
 
-
-def _check(x, name):
-    if not x.is_cuda:
-        raise RuntimeError("b200wave_losses::%s is CUDA-only (sm_100a); there is no CPU fallback -- got a %s tensor"
-                           % (name, x.device))
-    if x.dtype != torch.float32:
-        raise RuntimeError("b200wave_losses::%s: expected scalar type Float but found %s" % (name, x.dtype))
+def _check_tv(p, x, name):
+    _require(p, x, name)
     if x.dim() != 4:
-        raise IndexError("b200wave_losses::%s expects a 4-D (N, C, H, W) tensor, got %d-D" % (name, x.dim()))
+        raise IndexError("%s::%s expects a 4-D (N, C, H, W) tensor, got %d-D" % (p.ns, name, x.dim()))
 
 
-def _tv_sums_cuda(x):
+def _tv_sums_cuda(p, x):
     """(2,) tensor: sum of squared vertical / horizontal forward differences (model.py:28-29)."""
-    _check(x, "tv_sums")
+    _check_tv(p, x, "tv_sums")
     lib = _cabi.load()
     xc = x.contiguous()
     n, c, h, w = xc.shape
-    out = torch.zeros(2, device=x.device, dtype=torch.float32)
+    out = torch.zeros(2, device=x.device, dtype=p.dtype)
     if xc.numel() == 0:
         return out
-    ws = torch.empty(int(lib.b200w_tv_workspace_bytes(n * c, h)), device=x.device, dtype=torch.uint8)
+    nbytes = (lib.b200w_tv_workspace_bytes_f64 if p.dtype == torch.float64 else lib.b200w_tv_workspace_bytes)(n * c, h)
+    ws = torch.empty(int(nbytes), device=x.device, dtype=torch.uint8)
     with torch.cuda.device(x.device):
-        rc = lib.b200w_tv_fwd_f32(xc.data_ptr(), n * c, h, w, ws.data_ptr(), ws.numel(), out.data_ptr(), _stream())
+        rc = p.lib.b200w_tv_fwd(xc.data_ptr(), n * c, h, w, ws.data_ptr(), ws.numel(), out.data_ptr(), _stream())
     _cabi.check(rc, "tv")
     return out
 
 
-def _tv_grad_cuda(x, grad_out, ch, cw):
-    _check(x, "tv_grad")
-    lib = _cabi.load()
+def _tv_sums_fake(x):
+    return x.new_empty((2,))
+
+
+def _tv_grad_cuda(p, x, grad_out, ch, cw):
+    _check_tv(p, x, "tv_grad")
     xc = x.contiguous()
     n, c, h, w = xc.shape
     dx = torch.empty_like(xc)
     if xc.numel() == 0:
         return dx
-    g = grad_out.reshape(-1)[:1].to(torch.float32).contiguous()
+    g = grad_out.reshape(-1)[:1].to(p.dtype).contiguous()
     with torch.cuda.device(x.device):
-        rc = lib.b200w_tv_bwd_f32(xc.data_ptr(), g.data_ptr(), float(ch), float(cw), n * c, h, w, dx.data_ptr(),
-                                  _stream())
+        rc = p.lib.b200w_tv_bwd(xc.data_ptr(), g.data_ptr(), float(ch), float(cw), n * c, h, w, dx.data_ptr(),
+                                _stream())
     _cabi.check(rc, "tv")
     return dx
 
 
+def _tv_grad_fake(x, grad_out, ch, cw):
+    return torch.empty_like(x)
+
+
 def _check_spec(f, name):
-    if not f.is_cuda:
-        raise RuntimeError("b200wave_losses::%s is CUDA-only (sm_100a); there is no CPU fallback -- got a %s tensor"
-                           % (name, f.device))
-    if f.dtype != torch.float32 or f.dim() != 4 or f.shape[-1] != 2:
+    _require(_F32, f, name)
+    if f.dim() != 4 or f.shape[-1] != 2:
         raise RuntimeError("b200wave_losses::%s expects view_as_real of a (C, rows, cols/2+1) complex64 half spectrum"
                            % name)
 
@@ -120,27 +123,18 @@ def _phase_grad_cuda(fx, fy, cols, radius, sums, grad_out, eps):
     return gx, gy
 
 
-def _cpu_refuse(name):
-    def impl(*args, **kwargs):
-        raise RuntimeError("b200wave_losses::%s is CUDA-only (sm_100a): there is no CPU fallback. Move the tensors "
-                           "to a B200 (`.cuda()`)." % name)
-    return impl
-
-
-_LIB.impl("tv_sums", _tv_sums_cuda, "CUDA")
-_LIB.impl("tv_grad", _tv_grad_cuda, "CUDA")
-_LIB.impl("tv_sums", _cpu_refuse("tv_sums"), "CPU")
-_LIB.impl("tv_grad", _cpu_refuse("tv_grad"), "CPU")
+_LIB.impl("tv_sums", functools.partial(_tv_sums_cuda, _F32), "CUDA")
+_LIB.impl("tv_grad", functools.partial(_tv_grad_cuda, _F32), "CUDA")
 _LIB.impl("phase_sums", _phase_sums_cuda, "CUDA")
 _LIB.impl("phase_grad", _phase_grad_cuda, "CUDA")
-_LIB.impl("phase_sums", _cpu_refuse("phase_sums"), "CPU")
-_LIB.impl("phase_grad", _cpu_refuse("phase_grad"), "CPU")
+for _name in ("tv_sums", "tv_grad", "phase_sums", "phase_grad"):
+    _LIB.impl(_name, _cpu_refuse(_F32.ns, _name), "CPU")
 torch.library.register_fake("b200wave_losses::phase_sums", lambda fx, fy, cols, radius: fx.new_empty((3,)), lib=_LIB)
 torch.library.register_fake("b200wave_losses::phase_grad",
                             lambda fx, fy, cols, radius, sums, g, eps: (torch.empty_like(fx), torch.empty_like(fy)),
                             lib=_LIB)
-torch.library.register_fake("b200wave_losses::tv_sums", lambda x: x.new_empty((2,)), lib=_LIB)
-torch.library.register_fake("b200wave_losses::tv_grad", lambda x, g, ch, cw: torch.empty_like(x), lib=_LIB)
+torch.library.register_fake("b200wave_losses::tv_sums", _tv_sums_fake, lib=_LIB)
+torch.library.register_fake("b200wave_losses::tv_grad", _tv_grad_fake, lib=_LIB)
 
 
 class _TV(torch.autograd.Function):
@@ -150,7 +144,7 @@ class _TV(torch.autograd.Function):
         count_h = c * (h - 1) * w          # model.py:26-27 via _tensor_size
         count_w = c * h * (w - 1)
         f64 = x.dtype == torch.float64
-        sums = ops64.tv_sums(x) if f64 else torch.ops.b200wave_losses.tv_sums(x)
+        sums = torch.ops.b200wave64.tv_sums(x) if f64 else torch.ops.b200wave_losses.tv_sums(x)
         ctx.save_for_backward(x)
         ctx.f64 = f64
         ctx.scales = (weight, n, count_h, count_w)
@@ -164,7 +158,7 @@ class _TV(torch.autograd.Function):
         weight, n, count_h, count_w = ctx.scales
         ch = weight * 2.0 / (n * count_h) if count_h else float("nan")
         cw = weight * 2.0 / (n * count_w) if count_w else float("nan")
-        grad = ops64.tv_grad if ctx.f64 else torch.ops.b200wave_losses.tv_grad
+        grad = torch.ops.b200wave64.tv_grad if ctx.f64 else torch.ops.b200wave_losses.tv_grad
         return grad(x, g, ch, cw), None
 
 

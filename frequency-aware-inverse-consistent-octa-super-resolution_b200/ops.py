@@ -6,6 +6,10 @@ outputs with torch (the library never allocates) and launches on torch's
 current stream, so the ops are asynchronous and CUDA-graph capturable.
 CUDA-only: there is deliberately no CPU implementation.
 
+The ops that have a float64 twin in ``b200wave64::*`` (``ops64.py``) are written once here: every CUDA body and
+backward takes a ``Precision`` as its first argument, and each namespace registers them with
+``functools.partial(body, F32)`` / ``functools.partial(body, F64)``.
+
 Autograd follows the reference's hand-written backward passes, not the
 mathematical adjoint (SURVEY.md 8a-Q1):
 
@@ -18,11 +22,41 @@ mathematical adjoint (SURVEY.md 8a-Q1):
   plus the transpose of the 2x2 pooling applied to the gradients of the pooled outputs
 """
 import ctypes
+import functools
+from typing import Callable, NamedTuple
 
 import torch
 from torch.autograd.function import once_differentiable
 
 from . import _cabi
+
+
+class _Suffixed:
+    """The C library seen through one precision's symbol suffix: ``F64.lib.b200w_afb2d`` is ``b200w_afb2d_f64``.
+    Each entry point is looked up once, on first use, so that no call formats a symbol name."""
+
+    def __init__(self, suffix):
+        self.suffix = suffix
+
+    def __getattr__(self, name):
+        fn = getattr(_cabi.load(), name + self.suffix)
+        setattr(self, name, fn)
+        return fn
+
+
+class Precision(NamedTuple):
+    """What an fp32 op and its float64 twin differ in."""
+    ns: str               # op namespace, as messages name it
+    dtype: torch.dtype
+    scalar: str           # the dtype as messages name it
+    taps: Callable        # host taps -> (ctypes array, count)
+    lib: _Suffixed        # the C library under the entry points' names without their _f32 / _f64 suffix
+    elem: int             # bytes per element of the SSIM workspace
+    dense_win: bool       # SSIM window: 1-D separable taps (False) or the dense ws x ws window, row-major (True)
+
+
+F32 = Precision("b200wave", torch.float32, "Float", _cabi.taps_array, _Suffixed("_f32"), 4, False)
+F64 = Precision("b200wave64", torch.float64, "Double", _cabi.taps_array_f64, _Suffixed("_f64"), 8, True)
 
 _LIB = torch.library.Library("b200wave", "DEF")
 
@@ -77,12 +111,20 @@ def _stream():
     return ctypes.c_void_p(torch.cuda.current_stream().cuda_stream)
 
 
-def _require_cuda_f32(t, name):
+def _require(p, t, name, dtype=None):
+    """``t`` must be a CUDA tensor of the precision's dtype, or of ``dtype`` (the complex spectrum of ``freq``)."""
     if not t.is_cuda:
-        raise RuntimeError("b200wave::%s is CUDA-only (sm_100a); there is no CPU fallback -- got a %s tensor"
-                           % (name, t.device))
-    if t.dtype != torch.float32:
-        raise RuntimeError("b200wave::%s: expected scalar type Float but found %s" % (name, t.dtype))
+        raise RuntimeError("%s::%s is CUDA-only (sm_100a); there is no CPU fallback -- got a %s tensor"
+                           % (p.ns, name, t.device))
+    if t.dtype != (dtype or p.dtype):
+        raise RuntimeError("%s::%s: expected scalar type %s but found %s" % (p.ns, name, dtype or p.scalar, t.dtype))
+
+
+def _cpu_refuse(ns, name):
+    def impl(*args, **kwargs):
+        raise RuntimeError("%s::%s is CUDA-only (sm_100a): there is no CPU fallback. Move the tensors to a B200 "
+                           "(`.cuda()`)." % (ns, name))
+    return impl
 
 
 def _planes_view(t):
@@ -99,29 +141,28 @@ def _planes_view(t):
 
 
 # ------------------------------------------------------------------------------------------- afb2d
-def _afb2d_cuda(x, w_lo, w_hi, h_lo, h_hi, mode):
+def _afb2d_cuda(p, x, w_lo, w_hi, h_lo, h_hi, mode):
     _check_mode(mode)
-    _require_cuda_f32(x, "afb2d")
+    _require(p, x, "afb2d")
     if x.dim() != 4:
-        raise IndexError("b200wave::afb2d expects a 4-D (N, C, H, W) tensor, got %d-D" % x.dim())
-    lib = _cabi.load()
+        raise IndexError("%s::afb2d expects a 4-D (N, C, H, W) tensor, got %d-D" % (p.ns, x.dim()))
     N, C, H, W = x.shape
     Lw, Lh = len(w_lo), len(h_lo)
     if len(w_hi) != Lw or len(h_hi) != Lh:
         raise RuntimeError("low- and high-pass filters must have the same length along an axis")
     Ho, Wo = coeff_len(H, Lh, mode), coeff_len(W, Lw, mode)
-    low = torch.empty((N, C, Ho, Wo), device=x.device, dtype=torch.float32)
-    highs = torch.empty((N, C, 3, Ho, Wo), device=x.device, dtype=torch.float32)
+    low = torch.empty((N, C, Ho, Wo), device=x.device, dtype=p.dtype)
+    highs = torch.empty((N, C, 3, Ho, Wo), device=x.device, dtype=p.dtype)
     if low.numel() == 0:
         return low, highs
     xk, ps, rs = _planes_view(x)
-    a_wl, _ = _cabi.taps_array(w_lo)
-    a_wh, _ = _cabi.taps_array(w_hi)
-    a_hl, _ = _cabi.taps_array(h_lo)
-    a_hh, _ = _cabi.taps_array(h_hi)
+    a_wl, _ = p.taps(w_lo)
+    a_wh, _ = p.taps(w_hi)
+    a_hl, _ = p.taps(h_lo)
+    a_hh, _ = p.taps(h_hi)
     with torch.cuda.device(x.device):
-        rc = lib.b200w_afb2d_f32(xk.data_ptr(), ps, rs, N * C, H, W, a_wl, a_wh, Lw, a_hl, a_hh, Lh, int(mode),
-                                 low.data_ptr(), highs.data_ptr(), _stream())
+        rc = p.lib.b200w_afb2d(xk.data_ptr(), ps, rs, N * C, H, W, a_wl, a_wh, Lw, a_hl, a_hh, Lh, int(mode),
+                               low.data_ptr(), highs.data_ptr(), _stream())
     _cabi.check(rc, _mode_name(mode))
     return low, highs
 
@@ -133,35 +174,34 @@ def _afb2d_fake(x, w_lo, w_hi, h_lo, h_hi, mode):
 
 
 # ------------------------------------------------------------------------------------------- afb2d_select
-def _afb2d_select_cuda(x, w_lo, w_hi, h_lo, h_hi, mode, want_low, want_highs, hi_scale, hi_shift):
+def _afb2d_select_cuda(p, x, w_lo, w_hi, h_lo, h_hi, mode, want_low, want_highs, hi_scale, hi_shift):
     """One analysis level that writes only the sub-bands asked for, the detail bands as hi_scale*v + hi_shift
     (FS_Discriminator.filter_wavelet, model.py:166-179): an output that is not wanted comes back with 0 elements
     and costs no HBM traffic."""
     _check_mode(mode)
-    _require_cuda_f32(x, "afb2d_select")
+    _require(p, x, "afb2d_select")
     if x.dim() != 4:
-        raise IndexError("b200wave::afb2d_select expects a 4-D (N, C, H, W) tensor, got %d-D" % x.dim())
+        raise IndexError("%s::afb2d_select expects a 4-D (N, C, H, W) tensor, got %d-D" % (p.ns, x.dim()))
     if not (want_low or want_highs):
         raise ValueError("afb2d_select: at least one of the low-pass / detail outputs must be requested")
-    lib = _cabi.load()
     N, C, H, W = x.shape
     Lw, Lh = len(w_lo), len(h_lo)
     if len(w_hi) != Lw or len(h_hi) != Lh:
         raise RuntimeError("low- and high-pass filters must have the same length along an axis")
     Ho, Wo = coeff_len(H, Lh, mode), coeff_len(W, Lw, mode)
-    low = torch.empty((N, C, Ho, Wo) if want_low else (0,), device=x.device, dtype=torch.float32)
-    highs = torch.empty((N, C, 3, Ho, Wo) if want_highs else (0,), device=x.device, dtype=torch.float32)
+    low = torch.empty((N, C, Ho, Wo) if want_low else (0,), device=x.device, dtype=p.dtype)
+    highs = torch.empty((N, C, 3, Ho, Wo) if want_highs else (0,), device=x.device, dtype=p.dtype)
     if N * C * Ho * Wo == 0:
         return low, highs
     xk, ps, rs = _planes_view(x)
-    a_wl, _ = _cabi.taps_array(w_lo)
-    a_wh, _ = _cabi.taps_array(w_hi)
-    a_hl, _ = _cabi.taps_array(h_lo)
-    a_hh, _ = _cabi.taps_array(h_hi)
+    a_wl, _ = p.taps(w_lo)
+    a_wh, _ = p.taps(w_hi)
+    a_hl, _ = p.taps(h_lo)
+    a_hh, _ = p.taps(h_hi)
     with torch.cuda.device(x.device):
-        rc = lib.b200w_afb2d_ex_f32(xk.data_ptr(), ps, rs, N * C, H, W, a_wl, a_wh, Lw, a_hl, a_hh, Lh, int(mode),
-                                    low.data_ptr() if want_low else None, highs.data_ptr() if want_highs else None,
-                                    float(hi_scale), float(hi_shift), _stream())
+        rc = p.lib.b200w_afb2d_ex(xk.data_ptr(), ps, rs, N * C, H, W, a_wl, a_wh, Lw, a_hl, a_hh, Lh, int(mode),
+                                  low.data_ptr() if want_low else None, highs.data_ptr() if want_highs else None,
+                                  float(hi_scale), float(hi_shift), _stream())
     _cabi.check(rc, _mode_name(mode))
     return low, highs
 
@@ -183,7 +223,7 @@ def _afb2d_select_setup(ctx, inputs, output):
     ctx.set_materialize_grads(False)
 
 
-def _afb2d_select_backward(ctx, dlow, dhighs):
+def _afb2d_select_backward(p, ctx, dlow, dhighs):
     none = (None,) * 10
     if not ctx.needs_input_grad[0]:
         return none
@@ -199,41 +239,40 @@ def _afb2d_select_backward(ctx, dlow, dhighs):
     if dhighs is not None and ctx.hi_scale != 1.0:
         dhighs = dhighs * ctx.hi_scale   # d(hi_scale * v + hi_shift) / dv
     # same pseudo-adjoint as AFB2D.backward (lowlevel.py:356-364); a missing detail gradient is never materialised
-    dx = torch.ops.b200wave.sfb2d(dlow, dhighs, w_lo, w_hi, h_lo, h_hi, ctx.mode, H, W)
+    dx = getattr(torch.ops, p.ns).sfb2d(dlow, dhighs, w_lo, w_hi, h_lo, h_hi, ctx.mode, H, W)
     return (dx,) + none[1:]
 
 
 # ------------------------------------------------------------------------------------------- sfb2d
-def _sfb2d_cuda(low, highs, w_lo, w_hi, h_lo, h_hi, mode, out_h, out_w):
+def _sfb2d_cuda(p, low, highs, w_lo, w_hi, h_lo, h_hi, mode, out_h, out_w):
     _check_mode(mode)
-    _require_cuda_f32(low, "sfb2d")
+    _require(p, low, "sfb2d")
     if low.dim() != 4:
-        raise IndexError("b200wave::sfb2d expects a 4-D (N, C, h, w) lowpass tensor, got %d-D" % low.dim())
-    lib = _cabi.load()
+        raise IndexError("%s::sfb2d expects a 4-D (N, C, h, w) lowpass tensor, got %d-D" % (p.ns, low.dim()))
     N, C, h, w = low.shape
     Lw, Lh = len(w_lo), len(h_lo)
     if len(w_hi) != Lw or len(h_hi) != Lh:
         raise RuntimeError("low- and high-pass filters must have the same length along an axis")
     if highs is not None:
-        _require_cuda_f32(highs, "sfb2d")
+        _require(p, highs, "sfb2d")
         if tuple(highs.shape) != (N, C, 3, h, w):
-            raise RuntimeError("b200wave::sfb2d: highs must have shape %s, got %s"
-                               % ((N, C, 3, h, w), tuple(highs.shape)))
+            raise RuntimeError("%s::sfb2d: highs must have shape %s, got %s"
+                               % (p.ns, (N, C, 3, h, w), tuple(highs.shape)))
         highs = highs.contiguous()
     full_h, full_w = idwt_len(h, Lh, mode), idwt_len(w, Lw, mode)
     oh = full_h if out_h < 0 else out_h
     ow = full_w if out_w < 0 else out_w
-    y = torch.empty((N, C, oh, ow), device=low.device, dtype=torch.float32)
+    y = torch.empty((N, C, oh, ow), device=low.device, dtype=p.dtype)
     if y.numel() == 0:
         return y
     lk, ps, rs = _planes_view(low)
-    a_wl, _ = _cabi.taps_array(w_lo)
-    a_wh, _ = _cabi.taps_array(w_hi)
-    a_hl, _ = _cabi.taps_array(h_lo)
-    a_hh, _ = _cabi.taps_array(h_hi)
+    a_wl, _ = p.taps(w_lo)
+    a_wh, _ = p.taps(w_hi)
+    a_hl, _ = p.taps(h_lo)
+    a_hh, _ = p.taps(h_hi)
     with torch.cuda.device(low.device):
-        rc = lib.b200w_sfb2d_f32(lk.data_ptr(), ps, rs, None if highs is None else highs.data_ptr(), N * C, h, w,
-                                 a_wl, a_wh, Lw, a_hl, a_hh, Lh, int(mode), y.data_ptr(), oh, ow, _stream())
+        rc = p.lib.b200w_sfb2d(lk.data_ptr(), ps, rs, None if highs is None else highs.data_ptr(), N * C, h, w,
+                               a_wl, a_wh, Lw, a_hl, a_hh, Lh, int(mode), y.data_ptr(), oh, ow, _stream())
     _cabi.check(rc, _mode_name(mode))
     return y
 
@@ -260,7 +299,7 @@ def dwt2_level_dims(H, W, Lh, Lw, mode, J, pad_hw=()):
 def _dwt2_cuda(x, w_lo, w_hi, h_lo, h_hi, mode, J, pad_hw):
     """J analysis levels in one launch; returns [yl, yh_0 (finest), ..., yh_{J-1}]."""
     _check_mode(mode)
-    _require_cuda_f32(x, "dwt2")
+    _require(F32, x, "dwt2")
     if x.dim() != 4:
         raise IndexError("b200wave::dwt2 expects a 4-D (N, C, H, W) tensor, got %d-D" % x.dim())
     if not 1 <= J <= _cabi.MAX_LEVELS:
@@ -303,7 +342,7 @@ def _idwt2_cuda(yl, yh, hw, w_lo, w_hi, h_lo, h_hi, mode, out_hw):
     """J synthesis levels in one launch.  hw = 2*J ints (h_j, w_j): sub-band size of level j (yh index, finest
     first); out_hw = 2*J ints (per-level output size, a crop of the natural one) or [] for the natural sizes."""
     _check_mode(mode)
-    _require_cuda_f32(yl, "idwt2")
+    _require(F32, yl, "idwt2")
     if yl.dim() != 4:
         raise IndexError("b200wave::idwt2 expects a 4-D (N, C, h, w) lowpass tensor, got %d-D" % yl.dim())
     J = len(yh)
@@ -323,7 +362,7 @@ def _idwt2_cuda(yl, yh, hw, w_lo, w_hi, h_lo, h_hi, mode, out_hw):
     kept = []
     for j, h in enumerate(yh):
         if h is not None:
-            _require_cuda_f32(h, "idwt2")
+            _require(F32, h, "idwt2")
             if tuple(h.shape) != (N, C, 3, hs[j], ws[j]):
                 raise RuntimeError("b200wave::idwt2: yh[%d] must have shape %s, got %s"
                                    % (j, (N, C, 3, hs[j], ws[j]), tuple(h.shape)))
@@ -459,7 +498,7 @@ def _afb2d_setup(ctx, inputs, output):
     ctx.set_materialize_grads(False)
 
 
-def _afb2d_backward(ctx, dlow, dhighs):
+def _afb2d_backward(p, ctx, dlow, dhighs):
     dx = None
     if ctx.needs_input_grad[0]:
         if dlow is None and dhighs is None:
@@ -470,7 +509,7 @@ def _afb2d_backward(ctx, dlow, dhighs):
         w_lo, w_hi, h_lo, h_hi = ctx.taps
         H, W = ctx.in_hw
         # synthesis with the saved analysis taps, cropped to the forward input (lowlevel.py:356-364)
-        dx = torch.ops.b200wave.sfb2d(dlow, dhighs, w_lo, w_hi, h_lo, h_hi, ctx.mode, H, W)
+        dx = getattr(torch.ops, p.ns).sfb2d(dlow, dhighs, w_lo, w_hi, h_lo, h_hi, ctx.mode, H, W)
     return dx, None, None, None, None, None
 
 
@@ -483,17 +522,17 @@ def _sfb2d_setup(ctx, inputs, output):
                                                idwt_len(low.shape[-1], len(w_lo), mode))
 
 
-def _sfb2d_backward(ctx, dy):
+def _sfb2d_backward(p, ctx, dy):
     dlow = dhighs = None
     need_low = ctx.needs_input_grad[0]
     need_high = ctx.has_highs and ctx.needs_input_grad[1]
     if need_low or need_high:
         if ctx.cropped:
-            raise RuntimeError("b200wave::sfb2d: backward through a cropped synthesis is not defined "
-                               "(the crop only exists inside AFB2D.backward)")
+            raise RuntimeError("%s::sfb2d: backward through a cropped synthesis is not defined "
+                               "(the crop only exists inside AFB2D.backward)" % p.ns)
         w_lo, w_hi, h_lo, h_hi = ctx.taps
         # analysis of dy with the un-reversed synthesis taps as correlators (lowlevel.py:687-693)
-        dlow, dhighs = torch.ops.b200wave.afb2d(dy, w_lo, w_hi, h_lo, h_hi, ctx.mode)
+        dlow, dhighs = getattr(torch.ops, p.ns).afb2d(dy, w_lo, w_hi, h_lo, h_hi, ctx.mode)
         if not need_low:
             dlow = None
         if not need_high:
@@ -513,26 +552,25 @@ def _rows_view(t):
     return t, (sc if c > 1 else (sn if n > 1 else l))
 
 
-def _afb1d_cuda(x, h0, h1, mode):
+def _afb1d_cuda(p, x, h0, h1, mode):
     _check_mode(mode)
-    _require_cuda_f32(x, "afb1d")
+    _require(p, x, "afb1d")
     if x.dim() != 3:
-        raise IndexError("b200wave::afb1d expects a 3-D (N, C, L) tensor, got %d-D" % x.dim())
+        raise IndexError("%s::afb1d expects a 3-D (N, C, L) tensor, got %d-D" % (p.ns, x.dim()))
     if len(h0) != len(h1):
         raise RuntimeError("low- and high-pass filters must have the same length")
-    lib = _cabi.load()
     N, C, n = x.shape
     m = coeff_len(n, len(h0), mode)
-    lo = torch.empty((N, C, m), device=x.device, dtype=torch.float32)
-    hi = torch.empty((N, C, m), device=x.device, dtype=torch.float32)
+    lo = torch.empty((N, C, m), device=x.device, dtype=p.dtype)
+    hi = torch.empty((N, C, m), device=x.device, dtype=p.dtype)
     if lo.numel() == 0:
         return lo, hi
     xk, rs = _rows_view(x)
-    a0, _ = _cabi.taps_array(h0)
-    a1, _ = _cabi.taps_array(h1)
+    a0, _ = p.taps(h0)
+    a1, _ = p.taps(h1)
     with torch.cuda.device(x.device):
-        rc = lib.b200w_afb1d_f32(xk.data_ptr(), rs, N * C, n, a0, a1, len(h0), int(mode), lo.data_ptr(), hi.data_ptr(),
-                                 _stream())
+        rc = p.lib.b200w_afb1d(xk.data_ptr(), rs, N * C, n, a0, a1, len(h0), int(mode), lo.data_ptr(), hi.data_ptr(),
+                               _stream())
     _cabi.check(rc, _mode_name(mode))
     return lo, hi
 
@@ -543,30 +581,29 @@ def _afb1d_fake(x, h0, h1, mode):
     return x.new_empty((N, C, m)), x.new_empty((N, C, m))
 
 
-def _sfb1d_cuda(low, high, g0, g1, mode, out_len):
+def _sfb1d_cuda(p, low, high, g0, g1, mode, out_len):
     _check_mode(mode)
-    _require_cuda_f32(low, "sfb1d")
+    _require(p, low, "sfb1d")
     if low.dim() != 3:
-        raise IndexError("b200wave::sfb1d expects 3-D (N, C, L) tensors, got %d-D" % low.dim())
+        raise IndexError("%s::sfb1d expects 3-D (N, C, L) tensors, got %d-D" % (p.ns, low.dim()))
     if high is not None:
-        _require_cuda_f32(high, "sfb1d")
+        _require(p, high, "sfb1d")
         if high.shape != low.shape:
-            raise RuntimeError("b200wave::sfb1d: low %s and high %s must have the same shape"
-                               % (tuple(low.shape), tuple(high.shape)))
-    lib = _cabi.load()
+            raise RuntimeError("%s::sfb1d: low %s and high %s must have the same shape"
+                               % (p.ns, tuple(low.shape), tuple(high.shape)))
     N, C, m = low.shape
     full = idwt_len(m, len(g0), mode)
     n = full if out_len < 0 else out_len
-    y = torch.empty((N, C, n), device=low.device, dtype=torch.float32)
+    y = torch.empty((N, C, n), device=low.device, dtype=p.dtype)
     if y.numel() == 0:
         return y
     lk, rs = _rows_view(low)
     hk = None if high is None else high.contiguous()
-    a0, _ = _cabi.taps_array(g0)
-    a1, _ = _cabi.taps_array(g1)
+    a0, _ = p.taps(g0)
+    a1, _ = p.taps(g1)
     with torch.cuda.device(low.device):
-        rc = lib.b200w_sfb1d_f32(lk.data_ptr(), rs, None if hk is None else hk.data_ptr(), N * C, m, a0, a1, len(g0),
-                                 int(mode), n, y.data_ptr(), _stream())
+        rc = p.lib.b200w_sfb1d(lk.data_ptr(), rs, None if hk is None else hk.data_ptr(), N * C, m, a0, a1, len(g0),
+                               int(mode), n, y.data_ptr(), _stream())
     _cabi.check(rc, _mode_name(mode))
     return y
 
@@ -584,7 +621,7 @@ def _afb1d_setup(ctx, inputs, output):
     ctx.set_materialize_grads(False)
 
 
-def _afb1d_backward(ctx, dlo, dhi):
+def _afb1d_backward(p, ctx, dlo, dhi):
     dx = None
     if ctx.needs_input_grad[0]:
         if dlo is None and dhi is None:
@@ -592,7 +629,7 @@ def _afb1d_backward(ctx, dlo, dhi):
         if dlo is None:
             dlo = torch.zeros_like(dhi)
         # synthesis with the saved analysis taps, cropped to the forward input (lowlevel.py:417-422)
-        dx = torch.ops.b200wave.sfb1d(dlo, dhi, ctx.taps[0], ctx.taps[1], ctx.mode, ctx.n)
+        dx = getattr(torch.ops, p.ns).sfb1d(dlo, dhi, ctx.taps[0], ctx.taps[1], ctx.mode, ctx.n)
     return dx, None, None, None
 
 
@@ -604,16 +641,16 @@ def _sfb1d_setup(ctx, inputs, output):
     ctx.cropped = output.shape[-1] != idwt_len(low.shape[-1], len(g0), mode)
 
 
-def _sfb1d_backward(ctx, dy):
+def _sfb1d_backward(p, ctx, dy):
     dlo = dhi = None
     need_lo = ctx.needs_input_grad[0]
     need_hi = ctx.has_high and ctx.needs_input_grad[1]
     if need_lo or need_hi:
         if ctx.cropped:
-            raise RuntimeError("b200wave::sfb1d: backward through a cropped synthesis is not defined "
-                               "(the crop only exists inside AFB1D.backward)")
+            raise RuntimeError("%s::sfb1d: backward through a cropped synthesis is not defined "
+                               "(the crop only exists inside AFB1D.backward)" % p.ns)
         # analysis of dy with the un-reversed synthesis taps as correlators (lowlevel.py:736-742)
-        dlo, dhi = torch.ops.b200wave.afb1d(dy, ctx.taps[0], ctx.taps[1], ctx.mode)
+        dlo, dhi = getattr(torch.ops, p.ns).afb1d(dy, ctx.taps[0], ctx.taps[1], ctx.mode)
         if not need_lo:
             dlo = None
         if not need_hi:
@@ -627,40 +664,48 @@ def _check_swt_mode(mode):
         raise ValueError("Unkown pad type: {}".format(_mode_name(mode)))
 
 
-def _swt_call(fn_name, t, w_lo, w_hi, h_lo, h_hi, mode, dilation, planes, H, W, out):
-    lib = _cabi.load()
+def _swt_call(p, fn, t, w_lo, w_hi, h_lo, h_hi, mode, dilation, planes, H, W, out):
     if not (len(w_lo) == len(w_hi) == len(h_lo) == len(h_hi)):
-        raise RuntimeError("b200wave::swt2d: all four filters must have the same length")
-    a_wl, _ = _cabi.taps_array(w_lo)
-    a_wh, _ = _cabi.taps_array(w_hi)
-    a_hl, _ = _cabi.taps_array(h_lo)
-    a_hh, _ = _cabi.taps_array(h_hi)
+        raise RuntimeError("%s::swt2d: all four filters must have the same length" % p.ns)
+    a_wl, _ = p.taps(w_lo)
+    a_wh, _ = p.taps(w_hi)
+    a_hl, _ = p.taps(h_lo)
+    a_hh, _ = p.taps(h_hi)
     with torch.cuda.device(t.device):
-        rc = getattr(lib, fn_name)(t.data_ptr(), planes, H, W, a_wl, a_wh, a_hl, a_hh, len(w_lo), int(dilation),
-                                   int(mode), out.data_ptr(), _stream())
+        rc = fn(t.data_ptr(), planes, H, W, a_wl, a_wh, a_hl, a_hh, len(w_lo), int(dilation), int(mode), out.data_ptr(),
+                _stream())
     _cabi.check(rc, _mode_name(mode))
 
 
-def _swt2d_cuda(x, w_lo, w_hi, h_lo, h_hi, mode, dilation):
+def _swt2d_cuda(p, x, w_lo, w_hi, h_lo, h_hi, mode, dilation):
     _check_swt_mode(mode)
-    _require_cuda_f32(x, "swt2d")
+    _require(p, x, "swt2d")
     if x.dim() != 4:
-        raise IndexError("b200wave::swt2d expects a 4-D (N, C, H, W) tensor, got %d-D" % x.dim())
+        raise IndexError("%s::swt2d expects a 4-D (N, C, H, W) tensor, got %d-D" % (p.ns, x.dim()))
     N, C, H, W = x.shape
-    y = torch.empty((N, 4 * C, H, W), device=x.device, dtype=torch.float32)
+    y = torch.empty((N, 4 * C, H, W), device=x.device, dtype=p.dtype)
     if y.numel():
-        _swt_call("b200w_swt2d_fwd_f32", x.contiguous(), w_lo, w_hi, h_lo, h_hi, mode, dilation, N * C, H, W, y)
+        _swt_call(p, p.lib.b200w_swt2d_fwd, x.contiguous(), w_lo, w_hi, h_lo, h_hi, mode, dilation, N * C, H, W, y)
     return y
 
 
-def _swt2d_adjoint_cuda(dy, w_lo, w_hi, h_lo, h_hi, mode, dilation):
+def _swt2d_fake(x, w_lo, w_hi, h_lo, h_hi, mode, dilation):
+    return x.new_empty((x.shape[0], 4 * x.shape[1], x.shape[2], x.shape[3]))
+
+
+def _swt2d_adjoint_cuda(p, dy, w_lo, w_hi, h_lo, h_hi, mode, dilation):
     _check_swt_mode(mode)
-    _require_cuda_f32(dy, "swt2d_adjoint")
+    _require(p, dy, "swt2d_adjoint")
     N, C4, H, W = dy.shape
-    dx = torch.empty((N, C4 // 4, H, W), device=dy.device, dtype=torch.float32)
+    dx = torch.empty((N, C4 // 4, H, W), device=dy.device, dtype=p.dtype)
     if dx.numel():
-        _swt_call("b200w_swt2d_bwd_f32", dy.contiguous(), w_lo, w_hi, h_lo, h_hi, mode, dilation, N * (C4 // 4), H, W, dx)
+        _swt_call(p, p.lib.b200w_swt2d_bwd, dy.contiguous(), w_lo, w_hi, h_lo, h_hi, mode, dilation, N * (C4 // 4),
+                  H, W, dx)
     return dx
+
+
+def _swt2d_adjoint_fake(dy, w_lo, w_hi, h_lo, h_hi, mode, dilation):
+    return dy.new_empty((dy.shape[0], dy.shape[1] // 4, dy.shape[2], dy.shape[3]))
 
 
 def _swt2d_setup(ctx, inputs, output):
@@ -668,10 +713,10 @@ def _swt2d_setup(ctx, inputs, output):
     ctx.args = (w_lo, w_hi, h_lo, h_hi, mode, dilation)
 
 
-def _swt2d_backward(ctx, dy):
+def _swt2d_backward(p, ctx, dy):
     dx = None
     if ctx.needs_input_grad[0]:
-        dx = torch.ops.b200wave.swt2d_adjoint(dy, *ctx.args)
+        dx = getattr(torch.ops, p.ns).swt2d_adjoint(dy, *ctx.args)
     return dx, None, None, None, None, None, None
 
 
@@ -679,16 +724,16 @@ def _swt2d_backward(ctx, dy):
 PERIODIC = 6
 
 
-def iswt_layout(ll, y, name):
+def iswt_layout(p, ll, y):
     """Checks the shapes of one inverse-SWT level and returns (ll as (tensor, plane stride), dense y); copies only what
     the kernel cannot read in place: ll needs unit column stride, row stride W and uniform plane spacing."""
     if ll.dim() != 4 or y.dim() != 4:
-        raise IndexError("%s expects 4-D ll (N, C, H, W) and y (N, 4C, H, W), got %d-D and %d-D"
-                         % (name, ll.dim(), y.dim()))
+        raise IndexError("%s::iswt2d expects 4-D ll (N, C, H, W) and y (N, 4C, H, W), got %d-D and %d-D"
+                         % (p.ns, ll.dim(), y.dim()))
     N, C4, H, W = y.shape
     if C4 % 4 or tuple(ll.shape) != (N, C4 // 4, H, W):
-        raise RuntimeError("%s: y must be (N, 4C, H, W) and ll (N, C, H, W), got %s and %s"
-                           % (name, tuple(y.shape), tuple(ll.shape)))
+        raise RuntimeError("%s::iswt2d: y must be (N, 4C, H, W) and ll (N, C, H, W), got %s and %s"
+                           % (p.ns, tuple(y.shape), tuple(ll.shape)))
     lk, ps, rs = _planes_view(ll)
     if rs != W and H > 1:
         lk = ll.contiguous()
@@ -701,23 +746,26 @@ def iswt_adjoint_taps(w_lo, w_hi, h_lo, h_hi):
     return [[0.5 * float(v) for v in t] for t in (w_lo, w_hi, h_lo, h_hi)]
 
 
-def _iswt2d_cuda(ll, y, w_lo, w_hi, h_lo, h_hi, dilation):
-    _require_cuda_f32(ll, "iswt2d")
-    _require_cuda_f32(y, "iswt2d")
+def _iswt2d_cuda(p, ll, y, w_lo, w_hi, h_lo, h_hi, dilation):
+    _require(p, ll, "iswt2d")
+    _require(p, y, "iswt2d")
     if not (len(w_lo) == len(w_hi) == len(h_lo) == len(h_hi)):
-        raise RuntimeError("b200wave::iswt2d: all four filters must have the same length")
-    lk, ps, yk = iswt_layout(ll, y, "b200wave::iswt2d")
+        raise RuntimeError("%s::iswt2d: all four filters must have the same length" % p.ns)
+    lk, ps, yk = iswt_layout(p, ll, y)
     N, C4, H, W = yk.shape
-    x = torch.empty((N, C4 // 4, H, W), device=y.device, dtype=torch.float32)
+    x = torch.empty((N, C4 // 4, H, W), device=y.device, dtype=p.dtype)
     if x.numel() == 0:
         return x
-    lib = _cabi.load()
-    a = [_cabi.taps_array(t)[0] for t in (w_lo, w_hi, h_lo, h_hi)]
+    a = [p.taps(t)[0] for t in (w_lo, w_hi, h_lo, h_hi)]
     with torch.cuda.device(y.device):
-        rc = lib.b200w_iswt2d_f32(lk.data_ptr(), ps, yk.data_ptr(), N * (C4 // 4), H, W, a[0], a[1], a[2], a[3],
-                                  len(w_lo), int(dilation), x.data_ptr(), _stream())
+        rc = p.lib.b200w_iswt2d(lk.data_ptr(), ps, yk.data_ptr(), N * (C4 // 4), H, W, a[0], a[1], a[2], a[3],
+                                len(w_lo), int(dilation), x.data_ptr(), _stream())
     _cabi.check(rc)
     return x
+
+
+def _iswt2d_fake(ll, y, w_lo, w_hi, h_lo, h_hi, dilation):
+    return y.new_empty((y.shape[0], y.shape[1] // 4, y.shape[2], y.shape[3]))
 
 
 def _iswt2d_setup(ctx, inputs, output):
@@ -726,13 +774,13 @@ def _iswt2d_setup(ctx, inputs, output):
     ctx.dilation = dilation
 
 
-def iswt2d_backward(swt2d_op, ctx, dx):
+def _iswt2d_backward(p, ctx, dx):
     """Transpose of the level: the analysis kernel with the halved synthesis taps; band 0 of its output is the gradient
     of ll, bands 1..3 that of y (whose band 0 the level never reads)."""
     need_ll, need_y = ctx.needs_input_grad[0], ctx.needs_input_grad[1]
     if dx is None or not (need_ll or need_y):
         return (None,) * 7
-    g = swt2d_op(dx, *ctx.taps, PERIODIC, ctx.dilation)
+    g = getattr(torch.ops, p.ns).swt2d(dx, *ctx.taps, PERIODIC, ctx.dilation)
     N, C4, H, W = g.shape
     g5 = g.view(N, C4 // 4, 4, H, W)
     dll = g5[:, :, 0].clone() if need_ll else None
@@ -743,36 +791,41 @@ def iswt2d_backward(swt2d_op, ctx, dx):
     return (dll, dy) + (None,) * 5
 
 
-def _iswt2d_backward(ctx, dx):
-    return iswt2d_backward(torch.ops.b200wave.swt2d, ctx, dx)
-
-
 # ------------------------------------------------------------------------------------------- ssim
-def _ssim_common(img1, img2, win, name):
-    _require_cuda_f32(img1, name)
-    _require_cuda_f32(img2, name)
+def _ssim_common(p, img1, img2, win, name):
+    """Checks the images and the window; returns the window size the kernels take: the tap count of the 1-D window,
+    or the side ws of the dense ws x ws one."""
+    _require(p, img1, name)
+    _require(p, img2, name)
     if img1.dim() != 4 or img1.shape != img2.shape:
-        raise RuntimeError("b200wave::%s expects two (N, C, H, W) tensors of equal shape, got %s and %s"
-                           % (name, tuple(img1.shape), tuple(img2.shape)))
+        raise RuntimeError("%s::%s expects two (N, C, H, W) tensors of equal shape, got %s and %s"
+                           % (p.ns, name, tuple(img1.shape), tuple(img2.shape)))
+    if p.dense_win:
+        ws = int(round(len(win) ** 0.5))
+        if ws * ws != len(win) or ws % 2 == 0 or ws > _cabi.SSIM_MAX_WINDOW:
+            raise RuntimeError("%s::%s: the window must be ws x ws taps with ws odd and <= %d, got %d taps"
+                               % (p.ns, name, _cabi.SSIM_MAX_WINDOW, len(win)))
+        return ws
     if len(win) % 2 == 0 or len(win) > _cabi.SSIM_MAX_WINDOW:
-        raise RuntimeError("b200wave::%s: window size must be odd and <= %d, got %d"
-                           % (name, _cabi.SSIM_MAX_WINDOW, len(win)))
+        raise RuntimeError("%s::%s: window size must be odd and <= %d, got %d"
+                           % (p.ns, name, _cabi.SSIM_MAX_WINDOW, len(win)))
+    return len(win)
 
 
-def _ssim_fwd_cuda(img1, img2, win, size_average, n_maps):
-    _ssim_common(img1, img2, win, "ssim_fwd")
+def _ssim_fwd_cuda(p, img1, img2, win, size_average, n_maps):
+    nwin = _ssim_common(p, img1, img2, win, "ssim_fwd")
     lib = _cabi.load()
     img1, img2 = img1.contiguous(), img2.contiguous()
     N, C, H, W = img1.shape
-    out = torch.empty(() if size_average else (N,), device=img1.device, dtype=torch.float32)
-    maps = torch.empty((n_maps, N, C, H, W), device=img1.device, dtype=torch.float32)
-    ws_bytes = lib.b200w_ssim_workspace_bytes(N, C, H, W)
-    work = torch.empty((max(ws_bytes, 4) // 4,), device=img1.device, dtype=torch.float32)
-    a_win, nwin = _cabi.taps_array(win)
+    out = torch.empty(() if size_average else (N,), device=img1.device, dtype=p.dtype)
+    maps = torch.empty((n_maps, N, C, H, W), device=img1.device, dtype=p.dtype)
+    ws_bytes = (lib.b200w_ssim_workspace_bytes_f64 if p.dense_win else lib.b200w_ssim_workspace_bytes)(N, C, H, W)
+    work = torch.empty((max(ws_bytes, p.elem) // p.elem,), device=img1.device, dtype=p.dtype)
+    a_win, _ = p.taps(win)
     with torch.cuda.device(img1.device):
-        rc = lib.b200w_ssim_fwd_f32(img1.data_ptr(), img2.data_ptr(), N, C, H, W, a_win, nwin, int(size_average),
-                                    int(n_maps), maps.data_ptr() if n_maps else None, out.data_ptr(),
-                                    work.data_ptr(), ws_bytes, _stream())
+        rc = p.lib.b200w_ssim_fwd(img1.data_ptr(), img2.data_ptr(), N, C, H, W, a_win, nwin, int(size_average),
+                                  int(n_maps), maps.data_ptr() if n_maps else None, out.data_ptr(),
+                                  work.data_ptr(), ws_bytes, _stream())
     _cabi.check(rc)
     return out, maps
 
@@ -782,25 +835,24 @@ def _ssim_fwd_fake(img1, img2, win, size_average, n_maps):
     return img1.new_empty(() if size_average else (N,)), img1.new_empty((n_maps, N, C, H, W))
 
 
-def _ssim_bwd_cuda(img1, img2, maps, grad_out, win, size_average, need_d2):
-    _ssim_common(img1, img2, win, "ssim_bwd")
-    lib = _cabi.load()
+def _ssim_bwd_cuda(p, img1, img2, maps, grad_out, win, size_average, need_d2):
+    nwin = _ssim_common(p, img1, img2, win, "ssim_bwd")
     img1, img2, maps = img1.contiguous(), img2.contiguous(), maps.contiguous()
     N, C, H, W = img1.shape
     n_maps = maps.shape[0]
     if n_maps not in (3, 4) or (need_d2 and n_maps != 4):
-        raise RuntimeError("b200wave::ssim_bwd: forward saved %d derivative maps, not enough for this backward"
-                           % n_maps)
-    g = grad_out.to(device=img1.device, dtype=torch.float32).contiguous()
+        raise RuntimeError("%s::ssim_bwd: forward saved %d derivative maps, not enough for this backward"
+                           % (p.ns, n_maps))
+    g = grad_out.to(device=img1.device, dtype=p.dtype).contiguous()
     if g.numel() != (1 if size_average else N):
-        raise RuntimeError("b200wave::ssim_bwd: grad_out has %d elements" % g.numel())
+        raise RuntimeError("%s::ssim_bwd: grad_out has %d elements" % (p.ns, g.numel()))
     d1 = torch.empty_like(img1)
-    d2 = torch.empty_like(img2) if need_d2 else torch.empty((0,), device=img1.device, dtype=torch.float32)
-    a_win, nwin = _cabi.taps_array(win)
+    d2 = torch.empty_like(img2) if need_d2 else torch.empty((0,), device=img1.device, dtype=p.dtype)
+    a_win, _ = p.taps(win)
     with torch.cuda.device(img1.device):
-        rc = lib.b200w_ssim_bwd_f32(img1.data_ptr(), img2.data_ptr(), maps.data_ptr(), n_maps, g.data_ptr(),
-                                    N, C, H, W, a_win, nwin, int(size_average), d1.data_ptr(),
-                                    d2.data_ptr() if need_d2 else None, _stream())
+        rc = p.lib.b200w_ssim_bwd(img1.data_ptr(), img2.data_ptr(), maps.data_ptr(), n_maps, g.data_ptr(),
+                                  N, C, H, W, a_win, nwin, int(size_average), d1.data_ptr(),
+                                  d2.data_ptr() if need_d2 else None, _stream())
     _cabi.check(rc)
     return d1, d2
 
@@ -819,15 +871,15 @@ def _ssim_setup(ctx, inputs, output):
     ctx.set_materialize_grads(False)
 
 
-def _ssim_backward(ctx, dval, dmaps):
+def _ssim_backward(p, ctx, dval, dmaps):
     need1, need2 = ctx.needs_input_grad[0], ctx.needs_input_grad[1]
     if not (need1 or need2) or dval is None:
         return None, None, None, None, None
     if ctx.n_maps < 3 or (need2 and ctx.n_maps < 4):
-        raise RuntimeError("b200wave::ssim_fwd was called with n_maps=%d, which does not support the requested "
-                           "gradient (use 3 for d/dimg1, 4 for both)" % ctx.n_maps)
+        raise RuntimeError("%s::ssim_fwd was called with n_maps=%d, which does not support the requested "
+                           "gradient (use 3 for d/dimg1, 4 for both)" % (p.ns, ctx.n_maps))
     img1, img2, maps = ctx.saved_tensors
-    d1, d2 = torch.ops.b200wave.ssim_bwd(img1, img2, maps, dval, ctx.win, ctx.size_average, bool(need2))
+    d1, d2 = getattr(torch.ops, p.ns).ssim_bwd(img1, img2, maps, dval, ctx.win, ctx.size_average, bool(need2))
     return (d1 if need1 else None), (d2 if need2 else None), None, None, None
 
 
@@ -837,69 +889,72 @@ def pooled_shape(img, pool):
     return (N, C, H // 2, W // 2) if pool else (0,)
 
 
-def msssim_up(t, img, name):
+def msssim_up(p, t, img, name):
     """The gradient of a pooled output as the backward kernel reads it (or None)."""
     if t is None:
         return None
     if tuple(t.shape) != pooled_shape(img, True):
-        raise RuntimeError("b200wave::%s: the gradient of a pooled image has shape %s, expected %s"
-                           % (name, tuple(t.shape), pooled_shape(img, True)))
+        raise RuntimeError("%s::%s: the gradient of a pooled image has shape %s, expected %s"
+                           % (p.ns, name, tuple(t.shape), pooled_shape(img, True)))
     return t.to(dtype=img.dtype).contiguous()
 
 
-def _msssim_scale_cuda(img1, img2, win, cs, pool, n_maps):
-    _ssim_common(img1, img2, win, "msssim_scale")
+def _msssim_scale_cuda(p, img1, img2, win, cs, pool, n_maps):
+    nwin = _ssim_common(p, img1, img2, win, "msssim_scale")
     lib = _cabi.load()
     img1, img2 = img1.contiguous(), img2.contiguous()
     N, C, H, W = img1.shape
-    out = torch.empty((N,), device=img1.device, dtype=torch.float32)
-    maps = torch.empty((n_maps, N, C, H, W), device=img1.device, dtype=torch.float32)
-    p1 = torch.empty(pooled_shape(img1, pool), device=img1.device, dtype=torch.float32)
+    out = torch.empty((N,), device=img1.device, dtype=p.dtype)
+    maps = torch.empty((n_maps, N, C, H, W), device=img1.device, dtype=p.dtype)
+    p1 = torch.empty(pooled_shape(img1, pool), device=img1.device, dtype=p.dtype)
     p2 = torch.empty_like(p1)
-    ws_bytes = lib.b200w_ssim_workspace_bytes(N, C, H, W)
-    work = torch.empty((max(ws_bytes, 4) // 4,), device=img1.device, dtype=torch.float32)
-    a_win, nwin = _cabi.taps_array(win)
+    ws_bytes = (lib.b200w_ssim_workspace_bytes_f64 if p.dense_win else lib.b200w_ssim_workspace_bytes)(N, C, H, W)
+    work = torch.empty((max(ws_bytes, p.elem) // p.elem,), device=img1.device, dtype=p.dtype)
+    a_win, _ = p.taps(win)
     with torch.cuda.device(img1.device):
-        rc = lib.b200w_msssim_scale_fwd_f32(img1.data_ptr(), img2.data_ptr(), N, C, H, W, a_win, nwin, int(cs),
-                                            int(n_maps), maps.data_ptr() if n_maps else None, out.data_ptr(),
-                                            p1.data_ptr() if pool else None, p2.data_ptr() if pool else None,
-                                            work.data_ptr(), ws_bytes, _stream())
+        rc = p.lib.b200w_msssim_scale_fwd(img1.data_ptr(), img2.data_ptr(), N, C, H, W, a_win, nwin, int(cs),
+                                          int(n_maps), maps.data_ptr() if n_maps else None, out.data_ptr(),
+                                          p1.data_ptr() if pool else None, p2.data_ptr() if pool else None,
+                                          work.data_ptr(), ws_bytes, _stream())
     _cabi.check(rc)
     return out, maps, p1, p2
 
 
-def msssim_scale_fake(img1, img2, win, cs, pool, n_maps):
+def _msssim_scale_fake(img1, img2, win, cs, pool, n_maps):
     N, C, H, W = img1.shape
     p = img1.new_empty(pooled_shape(img1, pool))
     return img1.new_empty((N,)), img1.new_empty((n_maps, N, C, H, W)), p, torch.empty_like(p)
 
 
-def _msssim_scale_bwd_cuda(img1, img2, maps, grad_out, win, up1, up2, need_d2):
-    _ssim_common(img1, img2, win, "msssim_scale_bwd")
-    lib = _cabi.load()
+def _msssim_scale_bwd_cuda(p, img1, img2, maps, grad_out, win, up1, up2, need_d2):
+    nwin = _ssim_common(p, img1, img2, win, "msssim_scale_bwd")
     img1, img2, maps = img1.contiguous(), img2.contiguous(), maps.contiguous()
     N, C, H, W = img1.shape
     n_maps = maps.shape[0]
     if n_maps not in (3, 4) or (need_d2 and n_maps != 4):
-        raise RuntimeError("b200wave::msssim_scale_bwd: forward saved %d derivative maps, not enough for this backward"
-                           % n_maps)
-    g = grad_out.to(device=img1.device, dtype=torch.float32).contiguous()
+        raise RuntimeError("%s::msssim_scale_bwd: forward saved %d derivative maps, not enough for this backward"
+                           % (p.ns, n_maps))
+    g = grad_out.to(device=img1.device, dtype=p.dtype).contiguous()
     if g.numel() != N:
-        raise RuntimeError("b200wave::msssim_scale_bwd: grad_out has %d elements" % g.numel())
-    up1, up2 = msssim_up(up1, img1, "msssim_scale_bwd"), msssim_up(up2, img1, "msssim_scale_bwd")
+        raise RuntimeError("%s::msssim_scale_bwd: grad_out has %d elements" % (p.ns, g.numel()))
+    up1, up2 = msssim_up(p, up1, img1, "msssim_scale_bwd"), msssim_up(p, up2, img1, "msssim_scale_bwd")
     d1 = torch.empty_like(img1)
-    d2 = torch.empty_like(img2) if need_d2 else torch.empty((0,), device=img1.device, dtype=torch.float32)
-    a_win, nwin = _cabi.taps_array(win)
+    d2 = torch.empty_like(img2) if need_d2 else torch.empty((0,), device=img1.device, dtype=p.dtype)
+    a_win, _ = p.taps(win)
     with torch.cuda.device(img1.device):
-        rc = lib.b200w_msssim_scale_bwd_f32(img1.data_ptr(), img2.data_ptr(), maps.data_ptr(), n_maps, g.data_ptr(),
-                                            N, C, H, W, a_win, nwin, None if up1 is None else up1.data_ptr(),
-                                            None if up2 is None else up2.data_ptr(), d1.data_ptr(),
-                                            d2.data_ptr() if need_d2 else None, _stream())
+        rc = p.lib.b200w_msssim_scale_bwd(img1.data_ptr(), img2.data_ptr(), maps.data_ptr(), n_maps, g.data_ptr(),
+                                          N, C, H, W, a_win, nwin, None if up1 is None else up1.data_ptr(),
+                                          None if up2 is None else up2.data_ptr(), d1.data_ptr(),
+                                          d2.data_ptr() if need_d2 else None, _stream())
     _cabi.check(rc)
     return d1, d2
 
 
-def msssim_scale_setup(ctx, inputs, output):
+def _msssim_scale_bwd_fake(img1, img2, maps, grad_out, win, up1, up2, need_d2):
+    return _ssim_bwd_fake(img1, img2, maps, grad_out, win, False, need_d2)
+
+
+def _msssim_scale_setup(ctx, inputs, output):
     img1, img2, win, cs, pool, n_maps = inputs
     ctx.save_for_backward(img1, img2, output[1])
     ctx.win = win
@@ -907,7 +962,7 @@ def msssim_scale_setup(ctx, inputs, output):
     ctx.set_materialize_grads(False)
 
 
-def msssim_scale_backward(bwd_op, ctx, dval, dmaps, dp1, dp2):
+def _msssim_scale_backward(p, ctx, dval, dmaps, dp1, dp2):
     """One backward launch: the closed form for ``dval`` plus 0.25 ``dp`` spread over each 2x2 block."""
     need1, need2 = ctx.needs_input_grad[0], ctx.needs_input_grad[1]
     if not (need1 or need2):
@@ -918,70 +973,62 @@ def msssim_scale_backward(bwd_op, ctx, dval, dmaps, dp1, dp2):
     img1, img2, maps = ctx.saved_tensors
     if dval is None:
         dval = img1.new_zeros((img1.shape[0],))
-    d1, d2 = bwd_op(img1, img2, maps, dval, ctx.win, dp1 if need1 else None, dp2 if need2 else None, bool(need2))
+    d1, d2 = getattr(torch.ops, p.ns).msssim_scale_bwd(img1, img2, maps, dval, ctx.win, dp1 if need1 else None,
+                                                         dp2 if need2 else None, bool(need2))
     return (d1 if need1 else None), (d2 if need2 else None), None, None, None, None
 
 
-def _msssim_scale_backward(ctx, dval, dmaps, dp1, dp2):
-    return msssim_scale_backward(torch.ops.b200wave.msssim_scale_bwd, ctx, dval, dmaps, dp1, dp2)
-
-
-_LIB.impl("afb2d", _afb2d_cuda, "CUDA")
-_LIB.impl("sfb2d", _sfb2d_cuda, "CUDA")
+_LIB.impl("afb2d", functools.partial(_afb2d_cuda, F32), "CUDA")
+_LIB.impl("sfb2d", functools.partial(_sfb2d_cuda, F32), "CUDA")
 _LIB.impl("dwt2", _dwt2_cuda, "CUDA")
 _LIB.impl("idwt2", _idwt2_cuda, "CUDA")
-_LIB.impl("ssim_fwd", _ssim_fwd_cuda, "CUDA")
-_LIB.impl("ssim_bwd", _ssim_bwd_cuda, "CUDA")
-_LIB.impl("afb2d_select", _afb2d_select_cuda, "CUDA")
-_LIB.impl("afb1d", _afb1d_cuda, "CUDA")
-_LIB.impl("swt2d", _swt2d_cuda, "CUDA")
-_LIB.impl("swt2d_adjoint", _swt2d_adjoint_cuda, "CUDA")
-_LIB.impl("sfb1d", _sfb1d_cuda, "CUDA")
-_LIB.impl("iswt2d", _iswt2d_cuda, "CUDA")
-_LIB.impl("msssim_scale", _msssim_scale_cuda, "CUDA")
-_LIB.impl("msssim_scale_bwd", _msssim_scale_bwd_cuda, "CUDA")
-
-
-def _cpu_refuse(name):
-    def impl(*args, **kwargs):
-        raise RuntimeError("b200wave::%s is CUDA-only (sm_100a): there is no CPU fallback. Move the tensors to "
-                           "a B200 (`.cuda()`)." % name)
-    return impl
-
+_LIB.impl("ssim_fwd", functools.partial(_ssim_fwd_cuda, F32), "CUDA")
+_LIB.impl("ssim_bwd", functools.partial(_ssim_bwd_cuda, F32), "CUDA")
+_LIB.impl("afb2d_select", functools.partial(_afb2d_select_cuda, F32), "CUDA")
+_LIB.impl("afb1d", functools.partial(_afb1d_cuda, F32), "CUDA")
+_LIB.impl("swt2d", functools.partial(_swt2d_cuda, F32), "CUDA")
+_LIB.impl("swt2d_adjoint", functools.partial(_swt2d_adjoint_cuda, F32), "CUDA")
+_LIB.impl("sfb1d", functools.partial(_sfb1d_cuda, F32), "CUDA")
+_LIB.impl("iswt2d", functools.partial(_iswt2d_cuda, F32), "CUDA")
+_LIB.impl("msssim_scale", functools.partial(_msssim_scale_cuda, F32), "CUDA")
+_LIB.impl("msssim_scale_bwd", functools.partial(_msssim_scale_bwd_cuda, F32), "CUDA")
 
 for _name in ("afb2d", "afb2d_select", "sfb2d", "dwt2", "idwt2", "ssim_fwd", "ssim_bwd", "afb1d", "sfb1d", "swt2d",
               "swt2d_adjoint", "iswt2d", "msssim_scale", "msssim_scale_bwd"):
-    _LIB.impl(_name, _cpu_refuse(_name), "CPU")
+    _LIB.impl(_name, _cpu_refuse(F32.ns, _name), "CPU")
 
 torch.library.register_fake("b200wave::afb2d", _afb2d_fake, lib=_LIB)
 torch.library.register_fake("b200wave::sfb2d", _sfb2d_fake, lib=_LIB)
 torch.library.register_fake("b200wave::afb2d_select", _afb2d_select_fake, lib=_LIB)
-torch.library.register_autograd("b200wave::afb2d_select", _afb2d_select_backward, setup_context=_afb2d_select_setup,
-                                lib=_LIB)
+torch.library.register_autograd("b200wave::afb2d_select", functools.partial(_afb2d_select_backward, F32),
+                                setup_context=_afb2d_select_setup, lib=_LIB)
 torch.library.register_fake("b200wave::dwt2", _dwt2_fake, lib=_LIB)
 torch.library.register_fake("b200wave::afb1d", _afb1d_fake, lib=_LIB)
-torch.library.register_fake("b200wave::swt2d", lambda x, wl, wh, hl, hh, mode, d:
-                            x.new_empty((x.shape[0], 4 * x.shape[1], x.shape[2], x.shape[3])), lib=_LIB)
-torch.library.register_fake("b200wave::swt2d_adjoint", lambda dy, wl, wh, hl, hh, mode, d:
-                            dy.new_empty((dy.shape[0], dy.shape[1] // 4, dy.shape[2], dy.shape[3])), lib=_LIB)
-torch.library.register_autograd("b200wave::swt2d", _swt2d_backward, setup_context=_swt2d_setup, lib=_LIB)
+torch.library.register_fake("b200wave::swt2d", _swt2d_fake, lib=_LIB)
+torch.library.register_fake("b200wave::swt2d_adjoint", _swt2d_adjoint_fake, lib=_LIB)
+torch.library.register_autograd("b200wave::swt2d", functools.partial(_swt2d_backward, F32), setup_context=_swt2d_setup,
+                                lib=_LIB)
 torch.library.register_fake("b200wave::sfb1d", _sfb1d_fake, lib=_LIB)
-torch.library.register_fake("b200wave::iswt2d", lambda ll, y, wl, wh, hl, hh, d:
-                            y.new_empty((y.shape[0], y.shape[1] // 4, y.shape[2], y.shape[3])), lib=_LIB)
-torch.library.register_autograd("b200wave::iswt2d", _iswt2d_backward, setup_context=_iswt2d_setup, lib=_LIB)
-torch.library.register_autograd("b200wave::afb1d", _afb1d_backward, setup_context=_afb1d_setup, lib=_LIB)
-torch.library.register_autograd("b200wave::sfb1d", _sfb1d_backward, setup_context=_sfb1d_setup, lib=_LIB)
+torch.library.register_fake("b200wave::iswt2d", _iswt2d_fake, lib=_LIB)
+torch.library.register_autograd("b200wave::iswt2d", functools.partial(_iswt2d_backward, F32),
+                                setup_context=_iswt2d_setup, lib=_LIB)
+torch.library.register_autograd("b200wave::afb1d", functools.partial(_afb1d_backward, F32), setup_context=_afb1d_setup,
+                                lib=_LIB)
+torch.library.register_autograd("b200wave::sfb1d", functools.partial(_sfb1d_backward, F32), setup_context=_sfb1d_setup,
+                                lib=_LIB)
 torch.library.register_fake("b200wave::idwt2", _idwt2_fake, lib=_LIB)
 torch.library.register_fake("b200wave::ssim_fwd", _ssim_fwd_fake, lib=_LIB)
 torch.library.register_fake("b200wave::ssim_bwd", _ssim_bwd_fake, lib=_LIB)
-torch.library.register_autograd("b200wave::afb2d", _afb2d_backward, setup_context=_afb2d_setup, lib=_LIB)
-torch.library.register_autograd("b200wave::sfb2d", _sfb2d_backward, setup_context=_sfb2d_setup, lib=_LIB)
-torch.library.register_autograd("b200wave::ssim_fwd", _ssim_backward, setup_context=_ssim_setup, lib=_LIB)
-torch.library.register_fake("b200wave::msssim_scale", msssim_scale_fake, lib=_LIB)
-torch.library.register_fake("b200wave::msssim_scale_bwd", lambda img1, img2, maps, g, win, up1, up2, need_d2:
-                            _ssim_bwd_fake(img1, img2, maps, g, win, False, need_d2), lib=_LIB)
-torch.library.register_autograd("b200wave::msssim_scale", _msssim_scale_backward, setup_context=msssim_scale_setup,
+torch.library.register_autograd("b200wave::afb2d", functools.partial(_afb2d_backward, F32), setup_context=_afb2d_setup,
                                 lib=_LIB)
+torch.library.register_autograd("b200wave::sfb2d", functools.partial(_sfb2d_backward, F32), setup_context=_sfb2d_setup,
+                                lib=_LIB)
+torch.library.register_autograd("b200wave::ssim_fwd", functools.partial(_ssim_backward, F32),
+                                setup_context=_ssim_setup, lib=_LIB)
+torch.library.register_fake("b200wave::msssim_scale", _msssim_scale_fake, lib=_LIB)
+torch.library.register_fake("b200wave::msssim_scale_bwd", _msssim_scale_bwd_fake, lib=_LIB)
+torch.library.register_autograd("b200wave::msssim_scale", functools.partial(_msssim_scale_backward, F32),
+                                setup_context=_msssim_scale_setup, lib=_LIB)
 
 afb2d = torch.ops.b200wave.afb2d
 afb2d_select = torch.ops.b200wave.afb2d_select

@@ -160,7 +160,7 @@ def freq_and_fsd(it, wu):
         key = "64x%d^2" % side
         r = {}
         for name, dt in (("f64", torch.float64), ("f32", torch.float32)):
-            mask_, abs_sign = freq._OPS[dt][0], freq._OPS[dt][1]
+            mask_, abs_sign = freq._ops(dt)[:2]
             es = torch.finfo(dt).bits // 8
             x = torch.rand((64, 1, side, side), device=dev, dtype=dt)
             spec = torch.fft.rfft2(x).contiguous()
